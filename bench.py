@@ -18,6 +18,14 @@ mox_render(ctx, 8, seed): +8 samples for every pixel, rendered in wavefronts of 
   e2e     same metric through the C ABI with host buffers: per step set_camera (host struct),
           launch(seed), gather to rank 0, read_accum into a host array (device->host of the whole
           accumulation buffer inside the timed region).
+
+  --dump-outputs DIR  after the timed steps, rank 0 writes what they computed, so that two builds can
+          be compared output for output (the inputs are the same from run to run):
+            accum.npy        float32 (N, 3): the gathered accumulation buffer (warm-up + timed steps, 8 spp
+                             each) at N pixels: all of them when width*height <= 2^21, else a seeded
+                             sample of 2^21 pixels
+            accum_pixel.npy  float64 (N,): the row-major pixel index (y * width + x) of each row
+            ray_counts.npy   float64 [primary + bounce rays, shadow rays] of the K timed steps, all ranks
 """
 import argparse
 import json
@@ -38,13 +46,24 @@ WIDTH, HEIGHT, MAX_DEPTH, SEED = 3840, 2160, 5, 0xD1A1A6
 SPP_PER_STEP = 8
 TRIS = 1_000_000
 WORKLOAD = f"interior ~1M-triangle Disney scene (BASELINE configs[3]), 3840x2160, {SPP_PER_STEP} spp per step, max depth 5, rng=ref"
+DUMP_PIXELS = 1 << 21   # 2^21 pixels: 24 MiB of float32 RGB + 16 MiB of float64 indices, under 64 MB in all
+
+
+def positive(text):
+    v = int(text)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return v
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=8)
+    ap.add_argument("--steps", type=positive, default=8)
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the accumulation buffer (warm-up + timed steps; a seeded sample of "
+                         "2^21 pixels when larger) and the ray counts of the timed steps to DIR/*.npy (see the module docstring)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--width", type=int, default=WIDTH)
     ap.add_argument("--height", type=int, default=HEIGHT)
@@ -52,7 +71,27 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--emulate-world", type=int, default=0,
                     help="experiment: render only rank 0's tile set of an N-rank partition on this one GPU (what each GPU of an N-GPU run does)")
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
+
+
+def dump_arrays(img, rays, shadow):
+    """The arrays of --dump-outputs from the gathered (H, W, 3) accumulation buffer and the timed steps' ray counts."""
+    import numpy as np
+    flat = img.reshape(-1, 3)
+    n = len(flat)
+    pix = np.arange(n) if n <= DUMP_PIXELS else np.sort(np.random.default_rng(SEED).choice(n, DUMP_PIXELS, replace=False))
+    return {"accum": flat[pix].astype(np.float32), "accum_pixel": pix.astype(np.float64),
+            "ray_counts": np.array([rays, shadow], dtype=np.float64)}
+
+
+def write_dump(directory, arrays):
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -303,6 +342,10 @@ def main():
     rays_all, shadow_all, launches_all = cnt.tolist()
     value = rays_all / (dev_ms * 1e3)
 
+    dump = None
+    if args.dump_outputs and rank == 0:   # read now: the e2e run below clears the accumulation buffer
+        dump = dump_arrays(tiles.read(), rays_all, shadow_all)
+
     # dominant kernel: closest-hit traversal (k_extend), timed live with CUDA events on its stream
     ext_ms = s1["ms_extend"] - s0["ms_extend"]
     ext_launches = s1["extend_launches"] - s0["extend_launches"]
@@ -464,6 +507,8 @@ def main():
                 "gather_bytes": tiles.bytes_on_the_wire(), "gather_transport": tiles.transport(), "gather_ms": g0.elapsed_time(g1), "render_ms_rank0": s1["ms_render"] - s0["ms_render"], "render_ms_per_rank": render_per_rank, "tile": TILE, "gpu_launches": int(launches_all), "clocks": clocks, "roofline": roofline_shadow if (roofline_shadow and roofline and roofline_shadow["share_of_step"] > roofline["share_of_step"]) else roofline,
                 "roofline_closest": roofline, "roofline_shadow": roofline_shadow, "roofline_build": roofline_build,
                 "serial_pass": serial, "per_depth": per_depth, "cpu_baseline": cpu_baseline}
+        if dump is not None:
+            write_dump(args.dump_outputs, dump)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
