@@ -88,11 +88,6 @@ struct BuildOutput {
 bool buildBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::string& err);
 bool radixSortPairs(uint32_t* keys, uint32_t* vals, int n, cudaStream_t stream, std::string& err);
 
-// Allocation-free sorter used by the render loop (see bvh_build.cu).
-size_t radixSortScratchBytes(size_t maxN);
-void radixSortAsync(uint32_t* keysA, uint32_t* valsA, uint32_t* keysB, uint32_t* valsB, int n, int passes, uint32_t* scratch,
-                    cudaStream_t stream);
-
 // Collapse of the PLOC tree into the compressed wide BVH (bvh_wide.cu).
 size_t wideScratchBytes(int n);
 bool wideCollapse(const PlocScratch& s, int n, uint32_t root, DeviceArena& arena, BvhNode8* outNodes, uint32_t** orderedIds8Out,

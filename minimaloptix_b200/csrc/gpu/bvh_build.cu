@@ -606,27 +606,3 @@ bool radixSortPairs(uint32_t* keys, uint32_t* vals, int n, cudaStream_t stream, 
   if (flag) { err = "radix sort look-back timed out"; return false; }
   return true;
 }
-
-// Pre-allocated sorter for the render loop (ray reordering): `passes` 8-bit digits starting at
-// bit 0; the sorted pairs end up in (keysB, valsB) when `passes` is odd, in (keysA, valsA)
-// otherwise.  Nothing is allocated or synchronised here.
-size_t radixSortScratchBytes(size_t maxN) {
-  return ((size_t)(16 + 1024) + (size_t)4 * divUp(std::max<size_t>(maxN, 1), SORT_TILE) * 256) * 4;
-}
-void radixSortAsync(uint32_t* keysA, uint32_t* valsA, uint32_t* keysB, uint32_t* valsB, int n, int passes, uint32_t* scratch,
-                    cudaStream_t stream) {
-  if (n <= 0 || passes <= 0) return;
-  if (passes > 4) passes = 4;
-  const int nTiles = divUp(n, SORT_TILE);
-  uint32_t* small = scratch;
-  uint32_t* status = scratch + 16 + 1024;
-  cudaMemsetAsync(scratch, 0, ((size_t)(16 + 1024) + (size_t)passes * nTiles * 256) * 4, stream);
-  k_sort_hist<<<std::min(divUp(n, 256 * 8), histGridCap()), 256, 0, stream>>>(keysA, n, small + 16);
-  k_sort_scan_hist<<<1, 256, 0, stream>>>(small + 16);
-  uint32_t *kin = keysA, *vin = valsA, *kout = keysB, *vout = valsB;
-  for (int p = 0; p < passes; ++p) {
-    k_sort_pass<<<nTiles, SORT_THREADS, 0, stream>>>(kin, vin, kout, vout, n, 8 * p, small + 16 + 256 * p, small + 8 + p,
-                                                     status + (size_t)p * nTiles * 256, small + 7);
-    std::swap(kin, kout); std::swap(vin, vout);
-  }
-}

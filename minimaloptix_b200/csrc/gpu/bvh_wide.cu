@@ -162,7 +162,6 @@ k_collapse_level(int nItems, const WorkItem* __restrict__ items, int nLeaves, co
       ch[best] = c.x;
       ch[n++] = c.y;
     }
-#ifndef MOX_WIDE_NO_FILL
     // free slots left: also open small leaf subtrees (largest first), so the bottom nodes give every
     // primitive its own 8-bit box instead of leaving slots empty
     while (n < 8) {
@@ -178,7 +177,6 @@ k_collapse_level(int nItems, const WorkItem* __restrict__ items, int nLeaves, co
       ch[best] = c.x;
       ch[n++] = c.y;
     }
-#endif
   }
   // ---- node box and grid
   const float4 blo = nodeLo[it.binNode], bhi = nodeHi[it.binNode];
@@ -214,13 +212,13 @@ k_collapse_level(int nItems, const WorkItem* __restrict__ items, int nLeaves, co
   const uint32_t primBase = nPrims ? atomicAdd(&counters[1], nPrims) : 0u;
   const uint32_t nextBase = nInner ? atomicAdd(const_cast<uint32_t*>(levelCount) + 1, nInner) : 0u;
   // ---- emit
-  uint32_t meta[8], qlx[8], qly[8], qlz[8], qhx[8], qhy[8], qhz[8];
+  uint32_t qlx[8], qly[8], qlz[8], qhx[8], qhy[8], qhz[8];
   uint32_t innerRank = 0, primOff = 0;
-  uint32_t validPrims = 0;   // fixed-slot layout: bits 2s, 2s + 1 = the primitives of the leaf child in slot s
+  uint32_t validPrims = 0;   // bits 2s, 2s + 1 = the primitives of the leaf child in slot s
   for (int s = 0; s < 8; ++s) {
     int i = childAt[s];
     if (i < 0) {  // empty slot: inverted box, never hit
-      meta[s] = 0; qlx[s] = qly[s] = qlz[s] = 255; qhx[s] = qhy[s] = qhz[s] = 0;
+      qlx[s] = qly[s] = qlz[s] = 255; qhx[s] = qhy[s] = qhz[s] = 0;
       continue;
     }
     const uint32_t c = ch[i];
@@ -237,7 +235,6 @@ k_collapse_level(int nItems, const WorkItem* __restrict__ items, int nLeaves, co
     qh = (int)ceilf((hi.z - blo.z) / sz); qh = max(0, min(255, qh)); while (qh < 255 && blo.z + qh * sz < hi.z) ++qh;
     qlz[s] = ql; qhz[s] = qh;
     if (imask & (1u << s)) {
-      meta[s] = (1u << 5) | (24u + (uint32_t)s);
       nextItems[nextBase + innerRank] = WorkItem{c, childBase + innerRank};
       innerRank++;
     } else {
@@ -247,7 +244,6 @@ k_collapse_level(int nItems, const WorkItem* __restrict__ items, int nLeaves, co
       if (c < (uint32_t)nLeaves) first = leafPos[c];
       else first = firstPos[c - nLeaves];   // leaf-order position of the subtree's first primitive (k_ploc_leaf_order)
       for (uint32_t k = 0; k < cnt; ++k) orderedIds8[primBase + primOff + k] = orderedIds[first + k];
-      meta[s] = (((1u << cnt) - 1u) << 5) | primOff;
       validPrims |= ((1u << cnt) - 1u) << (2 * s);
       primOff += cnt;
     }
@@ -255,12 +251,8 @@ k_collapse_level(int nItems, const WorkItem* __restrict__ items, int nLeaves, co
   auto pack4 = [](const uint32_t* v) { return v[0] | (v[1] << 8) | (v[2] << 16) | (v[3] << 24); };
   BvhNode8 nd;
   nd.n0 = make_float4(blo.x, blo.y, blo.z, __uint_as_float(ex | (ey << 8) | (ez << 16) | (imask << 24)));
-#ifdef MOX_NODE_META
-  nd.n1 = make_float4(__uint_as_float(childBase), __uint_as_float(primBase), __uint_as_float(pack4(meta)), __uint_as_float(pack4(meta + 4)));
-#else
-  nd.n1 = make_float4(__uint_as_float(childBase), __uint_as_float(primBase), __uint_as_float((imask << MOX_NODE_VALID_INNER_SHIFT) | validPrims),
+  nd.n1 = make_float4(__uint_as_float(childBase), __uint_as_float(primBase), __uint_as_float((imask << 24) | validPrims),
                       __uint_as_float((validPrims << 8) | imask));
-#endif
   nd.n2 = make_float4(__uint_as_float(pack4(qlx)), __uint_as_float(pack4(qlx + 4)), __uint_as_float(pack4(qly)), __uint_as_float(pack4(qly + 4)));
   nd.n3 = make_float4(__uint_as_float(pack4(qlz)), __uint_as_float(pack4(qlz + 4)), __uint_as_float(pack4(qhx)), __uint_as_float(pack4(qhx + 4)));
   nd.n4 = make_float4(__uint_as_float(pack4(qhy)), __uint_as_float(pack4(qhy + 4)), __uint_as_float(pack4(qhz)), __uint_as_float(pack4(qhz + 4)));

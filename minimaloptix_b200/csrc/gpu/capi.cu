@@ -58,7 +58,7 @@ struct DevBuf {
 struct mox_ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
-  cudaEvent_t ev0 = nullptr, ev1 = nullptr, evFork = nullptr;
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   std::string err;
 
   RenderParams rp{};
@@ -108,30 +108,20 @@ struct mox_ctx {
   std::vector<DevBuf> otherOwned;  // cached owned lists of other ranks (unpack)
   std::vector<uint64_t> ownedCount; // cached |owned pixels| per rank of the current partition
 
-  // The owned pixels of a batch can be rendered as `nSlices` independent sub-batches ("slices"), each with its own
-  // path buffers and stream: while the host reads one slice's material counts back, and while that slice's
-  // persistent traversal kernel drains its last rays, the other slice's kernels keep the SMs busy.  Since the
-  // shadow rays of a bounce run on their own stream (overlapShadow) a single slice already has two traversal
-  // launches in flight, and one slice measures as fast at full frame (1347 vs 1350 Mrays/s), faster on an eighth
-  // of the frame (14.99 vs 15.16 ms per step) and end to end (1340 vs 1262): the default is 1 (MOX_SLICES=2..4).
-  struct Slice {
-    PathBuffers pb;
-    cudaStream_t stream = nullptr;   // slice 0 uses the context stream
-    cudaStream_t shadowStream = nullptr;  // shadow traversal + k_apply of bounce b, overlapping extend + classify of bounce b+1
-    cudaEvent_t evShaded = nullptr, evApplied = nullptr;
-    bool applyPending = false;       // evApplied must be waited for before the next kernel that touches rad / the shadow buffers
-    cudaEvent_t evReady = nullptr;   // the counters of the bounce in flight have landed in hostCnt
-    uint32_t* hostCnt = nullptr;     // pinned: C_WORDS + BOUNCE_RING * C_BOUNCE_WORDS
-    StageTimer timer;
-    // state of the batch in flight
-    LaunchCtx lc;
-    uint32_t S = 0, bound = 0, depth = 0, matCount[Q_COUNT] = {0, 0, 0, 0};
-    int iCur = 0, iNext = 1, iSpare = 2;
-    bool done = true;
-  };
-  static constexpr int kMaxSlices = 4;
-  Slice slices[kMaxSlices];
-  int nSlices = 1;
+  // Wavefront state of the batch in flight.  The shadow rays of a bounce run on their own stream (overlapShadow), so
+  // two persistent traversal launches are in flight while the host waits for a bounce's material counts.  Splitting
+  // a batch into sub-batches on further streams measured no faster (1347 vs 1350 Mrays/s at full frame, slower on an
+  // eighth of it) and was removed (DESIGN.md section 4; the code is in the git history).
+  PathBuffers pb;
+  cudaStream_t shadowStream = nullptr;  // shadow traversal + k_apply of bounce b, overlapping extend + classify of bounce b+1
+  cudaEvent_t evShaded = nullptr, evApplied = nullptr;
+  bool applyPending = false;       // evApplied must be waited for before the next kernel that touches rad / the shadow buffers
+  cudaEvent_t evReady = nullptr;   // the counters of the bounce in flight have landed in hostCnt
+  uint32_t* hostCnt = nullptr;     // pinned: C_WORDS + BOUNCE_RING * C_BOUNCE_WORDS
+  StageTimer timer;
+  LaunchCtx lc;
+  uint32_t batchSamples = 0, bound = 0, depth = 0, matCount[Q_COUNT] = {0, 0, 0, 0};
+  bool batchDone = true;
   float* pinned = nullptr;
   size_t pinnedBytes = 0;
 
@@ -156,14 +146,9 @@ struct mox_ctx {
   double msRender = 0, msBuild = 0;
   double msStage[ST_COUNT] = {0, 0, 0, 0, 0};
   uint64_t extendLaunches = 0, kernelLaunches = 0;
-  size_t maxBatchPaths = 32u << 20;  // paths per wavefront (~280 B each with 4 lights); measured 4 Mi -> 947, 32 Mi -> 980 Mrays/s at 4K
+  size_t maxBatchPaths = 32u << 20;  // paths per wavefront (264 B each with 4 lights, bytesPerPath); measured 4 Mi -> 947, 32 Mi -> 980 Mrays/s at 4K
   bool overlapShadow = true;     // shadow rays of bounce b on a second stream, concurrent with the extend launch of bounce b+1 (MOX_OVERLAP_SHADOW=0: serial)
-  bool disneySplit = false;      // Disney NORMAL shading as two kernels sharing a per-hit record (MOX_DISNEY_SPLIT=0: one kernel)
   bool brdfFast = true;          // approximate reciprocal / square root inside BRDF values (MOX_BRDF_IEEE=1: IEEE, the oracle's operations)
-  bool hasDisneyNormal = false;  // some material runs the Disney NORMAL program (set by mox_build_accel)
-  bool sortRays = false;         // reorder the extend queue by (direction octant, origin cell) from bounce 2 on
-  int sortPasses = 3;            // 3: the whole 24-bit key; 1: octant + the 5 top bits of the cell (MOX_SORT_PASSES)
-  float sceneLo[3] = {0, 0, 0}, sceneHi[3] = {1, 1, 1};
 };
 
 namespace {
@@ -249,23 +234,21 @@ int refreshOwned(mox_ctx* c) {
 void freePaths(PathBuffers& pb) {
   cudaFree(pb.rayO); cudaFree(pb.rayD); cudaFree(pb.hit); cudaFree(pb.thr); cudaFree(pb.rad); cudaFree(pb.state);
   for (auto& q : pb.qBuf) cudaFree(q);
-  for (auto& k : pb.kBuf) cudaFree(k);
-  cudaFree(pb.sortScratch);
   for (auto& q : pb.qMat) cudaFree(q);
-  cudaFree(pb.shO); cudaFree(pb.shD); cudaFree(pb.shC); cudaFree(pb.shQueue); cudaFree(pb.counters); cudaFree(pb.seeds); cudaFree(pb.disneyRec); cudaFree(pb.qDisneyAlt);
+  cudaFree(pb.shO); cudaFree(pb.shD); cudaFree(pb.shC); cudaFree(pb.shQueue); cudaFree(pb.counters); cudaFree(pb.seeds); cudaFree(pb.qDisneyAlt);
   pb = PathBuffers();
 }
 
 constexpr size_t kCounterWords = C_WORDS + BOUNCE_RING * C_BOUNCE_WORDS;
 
-// Bytes of wavefront state per path (see PathBuffers): rays, hit, throughput, radiance, RNG state, three queue
-// buffers, two key buffers, four material queues; per light a direction, a contribution and a queue entry; one
-// shadow origin when there are lights.
-size_t bytesPerPath(size_t nLights) { return 16 * 4 + 8 + 4 + 3 * 4 + 2 * 4 + 5 * 4 + (nLights ? 16 + nLights * 36 : 0) + 16 * MOX_DISNEY_REC_F4; }
+// Bytes of wavefront state per path (see PathBuffers): rays, hit, throughput, radiance, RNG state, two queue
+// buffers, four material queues and the second Disney queue; per light a direction, a contribution and a queue
+// entry; one shadow origin when there are lights.
+size_t bytesPerPath(size_t nLights) { return 16 * 4 + 8 + 4 + 2 * 4 + 5 * 4 + (nLights ? 16 + nLights * 36 : 0); }
 
 int ensurePaths(mox_ctx* c, PathBuffers& pb, cudaStream_t stream, size_t paths, size_t nLights, size_t nSeeds) {
   size_t slots = paths * nLights;
-  if (pb.capacity < paths || pb.shadowSlots < slots || !pb.counters || (c->disneySplit && c->hasDisneyNormal && !pb.disneyRec)) {
+  if (pb.capacity < paths || pb.shadowSlots < slots || !pb.counters) {
     cudaStreamSynchronize(stream);
     // grow geometrically so that a slowly growing sample count does not reallocate on every call
     if (pb.capacity && paths > pb.capacity) paths = std::max(paths, pb.capacity + pb.capacity / 2);
@@ -279,17 +262,12 @@ int ensurePaths(mox_ctx* c, PathBuffers& pb, cudaStream_t stream, size_t paths, 
     CUCK(c, cudaMalloc(&pb.hit, paths * 8)); CUCK(c, cudaMalloc(&pb.thr, paths * 16));
     CUCK(c, cudaMalloc(&pb.rad, paths * 16)); CUCK(c, cudaMalloc(&pb.state, paths * 4));
     for (auto& q : pb.qBuf) CUCK(c, cudaMalloc(&q, paths * 4));
-    if (c->sortRays) {
-      for (auto& k : pb.kBuf) CUCK(c, cudaMalloc(&k, paths * 4));
-      CUCK(c, cudaMalloc(&pb.sortScratch, radixSortScratchBytes(paths)));
-    }
     for (auto& q : pb.qMat) CUCK(c, cudaMalloc(&q, paths * 4));
     CUCK(c, cudaMalloc(&pb.qDisneyAlt, paths * 4));
     if (slots) {
       CUCK(c, cudaMalloc(&pb.shO, paths * 16)); CUCK(c, cudaMalloc(&pb.shD, slots * 16)); CUCK(c, cudaMalloc(&pb.shC, slots * 16));
       CUCK(c, cudaMalloc(&pb.shQueue, slots * 4));
     }
-    if (c->disneySplit && c->hasDisneyNormal) CUCK(c, cudaMalloc(&pb.disneyRec, paths * 16 * MOX_DISNEY_REC_F4));
     CUCK(c, cudaMalloc(&pb.counters, kCounterWords * 4));
     CUCK(c, cudaMemset(pb.counters, 0, kCounterWords * 4));
     pb.capacity = paths; pb.shadowSlots = slots;
@@ -384,230 +362,155 @@ int syncLights(mox_ctx* c) {
 
 inline uint32_t* bounceBlock(const PathBuffers& pb, uint32_t depth) { return pb.counters + C_WORDS + (depth % BOUNCE_RING) * C_BOUNCE_WORDS; }
 
-int ensureSlice(mox_ctx* c, int k) {
-  mox_ctx::Slice& sl = c->slices[k];
-  if (!sl.stream) {
-    if (k == 0) sl.stream = c->stream;
-    else CUCK(c, cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
-  }
-  if (!sl.evReady) CUCK(c, cudaEventCreateWithFlags(&sl.evReady, cudaEventDisableTiming));
-  if (c->overlapShadow && !sl.shadowStream) {
-    CUCK(c, cudaStreamCreateWithFlags(&sl.shadowStream, cudaStreamNonBlocking));
-    CUCK(c, cudaEventCreateWithFlags(&sl.evShaded, cudaEventDisableTiming));
-    CUCK(c, cudaEventCreateWithFlags(&sl.evApplied, cudaEventDisableTiming));
-  }
-  if (!sl.hostCnt) CUCK(c, cudaMallocHost(&sl.hostCnt, kCounterWords * 4));
-  return MOX_OK;
-}
-
-// Enqueue one bounce of a slice up to the point where the host needs numbers: extend (persistent traversal, ray
-// count read on the device), classify, and the read-back of the counters.
-int sliceEnqueueExtend(mox_ctx* c, mox_ctx::Slice& sl) {
-  LaunchCtx& lc = sl.lc;
-  StageTimer& tm = sl.timer;
-  const uint32_t depth = sl.depth;
-  lc.bc = bounceBlock(sl.pb, depth);
-  lc.pb.qMat[Q_DISNEY] = (depth & 1u) ? sl.pb.qMat[Q_DISNEY] : sl.pb.qDisneyAlt;   // k_apply of bounce depth-1 may still read the other one
+// Enqueue one bounce up to the point where the host needs numbers: extend (persistent traversal, ray count read on
+// the device), classify, and the read-back of the counters.
+int enqueueExtend(mox_ctx* c) {
+  LaunchCtx& lc = c->lc;
+  StageTimer& tm = c->timer;
+  const uint32_t depth = c->depth;
+  lc.bc = bounceBlock(c->pb, depth);
+  lc.pb.qMat[Q_DISNEY] = (depth & 1u) ? c->pb.qMat[Q_DISNEY] : c->pb.qDisneyAlt;   // k_apply of bounce depth-1 may still read the other one
   // bounce 1 traces exactly `bound` camera rays; later bounces read the number of spawned rays from the previous
   // bounce's counter block, `bound` (what was shaded) only sizes the grids
-  const uint32_t* countPtr = depth == 1 ? nullptr : bounceBlock(sl.pb, depth - 1) + C_NEXT;
-  tm.begin(ST_EXTEND, sl.stream, depth);
+  const uint32_t* countPtr = depth == 1 ? nullptr : bounceBlock(c->pb, depth - 1) + C_NEXT;
+  tm.begin(ST_EXTEND, c->stream, depth);
   // camera rays are queued in path order (k_generate: qCur[p] = p): the traversal kernel skips the indirection
-  launchExtend(lc, depth == 1 ? nullptr : lc.pb.qCur, sl.bound, countPtr, depth);
-  tm.end(sl.stream);
-  tm.begin(ST_SHADE, sl.stream);
-  launchClassify(lc, lc.pb.qCur, sl.bound, countPtr, depth);
-  tm.end(sl.stream);
+  launchExtend(lc, depth == 1 ? nullptr : lc.pb.qCur, c->bound, countPtr, depth);
+  tm.end(c->stream);
+  tm.begin(ST_SHADE, c->stream);
+  launchClassify(lc, lc.pb.qCur, c->bound, countPtr, depth);
+  tm.end(c->stream);
   c->extendLaunches++; c->kernelLaunches += 2;
-  CUCK(c, cudaMemcpyAsync(sl.hostCnt, sl.pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, sl.stream));
-  CUCK(c, cudaEventRecord(sl.evReady, sl.stream));
+  CUCK(c, cudaMemcpyAsync(c->hostCnt, c->pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, c->stream));
+  CUCK(c, cudaEventRecord(c->evReady, c->stream));
   return MOX_OK;
 }
 
-int sliceFinish(mox_ctx* c, mox_ctx::Slice& sl) {
-  StageTimer& tm = sl.timer;
-  if (sl.applyPending) { CUCK(c, cudaStreamWaitEvent(sl.stream, sl.evApplied, 0)); sl.applyPending = false; }
-  tm.begin(ST_ACCUMULATE, sl.stream);
-  launchAccumulate(sl.lc, sl.S);
-  tm.end(sl.stream);
+int finishBatch(mox_ctx* c) {
+  StageTimer& tm = c->timer;
+  if (c->applyPending) { CUCK(c, cudaStreamWaitEvent(c->stream, c->evApplied, 0)); c->applyPending = false; }
+  tm.begin(ST_ACCUMULATE, c->stream);
+  launchAccumulate(c->lc, c->batchSamples);
+  tm.end(c->stream);
   c->kernelLaunches++;
-  CUCK(c, cudaMemcpyAsync(sl.hostCnt, sl.pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, sl.stream));
-  CUCK(c, cudaEventRecord(sl.evReady, sl.stream));
-  sl.done = true;
+  CUCK(c, cudaMemcpyAsync(c->hostCnt, c->pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, c->stream));
+  CUCK(c, cudaEventRecord(c->evReady, c->stream));
+  c->batchDone = true;
   return MOX_OK;
 }
 
 // The counters of the bounce in flight have arrived: shade what was binned, trace the shadow rays, and enqueue
 // the next bounce — or the accumulation when nothing is left.
-int sliceAdvance(mox_ctx* c, mox_ctx::Slice& sl) {
-  LaunchCtx& lc = sl.lc;
-  StageTimer& tm = sl.timer;
-  PathBuffers& pb = sl.pb;
-  const uint32_t depth = sl.depth;
-  const uint32_t* hostBounce = sl.hostCnt + C_WORDS + (depth % BOUNCE_RING) * C_BOUNCE_WORDS;
+int advanceBounce(mox_ctx* c) {
+  LaunchCtx& lc = c->lc;
+  StageTimer& tm = c->timer;
+  PathBuffers& pb = c->pb;
+  const uint32_t depth = c->depth;
+  const uint32_t* hostBounce = c->hostCnt + C_WORDS + (depth % BOUNCE_RING) * C_BOUNCE_WORDS;
   const uint32_t dIdx = std::min<uint32_t>(depth, MOX_STATS_DEPTHS - 1);
-  if (depth == 1) { c->raysPrimary += sl.bound; c->raysDepth[1] += sl.bound; }
+  if (depth == 1) { c->raysPrimary += c->bound; c->raysDepth[1] += c->bound; }
   else {  // exact number of rays this bounce traced, and of shadow rays the previous one queued
-    const uint32_t* prev = sl.hostCnt + C_WORDS + ((depth - 1) % BOUNCE_RING) * C_BOUNCE_WORDS;
+    const uint32_t* prev = c->hostCnt + C_WORDS + ((depth - 1) % BOUNCE_RING) * C_BOUNCE_WORDS;
     c->raysBounce += prev[C_NEXT];
     c->raysShadowTraced += prev[C_SHQ];
     c->raysDepth[dIdx] += prev[C_NEXT];
     c->shadowDepth[std::min<uint32_t>(depth - 1, MOX_STATS_DEPTHS - 1)] += prev[C_SHQ];
   }
   uint32_t any = 0;
-  for (int k = 0; k < Q_COUNT; ++k) { sl.matCount[k] = hostBounce[C_MAT0 + k]; any += sl.matCount[k]; }
-  if (!any) return sliceFinish(c, sl);
+  for (int k = 0; k < Q_COUNT; ++k) { c->matCount[k] = hostBounce[C_MAT0 + k]; any += c->matCount[k]; }
+  if (!any) return finishBatch(c);
   // the shade kernels touch the radiance and rewrite the shadow-ray buffers: the previous bounce's k_apply first
-  if (sl.applyPending) { CUCK(c, cudaStreamWaitEvent(sl.stream, sl.evApplied, 0)); sl.applyPending = false; }
-  tm.begin(ST_SHADE, sl.stream);
-  for (int k = 0; k < Q_COUNT; ++k) { launchShade(lc, k, sl.matCount[k], depth); if (sl.matCount[k]) c->kernelLaunches += (k == Q_DISNEY && lc.disneySplit) ? 2 : 1; }
-  tm.end(sl.stream);
-  if (sl.matCount[Q_DISNEY] && lc.scene.nLights) {
+  if (c->applyPending) { CUCK(c, cudaStreamWaitEvent(c->stream, c->evApplied, 0)); c->applyPending = false; }
+  tm.begin(ST_SHADE, c->stream);
+  for (int k = 0; k < Q_COUNT; ++k) { launchShade(lc, k, c->matCount[k], depth); if (c->matCount[k]) c->kernelLaunches++; }
+  tm.end(c->stream);
+  if (c->matCount[Q_DISNEY] && lc.scene.nLights) {
     // Shadow rays and the NEE sum depend only on this bounce's shade kernels; the next extend launch does not
     // depend on them.  On a second stream the two persistent traversal launches overlap: each one's last CTAs
     // drain while the other's first CTAs already run.
-    cudaStream_t ss = sl.stream;
-    if (c->overlapShadow && sl.shadowStream) {
-      ss = sl.shadowStream;
-      CUCK(c, cudaEventRecord(sl.evShaded, sl.stream));
-      CUCK(c, cudaStreamWaitEvent(ss, sl.evShaded, 0));
+    cudaStream_t ss = c->stream;
+    if (c->overlapShadow && c->shadowStream) {
+      ss = c->shadowStream;
+      CUCK(c, cudaEventRecord(c->evShaded, c->stream));
+      CUCK(c, cudaStreamWaitEvent(ss, c->evShaded, 0));
     }
     tm.begin(ST_SHADOW, ss, depth);
-    launchShadow(lc, sl.matCount[Q_DISNEY], ss);
+    launchShadow(lc, c->matCount[Q_DISNEY], ss);
     tm.end(ss);
     tm.begin(ST_SHADE, ss);
-    launchApply(lc, sl.matCount[Q_DISNEY], ss);
+    launchApply(lc, c->matCount[Q_DISNEY], ss);
     tm.end(ss);
-    if (ss != sl.stream) { CUCK(c, cudaEventRecord(sl.evApplied, ss)); sl.applyPending = true; }
+    if (ss != c->stream) { CUCK(c, cudaEventRecord(c->evApplied, ss)); c->applyPending = true; }
     c->kernelLaunches += 2;
   }
   // the block bounce depth+1 will use was last written BOUNCE_RING bounces ago
-  CUCK(c, cudaMemsetAsync(bounceBlock(pb, depth + 1), 0, C_BOUNCE_WORDS * 4, sl.stream));
-  uint32_t bound = any;   // every shaded path spawns at most one ray
-  if (c->sortRays) {
-    // reordering needs the exact count on the host: one more round trip (this mode is an experiment, off by default)
-    CUCK(c, cudaMemcpyAsync(sl.hostCnt, pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, sl.stream));
-    CUCK(c, cudaStreamSynchronize(sl.stream));
-    bound = hostBounce[C_NEXT];
-  }
-  if (c->sortRays && bound > 4096) {
-    // 24-bit keys -> 3 passes (or their top 8 bits -> 1): the sorted queue lands in (kBuf[1], qBuf[iSpare])
-    tm.begin(ST_SHADE, sl.stream);
-    radixSortAsync(pb.kBuf[0], pb.qBuf[sl.iNext], pb.kBuf[1], pb.qBuf[sl.iSpare], (int)bound, c->sortPasses, pb.sortScratch, sl.stream);
-    tm.end(sl.stream);
-    c->kernelLaunches += 5;
-    int t = sl.iCur; sl.iCur = sl.iSpare; sl.iSpare = sl.iNext; sl.iNext = t;
-  } else {
-    int t = sl.iCur; sl.iCur = sl.iNext; sl.iNext = t;
-  }
-  lc.pb.qCur = pb.qBuf[sl.iCur]; lc.pb.qNext = pb.qBuf[sl.iNext];
-  sl.bound = bound;
-  sl.depth = depth + 1;
-  if (!bound) return sliceFinish(c, sl);
-  return sliceEnqueueExtend(c, sl);
+  CUCK(c, cudaMemsetAsync(bounceBlock(pb, depth + 1), 0, C_BOUNCE_WORDS * 4, c->stream));
+  std::swap(lc.pb.qCur, lc.pb.qNext);
+  c->bound = any;   // every shaded path spawns at most one ray
+  c->depth = depth + 1;
+  return enqueueExtend(c);
 }
 
-int slicesFor(const mox_ctx* c, size_t paths) {
-  int K = c->nSlices;
-  if (paths < (size_t)K * 65536 || c->nOwned < (uint32_t)K) K = 1;   // tiny batches: the second stream buys nothing
-  return K;
-}
-
-// Streams, events, pinned counters and wavefront buffers for a batch of S samples per owned pixel.  renderSeeds
-// calls it before its timed region, so the first launch of a context does not time its own allocations.
+// Events, pinned counters and wavefront buffers for a batch of S samples per owned pixel.  renderSeeds calls it
+// before its timed region, so the first launch of a context does not time its own allocations.
 int prepareBatch(mox_ctx* c, uint32_t S) {
-  const size_t P = (size_t)S * c->nOwned;
-  const int K = slicesFor(c, P);
-  for (int k = 0; k < K; ++k) {
-    int rc = ensureSlice(c, k);
-    if (rc) return rc;
-    const uint32_t nPix = (uint32_t)((uint64_t)c->nOwned * (k + 1) / K) - (uint32_t)((uint64_t)c->nOwned * k / K);
-    if ((rc = ensurePaths(c, c->slices[k].pb, c->slices[k].stream, (size_t)S * nPix, c->lights.size(), S))) return rc;
+  if (!c->evReady) CUCK(c, cudaEventCreateWithFlags(&c->evReady, cudaEventDisableTiming));
+  if (c->overlapShadow && !c->shadowStream) {
+    CUCK(c, cudaStreamCreateWithFlags(&c->shadowStream, cudaStreamNonBlocking));
+    CUCK(c, cudaEventCreateWithFlags(&c->evShaded, cudaEventDisableTiming));
+    CUCK(c, cudaEventCreateWithFlags(&c->evApplied, cudaEventDisableTiming));
   }
-  return MOX_OK;
+  if (!c->hostCnt) CUCK(c, cudaMallocHost(&c->hostCnt, kCounterWords * 4));
+  return ensurePaths(c, c->pb, c->stream, (size_t)S * c->nOwned, c->lights.size(), S);
 }
 
-// One wavefront batch: `seeds.size()` samples of every owned pixel, rendered as nSlices interleaved sub-batches.
+// One wavefront batch: `seeds.size()` samples of every owned pixel.  Generate, then advance bounce by bounce until
+// no path is left, then collect the counters.
 int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds) {
   const uint32_t S = (uint32_t)seeds.size();
   const size_t P = (size_t)S * c->nOwned;
   if (P == 0) return MOX_OK;
   if (P > 0xfffffff0ull) return fail(c, MOX_ERR_INVALID, "batch too large");
-  const int K = slicesFor(c, P);
   int rc;
-  // slice k renders the owned pixels [first_k, first_k+1) — all S samples of a pixel stay in one slice, in launch
-  // order, so the accumulated sums do not depend on the number of slices
-  uint32_t first[mox_ctx::kMaxSlices + 1];
-  for (int k = 0; k <= K; ++k) first[k] = (uint32_t)((uint64_t)c->nOwned * k / K);
-  // all allocations first: a failure (MOX_ERR_OOM -> the caller retries with a smaller batch) must not leave
-  // work of another slice in flight
+  // all allocations first: a failure (MOX_ERR_OOM -> the caller retries with a smaller batch) must not leave work
+  // in flight
   if ((rc = prepareBatch(c, S))) return rc;
-  cudaEvent_t evStart = c->evFork;
-  CUCK(c, cudaEventRecord(evStart, c->stream));
-  for (int k = 0; k < K; ++k) {
-    mox_ctx::Slice& sl = c->slices[k];
-    const uint32_t nPix = first[k + 1] - first[k];
-    const size_t paths = (size_t)S * nPix;
-    if (k) CUCK(c, cudaStreamWaitEvent(sl.stream, evStart, 0));   // scene uploads happened on the context stream
-    PathBuffers& pb = sl.pb;
-    CUCK(c, cudaMemcpyAsync(pb.seeds, seeds.data(), S * 4, cudaMemcpyHostToDevice, sl.stream));
-    LaunchCtx& lc = sl.lc;
-    lc.scene = sceneView(c);
-    lc.rp = c->rp;
-    lc.pb = pb;
-    lc.ownedPix = c->dOwned + first[k];
-    lc.nOwned = nPix;
-    lc.accu = c->dAccu;
-    lc.countTraversal = (c->accelFlags & MOX_ACCEL_COUNTERS) != 0;
-    lc.disneySplit = c->disneySplit && pb.disneyRec != nullptr;
-    lc.brdfFast = c->brdfFast;
-    lc.stream = sl.stream;
-    lc.sceneLo = make_float3(c->sceneLo[0], c->sceneLo[1], c->sceneLo[2]);
-    {
-      float ex = c->sceneHi[0] - c->sceneLo[0], ey = c->sceneHi[1] - c->sceneLo[1], ez = c->sceneHi[2] - c->sceneLo[2];
-      lc.sceneInvExt = make_float3(ex > 0 ? 128.f / ex : 0.f, ey > 0 ? 128.f / ey : 0.f, ez > 0 ? 128.f / ez : 0.f);
-    }
-    sl.iCur = 0; sl.iNext = 1; sl.iSpare = 2;
-    lc.pb.qCur = pb.qBuf[sl.iCur]; lc.pb.qNext = pb.qBuf[sl.iNext];
-    lc.pb.qKey = c->sortRays ? pb.kBuf[0] : nullptr;
-    lc.sortShift = c->sortPasses == 1 ? 16u : 0u;
-    lc.bc = bounceBlock(pb, 1);
-    sl.S = S; sl.bound = (uint32_t)paths; sl.depth = 1; sl.done = false; sl.applyPending = false;
-    CUCK(c, cudaMemsetAsync(pb.counters, 0, kCounterWords * 4, sl.stream));
-    sl.timer.begin(ST_GENERATE, sl.stream);
-    launchGenerate(lc, S);
-    sl.timer.end(sl.stream);
-    c->kernelLaunches++;
-    if (!paths) { sl.done = true; CUCK(c, cudaEventRecord(sl.evReady, sl.stream)); continue; }
-    if ((rc = sliceEnqueueExtend(c, sl))) return rc;
+  PathBuffers& pb = c->pb;
+  CUCK(c, cudaMemcpyAsync(pb.seeds, seeds.data(), S * 4, cudaMemcpyHostToDevice, c->stream));
+  LaunchCtx& lc = c->lc;
+  lc.scene = sceneView(c);
+  lc.rp = c->rp;
+  lc.pb = pb;
+  lc.ownedPix = c->dOwned;
+  lc.nOwned = c->nOwned;
+  lc.accu = c->dAccu;
+  lc.countTraversal = (c->accelFlags & MOX_ACCEL_COUNTERS) != 0;
+  lc.brdfFast = c->brdfFast;
+  lc.stream = c->stream;
+  lc.pb.qCur = pb.qBuf[0]; lc.pb.qNext = pb.qBuf[1];
+  lc.bc = bounceBlock(pb, 1);
+  c->batchSamples = S; c->bound = (uint32_t)P; c->depth = 1; c->batchDone = false; c->applyPending = false;
+  CUCK(c, cudaMemsetAsync(pb.counters, 0, kCounterWords * 4, c->stream));
+  c->timer.begin(ST_GENERATE, c->stream);
+  launchGenerate(lc, S);
+  c->timer.end(c->stream);
+  c->kernelLaunches++;
+  if ((rc = enqueueExtend(c))) return rc;
+  while (!c->batchDone) {
+    CUCK(c, cudaEventSynchronize(c->evReady));
+    if ((rc = advanceBounce(c))) return rc;
   }
-  // Round-robin over the slices: wait for one slice's counters, enqueue its next stage, move on.  While the host
-  // sits in cudaEventSynchronize for slice A, slice B's kernels are already queued on the GPU.
-  for (int live = K; live > 0;) {
-    live = 0;
-    for (int k = 0; k < K; ++k) {
-      mox_ctx::Slice& sl = c->slices[k];
-      if (sl.done) continue;
-      CUCK(c, cudaEventSynchronize(sl.evReady));
-      if ((rc = sliceAdvance(c, sl))) return rc;
-      if (!sl.done) live++;
-    }
-  }
-  // join: every slice's accumulation and final counter read-back
-  for (int k = 0; k < K; ++k) {
-    mox_ctx::Slice& sl = c->slices[k];
-    CUCK(c, cudaEventSynchronize(sl.evReady));
-    if (k) CUCK(c, cudaStreamWaitEvent(c->stream, sl.evReady, 0));
-    const uint32_t* host = sl.hostCnt;
-    sl.timer.collect(c->msStage, c->msDepth);
-    c->nonfinite += host[C_NONFINITE];
-    c->shadowBlocked += host[C_SH_BLOCKED]; c->shadowTinted += host[C_SH_TINTED];
-    c->raysShadow += host[C_SHADOW];
-    c->nodeVisits += ((uint64_t)host[C_NODEVIS_HI] << 32) | host[C_NODEVIS_LO];
-    c->primTests += ((uint64_t)host[C_PRIMTEST_HI] << 32) | host[C_PRIMTEST_LO];
-    c->nodeVisitsShadow += ((uint64_t)host[C_NODEVIS_SH_LO + 1] << 32) | host[C_NODEVIS_SH_LO];
-    c->primTestsShadow += ((uint64_t)host[C_PRIMTEST_SH_LO + 1] << 32) | host[C_PRIMTEST_SH_LO];
-  }
+  // the accumulation and the final counter read-back
+  CUCK(c, cudaEventSynchronize(c->evReady));
+  const uint32_t* host = c->hostCnt;
+  c->timer.collect(c->msStage, c->msDepth);
+  c->nonfinite += host[C_NONFINITE];
+  c->shadowBlocked += host[C_SH_BLOCKED]; c->shadowTinted += host[C_SH_TINTED];
+  c->raysShadow += host[C_SHADOW];
+  c->nodeVisits += ((uint64_t)host[C_NODEVIS_HI] << 32) | host[C_NODEVIS_LO];
+  c->primTests += ((uint64_t)host[C_PRIMTEST_HI] << 32) | host[C_PRIMTEST_LO];
+  c->nodeVisitsShadow += ((uint64_t)host[C_NODEVIS_SH_LO + 1] << 32) | host[C_NODEVIS_SH_LO];
+  c->primTestsShadow += ((uint64_t)host[C_PRIMTEST_SH_LO + 1] << 32) | host[C_PRIMTEST_SH_LO];
   CUCK(c, cudaGetLastError());
   c->launches += S;
   return MOX_OK;
@@ -617,23 +520,17 @@ int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds) {
 // memory for this scene's light count (36 bytes per path and light).
 size_t batchCap(mox_ctx* c, size_t wanted /* samples per pixel of this call */) {
   size_t cap = c->maxBatchPaths;
+  const PathBuffers& pb = c->pb;
   // The buffers of an earlier call already hold such a batch: nothing will be allocated, so there is nothing to
   // budget.  (cudaMemGetInfo is a slow driver call — it was the 20-70 ms hiccup in front of some steps.)
   if (c->nOwned) {
     const size_t S = std::min(std::max<size_t>(1, cap / c->nOwned), wanted), nL = c->lights.size();   // samples per batch at the full cap
-    const int K = slicesFor(c, S * c->nOwned);
-    bool fits = true;
-    for (int k = 0; k < K && fits; ++k) {
-      const PathBuffers& pb = c->slices[k].pb;
-      const size_t nPix = (size_t)((uint64_t)c->nOwned * (k + 1) / K) - (size_t)((uint64_t)c->nOwned * k / K);   // as prepareBatch splits them
-      fits = pb.counters && pb.capacity >= S * nPix && pb.shadowSlots >= S * nPix * nL && pb.seedCap >= S;
-    }
-    if (fits) return cap;
+    const size_t P = S * c->nOwned;
+    if (pb.counters && pb.capacity >= P && pb.shadowSlots >= P * nL && pb.seedCap >= S) return cap;
   }
   size_t freeB = 0, totalB = 0;
   if (cudaMemGetInfo(&freeB, &totalB) == cudaSuccess) {
-    size_t have = 0;
-    for (auto& sl : c->slices) have += sl.pb.capacity * bytesPerPath(sl.pb.capacity ? sl.pb.shadowSlots / sl.pb.capacity : 0);
+    const size_t have = pb.capacity * bytesPerPath(pb.capacity ? pb.shadowSlots / pb.capacity : 0);
     size_t budget = (size_t)((freeB + have) * 0.6);
     cap = std::min(cap, std::max<size_t>(budget / bytesPerPath(c->lights.size()), 65536));
   }
@@ -662,7 +559,7 @@ int renderSeeds(mox_ctx* c, const std::vector<int32_t>& seeds) {
       // the allocation failed after all (fragmentation, another context on the device): free the wavefront
       // state, halve the batch and render this chunk again (nothing of it was enqueued)
       cudaGetLastError();
-      for (auto& sl : c->slices) { int32_t* sd = sl.pb.seeds; sl.pb.seeds = nullptr; freePaths(sl.pb); cudaFree(sd); }
+      { int32_t* sd = c->pb.seeds; c->pb.seeds = nullptr; freePaths(c->pb); cudaFree(sd); }
       perBatch = std::max<size_t>(1, perBatch / 2);
       continue;
     }
@@ -786,19 +683,14 @@ int mox_create(mox_ctx** out, int device_id) {
   mox_ctx* c = new mox_ctx();
   c->device = device_id;
   if ((e = cudaSetDevice(device_id)) != cudaSuccess || (e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking)) != cudaSuccess ||
-      (e = cudaEventCreate(&c->ev0)) != cudaSuccess || (e = cudaEventCreate(&c->ev1)) != cudaSuccess ||
-      (e = cudaEventCreateWithFlags(&c->evFork, cudaEventDisableTiming)) != cudaSuccess) {
+      (e = cudaEventCreate(&c->ev0)) != cudaSuccess || (e = cudaEventCreate(&c->ev1)) != cudaSuccess) {
     std::string msg = cudaGetErrorString(e);
     delete c;
     return fail(nullptr, MOX_ERR_CUDA, msg);
   }
-  if (const char* env = getenv("MOX_SORT_RAYS")) c->sortRays = atoi(env) != 0;
-  if (const char* env = getenv("MOX_SORT_PASSES")) c->sortPasses = atoi(env) == 1 ? 1 : 3;
   if (const char* env = getenv("MOX_MAX_BATCH_PATHS")) { long long v = atoll(env); if (v > 0) c->maxBatchPaths = (size_t)v; }
-  if (const char* env = getenv("MOX_DISNEY_SPLIT")) c->disneySplit = atoi(env) != 0;
   if (const char* env = getenv("MOX_OVERLAP_SHADOW")) c->overlapShadow = atoi(env) != 0;
   if (const char* env = getenv("MOX_BRDF_IEEE")) c->brdfFast = atoi(env) == 0;
-  if (const char* env = getenv("MOX_SLICES")) c->nSlices = std::min(std::max(atoi(env), 1), (int)mox_ctx::kMaxSlices);
   memset(&c->rp, 0, sizeof c->rp);
   c->rp.maxDepth = 256; c->rp.eps = 0.001f; c->rp.minIntensity = 0.001f;
   c->rp.bad = make_float3(1.f, 1.f, 1.f);
@@ -818,17 +710,13 @@ void mox_destroy(mox_ctx* c) {
   c->dTexObjs.release();
   c->buildArena.release();
   cudaFree(c->dNodes); cudaFree(c->dPacked); cudaFree(c->dNodes8); cudaFree(c->dPacked8); cudaFree(c->dAccu); cudaFree(c->dOwned);
-  for (int k = 0; k < mox_ctx::kMaxSlices; ++k) {
-    mox_ctx::Slice& sl = c->slices[k];
-    if (sl.stream && k) { cudaStreamSynchronize(sl.stream); cudaStreamDestroy(sl.stream); }
-    if (sl.shadowStream) { cudaStreamSynchronize(sl.shadowStream); cudaStreamDestroy(sl.shadowStream); }
-    if (sl.evShaded) cudaEventDestroy(sl.evShaded);
-    if (sl.evApplied) cudaEventDestroy(sl.evApplied);
-    freePaths(sl.pb);
-    sl.timer.release();
-    if (sl.evReady) cudaEventDestroy(sl.evReady);
-    if (sl.hostCnt) cudaFreeHost(sl.hostCnt);
-  }
+  if (c->shadowStream) { cudaStreamSynchronize(c->shadowStream); cudaStreamDestroy(c->shadowStream); }
+  if (c->evShaded) cudaEventDestroy(c->evShaded);
+  if (c->evApplied) cudaEventDestroy(c->evApplied);
+  freePaths(c->pb);
+  c->timer.release();
+  if (c->evReady) cudaEventDestroy(c->evReady);
+  if (c->hostCnt) cudaFreeHost(c->hostCnt);
   if (c->pinned) cudaFreeHost(c->pinned);
   freeGather(c);
   if (c->copyStream) cudaStreamDestroy(c->copyStream);
@@ -836,7 +724,6 @@ void mox_destroy(mox_ctx* c) {
   for (auto e : c->evCopied) if (e) cudaEventDestroy(e);
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
-  if (c->evFork) cudaEventDestroy(c->evFork);
   if (c->stream) cudaStreamDestroy(c->stream);
   delete c;
 }
@@ -1032,11 +919,9 @@ int mox_build_accel(mox_ctx* c, uint32_t flags, float* out_ms) {
   }
   if ((rc = syncLights(c))) return rc;
   if ((rc = syncTextures(c))) return rc;
-  c->hasDisneyNormal = false;
   for (auto& m : c->mats) {
     if (m.kind == MOX_MAT_DISNEY && (m.dis.albedoID < 0 || m.dis.albedoID > (int)c->textures.size()))
       return fail(c, MOX_ERR_INVALID, "DisneyParams.albedoID refers to a texture that was not added");
-    if (m.kind == MOX_MAT_DISNEY && m.dis.brdfType != GLASS) c->hasDisneyNormal = true;
   }
   BuildInput in;
   in.arena = &c->buildArena;
@@ -1068,7 +953,6 @@ int mox_build_accel(mox_ctx* c, uint32_t flags, float* out_ms) {
   float ms = 0;
   CUCK(c, cudaEventElapsedTime(&ms, c->ev0, c->ev1));
   c->dNodes = out.nodes; c->dPacked = out.packed; c->nNodes = out.nNodes; c->nValid = out.nValid;
-  for (int k = 0; k < 3; ++k) { c->sceneLo[k] = out.sceneLo[k]; c->sceneHi[k] = out.sceneHi[k]; }
   c->msBuild = ms;
   c->accelFlags = flags;
   c->built = true;

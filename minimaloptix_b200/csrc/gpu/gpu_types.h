@@ -60,8 +60,7 @@ static_assert(sizeof(BvhNode2) == 64, "BvhNode2");
 //        traversal ORs one compile-time constant per hit child and masks the result once:
 //        valid = imask << 24 | V,  V = the primitive bits that exist (16 bits);  group = V << 8 | imask (the low
 //        24 bits of the lane's node-group word).  The rank of primitive bit k among V's set bits is its offset
-//        from primBase.  (Round 1 and most of round 2 kept a position + count byte per child instead:
-//        MOX_NODE_META restores that layout, five more instructions per child in the node test.)
+//        from primBase.
 //   n2 = (qlo.x[0..3], qlo.x[4..7], qlo.y[0..3], qlo.y[4..7])      child boxes, 8 bit per plane:
 //   n3 = (qlo.z[0..3], qlo.z[4..7], qhi.x[0..3], qhi.x[4..7])      lo = p + qlo * scale (rounded down),
 //   n4 = (qhi.y[0..3], qhi.y[4..7], qhi.z[0..3], qhi.z[4..7])      hi = p + qhi * scale (rounded up)
@@ -72,19 +71,7 @@ static_assert(sizeof(BvhNode8) == 80, "BvhNode8");
 #ifndef MOX_WIDE_LEAF_MAX
 #define MOX_WIDE_LEAF_MAX 2  // measured: 2 -> 1037, 1 -> 1036, 3 -> 1013 Mrays/s (binary BVH: 1029)
 #endif
-// How the traversal turns a child's box test into hit bits (traverse_wide.cuh); form 3 accumulates the mask as a
-// float and wants the inner-child bits of the node's valid word at 16..23 instead of 24..31.
-#ifndef MOX_HIT_SIGN
-#define MOX_HIT_SIGN 1
-#endif
-#if MOX_HIT_SIGN == 3
-#define MOX_NODE_VALID_INNER_SHIFT 16
-#else
-#define MOX_NODE_VALID_INNER_SHIFT 24
-#endif
-#if !defined(MOX_NODE_META) && MOX_WIDE_LEAF_MAX > 2
-#error "the fixed-slot node layout has two primitive bits per slot: MOX_WIDE_LEAF_MAX > 2 needs MOX_NODE_META"
-#endif
+static_assert(MOX_WIDE_LEAF_MAX <= 2, "the fixed-slot node layout has two primitive bits per slot: a wide leaf holds at most two primitives");
 
 // Leaf-ordered packed primitive, 3 x float4 = 48 bytes per slot.
 //   triangle: (p0, idbits) (e0 = p1 - p0, -) (e1 = p0 - p2, -); with MOX_ACCEL_WATERTIGHT the raw vertices (p0) (p1) (p2)

@@ -76,14 +76,8 @@ template <bool F> MOX_D float powerHeuristic(float a, float b) { float t = a * a
 
 // disney.h:9-30; draws: lobe, then (u1,u2) | (phi, xi).
 template <class R>
-MOX_D void disneySample(R& rng, float metallic, float roughness, const float3& N, float3& L, const float3& V, float3& H);
-template <class R>
 MOX_D void disneySample(R& rng, const DisneyParams& mp, const float3& N, float3& L, const float3& V, float3& H) {
-  disneySample(rng, mp.metallic, mp.roughness, N, L, V, H);
-}
-template <class R>
-MOX_D void disneySample(R& rng, float metallic, float roughness, const float3& N, float3& L, const float3& V, float3& H) {
-  float diffuseRatio = 0.5f * (1.0f - metallic);
+  float diffuseRatio = 0.5f * (1.0f - mp.metallic);
   Onb3 onb(N);
   float r0 = rng.rnd();
   if (r0 < diffuseRatio) {
@@ -96,7 +90,7 @@ MOX_D void disneySample(R& rng, float metallic, float roughness, const float3& N
     L = normalize(onb.toWorld(p));
     H = normalize(L + V);
   } else {
-    float a = fmaxf(0.001f, roughness);
+    float a = fmaxf(0.001f, mp.roughness);
     float phi = rng.rnd() * 2.0f * MOX_PI_F;
     float xi = rng.rnd();
     float cosTheta = sqrtf((1.f - xi) / (1.0f + (a * a - 1.f) * xi));
@@ -116,21 +110,6 @@ template <bool F>
 struct DisneyHit {
   float3 N, X, Y, Cdlin, Cspec0, Csheen;
   float metallic, subsurface, roughness, sheen, clearcoat, ax, ay, clearcoatAlpha, specularAlpha, diffuseRatio, pdfRatio;
-
-  // Rebuilt from the 7-word record the light-sampling kernel stored for the BSDF-sampling kernel (wavefront.cu):
-  // the tangent frame is a function of N alone and is recomputed with the same operations.
-  MOX_D DisneyHit(const float4& r0, const float4& r1, const float4& r2, const float4& r3, float clearcoat_, const float4& r5, const float4& r6) {
-    N = mk3(r0); metallic = r0.w;
-    Cdlin = mk3(r1); subsurface = r1.w;
-    Cspec0 = mk3(r2); roughness = r2.w;
-    Csheen = mk3(r3); sheen = r3.w;
-    clearcoat = clearcoat_;
-    ax = r5.x; ay = r5.y; clearcoatAlpha = r5.z; specularAlpha = r5.w;
-    diffuseRatio = r6.x; pdfRatio = r6.y;
-    Onb3 onb(N);
-    X = bnormalize<F>(onb.tangent);
-    Y = bnormalize<F>(cross(N, X));
-  }
 
   MOX_D DisneyHit(const DisneyParams& mp, const float3& baseColor, const float3& n) {
     N = n;

@@ -107,13 +107,9 @@ struct RayPre { float3 o, d, idir; float tmin; };
 // addends moved by 2^-21 of the origin term): the hardware reciprocal (1 ulp) instead of the IEEE sequence and its
 // slow-path branch, three times per ray.  Primitive tests never see it.
 MOX_D float slabRcp(float x) {
-#ifdef MOX_IDIR_IEEE
-  return 1.0f / x;
-#else
   float r;
   asm("rcp.approx.f32 %0, %1;" : "=f"(r) : "f"(x));
   return r;
-#endif
 }
 MOX_D RayPre prepRay(const float3& o, const float3& d, float tmin) {
   RayPre r;
@@ -147,13 +143,8 @@ MOX_D float boxEntry(const RayPre& r, float lox, float hix, float loy, float hiy
 #define MOX_STACK MOX_TRAVERSAL_STACK
 // Ray / hit records are touched once per launch: stream them (evict-first) so they do not push
 // the BVH and the triangles out of L2.
-#ifdef MOX_NO_STREAM_HINTS
-#define MOX_LD_STREAM(p) __ldg(p)
-#define MOX_ST_STREAM(p, v) (*(p) = (v))
-#else
 #define MOX_LD_STREAM(p) __ldcs(p)
 #define MOX_ST_STREAM(p, v) __stcs((p), (v))
-#endif
 #define MOX_DONE ((int)0x80000000)   // sentinel "no more nodes" (same bit pattern as an empty child)
 #define MOX_FETCH_THRESHOLD 20       // refill a warp's idle lanes when fewer than this many are traversing
 

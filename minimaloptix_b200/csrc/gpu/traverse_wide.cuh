@@ -16,49 +16,22 @@
 
 #define MOX_WIDE_STACK MOX_TRAVERSAL_STACK
 
-// Four small savings of the node / primitive step, adopted together at the very end of round 2 (1 662 -> 1 720 Mrays/s in
-// one A/B call, all GPU tests green on that library); MOX_NODE_STEP_R2A restores the forms measured until then:
-//   MOX_ADDEND_DIRECTED   PRMT-plane addends by directed rounding instead of an extra error bound (planeTerms)
-//   MOX_BFIND             highest set bit by FLO directly
-//   MOX_SWAP_PREDICATED   the octant swaps predicated on the signs of 1/d the node step tests anyway
-//   MOX_ONE_FMA           the 1.0f pattern of the PRMT conversion from one FMA
-#ifndef MOX_NODE_STEP_R2A
-#define MOX_ADDEND_DIRECTED
-#define MOX_BFIND
-#define MOX_SWAP_PREDICATED
-#define MOX_ONE_FMA
-#endif
-
-
 // Quantised plane byte -> float, two ways, mixed per plane so that neither pipe is the bottleneck:
 //  * I2F.U8 on the conversion pipe (15.4 results/clk/SM measured, scripts/microbench/pipe_rates.cu, against 124
 //    FFMA): with all 48 conversions of a node step on it that pipe was ~70 % busy and 15-19 % of the stall samples
 //    were mio_throttle;
 //  * one PRMT on the ALU pipe: m = 1 + b * 2^-15 — byte b dropped into mantissa bits 8..15 of 1.0f — with the
 //    affine map folded back into the plane FMA:   b * ia + on  ==  m * (2^15 ia) + (on - 2^15 ia).
-//    The addend's rounding error (<= 2^-24 of 2^15 |ia|, i.e. 2^-9 of one quantisation step) is added to the
-//    conservative margin, so boxes only ever grow.
+//    The subtraction of 2^15 ia from the addend is rounded towards the outside of the box, so boxes only ever grow.
 // MOX_BYTE_MIX: bit 0..2 = near plane x, y, z, bit 3..5 = far plane x, y, z; a set bit converts that plane's eight
-// bytes with PRMT.  Measured (1 M-triangle bench, Mrays/s, with the select form of the hit mask): 0 (all I2F) 1 582,
-// 0x3f (all PRMT) 1 599, 0x3b 1 591, 0x38 (far planes) 1 617, 0x39 1 625, 0x30 1 633, 0x18 1 632, 0x10 1 616;
-// with MOX_HIT_SIGN=1: 0x3f 1 612, 0x10 1 627, 0x39 1 632, 0x30 1 645, 0x28 1 647, 0x33 1 648 (0x38 and 0x31 spill).
-// MOX_HIT_SIGN: how a child's box test becomes its hit bits.  0: FSETP + SEL of the child's constant, OR-ed three at
-// a time (all on the ALU pipe, which also runs the 32 FMNMX, the PRMTs and the near/far selects of a node step).
-// 1 (default): the far-side widening and the comparison are one FMA, tf * 1.00001 - tn, whose sign bit times the
-// child's constant is subtracted from an all-hit mask by one IMAD — FFMA + SHF + IMAD instead of FMUL + FSETP + SEL +
-// half an IADD3, and only the shift is on the ALU pipe.  2: the same with an arithmetic shift and one LOP3 (1 588).
-// 3: no ALU-pipe instruction at all — s = saturate(dd * -3e38) is 1.0 for a miss and 0.0 for a hit (FMUL.SAT,
-// flush-to-zero so that a denormal difference counts as a hit), and the mask is accumulated as a float, all 24 bits
-// minus s * constant per child (integers below 2^24: exact), and converted once per node.
-// (the default is set in gpu_types.h: the builder lays out the node's valid word to match)
+// bytes with PRMT (0x33 measured best, DESIGN.md section 4).
+// A child's hit bits come from the sign of one FMA: tf * 1.00001 - tn < 0 is a miss, and the sign bit times the
+// child's constant is subtracted from an all-hit mask by one IMAD (FFMA + SHF + IMAD; only the shift is on the ALU
+// pipe, which also runs the 32 FMNMX, the PRMTs and the near/far selects of a node step).
 #ifndef MOX_BYTE_MIX
-#ifdef MOX_BYTE_PRMT
-#define MOX_BYTE_MIX 0x3f
-#else
 #define MOX_BYTE_MIX 0x33
 #endif
-#endif
-// `one` is 1.0f's bit pattern held in a register (see traverseWidePersistent): with the constant as an immediate
+// `one` is 1.0f's bit pattern held in a register (see the node step of traverseWidePersistent): with the constant as an immediate
 // ptxas needs the byte selector in a register and re-materialises four selectors per node.
 template <bool PRMT>
 MOX_D float byteToFloat(uint32_t w, int i, uint32_t one) {
@@ -71,33 +44,23 @@ MOX_D float byteToFloat(uint32_t w, int i, uint32_t one) {
   return __uint_as_float(r);
 }
 // Scale and addends of one axis for the plane FMAs  t = float(byte) * scale + addend  (near: rounded down, far:
-// rounded up): every axis gets its own rounding bound, 2^-21 of the local origin term (+ 2^-22 of the PRMT
-// form's 2^15 ia), folded into the addends so a plane costs one conversion and one FMA.
+// rounded up): every axis gets its own rounding bound, 2^-21 of the local origin term, folded into the addends so a
+// plane costs one conversion and one FMA.
 template <bool NEAR_PRMT, bool FAR_PRMT>
 MOX_D void planeTerms(float ia, float oa, float& sn, float& an, float& sf, float& af) {
   const float k = ia * 32768.f;
   // (I2F form: |oa| * 2^-21 is exact, so one FMA rounds the same sum once)
   const float an0 = fmaf(-4.76837158203125e-07f, fabsf(oa), oa), af0 = fmaf(4.76837158203125e-07f, fabsf(oa), oa);
-#ifdef MOX_ADDEND_DIRECTED
   // PRMT form: the only new rounding is the subtraction of 2^15 ia from the addend — rounded towards the outside of the
-  // box (FADD.RM / FADD.RP) it needs no bound of its own: two instructions per plane instead of four
+  // box (FADD.RM / FADD.RP) it needs no bound of its own
   if (NEAR_PRMT) { sn = k; an = __fsub_rd(an0, k); } else { sn = ia; an = an0; }
   if (FAR_PRMT) { sf = k; af = __fsub_ru(af0, k); } else { sf = ia; af = af0; }
-#else
-  const float e = fmaf(2.384185791015625e-07f, fabsf(k), 4.76837158203125e-07f * fabsf(oa));
-  if (NEAR_PRMT) { sn = k; an = (oa - e) - k; } else { sn = ia; an = an0; }
-  if (FAR_PRMT) { sf = k; af = (oa + e) - k; } else { sf = ia; af = af0; }
-#endif
 }
-// index of the highest set bit (x != 0): FLO directly — written as 31 - __clz(x), ptxas keeps both subtractions
+// index of the highest set bit (x != 0): FLO directly (written as 31 - __clz(x), ptxas keeps both subtractions)
 MOX_D uint32_t highestBit(uint32_t x) {
-#ifdef MOX_BFIND
   uint32_t r;
   asm("bfind.u32 %0, %1;" : "=r"(r) : "r"(x));
   return r;
-#else
-  return 31u - (uint32_t)__clz(x);
-#endif
 }
 
 // (a & m) | (b & ~m) as one LOP3 (written as two ANDs and an OR, ptxas spends two)
@@ -117,21 +80,6 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
   const int lane = threadIdx.x & 31;
   const unsigned ltMask = (1u << lane) - 1u;
   const uint32_t jobCount = job.countPtr ? __ldg(job.countPtr) : job.count;
-#ifdef MOX_TOP_SMEM
-  // Measured option (VERDICT r1 item 5a): the first MOX_TOP_SMEM nodes — the array is in level order, 73 = root + two
-  // levels — staged once per CTA in shared memory and read from there instead of through L1.
-  __shared__ float4 sTop[MOX_TOP_SMEM * 5];
-  {
-    const float4* src = (const float4*)s.nodes8;
-    const uint32_t nTop = min((uint32_t)MOX_TOP_SMEM, s.nNodes8) * 5u;
-    for (uint32_t k = threadIdx.x; k < nTop; k += blockDim.x) sTop[k] = __ldg(src + k);
-    __syncthreads();
-  }
-#endif
-  // 0x3f800000 that ptxas cannot fold into an immediate (a launch never has 2^31 rays)
-#ifndef MOX_ONE_FMA
-  const uint32_t one = 0x3f800000u | (job.count >> 31);
-#endif
   // Per-lane state.  A lane is busy exactly while it has a primitive group or a node group pending (a ray with
   // neither pops its stack or finishes in the same iteration), so there is no separate "active" flag.  CLASSIFY keeps
   // the winner's shade class in bits 28..30 of bPrim (the form the hit record has anyway).  A shadow ray's
@@ -160,13 +108,7 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
   // instead of three (cursor, queue entry, ray); the whole warp sits in that wait, busy lanes included.  Measured:
   // shadow 90.6 -> 90.0 ms per step; the closest-hit kernel lost with it (69.3 -> 70.1 ms) and keeps one atomic
   // per refill.
-#ifdef MOX_REFILL_PER_EVENT
-  constexpr bool CHUNKED = false;
-#elif defined(MOX_REFILL_CHUNK_ALL)
-  constexpr bool CHUNKED = true;
-#else
   constexpr bool CHUNKED = ANYHIT;
-#endif
   uint32_t poolId = 0, poolPos = 0, poolCount = 0;   // poolPos / poolCount are warp-uniform
   bool moreChunks = true;
   while (true) {
@@ -206,11 +148,7 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
             RayPre r = prepRay(mk3(ro), mk3(rd), ro.w);
             o = r.o; d = r.d; idir = r.idir; tmin = r.tmin;
             if (WT) wr = wtPrep(d);
-#ifdef MOX_SWAP_PREDICATED
             octinv = 7u ^ ((idir.x < 0.f ? 4u : 0u) | (idir.y < 0.f ? 2u : 0u) | (idir.z < 0.f ? 1u : 0u));   // (-0.0 counts as negative here)
-#else
-            octinv = 7u ^ ((d.x < 0.f ? 4u : 0u) | (d.y < 0.f ? 2u : 0u) | (d.z < 0.f ? 1u : 0u));
-#endif
             tBest = rd.w; bPrim = -1;
             if (!CLASSIFY) { bBeta = 0.f; bGamma = 0.f; }
             tinted = false;
@@ -248,20 +186,12 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
 #ifndef MOX_VOTE_TRI_WEIGHT
 #define MOX_VOTE_TRI_WEIGHT 3  // a primitive step costs less than half a node step: vote by cost, not by head count (round 1: 1: 1115, 2: 1191, 3: 1206, 4: 1214, 6: 1207, 32: 1069 Mrays/s; with the cheaper node step of round 2 and two primitives per step: 2: 1693-1696, 3: 1691-1692, 4: 1671)
 #endif
-#ifndef MOX_VOTE_POPC
       // one ballot + one warp reduction (REDUX) of the weighted vote instead of two ballots + two POPCs — POPC shares the
-      // slow conversion pipe with the 48 I2F of a node step (ncu: 15-19 % of the stall samples are mio_throttle):
-      // extend 71.6 -> 71.0 ms, shadow 92.2 -> 91.7 ms per step (MOX_VOTE_POPC restores the counted form)
+      // slow conversion pipe with the 48 I2F of a node step (ncu: 15-19 % of the stall samples are mio_throttle)
       const unsigned bm = __ballot_sync(FULL, isNode | isTri);
       const int score = __reduce_add_sync(FULL, isNode ? 1 : (isTri ? -MOX_VOTE_TRI_WEIGHT : 0));
       if (bm == 0u || (!exhausted && __popc(bm) < job.fetchThreshold)) break;
       if (score >= 0) {
-#else
-      const unsigned nm = __ballot_sync(FULL, isNode), tm = __ballot_sync(FULL, isTri);
-      const int nNode = __popc(nm), nTri = __popc(tm);  // disjoint masks: busy lanes = nNode + nTri (POPC shares the slow conversion pipe)
-      if ((nm | tm) == 0u || (!exhausted && nNode + nTri < job.fetchThreshold)) break;
-      if (nNode >= MOX_VOTE_TRI_WEIGHT * nTri) {
-#endif
         if (isNode) {
           // ---- pop the front-most pending child of G
           const uint32_t bit = highestBit(gBits & 0xff000000u);
@@ -271,54 +201,27 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
           const uint32_t nodeIdx = gBase + __popc(imaskG & ((1u << slot) - 1u));
           if (gBits & 0xff000000u) stack[sp++] = make_uint2(gBase, gBits);
           // ---- fetch and test the node
-#ifdef MOX_TOP_SMEM
-          float4 n0, n1, n2, n3, n4;
-          if (nodeIdx < (uint32_t)MOX_TOP_SMEM) {
-            const float4* t = sTop + nodeIdx * 5u;
-            n0 = t[0]; n1 = t[1]; n2 = t[2]; n3 = t[3]; n4 = t[4];
-          } else {
-            const BvhNode8* nd = s.nodes8 + nodeIdx;
-            n0 = __ldg(&nd->n0); n1 = __ldg(&nd->n1); n2 = __ldg(&nd->n2); n3 = __ldg(&nd->n3); n4 = __ldg(&nd->n4);
-          }
-#else
           const BvhNode8* nd = s.nodes8 + nodeIdx;
           const float4 n0 = __ldg(&nd->n0), n1 = __ldg(&nd->n1), n2 = __ldg(&nd->n2), n3 = __ldg(&nd->n3), n4 = __ldg(&nd->n4);
-#endif
           if (COUNT) nv++;
           const uint32_t ew = __float_as_uint(n0.w);
           const float iax = __uint_as_float((ew & 0xffu) << 23) * idir.x;
           const float iay = __uint_as_float(((ew >> 8) & 0xffu) << 23) * idir.y;
           const float iaz = __uint_as_float(((ew >> 16) & 0xffu) << 23) * idir.z;
           const float oax = (n0.x - o.x) * idir.x, oay = (n0.y - o.y) * idir.y, oaz = (n0.z - o.z) * idir.z;
-#ifdef MOX_ONE_FMA
-          // ... or one FMA per node step (0 * finite + 1; neither nvcc nor ptxas may fold it) instead of a constant
-          // load and an ALU instruction to rebuild the value ptxas does not keep in a register across the loop
+          // 1.0f's bit pattern for byteToFloat from one FMA per node step (0 * finite + 1; neither nvcc nor ptxas may
+          // fold it) instead of a constant load and an ALU instruction to rebuild the value ptxas does not keep in a
+          // register across the loop
           const uint32_t one = __float_as_uint(fmaf(0.f, idir.x, 1.0f));
-#endif
           // conservative plane terms (planeTerms above); the far side is additionally widened by 1e-5 relative
           constexpr unsigned MIX = MOX_BYTE_MIX;
           float snx, onx, sfx, ofx, sny, ony, sfy, ofy, snz, onz, sfz, ofz;
           planeTerms<(MIX & 1u) != 0, (MIX & 8u) != 0>(iax, oax, snx, onx, sfx, ofx);
           planeTerms<(MIX & 2u) != 0, (MIX & 16u) != 0>(iay, oay, sny, ony, sfy, ofy);
           planeTerms<(MIX & 4u) != 0, (MIX & 32u) != 0>(iaz, oaz, snz, onz, sfz, ofz);
-#if !defined(MOX_NODE_META) && MOX_HIT_SIGN == 3
-          float hitf = 16777215.f;   // inner children in bits 16..23 until the mask is an integer again
-          uint32_t hitmask;
-#elif !defined(MOX_NODE_META) && MOX_HIT_SIGN
           uint32_t hitmask = 0xff00ffffu;
-#else
-          uint32_t hitmask = 0;
-#endif
 #pragma unroll
           for (int half = 0; half < 2; ++half) {
-#ifdef MOX_NODE_META
-            const uint32_t meta4 = __float_as_uint(half ? n1.w : n1.z);
-            // four children at once: inner children (position field 24..31 = 0b11xxx) get their slot
-            // XOR-ed with the ray's octant mask, which orders them front to back
-            const uint32_t inner4 = (meta4 & (meta4 << 1)) & 0x10101010u;
-            const uint32_t pos4 = (meta4 ^ ((inner4 >> 4) * octinv)) & 0x1f1f1f1fu;
-            const uint32_t cnt4 = (meta4 >> 5) & 0x07070707u;
-#endif
             const uint32_t qlx = __float_as_uint(half ? n2.y : n2.x), qly = __float_as_uint(half ? n2.w : n2.z);
             const uint32_t qlz = __float_as_uint(half ? n3.y : n3.x), qhx = __float_as_uint(half ? n3.w : n3.z);
             const uint32_t qhy = __float_as_uint(half ? n4.y : n4.x), qhz = __float_as_uint(half ? n4.w : n4.z);
@@ -331,67 +234,29 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
               const float tny = fmaf(byteToFloat<(MIX & 2u) != 0>(ny, i, one), sny, ony), tfy = fmaf(byteToFloat<(MIX & 16u) != 0>(fy, i, one), sfy, ofy);
               const float tnz = fmaf(byteToFloat<(MIX & 4u) != 0>(nz, i, one), snz, onz), tfz = fmaf(byteToFloat<(MIX & 32u) != 0>(fz, i, one), sfz, ofz);
               const float tn = fmaxf(fmaxf(tnx, tny), fmaxf(tnz, tmin));
-#if !defined(MOX_NODE_META) && MOX_HIT_SIGN
               // hit <=> tf * 1.00001 - tn >= 0, read off the sign bit of one FMA (the FMA pipe has room, the ALU pipe
               // that runs FSETP / SEL does not): every miss clears the child's constant from an all-hit mask
               const float dd = fmaf(fminf(fminf(tfx, tfy), fminf(tfz, tBest)), 1.00001f, -tn);
               const uint32_t K = (1u << (24 + 4 * half + i)) | (3u << (2 * (4 * half + i)));
-#if MOX_HIT_SIGN == 1
               asm("mad.lo.u32 %0, %1, %2, %0;" : "+r"(hitmask) : "r"(__float_as_uint(dd) >> 31), "r"(0u - K));
-#elif MOX_HIT_SIGN == 3
-              float miss;
-              asm("mul.ftz.sat.f32 %0, %1, %2;" : "=f"(miss) : "f"(dd), "f"(-3.0e38f));
-              hitf = fmaf(miss, -(float)((1u << (16 + 4 * half + i)) | (3u << (2 * (4 * half + i)))), hitf);
-#else
-              hitmask &= ~((uint32_t)(__float_as_int(dd) >> 31) & K);
-#endif
-#else
-              const float tf = fminf(fminf(tfx, tfy), fminf(tfz, tBest)) * 1.00001f;
-#endif
-#ifdef MOX_NODE_META
-              // branch-free: an empty slot has count bits 0 (and an inverted box)
-              const uint32_t bitsI = tn <= tf ? ((cnt4 >> (8 * i)) & 0xffu) : 0u;
-              hitmask |= bitsI << ((pos4 >> (8 * i)) & 0xffu);
-#elif !MOX_HIT_SIGN
-              // fixed positions per slot: one select of a compile-time constant per child (gpu_types.h)
-              hitmask |= tn <= tf ? ((1u << (24 + 4 * half + i)) | (3u << (2 * (4 * half + i)))) : 0u;
-#endif
             }
           }
           gBase = __float_as_uint(n1.x);
           tBase = __float_as_uint(n1.y);
-#ifdef MOX_NODE_META
-          gBits = (hitmask & 0xff000000u) | (ew >> 24);
-          tBits = hitmask & 0x00ffffffu;
-#else
           // keep what exists (inner children: imask, primitives: V), then bring the inner byte into front-to-back
           // order: bit 24 + s moves to 24 + (s ^ octinv) — three conditional swaps (nibbles, pairs, neighbours) written
           // as shifts by 0 or 4 / 2 / 1, so there is no branch and no select: (x << 0 & m) | (x >> 0 & ~m) = x
-#if MOX_HIT_SIGN == 3
-          hitmask = __float2uint_rz(hitf) & __float_as_uint(n1.z);   // n1.z = imask << 16 | V in this build
-          tBits = hitmask & 0x0000ffffu;
-          hitmask <<= 8;
-#else
           hitmask &= __float_as_uint(n1.z);
           tBits = hitmask & 0x0000ffffu;
-#endif
           {
             uint32_t x = hitmask;
-#ifdef MOX_SWAP_PREDICATED
             // the octant mask is made of the signs of 1/d (see the refill), the predicates the near/far selects of this
             // node step hold anyway: three predicated instructions per swap
             if (!(idir.x < 0.f)) x = bitSelect(x << 4, x >> 4, 0xf0000000u);
             if (!(idir.y < 0.f)) x = bitSelect(x << 2, x >> 2, 0xcc000000u);
             if (!(idir.z < 0.f)) x = bitSelect(x << 1, x >> 1, 0xaa000000u);
-#else
-            const uint32_t s4 = octinv & 4u, s2 = octinv & 2u, s1 = octinv & 1u;
-            x = bitSelect(x << s4, x >> s4, 0xf0000000u);
-            x = bitSelect(x << s2, x >> s2, 0xcc000000u);
-            x = bitSelect(x << s1, x >> s1, 0xaa000000u);
-#endif
             gBits = (x & 0xff000000u) | __float_as_uint(n1.w);   // n1.w = V << 8 | imask
           }
-#endif
         }
       } else {
 #ifndef MOX_PRIMS_PER_STEP
@@ -399,21 +264,15 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
 #endif
         // ---- up to MOX_PRIMS_PER_STEP primitives of the current group.  Leaf children hold up to two primitives and a
         // ray often hits the boxes of several, so a lane that is in the primitive phase usually has more than one bit
-        // pending: testing two per step halves the vote / loop overhead per primitive, and (MOX_PRIM_PREFETCH) both
-        // records are fetched before the first test, so the second fetch hides behind the first test.
+        // pending: testing two per step halves the vote / loop overhead per primitive.
         // Measured (Mrays/s): 1 per step 1 656, 2 per step 1 691 (vote weight 3) / 1 696 (weight 2).
         auto recordOf = [&](uint32_t k) -> const float4* {
-#ifdef MOX_NODE_META
-          return s.packed8 + (size_t)(tBase + k) * MOX_PACKED_F4;
-#else
           // offset from the node's first primitive = rank of bit k among the primitive bits that exist (V sits in
           // bits 8..23 of the node-group word for as long as primitives of that node are pending)
           return s.packed8 + (size_t)(tBase + __popc((gBits >> 8) & ~(0xffffffffu << k))) * MOX_PACKED_F4;
-#endif
         };
-        // one primitive test; returns true when a shadow ray was blocked (the lane has nothing pending any more)
-        auto testPrimitive = [&](const float4 r0, const float4 r1, const float4 r2) -> bool {
-          bool blockedNow = false;
+        // one primitive test
+        auto testPrimitive = [&](const float4 r0, const float4 r1, const float4 r2) {
           if (COUNT) np++;
           const uint32_t idbits = __float_as_uint(r0.w);
           const uint32_t type = (idbits >> 30) | __float_as_uint(r2.w) | (__float_as_uint(r1.w) >> 8);
@@ -443,7 +302,6 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
                 MOX_ST_STREAM(job.shC + rayId, make_float4(0.f, 0.f, 0.f, 0.f));
                 tinted = false;
                 tBits = 0u; gBits = 0u; sp = 0;
-                blockedNow = true;
                 if (COUNT) shadowEnd = 1u;
               } else if (cls == MOX_SHADOW_TINTS) {
                 const GpuMaterial* m = s.mats + (__ldg(&s.prims[id].typeMat) >> 2);
@@ -463,24 +321,7 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
               else { bPrim = id; bBeta = be; bGamma = ga; }
             }
           }
-          return blockedNow;
         };
-#if MOX_PRIMS_PER_STEP == 2 && defined(MOX_PRIM_PREFETCH)
-        if (isTri) {
-          const uint32_t k1 = highestBit(tBits);
-          const float4* recA = recordOf(k1);
-          tBits &= ~(1u << k1);
-          const bool two = tBits != 0u;
-          const uint32_t k2 = two ? highestBit(tBits) : k1;
-          const float4* recB = recordOf(k2);
-          tBits &= ~(1u << k2);
-          // All words are fetched before a type is known (see below)
-          const float4 a0 = __ldg(recA), a1 = __ldg(recA + 1), a2 = __ldg(recA + 2);
-          const float4 b0 = __ldg(recB), b1 = __ldg(recB + 1), b2 = __ldg(recB + 2);
-          const bool blockedA = testPrimitive(a0, a1, a2);
-          if (two && !blockedA) testPrimitive(b0, b1, b2);
-        }
-#else
 #pragma unroll
         for (int rep = 0; rep < MOX_PRIMS_PER_STEP; ++rep)
         if (rep == 0 ? isTri : tBits != 0u) {
@@ -493,7 +334,6 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
           const float4 r0 = __ldg(rec), r1 = __ldg(rec + 1), r2 = __ldg(rec + 2);
           testPrimitive(r0, r1, r2);
         }
-#endif
       }
       // ---- out of work in the current groups: resume a postponed node group, or finish the ray.  Only a lane that
       // was busy when this iteration started can have run dry in it.

@@ -273,16 +273,6 @@ __device__ __forceinline__ void spawnAt(const LaunchCtx& c, uint32_t path, const
   c.pb.thr[path] = make_float4(t.x, t.y, t.z, 0.f);
   c.pb.state[path] = childState;
   c.pb.qNext[pos] = path;
-  if (c.pb.qKey) {
-    // reordering key: direction octant | 21-bit Morton cell of the origin (7 bits/axis of the scene box)
-    uint32_t x = (uint32_t)fminf(fmaxf((o.x - c.sceneLo.x) * c.sceneInvExt.x, 0.f), 127.f);
-    uint32_t y = (uint32_t)fminf(fmaxf((o.y - c.sceneLo.y) * c.sceneInvExt.y, 0.f), 127.f);
-    uint32_t z = (uint32_t)fminf(fmaxf((o.z - c.sceneLo.z) * c.sceneInvExt.z, 0.f), 127.f);
-    auto spread = [](uint32_t v) { v = (v | (v << 16)) & 0x030000FFu; v = (v | (v << 8)) & 0x0300F00Fu; v = (v | (v << 4)) & 0x030C30C3u; v = (v | (v << 2)) & 0x09249249u; return v; };
-    uint32_t cell = (spread(x) << 2) | (spread(y) << 1) | spread(z);
-    uint32_t oct = (d.x < 0.f ? 4u : 0u) | (d.y < 0.f ? 2u : 0u) | (d.z < 0.f ? 1u : 0u);
-    c.pb.qKey[pos] = ((oct << 21) | cell) >> c.sortShift;   // octant on top: a one-pass sort keeps it
-  }
 }
 __device__ __forceinline__ void spawn(const LaunchCtx& c, uint32_t path, const float3& o, const float3& d, const float3& A,
                                       int childState) {
@@ -350,11 +340,6 @@ __device__ __forceinline__ uint32_t blockReserve(uint32_t n, uint32_t* counter, 
   uint32_t incl = n;
 #pragma unroll
   for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= (uint32_t)o) incl += t; }
-#ifdef MOX_RESERVE_PER_WARP   // alternative for A/B runs: one atomic per warp
-  uint32_t wb = 0;
-  if (lane == 31u && incl) wb = atomicAdd(counter, incl);
-  return __shfl_sync(0xffffffffu, wb, 31) + incl - n;
-#endif
   if (lane == 31u) sWarp[warp] = incl;
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -468,124 +453,6 @@ __global__ void __launch_bounds__(DISNEY_TPB, MOX_DISNEY_MINBLOCKS) k_shade_disn
   if (spawned) spawnAt(c, s.path, a.front, L, A, s.rng.forkState((int)depth + 1), nextPos);
   // no indirect ray: the path ends with what it has; its (stale) hit record must not be read as a terminal hit
   else if (live) c.pb.hit[s.path].y = __int_as_float(MOX_HIT_DEAD);
-}
-
-// The same program as two kernels.  k_shade_disney is 3 440 instructions at 80 registers (36 % occupancy, 12-15 % of
-// its stall samples instruction-cache misses): each half below holds ONE copy of disneyPdf / disneyEval.
-//   k_disney_nee     attributes, per-hit constants, the light loop (Material.cu:172-203), emission; leaves the
-//                    per-hit constants and the advanced RNG state for
-//   k_disney_sample  disneySample + indirect term (Material.cu:205-220) and the spawn.
-// RNG draws happen in the reference's order: all lights first, then the BSDF sample.
-#ifndef MOX_DISNEY_NEE_MINBLOCKS
-#define MOX_DISNEY_NEE_MINBLOCKS 6
-#endif
-template <int RM, bool F>
-__global__ void __launch_bounds__(DISNEY_TPB, MOX_DISNEY_NEE_MINBLOCKS) k_disney_nee(LaunchCtx c, uint32_t count, uint32_t depth) {
-  uint32_t i = blockIdx.x * DISNEY_TPB + threadIdx.x;
-  if (i >= count) return;
-  ShadeIn<RM> s = loadShadeIn<RM>(c, c.pb.qMat[Q_DISNEY][i], depth);
-  Attr a = hitAttributes(c.scene, s.pd, s.o, s.d, s.t, true);
-  const DisneyParams dp = s.m->dis;
-  float3 N = faceforward3(a.Ns, -s.d, a.Ng);
-  float3 V = -s.d;
-  float3 baseColor = disneyBaseColor(c.scene, dp, a.u, a.v);
-  DisneyHit<F> dh(dp, baseColor, N);
-  dh.setView(V);
-  {  // what the BSDF-sampling kernel needs, word-major so that neighbouring hits store neighbouring words
-    float4* rec = c.pb.disneyRec + i;
-    const size_t cap = c.pb.capacity;
-    rec[0] = make_float4(N.x, N.y, N.z, dh.metallic);
-    rec[cap] = make_float4(dh.Cdlin.x, dh.Cdlin.y, dh.Cdlin.z, dh.subsurface);
-    rec[2 * cap] = make_float4(dh.Cspec0.x, dh.Cspec0.y, dh.Cspec0.z, dh.roughness);
-    rec[3 * cap] = make_float4(dh.Csheen.x, dh.Csheen.y, dh.Csheen.z, dh.sheen);
-    rec[4 * cap] = make_float4(a.front.x, a.front.y, a.front.z, dh.clearcoat);
-    rec[5 * cap] = make_float4(dh.ax, dh.ay, dh.clearcoatAlpha, dh.specularAlpha);
-    rec[6 * cap] = make_float4(dh.diffuseRatio, dh.pdfRatio, 0.f, 0.f);
-  }
-  float3 Tprev = mk3(c.pb.thr[s.path]);
-  float3 L, H;
-  const int nL = c.scene.nLights;
-  uint32_t shadowCount = 0;
-  for (int li = 0; li < nL; ++li) {
-    const LightParams* lp = c.scene.lights + li;
-    float3 lpos = mk3(__ldg(&lp->position.x), __ldg(&lp->position.y), __ldg(&lp->position.z));
-    float3 pointOnLight, normalOnLight;
-    if (__ldg((const int*)&lp->shape) == SPHERE) {
-      pointOnLight = lpos + randInUnitSphere(s.rng) * __ldg(&lp->radius);
-      normalOnLight = normalize(pointOnLight - lpos);
-    } else {
-      float r1 = s.rng.rnd();
-      float r2 = s.rng.rnd();
-      pointOnLight = lpos + f3(lp->u) * r1 + f3(lp->v) * r2;
-      normalOnLight = mk3(__ldg(c.scene.lightN + li));
-    }
-    L = pointOnLight - a.front;
-    float lightDst = length(L);
-    L = normalize(L);
-    size_t slot = (size_t)li * count + i;  // light-major: neighbouring lanes aim at the same light
-    float3 contrib = mk3(0.f);
-    if (dot(L, N) > 0.f && dot(L, normalOnLight) < 0.f) {
-      shadowCount++;
-      H = bnormalize<F>(L + V);
-      float lightPdf = bdiv<F>(bdiv<F>(lightDst * lightDst, __ldg(&lp->area)), dot(normalOnLight, -L));
-      float dr;
-      float objPdf = dh.pdf(L, H, dr);
-      if (lightPdf > 0 && objPdf > 0) {
-        float3 brdf = dh.eval(L, H, dr);
-        contrib = powerHeuristic<F>(lightPdf, objPdf) * brdf * f3(lp->emission) * bdiv<F>(1.0f, fmaxf(0.001f, lightPdf));
-      }
-    }
-    float3 pc = Tprev * contrib;
-    bool trace = pc.x != 0.f || pc.y != 0.f || pc.z != 0.f;
-    c.pb.shC[slot] = make_float4(pc.x, pc.y, pc.z, 0.f);
-    if (trace) {
-      c.pb.shD[slot] = make_float4(L.x, L.y, L.z, lightDst - c.rp.eps);
-      uint32_t pos = queuePush(c.bc + C_SHQ);
-      c.pb.shQueue[pos] = (uint32_t)slot;
-    }
-  }
-  if (nL) c.pb.shO[i] = make_float4(a.front.x, a.front.y, a.front.z, c.rp.eps);
-  if (shadowCount) atomicAdd(c.pb.counters + C_SHADOW, shadowCount);
-  {  // + emission
-    float3 e = f3(dp.emission);
-    if (e.x != 0.f || e.y != 0.f || e.z != 0.f) {
-      float3 r = mk3(c.pb.rad[s.path]) + Tprev * e;
-      c.pb.rad[s.path] = make_float4(r.x, r.y, r.z, 0.f);
-    }
-  }
-  c.pb.state[s.path] = s.rng.state;   // the sample kernel continues the stream where the light loop left it
-}
-
-#ifndef MOX_DISNEY_SAMPLE_MINBLOCKS
-#define MOX_DISNEY_SAMPLE_MINBLOCKS 8
-#endif
-template <int RM, bool F>
-__global__ void __launch_bounds__(DISNEY_TPB, MOX_DISNEY_SAMPLE_MINBLOCKS) k_disney_sample(LaunchCtx c, uint32_t count, uint32_t depth) {
-  uint32_t i = blockIdx.x * DISNEY_TPB + threadIdx.x;
-  if (i >= count) return;
-  const uint32_t path = c.pb.qMat[Q_DISNEY][i];
-  const float4* rec = c.pb.disneyRec + i;
-  const size_t cap = c.pb.capacity;
-  const float4 r0 = rec[0], r1 = rec[cap], r2 = rec[2 * cap], r3 = rec[3 * cap], r4 = rec[4 * cap], r5 = rec[5 * cap], r6 = rec[6 * cap];
-  DisneyHit<F> dh(r0, r1, r2, r3, r4.w, r5, r6);
-  const float3 N = dh.N, V = -mk3(c.pb.rayD[path]);
-  dh.setView(V);
-  RngT<RM> rng;
-  if (RM == 0) rng = makeRng<RM>(c.pb.state[path], 0u, 0u, depth);
-  else { PathCtx pc = pathCtx(c, path); rng = makeRng<RM>(c.pb.state[path], pc.pixel, (uint32_t)pc.launchSeed, depth); }
-  float3 L, H;
-  disneySample(rng, dh.metallic, dh.roughness, N, L, V, H);
-  bool spawned = false;
-  if (dot(N, L) > 0.0f && dot(N, V) > 0.0f) {
-    float dr;
-    float pdf = dh.pdf(L, H, dr);
-    if (pdf > 0) {
-      float3 brdf = dh.eval(L, H, dr);
-      spawn(c, path, mk3(r4), L, brdf * bdiv<F>(1.0f, pdf), rng.forkState((int)depth + 1));
-      spawned = true;
-    }
-  }
-  if (!spawned) c.pb.hit[path].y = __int_as_float(MOX_HIT_DEAD);
 }
 
 __global__ void __launch_bounds__(TPB) k_apply(LaunchCtx c, uint32_t count) {
@@ -817,14 +684,13 @@ void launchShade(const LaunchCtx& c, int kind, uint32_t count, uint32_t depth) {
       break;
     case Q_DISNEY: {
       const unsigned g = (count + DISNEY_TPB - 1) / DISNEY_TPB;
-#define MOX_LAUNCH_DISNEY(RM, F)                                                                              \
-  do {                                                                                                        \
-    if (c.disneySplit) { k_disney_nee<RM, F><<<g, DISNEY_TPB, 0, c.stream>>>(c, count, depth); k_disney_sample<RM, F><<<g, DISNEY_TPB, 0, c.stream>>>(c, count, depth); } \
-    else k_shade_disney<RM, F><<<g, DISNEY_TPB, 0, c.stream>>>(c, count, depth);                               \
-  } while (0)
-      if (ref) { if (c.brdfFast) MOX_LAUNCH_DISNEY(0, true); else MOX_LAUNCH_DISNEY(0, false); }
-      else { if (c.brdfFast) MOX_LAUNCH_DISNEY(1, true); else MOX_LAUNCH_DISNEY(1, false); }
-#undef MOX_LAUNCH_DISNEY
+      if (ref) {
+        if (c.brdfFast) k_shade_disney<0, true><<<g, DISNEY_TPB, 0, c.stream>>>(c, count, depth);
+        else k_shade_disney<0, false><<<g, DISNEY_TPB, 0, c.stream>>>(c, count, depth);
+      } else {
+        if (c.brdfFast) k_shade_disney<1, true><<<g, DISNEY_TPB, 0, c.stream>>>(c, count, depth);
+        else k_shade_disney<1, false><<<g, DISNEY_TPB, 0, c.stream>>>(c, count, depth);
+      }
       break;
     }
   }

@@ -28,35 +28,26 @@ struct PathBuffers {
   float2* hit = nullptr;    // (t, primitive id | shade class << 28 | MOX_HIT_MISS | MOX_HIT_DEAD)
   int* state = nullptr;
   uint32_t *qCur = nullptr, *qNext = nullptr;
-  uint32_t* qBuf[3] = {nullptr, nullptr, nullptr};   // queue storage; qCur / qNext point into it
-  uint32_t* kBuf[2] = {nullptr, nullptr};            // sort keys of qNext (ray reordering) + scratch
-  uint32_t* qKey = nullptr;                          // keys written next to qNext (null: reordering off)
-  uint32_t* sortScratch = nullptr;
+  uint32_t* qBuf[2] = {nullptr, nullptr};   // queue storage; qCur / qNext point into it
   uint32_t* qMat[Q_COUNT] = {nullptr, nullptr, nullptr, nullptr};
   uint32_t* qDisneyAlt = nullptr;   // second Disney queue: bounce b's k_apply may still read its queue while bounce b+1 is classified
   float4 *shO = nullptr, *shD = nullptr, *shC = nullptr;  // shadow rays: origin per Disney path, (dir, tmax) and contribution per slot
   uint32_t* shQueue = nullptr;                            // slots that need a shadow ray
-  float4* disneyRec = nullptr;                            // MOX_DISNEY_REC_F4 words per Disney hit, word-major (word * capacity + hit)
   uint32_t* counters = nullptr;   // C_WORDS per-batch words (0..7 unused) followed by BOUNCE_RING blocks of C_BOUNCE_WORDS
   int32_t* seeds = nullptr;       // launch seed per sample of the batch
   size_t seedCap = 0;
 };
-
-#define MOX_DISNEY_REC_F4 7
 
 struct LaunchCtx {
   SceneView scene;
   RenderParams rp;
   PathBuffers pb;
   uint32_t* bc;              // this bounce's counter block (C_NEXT, C_MAT0.., C_SHQ)
-  const uint32_t* ownedPix;  // device: the pixels this slice renders
+  const uint32_t* ownedPix;  // device: the pixels this context renders
   uint32_t nOwned;
   float* accu;               // device W*H*3
   bool countTraversal;
-  bool disneySplit;          // Disney NORMAL as two kernels (light sampling, then BSDF sampling) instead of one
   bool brdfFast;             // hardware reciprocal / square-root approximations inside BRDF values (shading.cuh::bdiv)
-  float3 sceneLo, sceneInvExt;  // ray-reordering key: 7-bit cell of the origin inside the scene box
-  uint32_t sortShift = 0;       // the key's low bits dropped: 0 = 24-bit key (3 sort passes), 16 = octant + 5 cell bits (1 pass)
   cudaStream_t stream;
 };
 

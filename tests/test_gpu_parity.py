@@ -499,43 +499,28 @@ def test_nonfinite_samples_become_bad_color(host, orc, gpu_backend):
     assert np.allclose(imgs[1][1, 1], 4 * 0.1)                                # corner: background only
 
 
-def test_sorted_ray_queue_is_bit_identical(host, api_tables, gpu_backend, monkeypatch):
-    """MOX_SORT_RAYS=1 reorders the extend queue (3-pass radix sort by origin cell + direction octant inside the
-    bounce loop): every per-path result is order-independent, so image and ray counts are bit-identical."""
-    sc = host.Scene.builtin("interior", 30000)
-    out = []
-    for sort in ("0", "1"):
-        monkeypatch.setenv("MOX_SORT_RAYS", sort)    # read by mox_create
-        g = gpu_backend.context(0)
-        sc.upload(api_tables.gpu, g, 200, 120, 5)
-        g.build_accel()
-        g.render(3, 31)
-        st = g.stats()
-        out.append((g.read_accum(), st["rays_bounce"], st["rays_shadow"], st["kernel_launches"]))
-    assert out[0][1:3] == out[1][1:3]
-    assert np.array_equal(out[0][0].view(np.uint32), out[1][0].view(np.uint32))
-    assert out[1][3] > out[0][3]    # the sort kernels did run
-
-
 def test_scheduling_variants_are_bit_identical(host, api_tables, gpu_backend, monkeypatch):
-    """How a batch is scheduled must not show in the result: 1 / 2 / 3 sub-batch slices on their own streams,
-    shadow rays on a second stream or in line, the Disney program as one kernel or as light-sampling + BSDF-sampling
-    kernels — same image bit for bit, same ray counts (all read by mox_create)."""
+    """How a render is scheduled must not show in the result: shadow rays on a second stream or in line, and all
+    samples in one batch or one sample per batch (MOX_MAX_BATCH_PATHS = the pixel count: three batches, whose
+    samples k_accumulate adds in launch order) — same image bit for bit, same ray counts (all read by mox_create)."""
     sc = host.Scene.builtin("interior", 30000)
     out = []
-    for slices, overlap, split in (("1", "1", "0"), ("1", "0", "0"), ("2", "1", "0"), ("3", "0", "0"), ("1", "1", "1"), ("2", "0", "1")):
-        monkeypatch.setenv("MOX_SLICES", slices)
+    for overlap, batch_paths in (("1", None), ("0", None), ("1", str(400 * 300))):
         monkeypatch.setenv("MOX_OVERLAP_SHADOW", overlap)
-        monkeypatch.setenv("MOX_DISNEY_SPLIT", split)
+        if batch_paths is None:
+            monkeypatch.delenv("MOX_MAX_BATCH_PATHS", raising=False)
+        else:
+            monkeypatch.setenv("MOX_MAX_BATCH_PATHS", batch_paths)
         g = gpu_backend.context(0)
         sc.upload(api_tables.gpu, g, 400, 300, 5)
         g.build_accel()
         g.render(3, 77)
         st = g.stats()
-        out.append((g.read_accum(), st["rays_bounce"], st["rays_shadow"]))
+        out.append((g.read_accum(), st["rays_bounce"], st["rays_shadow"], st["extend_launches"]))
     for o in out[1:]:
-        assert o[1:] == out[0][1:]
+        assert o[1:3] == out[0][1:3]
         assert np.array_equal(o[0].view(np.uint32), out[0][0].view(np.uint32))
+    assert out[2][3] > out[0][3]    # three batches: the bounce loop ran once per batch
 
 
 def test_wide_and_binary_traversal_render_identically(host, api_tables, gpu_backend):

@@ -7,7 +7,7 @@ step relies on, so that a change of the layout fails here first, on the CPU:
   * subtracting a missed child's constant from the all-hit mask (the IMAD form) equals OR-ing the hit children's
     constants (the select form), and masking with the node's valid word leaves exactly the children that exist;
   * the byte -> float conversion by PRMT (m = 1 + b * 2^-15) folded into the plane FMA is the affine map it replaces,
-    within the rounding bound the kernel adds to its conservative margin."""
+    with the addends rounded away from the box."""
 import itertools
 import struct
 
@@ -96,12 +96,6 @@ def test_imad_form_equals_select_form_and_valid_mask():
         for s in range(8):
             assert (got >> (24 + s) & 1) == int(bool(hit[s]) and kinds[s] == 1)
             assert (got >> (2 * s) & 3) == ((1 << (int(kinds[s]) - 1)) - 1 if hit[s] and kinds[s] >= 2 else 0)
-        # float accumulator of MOX_HIT_SIGN=3: the same sum with the inner bits at 16..23 stays below 2^24 (exact in fp32)
-        acc = np.float32(16777215.0)
-        for s in range(8):
-            if not hit[s]:
-                acc = np.float32(acc - np.float32((1 << (16 + s)) | (3 << (2 * s))))
-        assert int(acc) == ((selected >> 24) << 16) | (selected & 0xFFFF)
 
 
 def f32(x):
@@ -109,6 +103,7 @@ def f32(x):
 
 
 def test_prmt_byte_conversion_is_the_affine_map_within_the_stated_bound():
+    # stated bound: the I2F addends' 2^-21 of the origin term, then the subtraction of 2^15 ia rounded away from the box
     rng = np.random.default_rng(3)
     one = 0x3F800000
     for _ in range(4000):
@@ -119,9 +114,9 @@ def test_prmt_byte_conversion_is_the_affine_map_within_the_stated_bound():
         oa = f32(float(rng.normal()) * 2.0 ** int(rng.integers(-6, 12)))   # (node origin - ray origin) * 1/d
         k = f32(ia * 32768.0)
         exact = b * ia + oa
-        e = f32(2.0 ** -22 * abs(k) + 2.0 ** -21 * abs(oa))
-        near = f32(m * k + f32(f32(oa - e) - k))            # one FMA on the GPU: compare with its exact value
-        far = f32(m * k + f32(f32(oa + e) - k))
+        an0, af0 = f32(oa - 2.0 ** -21 * abs(oa)), f32(oa + 2.0 ** -21 * abs(oa))   # one FMA each (the product is exact)
+        near = f32(m * k + float(_round_directed(np.float64(an0) - k, up=False)))   # one FMA on the GPU: compare with its exact value
+        far = f32(m * k + float(_round_directed(np.float64(af0) - k, up=True)))
         slack = 2.0 ** -23 * (abs(near) + abs(far)) + 1e-30  # the FMA's own rounding, covered by the 1e-5 far-side widening
         assert near <= exact + slack and far >= exact - slack
 
@@ -161,9 +156,8 @@ def _round_directed(x64, up):
     return np.where(r.astype(np.float64) > x64, np.nextafter(r, np.float32(-np.inf)), r).astype(np.float32)
 
 
-@pytest.mark.parametrize("directed", [False, True], ids=["bounded", "directed"])
-@pytest.mark.parametrize("mix", [0x00, 0x33, 0x38, 0x3F])
-def test_quantised_box_test_is_conservative(mix, directed):
+@pytest.mark.parametrize("mix", [0x00, 0x10, 0x18, 0x30, 0x33, 0x38, 0x39, 0x3F])
+def test_quantised_box_test_is_conservative(mix):
     rng = np.random.default_rng(1000 + mix)
     n = 200000
     f = np.float32
@@ -217,20 +211,17 @@ def test_quantised_box_test_is_conservative(mix, directed):
     oa = ((blo - o).astype(f) * idir).astype(f)
     neg = idir < 0
     nb, fb = np.where(neg, qh, ql), np.where(neg, ql, qh)
-    c21, c22 = f(4.76837158203125e-07), f(2.384185791015625e-07)
+    c21 = f(4.76837158203125e-07)
     k = (ia * f(32768.0)).astype(f)
-    err = _fma(np.full_like(k, c22), np.abs(k), (c21 * np.abs(oa)).astype(f))
     tn_ax, tf_ax = np.empty_like(oa), np.empty_like(oa)
     for ax in range(3):
         for far in (False, True):
             byte = (fb if far else nb)[:, ax].astype(f)
             if mix >> (ax + (3 if far else 0)) & 1:                          # PRMT form
                 m = (f(1.0) + byte * f(2.0 ** -15)).astype(f)
-                if directed:   # MOX_ADDEND_DIRECTED: the I2F addend minus 2^15 ia, rounded away from the box
-                    add0 = _fma(np.full(n, c21 if far else -c21, f), np.abs(oa[:, ax]), oa[:, ax])
-                    add = _round_directed(add0.astype(np.float64) - k[:, ax].astype(np.float64), up=far)
-                else:
-                    add = (((oa[:, ax] + err[:, ax]) if far else (oa[:, ax] - err[:, ax])).astype(f) - k[:, ax]).astype(f)
+                # the I2F addend minus 2^15 ia, rounded away from the box
+                add0 = _fma(np.full(n, c21 if far else -c21, f), np.abs(oa[:, ax]), oa[:, ax])
+                add = _round_directed(add0.astype(np.float64) - k[:, ax].astype(np.float64), up=far)
                 t = _fma(m, k[:, ax], add)
             else:                                                            # I2F form
                 add = _fma(np.full(n, c21 if far else -c21, f), np.abs(oa[:, ax]), oa[:, ax])
@@ -238,7 +229,7 @@ def test_quantised_box_test_is_conservative(mix, directed):
             (tf_ax if far else tn_ax)[:, ax] = t
     tn = np.maximum(tn_ax.max(axis=1), tmin)
     tf = np.minimum(tf_ax.min(axis=1), tbest)
-    diff = _fma(tf, np.full(n, f(1.00001)), -tn)                             # MOX_HIT_SIGN: the sign bit decides
+    diff = _fma(tf, np.full(n, f(1.00001)), -tn)                             # the sign bit decides
     hit_kernel = ~np.signbit(diff)
     assert hit_true.sum() > n // 10                                          # the sample does exercise hits
     missed = hit_true & ~hit_kernel
