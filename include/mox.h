@@ -68,6 +68,15 @@ typedef enum mox_rng_mode { MOX_RNG_REF = 0, MOX_RNG_PHILOX = 1 } mox_rng_mode;
                                     an edge or a vertex.  t / beta / gamma then differ from the reference's in the last bits and
                                     the winner can differ on epsilon ties; the oracle has the same switch (also: env
                                     MOX_WATERTIGHT=1 at mox_build_accel, mox_cli --watertight) */
+#define MOX_ACCEL_REFIT 16u      /* refit the structure of the last full build in place: same topology, boxes and packed
+                                    records from the current vertex, normal and sphere data (what OptiX's Trbvh builder
+                                    does for an acceleration marked dirty with the "refit" property).  Needs a successful
+                                    full build with no mox_add_* / mox_clear_scene after it (else MOX_ERR_STATE), the other
+                                    flag bits equal to that build's, env switches applied (else MOX_ERR_INVALID), and every
+                                    primitive still valid or still invalid (zero-area / infinite primitives are not in the
+                                    BVH; else MOX_ERR_STATE and the context is not built: build again without this flag).
+                                    Unchanged geometry gives node and primitive arrays byte-identical to the full build's.
+                                    Tree quality falls as the geometry moves away from the built pose: rebuild now and then */
 
 typedef struct mox_stats {
   uint64_t rays_primary;      /* camera rays traced (closest hit)                 */
@@ -159,6 +168,14 @@ int mox_add_mesh(mox_ctx*, const float* vertices, size_t n_vertices, const float
  * next launch. */
 int mox_update_sphere(mox_ctx*, uint32_t prim_id, const SphereParams*);
 
+/* vertexBuffer / normalBuffer->map(), write, unmap() and acceleration->markDirty() for one OBJ shape
+ * (MinimalOptiX.cpp:398-411,441): new vertices (and, when normals is not NULL, normals) for the mesh whose face 0 is
+ * first_prim_id (the id mox_add_mesh returned).  n_vertices must equal the count the mesh was added with; normals
+ * need a mesh added with normals and their count.  Faces, indices and texcoords do not change.  The acceleration
+ * structure must be rebuilt or refitted (mox_build_accel, MOX_ACCEL_REFIT) before the next launch or trace. */
+int mox_update_mesh(mox_ctx*, uint32_t first_prim_id, const float* vertices, size_t n_vertices, const float* normals,
+                    size_t n_normals);
+
 /* context["lights"] buffer used by the Disney NEE loop (MinimalOptiX.cpp:523-531,
  * Material.cu:116,172). */
 int mox_set_lights(mox_ctx*, const LightParams*, size_t n);
@@ -168,7 +185,8 @@ int mox_clear_scene(mox_ctx*);
 
 /* The moment OptiX builds Trbvh (context->validate() + first launch,
  * MinimalOptiX.cpp:378,494,534,542): uploads the scene and builds the BVH on
- * the GPU.  *out_build_ms (may be NULL): device time of the build kernels. */
+ * the GPU.  *out_build_ms (may be NULL): device time of the build kernels (with
+ * MOX_ACCEL_REFIT: of the refit kernels). */
 int mox_build_accel(mox_ctx*, uint32_t flags, float* out_build_ms);
 
 /* ---- render -------------------------------------------------------------- */

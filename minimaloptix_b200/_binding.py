@@ -43,6 +43,7 @@ SIGNATURES = {
     "clear_accum": (C.c_int, [_vp]),
     "set_accum": (C.c_int, [_vp, _vp, _u64]),
     "update_sphere": (C.c_int, [_vp, _u32, C.POINTER(S.SphereParams)]),
+    "update_mesh": (C.c_int, [_vp, _u32, _vp, C.c_size_t, _vp, C.c_size_t]),
     "owned_pixels": (C.c_int, [_vp, _u32, C.POINTER(_u64)]),
     "pack_owned": (C.c_int, [_vp, _vp]),
     "unpack_owned": (C.c_int, [_vp, _u32, _vp]),
@@ -62,7 +63,10 @@ GPU_ONLY = {"create_multi": (C.c_int, [C.POINTER(_vp), C.POINTER(C.c_int), C.c_i
             "read_gathered_begin": (C.c_int, [_vp, C.c_int]),
             "read_gathered_end": (C.c_int, [_vp, C.c_int, C.POINTER(_fp)]),
             "trace_closest_device": (C.c_int, [_vp, _vp, C.c_size_t, _vp, C.POINTER(_f32)]),
-            "debug_radix_sort": (C.c_int, [_vp, _vp, _vp, C.c_size_t])}
+            "debug_radix_sort": (C.c_int, [_vp, _vp, _vp, C.c_size_t]),
+            "debug_read_accel": (C.c_int, [_vp, C.c_int, _vp, C.c_size_t, C.POINTER(C.c_size_t)])}
+# Arrays of a built acceleration structure, in the order of include/mox_debug.h's MOX_DEBUG_ACCEL_*.
+ACCEL_ARRAYS = ("nodes", "nodes8", "packed", "packed8")
 
 
 class MoxError(RuntimeError):
@@ -263,6 +267,12 @@ class Context:
     def update_sphere(self, prim_id, sphere):
         self._ck(self.b.update_sphere(self.h, prim_id, C.byref(sphere)), "update_sphere")
 
+    def update_mesh(self, first_prim_id, vertices, normals=None):
+        """New vertices (and normals) of the mesh whose first primitive id add_mesh returned; build or refit next."""
+        v = _f32c(vertices).reshape(-1, 3)
+        n = None if normals is None else _f32c(normals).reshape(-1, 3)
+        self._ck(self.b.update_mesh(self.h, first_prim_id, _ptr(v), len(v), _ptr(n), 0 if n is None else len(n)), "update_mesh")
+
     def clear_accum(self):
         self._ck(self.b.clear_accum(self.h), "clear_accum")
 
@@ -299,6 +309,15 @@ class Context:
         v = np.ascontiguousarray(vals, dtype=np.uint32).copy()
         self._ck(self.b.debug_radix_sort(self.h, _ptr(k), _ptr(v), len(k)), "debug_radix_sort")
         return k, v
+
+    def debug_read_accel(self, which):
+        """Bytes of one array of the built acceleration structure (a name of ACCEL_ARRAYS) as uint8."""
+        k = ACCEL_ARRAYS.index(which)
+        size = C.c_size_t()
+        self._ck(self.b.debug_read_accel(self.h, k, None, 0, C.byref(size)), "debug_read_accel")
+        out = np.empty(size.value, dtype=np.uint8)
+        self._ck(self.b.debug_read_accel(self.h, k, _ptr(out), len(out), C.byref(size)), "debug_read_accel")
+        return out
 
     def trace_shadow(self, rays):
         r = _f32c(rays).reshape(-1, 8)

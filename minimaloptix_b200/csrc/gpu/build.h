@@ -66,6 +66,27 @@ bool plocAlloc(PlocScratch& s, int n, DeviceArena& arena, std::string& err);
 bool plocBuild(PlocScratch& s, int n, const uint32_t* sortedIds, const float4* primLo, const float4* primHi, int radius,
                BvhNode2* outNodes, float rootLo[3], float rootHi[3], int* maxDepthOut, cudaStream_t stream, std::string& err);
 
+// What an in-place refit (refitBvh) needs from the last full build.  Every pointer is a slice of the build's
+// DeviceArena.  Nothing takes from the arena between two full builds, so the slices stay valid until the next
+// buildBvh, which overwrites them.  A refit keeps the topology (Morton order, tree, leaf orders, wide-node slots) and
+// recomputes the boxes only.
+struct RefitState {
+  enum Path { NONE = 0, TRIVIAL, PLOC, KARRAS };
+  Path path = NONE;          // TRIVIAL: at most one valid primitive, no hierarchy to refit (the caller rebuilds)
+  bool wide = false;         // the compressed 8-wide BVH was built from the PLOC tree
+  int nPrims = 0, nValid = 0, nNodes8 = 0;
+  float4 *primLo = nullptr, *primHi = nullptr;  // per primitive id, validity in primLo .w (1 / 0)
+  uint32_t* sortedIds = nullptr;                // primitive ids in Morton order, the valid ones first
+  uint32_t* flag = nullptr;                     // device word, set by the refit when a primitive's validity changed
+  PlocScratch ploc;                             // PLOC: children, parent, size, leafPos, firstPos, orderedIds, node boxes
+  int2 *children = nullptr, *range = nullptr;   // Karras radix tree ...
+  int *parentInternal = nullptr, *parentLeaf = nullptr;
+  float4 *nodeLo = nullptr, *nodeHi = nullptr;
+  uint32_t* arrivals = nullptr;                 // nValid - 1 counters (both binary refits)
+  uint32_t* orderedIds8 = nullptr;              // wide: primitives in wide-leaf order
+  uint32_t* wideSrc = nullptr;                  // wide: per node its binary node and the binary node of each slot (~0u: empty)
+};
+
 struct BuildOutput {
   // device, owned by the caller.  On entry they may hold buffers of nodesCap / packedCap records from a
   // previous build, which are reused when large enough.
@@ -83,12 +104,26 @@ struct BuildOutput {
   int maxDepth = 0;   // deepest leaf (PLOC); the traversal stack holds MOX_STACK entries
   float sceneLo[3] = {0, 0, 0}, sceneHi[3] = {0, 0, 0};
   float4 *scratchLo = nullptr, *scratchHi = nullptr;  // builder-internal
+  RefitState refit;   // what the build left for refitBvh
 };
 
 bool buildBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::string& err);
+// Refit of the structure out.refit describes (path PLOC or KARRAS), in place, from the current primitive data of
+// `in`: new primitive boxes, binary nodes, wide nodes and packed records, with the last build's topology.  Unchanged
+// geometry gives byte-identical nodes and records.  in.evStart / in.evStop are recorded around the kernels.
+// *validityChanged: a primitive became valid or invalid since the build; the result is then unusable.
+bool refitBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::string& err, bool* validityChanged);
 bool radixSortPairs(uint32_t* keys, uint32_t* vals, int n, cudaStream_t stream, std::string& err);
 
-// Collapse of the PLOC tree into the compressed wide BVH (bvh_wide.cu).
+// Refit of a PLOC tree built by plocBuild over n leaves: new leaf and inner boxes in s.nodeLo / s.nodeHi, then the
+// binary nodes again.  arrivals: n - 1 words of scratch.
+bool plocRefit(const PlocScratch& s, int n, const uint32_t* sortedIds, const float4* primLo, const float4* primHi, uint32_t* arrivals,
+               BvhNode2* outNodes, cudaStream_t stream, std::string& err);
+
+// Collapse of the PLOC tree into the compressed wide BVH (bvh_wide.cu).  *wideSrcOut: 9 words per wide node (its
+// binary node, then the binary node in each slot or ~0u), what wideRefit needs.
 size_t wideScratchBytes(int n);
 bool wideCollapse(const PlocScratch& s, int n, uint32_t root, DeviceArena& arena, BvhNode8* outNodes, uint32_t** orderedIds8Out,
-                  int* nNodesOut, int* levelsOut, cudaStream_t stream, std::string& err);
+                  uint32_t** wideSrcOut, int* nNodesOut, int* levelsOut, cudaStream_t stream, std::string& err);
+// New boxes for the nNodes wide nodes from the refitted binary boxes; slots, masks and bases stay.
+void wideRefit(const uint32_t* wideSrc, int nNodes, const float4* nodeLo, const float4* nodeHi, BvhNode8* nodes, cudaStream_t stream);

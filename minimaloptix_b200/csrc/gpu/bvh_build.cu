@@ -32,6 +32,44 @@ __host__ __device__ __forceinline__ float fromOrderedBits(uint32_t u) {
 #endif
 }
 
+// Box of primitive i and whether it takes part in the BVH (zero-area / infinite primitives do not; their box is
+// empty).  The build and the refit both store what this returns, so their boxes have the same bits.
+__device__ __forceinline__ bool primBounds(int i, const PrimDesc* __restrict__ prims, const TriIdx* __restrict__ tris,
+                                           const float* __restrict__ verts, const Analytic* __restrict__ analytic, float3& lo,
+                                           float3& hi) {
+  bool valid;
+  PrimDesc pd = prims[i];
+  uint32_t type = pd.typeMat & 3u;
+  if (type == PT_TRI) {
+    TriIdx t = tris[pd.geom];
+    float3 v0 = mk3(verts[3 * t.v[0]], verts[3 * t.v[0] + 1], verts[3 * t.v[0] + 2]);
+    float3 v1 = mk3(verts[3 * t.v[1]], verts[3 * t.v[1] + 1], verts[3 * t.v[1] + 2]);
+    float3 v2 = mk3(verts[3 * t.v[2]], verts[3 * t.v[2] + 1], verts[3 * t.v[2] + 2]);
+    float area = length(cross(v1 - v0, v2 - v0));
+    valid = area > 0.0f && !isinf(area);
+    lo = fmin3(fmin3(v0, v1), v2);
+    hi = fmax3(fmax3(v0, v1), v2);
+  } else if (type == PT_SPHERE) {
+    float4 cr = analytic[pd.geom].a;
+    lo = mk3(cr) + (-cr.w);
+    hi = mk3(cr) + cr.w;
+    valid = cr.w == cr.w && !isinf(cr.w);
+    if (cr.w < 0) { float3 t = lo; lo = hi; hi = t; }
+  } else {
+    Analytic q = analytic[pd.geom];
+    float3 v1 = mk3(q.b), v2 = mk3(q.c), a = mk3(q.d);
+    float3 tv1 = v1 / dot(v1, v1);
+    float3 tv2 = v2 / dot(v2, v2);
+    float3 p01 = a + tv1, p10 = a + tv2, p11 = a + tv1 + tv2;
+    float area = length(cross(tv1, tv2));
+    valid = area > 0.0f && !isinf(area);
+    lo = fmin3(fmin3(a, p01), fmin3(p10, p11));
+    hi = fmax3(fmax3(a, p01), fmax3(p10, p11));
+  }
+  if (!valid) { lo = mk3(kInf); hi = mk3(-kInf); }
+  return valid;
+}
+
 __global__ void k_prim_bounds(int n, const PrimDesc* __restrict__ prims, const TriIdx* __restrict__ tris,
                               const float* __restrict__ verts, const Analytic* __restrict__ analytic,
                               float4* __restrict__ boxLo, float4* __restrict__ boxHi, uint32_t* __restrict__ cbounds,
@@ -40,35 +78,7 @@ __global__ void k_prim_bounds(int n, const PrimDesc* __restrict__ prims, const T
   float3 lo = mk3(kInf), hi = mk3(-kInf);
   bool valid = false;
   if (i < n) {
-    PrimDesc pd = prims[i];
-    uint32_t type = pd.typeMat & 3u;
-    if (type == PT_TRI) {
-      TriIdx t = tris[pd.geom];
-      float3 v0 = mk3(verts[3 * t.v[0]], verts[3 * t.v[0] + 1], verts[3 * t.v[0] + 2]);
-      float3 v1 = mk3(verts[3 * t.v[1]], verts[3 * t.v[1] + 1], verts[3 * t.v[1] + 2]);
-      float3 v2 = mk3(verts[3 * t.v[2]], verts[3 * t.v[2] + 1], verts[3 * t.v[2] + 2]);
-      float area = length(cross(v1 - v0, v2 - v0));
-      valid = area > 0.0f && !isinf(area);
-      lo = fmin3(fmin3(v0, v1), v2);
-      hi = fmax3(fmax3(v0, v1), v2);
-    } else if (type == PT_SPHERE) {
-      float4 cr = analytic[pd.geom].a;
-      lo = mk3(cr) + (-cr.w);
-      hi = mk3(cr) + cr.w;
-      valid = cr.w == cr.w && !isinf(cr.w);
-      if (cr.w < 0) { float3 t = lo; lo = hi; hi = t; }
-    } else {
-      Analytic q = analytic[pd.geom];
-      float3 v1 = mk3(q.b), v2 = mk3(q.c), a = mk3(q.d);
-      float3 tv1 = v1 / dot(v1, v1);
-      float3 tv2 = v2 / dot(v2, v2);
-      float3 p01 = a + tv1, p10 = a + tv2, p11 = a + tv1 + tv2;
-      float area = length(cross(tv1, tv2));
-      valid = area > 0.0f && !isinf(area);
-      lo = fmin3(fmin3(a, p01), fmin3(p10, p11));
-      hi = fmax3(fmax3(a, p01), fmax3(p10, p11));
-    }
-    if (!valid) { lo = mk3(kInf); hi = mk3(-kInf); }
+    valid = primBounds(i, prims, tris, verts, analytic, lo, hi);
     boxLo[i] = make_float4(lo.x, lo.y, lo.z, valid ? 1.f : 0.f);
     boxHi[i] = make_float4(hi.x, hi.y, hi.z, 0.f);
   }
@@ -91,6 +101,20 @@ __global__ void k_prim_bounds(int n, const PrimDesc* __restrict__ prims, const T
     }
     if (inval) atomicAdd(invalidCount, inval);
   }
+}
+
+// Refit: the boxes of the current primitive data over the stored ones.  The topology of the last build holds only
+// while every primitive keeps its validity; a change raises *changed.
+__global__ void k_refit_bounds(int n, const PrimDesc* __restrict__ prims, const TriIdx* __restrict__ tris,
+                               const float* __restrict__ verts, const Analytic* __restrict__ analytic,
+                               float4* __restrict__ boxLo, float4* __restrict__ boxHi, uint32_t* __restrict__ changed) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  float3 lo, hi;
+  const bool valid = primBounds(i, prims, tris, verts, analytic, lo, hi);
+  if (valid != (boxLo[i].w != 0.f)) *changed = 1u;
+  boxLo[i] = make_float4(lo.x, lo.y, lo.z, valid ? 1.f : 0.f);
+  boxHi[i] = make_float4(hi.x, hi.y, hi.z, 0.f);
 }
 
 __device__ __forceinline__ uint32_t expandBits10(uint32_t v) {
@@ -433,6 +457,7 @@ bool buildBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::
     CK(cudaMemcpyAsync(out.nodes, &root, sizeof root, cudaMemcpyHostToDevice, stream));
     CK(cudaStreamSynchronize(stream));
     out.nNodes = 1;
+    out.refit.path = RefitState::TRIVIAL;
     if (in.evStart) CK(cudaEventRecord(in.evStart, stream));
     if (in.evStop) CK(cudaEventRecord(in.evStop, stream));
     return true;
@@ -514,6 +539,12 @@ bool buildBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::
   const int nValid = n - (int)hostSmall[6];
   out.nValid = nValid;
   out.nInvalid = (int)hostSmall[6];
+  RefitState& rs = out.refit;
+  rs.nPrims = n; rs.nValid = nValid;
+  rs.primLo = boxLo; rs.primHi = boxHi; rs.sortedIds = vin; rs.flag = small + 12;
+  rs.ploc = ploc;
+  rs.children = children; rs.range = range; rs.parentInternal = parentInternal; rs.parentLeaf = parentLeaf;
+  rs.nodeLo = nodeLo; rs.nodeHi = nodeHi; rs.arrivals = arrivals;
 
   if (nValid > 0 && (nValid <= 1 || !in.usePloc))
     k_pack<<<divUp(nValid, B), B, 0, stream>>>(nValid, vin, in.prims, in.tris, in.verts, in.analytic, in.mats, out.packed, in.watertight);
@@ -538,6 +569,7 @@ bool buildBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::
     if (in.evStop) CKB(cudaEventRecord(in.evStop, stream));
     CKB(cudaStreamSynchronize(stream));
     freeScratch();
+    rs.path = RefitState::TRIVIAL;
     return true;
   }
 
@@ -551,14 +583,17 @@ bool buildBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::
     if (wantWide) {
       uint32_t* ordered8 = nullptr;
       const uint32_t rootId = (uint32_t)(nValid + nValid - 2);  // the last node PLOC created
-      if (!wideCollapse(ploc, nValid, rootId, arena, out.nodes8, &ordered8, &out.nNodes8, &out.wideLevels, stream, perr)) return bail(perr);
+      if (!wideCollapse(ploc, nValid, rootId, arena, out.nodes8, &ordered8, &rs.wideSrc, &out.nNodes8, &out.wideLevels, stream, perr))
+        return bail(perr);
       k_pack<<<divUp(nValid, B), B, 0, stream>>>(nValid, ordered8, in.prims, in.tris, in.verts, in.analytic, in.mats, out.packed8, in.watertight);
+      rs.wide = true; rs.orderedIds8 = ordered8; rs.nNodes8 = out.nNodes8;
     }
     if (in.evStop) CKB(cudaEventRecord(in.evStop, stream));
     CKB(cudaStreamSynchronize(stream));
     CKB(cudaGetLastError());
     out.usedPloc = true;
     freeScratch();
+    rs.path = RefitState::PLOC;
     return true;
     }
     // too deep for the traversal stack: fall through to the radix tree (depth <= 62)
@@ -577,8 +612,41 @@ bool buildBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::
   out.sceneLo[0] = rlo.x; out.sceneLo[1] = rlo.y; out.sceneLo[2] = rlo.z;
   out.sceneHi[0] = rhi.x; out.sceneHi[1] = rhi.y; out.sceneHi[2] = rhi.z;
   freeScratch();
+  rs.path = RefitState::KARRAS;
   return true;
 #undef CKB
+}
+
+bool refitBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::string& err, bool* validityChanged) {
+  const RefitState& rs = out.refit;
+  if (rs.path != RefitState::PLOC && rs.path != RefitState::KARRAS) { err = "no hierarchy to refit"; return false; }
+  if (rs.nPrims != in.nPrims) { err = "primitive count differs from the build's"; return false; }
+  const int n = rs.nPrims, nValid = rs.nValid, nInner = nValid - 1;
+  const int B = 256;
+  uint32_t* host = (uint32_t*)in.arena->pinned;
+  if (in.evStart) CK(cudaEventRecord(in.evStart, stream));
+  CK(cudaMemsetAsync(rs.flag, 0, 4, stream));
+  k_refit_bounds<<<divUp(n, B), B, 0, stream>>>(n, in.prims, in.tris, in.verts, in.analytic, rs.primLo, rs.primHi, rs.flag);
+  if (rs.path == RefitState::PLOC) {
+    if (!plocRefit(rs.ploc, nValid, rs.sortedIds, rs.primLo, rs.primHi, rs.arrivals, out.nodes, stream, err)) return false;
+    k_pack<<<divUp(nValid, B), B, 0, stream>>>(nValid, rs.ploc.orderedIds, in.prims, in.tris, in.verts, in.analytic, in.mats, out.packed, in.watertight);
+    if (rs.wide) {
+      wideRefit(rs.wideSrc, rs.nNodes8, rs.ploc.nodeLo, rs.ploc.nodeHi, out.nodes8, stream);
+      k_pack<<<divUp(nValid, B), B, 0, stream>>>(nValid, rs.orderedIds8, in.prims, in.tris, in.verts, in.analytic, in.mats, out.packed8, in.watertight);
+    }
+  } else {
+    CK(cudaMemsetAsync(rs.arrivals, 0, (size_t)nInner * 4, stream));
+    k_refit<<<divUp(nValid, B), B, 0, stream>>>(nValid, rs.sortedIds, rs.primLo, rs.primHi, rs.children, rs.parentInternal, rs.parentLeaf,
+                                                 rs.nodeLo, rs.nodeHi, rs.arrivals);
+    k_emit2<<<divUp(nInner, B), B, 0, stream>>>(nValid, rs.sortedIds, rs.primLo, rs.primHi, rs.children, rs.range, rs.nodeLo, rs.nodeHi, out.nodes);
+    k_pack<<<divUp(nValid, B), B, 0, stream>>>(nValid, rs.sortedIds, in.prims, in.tris, in.verts, in.analytic, in.mats, out.packed, in.watertight);
+  }
+  if (in.evStop) CK(cudaEventRecord(in.evStop, stream));
+  CK(cudaMemcpyAsync(host, rs.flag, 4, cudaMemcpyDeviceToHost, stream));
+  CK(cudaStreamSynchronize(stream));
+  CK(cudaGetLastError());
+  *validityChanged = host[0] != 0u;
+  return true;
 }
 
 // Stand-alone sort entry used by the tests (keys/vals are device pointers, sorted in place).

@@ -36,6 +36,43 @@ __device__ __forceinline__ uint32_t gridExponent(float extent) {
   return (uint32_t)e;
 }
 
+// Grid of a wide node whose box is [blo, bhi]: biased exponents and the scales 2^(e-127) per axis.
+struct WideGrid { uint32_t ex, ey, ez; float sx, sy, sz; };
+__device__ __forceinline__ WideGrid wideGrid(const float4& blo, const float4& bhi) {
+  WideGrid g;
+  g.ex = gridExponent(bhi.x - blo.x); g.ey = gridExponent(bhi.y - blo.y); g.ez = gridExponent(bhi.z - blo.z);
+  g.sx = __uint_as_float(g.ex << 23); g.sy = __uint_as_float(g.ey << 23); g.sz = __uint_as_float(g.ez << 23);
+  return g;
+}
+
+// 8-bit planes of the child box [lo, hi] in slot s of a node with origin blo: outward rounding, then verified against
+// the float planes the traversal will reconstruct.  The collapse and the refit both quantise here.
+__device__ __forceinline__ void quantiseChild(const float4& lo, const float4& hi, const float4& blo, const WideGrid& g, int s,
+                                              uint32_t* qlx, uint32_t* qly, uint32_t* qlz, uint32_t* qhx, uint32_t* qhy, uint32_t* qhz) {
+  int ql, qh;
+  ql = (int)floorf((lo.x - blo.x) / g.sx); ql = max(0, min(255, ql)); while (ql > 0 && blo.x + ql * g.sx > lo.x) --ql;
+  qh = (int)ceilf((hi.x - blo.x) / g.sx); qh = max(0, min(255, qh)); while (qh < 255 && blo.x + qh * g.sx < hi.x) ++qh;
+  qlx[s] = ql; qhx[s] = qh;
+  ql = (int)floorf((lo.y - blo.y) / g.sy); ql = max(0, min(255, ql)); while (ql > 0 && blo.y + ql * g.sy > lo.y) --ql;
+  qh = (int)ceilf((hi.y - blo.y) / g.sy); qh = max(0, min(255, qh)); while (qh < 255 && blo.y + qh * g.sy < hi.y) ++qh;
+  qly[s] = ql; qhy[s] = qh;
+  ql = (int)floorf((lo.z - blo.z) / g.sz); ql = max(0, min(255, ql)); while (ql > 0 && blo.z + ql * g.sz > lo.z) --ql;
+  qh = (int)ceilf((hi.z - blo.z) / g.sz); qh = max(0, min(255, qh)); while (qh < 255 && blo.z + qh * g.sz < hi.z) ++qh;
+  qlz[s] = ql; qhz[s] = qh;
+}
+
+__device__ __forceinline__ uint32_t pack4(const uint32_t* v) { return v[0] | (v[1] << 8) | (v[2] << 16) | (v[3] << 24); }
+
+// n0 .xyz / .w and the planes n2 .. n4 of a node (n1 is the caller's)
+__device__ __forceinline__ void wideBoxWords(BvhNode8& nd, const float4& blo, const WideGrid& g, uint32_t imask, const uint32_t* qlx,
+                                             const uint32_t* qly, const uint32_t* qlz, const uint32_t* qhx, const uint32_t* qhy,
+                                             const uint32_t* qhz) {
+  nd.n0 = make_float4(blo.x, blo.y, blo.z, __uint_as_float(g.ex | (g.ey << 8) | (g.ez << 16) | (imask << 24)));
+  nd.n2 = make_float4(__uint_as_float(pack4(qlx)), __uint_as_float(pack4(qlx + 4)), __uint_as_float(pack4(qly)), __uint_as_float(pack4(qly + 4)));
+  nd.n3 = make_float4(__uint_as_float(pack4(qlz)), __uint_as_float(pack4(qlz + 4)), __uint_as_float(pack4(qhx)), __uint_as_float(pack4(qhx + 4)));
+  nd.n4 = make_float4(__uint_as_float(pack4(qhy)), __uint_as_float(pack4(qhy + 4)), __uint_as_float(pack4(qhz)), __uint_as_float(pack4(qhz + 4)));
+}
+
 // ---- optimal collapse (Ylitie et al. 2017, section 3.1) -----------------------------------------------------
 // C(n, i): cheapest way to represent the subtree of binary node n as a forest of at most i wide-BVH children,
 //   C(n, 1) = min(C_leaf(n), C_distribute(n, 8) + A_n c_node),   C_leaf(n) = A_n P_n c_prim if P_n <= leaf max
@@ -115,7 +152,7 @@ k_collapse_level(int nItems, const WorkItem* __restrict__ items, int nLeaves, co
                  const uint32_t* __restrict__ orderedIds, BvhNode8* __restrict__ out, uint32_t* __restrict__ orderedIds8,
                  WorkItem* __restrict__ nextItems, uint32_t* __restrict__ counters /* [0] nodes, [1] prims */,
                  const uint32_t* __restrict__ levelCount /* items of this level; [1]: of the next, filled here */,
-                 const uint32_t* __restrict__ decision /* null: greedy collapse */) {
+                 const uint32_t* __restrict__ decision /* null: greedy collapse */, uint32_t* __restrict__ wideSrc) {
   int w = blockIdx.x * blockDim.x + threadIdx.x;
   if (w >= nItems || w >= (int)__ldg(levelCount)) return;   // nItems: the host's upper bound (grid size)
   const WorkItem it = items[w];
@@ -180,8 +217,7 @@ k_collapse_level(int nItems, const WorkItem* __restrict__ items, int nLeaves, co
   }
   // ---- node box and grid
   const float4 blo = nodeLo[it.binNode], bhi = nodeHi[it.binNode];
-  const uint32_t ex = gridExponent(bhi.x - blo.x), ey = gridExponent(bhi.y - blo.y), ez = gridExponent(bhi.z - blo.z);
-  const float sx = __uint_as_float(ex << 23), sy = __uint_as_float(ey << 23), sz = __uint_as_float(ez << 23);
+  const WideGrid g = wideGrid(blo, bhi);
   const float cx = 0.5f * (blo.x + bhi.x), cy = 0.5f * (blo.y + bhi.y), cz = 0.5f * (blo.z + bhi.z);
   // ---- slots by centroid octant, nearest free slot (Hamming distance) when taken
   int slotOf[8];
@@ -215,25 +251,18 @@ k_collapse_level(int nItems, const WorkItem* __restrict__ items, int nLeaves, co
   uint32_t qlx[8], qly[8], qlz[8], qhx[8], qhy[8], qhz[8];
   uint32_t innerRank = 0, primOff = 0;
   uint32_t validPrims = 0;   // bits 2s, 2s + 1 = the primitives of the leaf child in slot s
+  uint32_t* srcOut = wideSrc + 9 * (size_t)it.wideIndex;   // for the refit: this node's binary node and each slot's
+  srcOut[0] = it.binNode;
   for (int s = 0; s < 8; ++s) {
     int i = childAt[s];
     if (i < 0) {  // empty slot: inverted box, never hit
       qlx[s] = qly[s] = qlz[s] = 255; qhx[s] = qhy[s] = qhz[s] = 0;
+      srcOut[1 + s] = ~0u;
       continue;
     }
     const uint32_t c = ch[i];
-    const float4 lo = nodeLo[c], hi = nodeHi[c];
-    // outward rounding, then verify against the float planes the traversal will reconstruct
-    int ql, qh;
-    ql = (int)floorf((lo.x - blo.x) / sx); ql = max(0, min(255, ql)); while (ql > 0 && blo.x + ql * sx > lo.x) --ql;
-    qh = (int)ceilf((hi.x - blo.x) / sx); qh = max(0, min(255, qh)); while (qh < 255 && blo.x + qh * sx < hi.x) ++qh;
-    qlx[s] = ql; qhx[s] = qh;
-    ql = (int)floorf((lo.y - blo.y) / sy); ql = max(0, min(255, ql)); while (ql > 0 && blo.y + ql * sy > lo.y) --ql;
-    qh = (int)ceilf((hi.y - blo.y) / sy); qh = max(0, min(255, qh)); while (qh < 255 && blo.y + qh * sy < hi.y) ++qh;
-    qly[s] = ql; qhy[s] = qh;
-    ql = (int)floorf((lo.z - blo.z) / sz); ql = max(0, min(255, ql)); while (ql > 0 && blo.z + ql * sz > lo.z) --ql;
-    qh = (int)ceilf((hi.z - blo.z) / sz); qh = max(0, min(255, qh)); while (qh < 255 && blo.z + qh * sz < hi.z) ++qh;
-    qlz[s] = ql; qhz[s] = qh;
+    srcOut[1 + s] = c;
+    quantiseChild(nodeLo[c], nodeHi[c], blo, g, s, qlx, qly, qlz, qhx, qhy, qhz);
     if (imask & (1u << s)) {
       nextItems[nextBase + innerRank] = WorkItem{c, childBase + innerRank};
       innerRank++;
@@ -248,15 +277,33 @@ k_collapse_level(int nItems, const WorkItem* __restrict__ items, int nLeaves, co
       primOff += cnt;
     }
   }
-  auto pack4 = [](const uint32_t* v) { return v[0] | (v[1] << 8) | (v[2] << 16) | (v[3] << 24); };
   BvhNode8 nd;
-  nd.n0 = make_float4(blo.x, blo.y, blo.z, __uint_as_float(ex | (ey << 8) | (ez << 16) | (imask << 24)));
+  wideBoxWords(nd, blo, g, imask, qlx, qly, qlz, qhx, qhy, qhz);
   nd.n1 = make_float4(__uint_as_float(childBase), __uint_as_float(primBase), __uint_as_float((imask << 24) | validPrims),
                       __uint_as_float((validPrims << 8) | imask));
-  nd.n2 = make_float4(__uint_as_float(pack4(qlx)), __uint_as_float(pack4(qlx + 4)), __uint_as_float(pack4(qly)), __uint_as_float(pack4(qly + 4)));
-  nd.n3 = make_float4(__uint_as_float(pack4(qlz)), __uint_as_float(pack4(qlz + 4)), __uint_as_float(pack4(qhx)), __uint_as_float(pack4(qhx + 4)));
-  nd.n4 = make_float4(__uint_as_float(pack4(qhy)), __uint_as_float(pack4(qhy + 4)), __uint_as_float(pack4(qhz)), __uint_as_float(pack4(qhz + 4)));
   out[it.wideIndex] = nd;
+}
+
+// Refit of the wide nodes after the binary boxes were refitted: one thread per node, no level order needed.  The box
+// comes from the node's binary node, the slot planes from the binary node in each slot; n1 (bases, valid bits) and the
+// inner mask stay.
+__global__ void __launch_bounds__(128)
+k_wide_refit(int nNodes, const uint32_t* __restrict__ wideSrc, const float4* __restrict__ nodeLo, const float4* __restrict__ nodeHi,
+             BvhNode8* __restrict__ nodes) {
+  int w = blockIdx.x * blockDim.x + threadIdx.x;
+  if (w >= nNodes) return;
+  const uint32_t* src = wideSrc + 9 * (size_t)w;
+  const float4 blo = nodeLo[src[0]], bhi = nodeHi[src[0]];
+  const WideGrid g = wideGrid(blo, bhi);
+  uint32_t qlx[8], qly[8], qlz[8], qhx[8], qhy[8], qhz[8];
+  for (int s = 0; s < 8; ++s) {
+    const uint32_t c = src[1 + s];
+    if (c == ~0u) { qlx[s] = qly[s] = qlz[s] = 255; qhx[s] = qhy[s] = qhz[s] = 0; continue; }
+    quantiseChild(nodeLo[c], nodeHi[c], blo, g, s, qlx, qly, qlz, qhx, qhy, qhz);
+  }
+  BvhNode8 nd = nodes[w];
+  wideBoxWords(nd, blo, g, __float_as_uint(nd.n0.w) >> 24, qlx, qly, qlz, qhx, qhy, qhz);
+  nodes[w] = nd;
 }
 
 inline int divUp(size_t a, size_t b) { return (int)((a + b - 1) / b); }
@@ -268,17 +315,19 @@ inline int divUp(size_t a, size_t b) { return (int)((a + b - 1) / b); }
 size_t wideScratchBytes(int n) {
   // two work queues of at most n/2 items (8 B each), 4 counters, 258 level counts, the wide-leaf order; slack for alignment
   // + the collapse programme: 2 float4 of costs, one decision word and one arrival counter per inner binary node
-  return (size_t)std::max(n, 2) * (8 + 8 + 4 + 32 + 4 + 4) + 9 * 256 + 1024 + 2048;   // + the per-level item counts
+  // + the refit's slot map: 36 bytes per wide node (at most n)
+  return (size_t)std::max(n, 2) * (8 + 8 + 4 + 32 + 4 + 4 + 36) + 10 * 256 + 1024 + 2048;   // + the per-level item counts
 }
 
 // Collapse the PLOC tree held in `s` (n >= 2 leaves) into outNodes (capacity >= n wide nodes) and
 // fill orderedIds8 (n entries).  *nNodesOut receives the number of wide nodes.
 bool wideCollapse(const PlocScratch& s, int n, uint32_t root, DeviceArena& arena, BvhNode8* outNodes, uint32_t** orderedIds8Out,
-                  int* nNodesOut, int* levelsOut, cudaStream_t stream, std::string& err) {
+                  uint32_t** wideSrcOut, int* nNodesOut, int* levelsOut, cudaStream_t stream, std::string& err) {
   WorkItem* q[2] = {arena.take<WorkItem>((size_t)n), arena.take<WorkItem>((size_t)n)};
   uint32_t* counters = arena.take<uint32_t>(4);
   uint32_t* orderedIds8 = arena.take<uint32_t>((size_t)n);
-  if (!orderedIds8 || !q[0] || !q[1] || !counters) { err = "wide-BVH scratch does not fit the build arena"; return false; }
+  uint32_t* wideSrc = arena.take<uint32_t>(9 * (size_t)n);
+  if (!orderedIds8 || !q[0] || !q[1] || !counters || !wideSrc) { err = "wide-BVH scratch does not fit the build arena"; return false; }
   // optimal collapse up to 4 M primitives (above, the greedy collapse keeps the build inside its time budget)
   const uint32_t* decision = nullptr;
   const char* env = getenv("MOX_WIDE_GREEDY");
@@ -312,7 +361,8 @@ bool wideCollapse(const PlocScratch& s, int n, uint32_t root, DeviceArena& arena
     if (levels + kLevelBatch >= kMaxLevels) { err = "wide collapse did not terminate"; return false; }
     for (int b = 0; b < kLevelBatch; ++b, ++levels) {
       k_collapse_level<<<divUp(bound, 128), 128, 0, stream>>>((int)bound, q[cur], n, s.children, s.nodeLo, s.nodeHi, s.size, s.parent, s.leafPos, s.firstPos,
-                                                             root, s.orderedIds, outNodes, orderedIds8, q[cur ^ 1], counters, levelCount + levels, decision);
+                                                             root, s.orderedIds, outNodes, orderedIds8, q[cur ^ 1], counters, levelCount + levels, decision,
+                                                             wideSrc);
       cur ^= 1;
       bound = std::min<size_t>(bound * 8, (size_t)std::max(n / 2, 1));
     }
@@ -329,6 +379,11 @@ bool wideCollapse(const PlocScratch& s, int n, uint32_t root, DeviceArena& arena
   if ((int)host[1] != n) { err = "wide collapse lost primitives (" + std::to_string(host[1]) + " of " + std::to_string(n) + ")"; return false; }
   WCK(cudaGetLastError());
   *orderedIds8Out = orderedIds8;
+  *wideSrcOut = wideSrc;
   *levelsOut = levels;
   return true;
+}
+
+void wideRefit(const uint32_t* wideSrc, int nNodes, const float4* nodeLo, const float4* nodeHi, BvhNode8* nodes, cudaStream_t stream) {
+  k_wide_refit<<<divUp((size_t)nNodes, 128), 128, 0, stream>>>(nNodes, wideSrc, nodeLo, nodeHi, nodes);
 }

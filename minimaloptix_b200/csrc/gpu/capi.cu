@@ -5,6 +5,7 @@
 //
 // There is no CPU path in this library: every compute entry point needs a usable sm_100 GPU.
 #include <algorithm>
+#include <cstdint>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -14,6 +15,7 @@
 #include "build.h"
 #include "group.h"
 #include "mox.h"
+#include "mox_debug.h"
 #include "rng.cuh"
 #include "wavefront.h"
 
@@ -79,6 +81,11 @@ struct mox_ctx {
   std::vector<cudaTextureObject_t> texObjects;
   bool texturesDirty = false;
   uint32_t nSpheres = 0, nQuads = 0;
+  // One record per mox_add_mesh: its primitives, and its vertices / normals in verts / normals (in vertices, not floats).
+  struct MeshRec { uint32_t firstPrim, nFaces; size_t vBase, nV, nBase, nN; };
+  std::vector<MeshRec> meshes;
+  // Float ranges of verts / normals changed by mox_update_mesh since the last upload: [lo, hi), empty when lo >= hi.
+  size_t vDirtyLo = SIZE_MAX, vDirtyHi = 0, nDirtyLo = SIZE_MAX, nDirtyHi = 0;
 
   // device scene
   DevBuf dPrims, dTris, dVerts, dNormals, dUvs, dAnalytic, dMats, dLights, dLightN, dShadeRec;
@@ -98,6 +105,9 @@ struct mox_ctx {
   int nNodes = 0, nValid = 0;
   bool built = false, lightsDirty = true;
   uint32_t accelFlags = 0;
+  // The last full build succeeded and no primitive was added or removed since: MOX_ACCEL_REFIT may reuse its topology.
+  bool refitOk = false;
+  RefitState refit;
 
   // image
   float* dAccu = nullptr;
@@ -614,6 +624,70 @@ int ensurePinned(mox_ctx* c, size_t bytes) {
   return MOX_OK;
 }
 
+// What the builder reads of the context's device scene; the flags set the rest.
+BuildInput buildInput(mox_ctx* c, uint32_t flags) {
+  BuildInput in;
+  in.arena = &c->buildArena;
+  in.nPrims = (int)c->prims.size();
+  in.prims = (const PrimDesc*)c->dPrims.p;
+  in.tris = (const TriIdx*)c->dTris.p;
+  in.verts = (const float*)c->dVerts.p;
+  in.analytic = (const Analytic*)c->dAnalytic.p;
+  in.mats = (const GpuMaterial*)c->dMats.p;
+  in.evStart = c->ev0; in.evStop = c->ev1;
+  in.watertight = (flags & MOX_ACCEL_WATERTIGHT) != 0;
+  return in;
+}
+
+void buildShadeRecords(mox_ctx* c) {
+  launchBuildShadeRecords((const TriIdx*)c->dTris.p, (const float*)c->dVerts.p, (const float*)c->dNormals.p, (const float*)c->dUvs.p,
+                          (uint32_t)c->tris.size(), (float4*)c->dShadeRec.p, c->stream);
+}
+
+constexpr int kRebuild = 1;   // refitAccel: nothing to refit, run the full build
+
+// MOX_ACCEL_REFIT (flags without it): refit the structure of the last full build in place.  Uploads only what
+// mox_update_mesh / mox_update_sphere can have changed.  Returns kRebuild when that build had at most one valid
+// primitive: there is no hierarchy to keep, and a full build is as cheap.
+int refitAccel(mox_ctx* c, uint32_t flags, float* out_ms) {
+  if (!c->refitOk)
+    return fail(c, MOX_ERR_STATE, "MOX_ACCEL_REFIT needs a successful full build with no mox_add_* / mox_clear_scene after it");
+  if (const char* env = getenv("MOX_WATERTIGHT")) { if (atoi(env)) flags |= MOX_ACCEL_WATERTIGHT; }
+  if (flags != c->accelFlags) return fail(c, MOX_ERR_INVALID, "MOX_ACCEL_REFIT: the other flags differ from those of the last full build");
+  if (c->refit.path == RefitState::TRIVIAL) return kRebuild;
+  // A failed refit must not leave a context that still claims to be built, nor one that offers a refit again.
+  c->built = false;
+  c->refitOk = false;
+  cudaStreamSynchronize(c->stream);
+  if (c->vDirtyLo < c->vDirtyHi)
+    CUCK(c, cudaMemcpyAsync((float*)c->dVerts.p + c->vDirtyLo, c->verts.data() + c->vDirtyLo, (c->vDirtyHi - c->vDirtyLo) * 4,
+                            cudaMemcpyHostToDevice, c->stream));
+  if (c->nDirtyLo < c->nDirtyHi)
+    CUCK(c, cudaMemcpyAsync((float*)c->dNormals.p + c->nDirtyLo, c->normals.data() + c->nDirtyLo, (c->nDirtyHi - c->nDirtyLo) * 4,
+                            cudaMemcpyHostToDevice, c->stream));
+  c->vDirtyLo = c->nDirtyLo = SIZE_MAX; c->vDirtyHi = c->nDirtyHi = 0;
+  int rc = upload(c, c->dAnalytic, c->analytic);
+  if (rc) return rc;
+  if (c->shadeRecBuilt) buildShadeRecords(c);   // ahead of the timed kernels, as in the full build
+  BuildInput in = buildInput(c, flags);
+  BuildOutput out;
+  out.nodes = c->dNodes; out.packed = c->dPacked; out.nodes8 = c->dNodes8; out.packed8 = c->dPacked8;
+  out.refit = c->refit;
+  std::string err;
+  bool changed = false;
+  if (!refitBvh(in, out, c->stream, err, &changed)) return fail(c, MOX_ERR_CUDA, "build_accel (refit): " + err);
+  if (changed)
+    return fail(c, MOX_ERR_STATE, "MOX_ACCEL_REFIT: a primitive became degenerate, or valid again, since the last full build; "
+                                  "build without MOX_ACCEL_REFIT");
+  float ms = 0;
+  CUCK(c, cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+  c->msBuild = ms;
+  c->built = true;
+  c->refitOk = true;
+  if (out_ms) *out_ms = ms;
+  return MOX_OK;
+}
+
 }  // namespace
 
 // A multi-GPU handle (mox_create_multi) is a shell: every call is forwarded to its per-device contexts.
@@ -806,7 +880,7 @@ int mox_add_sphere(mox_ctx* c, const SphereParams* s, int kind, const void* para
   c->prims.push_back({PT_SPHERE | ((uint32_t)m << 2), (uint32_t)c->analytic.size() - 1});
   c->nSpheres++;
   if (out_id) *out_id = (uint32_t)c->prims.size() - 1;
-  c->built = false;
+  c->built = false; c->refitOk = false;
   return MOX_OK;
 }
 
@@ -825,7 +899,7 @@ int mox_add_quad(mox_ctx* c, const QuadParams* q, int kind, const void* params, 
   c->prims.push_back({PT_QUAD | ((uint32_t)m << 2), (uint32_t)c->analytic.size() - 1});
   c->nQuads++;
   if (out_id) *out_id = (uint32_t)c->prims.size() - 1;
-  c->built = false;
+  c->built = false; c->refitOk = false;
   return MOX_OK;
 }
 
@@ -848,6 +922,7 @@ int mox_add_mesh(mox_ctx* c, const float* v, size_t nv, const float* n, size_t n
   if (hasN) c->normals.insert(c->normals.end(), n, n + nn * 3);
   if (hasT) c->uvs.insert(c->uvs.end(), uv, uv + nt * 2);
   if (out_first) *out_first = (uint32_t)c->prims.size();
+  c->meshes.push_back({(uint32_t)c->prims.size(), (uint32_t)nFaces, (size_t)vb, nv, (size_t)nb, hasN ? nn : 0});
   c->tris.reserve(c->tris.size() + nFaces);
   c->prims.reserve(c->prims.size() + nFaces);
   for (size_t f = 0; f < nFaces; ++f) {
@@ -860,7 +935,7 @@ int mox_add_mesh(mox_ctx* c, const float* v, size_t nv, const float* n, size_t n
     c->tris.push_back(t);
     c->prims.push_back({PT_TRI | ((uint32_t)m << 2), (uint32_t)c->tris.size() - 1});
   }
-  c->built = false;
+  c->built = false; c->refitOk = false;
   return MOX_OK;
 }
 
@@ -877,10 +952,10 @@ int mox_clear_scene(mox_ctx* c) {
   if (!c) return MOX_ERR_INVALID;
   GROUP_EACH(c, mox_clear_scene(k));
   c->prims.clear(); c->tris.clear(); c->verts.clear(); c->normals.clear(); c->uvs.clear(); c->analytic.clear();
-  c->mats.clear(); c->lights.clear();
+  c->mats.clear(); c->lights.clear(); c->meshes.clear();
   c->textures.clear(); c->texturesDirty = true;
   c->nSpheres = c->nQuads = 0;
-  c->built = false; c->lightsDirty = true;
+  c->built = false; c->refitOk = false; c->lightsDirty = true;
   return MOX_OK;
 }
 
@@ -895,8 +970,13 @@ int mox_build_accel(mox_ctx* c, uint32_t flags, float* out_ms) {
   }
   int rc = bind(c);
   if (rc) return rc;
+  if (flags & MOX_ACCEL_REFIT) {
+    flags &= ~MOX_ACCEL_REFIT;
+    if ((rc = refitAccel(c, flags, out_ms)) != kRebuild) return rc;
+  }
   // A failed rebuild must not leave a context that still claims to be built.
   c->built = false;
+  c->refitOk = false;
   c->wideBuilt = false;
   cudaStreamSynchronize(c->stream);
   if ((rc = upload(c, c->dPrims, c->prims))) return rc;
@@ -906,14 +986,14 @@ int mox_build_accel(mox_ctx* c, uint32_t flags, float* out_ms) {
   if ((rc = upload(c, c->dUvs, c->uvs))) return rc;
   if ((rc = upload(c, c->dAnalytic, c->analytic))) return rc;
   if ((rc = upload(c, c->dMats, c->mats))) return rc;
+  c->vDirtyLo = c->nDirtyLo = SIZE_MAX; c->vDirtyHi = c->nDirtyHi = 0;
   c->shadeRecBuilt = false;
   {
     bool want = !c->tris.empty();
     if (const char* env = getenv("MOX_SHADE_RECORDS")) want = want && atoi(env) != 0;
     if (want) {
       if ((rc = ensure(c, c->dShadeRec, c->tris.size() * MOX_SHADE_REC_F4 * sizeof(float4)))) return rc;
-      launchBuildShadeRecords((const TriIdx*)c->dTris.p, (const float*)c->dVerts.p, (const float*)c->dNormals.p, (const float*)c->dUvs.p,
-                              (uint32_t)c->tris.size(), (float4*)c->dShadeRec.p, c->stream);
+      buildShadeRecords(c);
       c->shadeRecBuilt = true;
     }
   }
@@ -923,23 +1003,14 @@ int mox_build_accel(mox_ctx* c, uint32_t flags, float* out_ms) {
     if (m.kind == MOX_MAT_DISNEY && (m.dis.albedoID < 0 || m.dis.albedoID > (int)c->textures.size()))
       return fail(c, MOX_ERR_INVALID, "DisneyParams.albedoID refers to a texture that was not added");
   }
-  BuildInput in;
-  in.arena = &c->buildArena;
-  in.nPrims = (int)c->prims.size();
-  in.prims = (const PrimDesc*)c->dPrims.p;
-  in.tris = (const TriIdx*)c->dTris.p;
-  in.verts = (const float*)c->dVerts.p;
-  in.analytic = (const Analytic*)c->dAnalytic.p;
-  in.mats = (const GpuMaterial*)c->dMats.p;
-  in.evStart = c->ev0; in.evStop = c->ev1;
+  if (const char* env = getenv("MOX_WATERTIGHT")) { if (atoi(env)) flags |= MOX_ACCEL_WATERTIGHT; }
+  BuildInput in = buildInput(c, flags);
   in.usePloc = (flags & MOX_ACCEL_LBVH) == 0;
   if (const char* env = getenv("MOX_PLOC_RADIUS")) in.plocRadius = atoi(env);
   if (const char* env = getenv("MOX_FORCE_LBVH")) { if (atoi(env)) in.usePloc = false; }
   c->useWide = (flags & MOX_ACCEL_BINARY) == 0;
   if (const char* env = getenv("MOX_FORCE_BINARY")) { if (atoi(env)) c->useWide = false; }
   in.useWide = c->useWide;
-  if (const char* env = getenv("MOX_WATERTIGHT")) { if (atoi(env)) flags |= MOX_ACCEL_WATERTIGHT; }
-  in.watertight = (flags & MOX_ACCEL_WATERTIGHT) != 0;
   BuildOutput out;
   out.nodes = c->dNodes; out.packed = c->dPacked; out.nodesCap = c->nodesCap; out.packedCap = c->packedCap;
   out.nodes8 = c->dNodes8; out.packed8 = c->dPacked8; out.nodes8Cap = c->nodes8Cap; out.packed8Cap = c->packed8Cap;
@@ -956,6 +1027,8 @@ int mox_build_accel(mox_ctx* c, uint32_t flags, float* out_ms) {
   c->msBuild = ms;
   c->accelFlags = flags;
   c->built = true;
+  c->refit = out.refit;
+  c->refitOk = true;
   if (out_ms) *out_ms = ms;
   return MOX_OK;
 }
@@ -1189,6 +1262,26 @@ int mox_update_sphere(mox_ctx* c, uint32_t prim_id, const SphereParams* s) {
   return MOX_OK;
 }
 
+int mox_update_mesh(mox_ctx* c, uint32_t first_prim_id, const float* v, size_t nv, const float* n, size_t nn) {
+  if (!c) return MOX_ERR_INVALID;
+  GROUP_EACH(c, mox_update_mesh(k, first_prim_id, v, nv, n, nn));
+  auto it = std::lower_bound(c->meshes.begin(), c->meshes.end(), first_prim_id,
+                             [](const mox_ctx::MeshRec& m, uint32_t id) { return m.firstPrim < id; });
+  while (it != c->meshes.end() && it + 1 != c->meshes.end() && (it + 1)->firstPrim == first_prim_id && it->nFaces == 0) ++it;  // skip empty meshes
+  if (it == c->meshes.end() || it->firstPrim != first_prim_id) return fail(c, MOX_ERR_INVALID, "not the first primitive id of a mesh");
+  const mox_ctx::MeshRec& m = *it;
+  if (nv != m.nV || (nv && !v)) return fail(c, MOX_ERR_INVALID, "vertex count differs from the one the mesh was added with");
+  if (n && (m.nN == 0 || nn != m.nN)) return fail(c, MOX_ERR_INVALID, "normal count differs from the one the mesh was added with");
+  std::copy(v, v + 3 * nv, c->verts.begin() + 3 * m.vBase);
+  c->vDirtyLo = std::min(c->vDirtyLo, 3 * m.vBase); c->vDirtyHi = std::max(c->vDirtyHi, 3 * (m.vBase + nv));
+  if (n) {
+    std::copy(n, n + 3 * nn, c->normals.begin() + 3 * m.nBase);
+    c->nDirtyLo = std::min(c->nDirtyLo, 3 * m.nBase); c->nDirtyHi = std::max(c->nDirtyHi, 3 * (m.nBase + nn));
+  }
+  c->built = false;
+  return MOX_OK;
+}
+
 int mox_owned_pixels(mox_ctx* c, uint32_t rank, uint64_t* out_n) {
   if (!c) return MOX_ERR_INVALID;
   GROUP_REFUSE(c, "the tile partition");
@@ -1381,4 +1474,28 @@ extern "C" int mox_debug_radix_sort(mox_ctx* c, uint32_t* keys, uint32_t* vals, 
   }
   cudaFree(dk); cudaFree(dv);
   return ok ? MOX_OK : fail(c, MOX_ERR_CUDA, err);
+}
+
+extern "C" int mox_debug_read_accel(mox_ctx* c, int which, void* dst, size_t cap, size_t* out_bytes) {
+  if (!c) return MOX_ERR_INVALID;
+  GROUP_FIRST(c, mox_debug_read_accel(k, which, dst, cap, out_bytes));
+  if (!c->built) return fail(c, MOX_ERR_STATE, "debug_read_accel before mox_build_accel");
+  const bool wide = c->wideBuilt && c->useWide;
+  const void* src = nullptr;
+  size_t bytes = 0;
+  switch (which) {
+    case MOX_DEBUG_ACCEL_NODES: src = c->dNodes; bytes = (size_t)c->nNodes * sizeof(BvhNode2); break;
+    case MOX_DEBUG_ACCEL_NODES8: src = c->dNodes8; bytes = wide ? (size_t)c->nNodes8 * sizeof(BvhNode8) : 0; break;
+    case MOX_DEBUG_ACCEL_PACKED: src = c->dPacked; bytes = (size_t)c->nValid * 16 * MOX_PACKED_F4; break;
+    case MOX_DEBUG_ACCEL_PACKED8: src = c->dPacked8; bytes = wide ? (size_t)c->nValid * 16 * MOX_PACKED_F4 : 0; break;
+    default: return fail(c, MOX_ERR_INVALID, "unknown acceleration array");
+  }
+  if (out_bytes) *out_bytes = bytes;
+  if (!dst || !bytes) return MOX_OK;
+  if (cap < bytes) return fail(c, MOX_ERR_INVALID, "destination too small");
+  int rc = bind(c);
+  if (rc) return rc;
+  CUCK(c, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, c->stream));
+  CUCK(c, cudaStreamSynchronize(c->stream));
+  return MOX_OK;
 }

@@ -334,6 +334,31 @@ __global__ void k_ploc_emit(int nLeaves, int nInner, uint32_t root, const uint32
   out[nInner - 1 - k] = nd;
 }
 
+// Refit of a finished tree: leaf i takes the box of sorted primitive i (as k_ploc_init), inner nodes are formed again
+// bottom-up; the second child to arrive at a node (per-node arrival counters, as k_refit) writes it.  The union takes
+// the same operands in the same order as k_ploc_merge / k_ploc_tail (children.x first), so unchanged boxes give the
+// same bits, signed zeros included.
+__global__ void k_ploc_refit(int nLeaves, uint32_t root, const uint32_t* __restrict__ sortedIds, const float4* __restrict__ primLo,
+                             const float4* __restrict__ primHi, const uint2* __restrict__ children, const uint32_t* __restrict__ parent,
+                             float4* __restrict__ nodeLo, float4* __restrict__ nodeHi, uint32_t* __restrict__ arrivals) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= nLeaves) return;
+  const uint32_t id = sortedIds[i];
+  __stcg(&nodeLo[i], primLo[id]);
+  __stcg(&nodeHi[i], primHi[id]);
+  __threadfence();
+  for (uint32_t node = (uint32_t)i; node != root;) {
+    const uint32_t p = parent[node];
+    if (atomicAdd(&arrivals[p - nLeaves], 1u) == 0u) return;  // the sibling subtree is not finished yet
+    const uint2 ch = children[p - nLeaves];
+    const float4 alo = __ldcg(&nodeLo[ch.x]), ahi = __ldcg(&nodeHi[ch.x]), blo = __ldcg(&nodeLo[ch.y]), bhi = __ldcg(&nodeHi[ch.y]);
+    __stcg(&nodeLo[p], make_float4(fminf(alo.x, blo.x), fminf(alo.y, blo.y), fminf(alo.z, blo.z), 0.f));
+    __stcg(&nodeHi[p], make_float4(fmaxf(ahi.x, bhi.x), fmaxf(ahi.y, bhi.y), fmaxf(ahi.z, bhi.z), 0.f));
+    __threadfence();
+    node = p;
+  }
+}
+
 inline int divUp(size_t a, size_t b) { return (int)((a + b - 1) / b); }
 
 }  // namespace
@@ -428,5 +453,15 @@ bool plocBuild(PlocScratch& s, int n, const uint32_t* sortedIds, const float4* p
   *maxDepthOut = (int)depth;
   rootLo[0] = lo.x; rootLo[1] = lo.y; rootLo[2] = lo.z;
   rootHi[0] = hi.x; rootHi[1] = hi.y; rootHi[2] = hi.z;
+  return true;
+}
+
+bool plocRefit(const PlocScratch& s, int n, const uint32_t* sortedIds, const float4* primLo, const float4* primHi, uint32_t* arrivals,
+               BvhNode2* outNodes, cudaStream_t stream, std::string& err) {
+  const int B = 256, nInner = n - 1;
+  const uint32_t root = (uint32_t)(n + nInner - 1);
+  PCK(cudaMemsetAsync(arrivals, 0, (size_t)nInner * 4, stream));
+  k_ploc_refit<<<divUp(n, B), B, 0, stream>>>(n, root, sortedIds, primLo, primHi, s.children, s.parent, s.nodeLo, s.nodeHi, arrivals);
+  k_ploc_emit<<<divUp(nInner, B), B, 0, stream>>>(n, nInner, root, s.parent, s.children, s.size, s.leafPos, s.firstPos, s.nodeLo, s.nodeHi, outNodes);
   return true;
 }

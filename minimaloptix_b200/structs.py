@@ -85,6 +85,7 @@ class Stats(C.Structure):
 MAT_LAMBERTIAN, MAT_METAL, MAT_GLASS, MAT_DISNEY, MAT_LIGHT = range(5)
 RNG_REF, RNG_PHILOX = 0, 1
 ACCEL_DEFAULT, ACCEL_LBVH, ACCEL_COUNTERS, ACCEL_BINARY, ACCEL_WATERTIGHT = 0, 1, 2, 4, 8
+ACCEL_REFIT = 16   # refit the last full build in place (mox.h MOX_ACCEL_REFIT)
 
 SIZES = {Payload: 32, CamParams: 76, SphereParams: 28, QuadParams: 64, LambertianParams: 12, MetalParams: 16,
          GlassParams: 16, DisneyParams: 72, LightParams: 72}
