@@ -114,6 +114,9 @@ bool buildBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::
 // *validityChanged: a primitive became valid or invalid since the build; the result is then unusable.
 bool refitBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::string& err, bool* validityChanged);
 bool radixSortPairs(uint32_t* keys, uint32_t* vals, int n, cudaStream_t stream, std::string& err);
+// Marks the entries of the terminal query's light list (n <= MOX_TERMINAL_LIGHTS_MAX, traverse_job.h) whose primitive
+// the last full build left out (rs.primLo .w == 0).  A refit keeps every primitive's validity, so the list stays.
+void excludeUnbuiltLights(uint4* list, int n, const RefitState& rs, cudaStream_t stream);
 
 // Refit of a PLOC tree built by plocBuild over n leaves: new leaf and inner boxes in s.nodeLo / s.nodeHi, then the
 // binary nodes again.  arrivals: n - 1 words of scratch.

@@ -12,6 +12,7 @@
 //   k_emit2         Aila–Laine 64-byte nodes, subtrees of <= MOX_LEAF_MAX prims folded into leaves
 //   k_pack          leaf-ordered 48-byte primitive records
 #include "build.h"
+#include "traverse_job.h"
 #include "vec.cuh"
 
 namespace {
@@ -408,6 +409,13 @@ __global__ void k_pack(int n, const uint32_t* __restrict__ sortedIds, const Prim
   }
 }
 
+// Light list of the terminal query: a primitive k_prim_bounds left out of the BVH (validity in boxLo .w) must not be
+// found by the list either.
+__global__ void k_terminal_lights(int n, const float4* __restrict__ boxLo, uint4* __restrict__ list) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n && boxLo[list[i].x & MOX_HIT_ID_MASK].w == 0.f) list[i].y = MOX_TERMINAL_EXCLUDED;
+}
+
 inline int divUp(size_t a, size_t b) { return (int)((a + b - 1) / b); }
 
 // Grid of the grid-stride histogram kernel: eight 256-thread blocks per SM of the current device.
@@ -647,6 +655,10 @@ bool refitBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::
   CK(cudaGetLastError());
   *validityChanged = host[0] != 0u;
   return true;
+}
+
+void excludeUnbuiltLights(uint4* list, int n, const RefitState& rs, cudaStream_t stream) {
+  if (n > 0) k_terminal_lights<<<1, MOX_TERMINAL_LIGHTS_MAX, 0, stream>>>(n, rs.primLo, list);
 }
 
 // Stand-alone sort entry used by the tests (keys/vals are device pointers, sorted in place).

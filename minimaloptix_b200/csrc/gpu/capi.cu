@@ -108,6 +108,10 @@ struct mox_ctx {
   // The last full build succeeded and no primitive was added or removed since: MOX_ACCEL_REFIT may reuse its topology.
   bool refitOk = false;
   RefitState refit;
+  // Light primitives of the terminal query (traverse_job.h), from the last full build; nTerminalLights < 0: the scene
+  // has a triangle-mesh light or more than MOX_TERMINAL_LIGHTS_MAX lights, and the terminal bounce runs closest hit.
+  DevBuf dTerminalLights;
+  int nTerminalLights = -1;
 
   // image
   float* dAccu = nullptr;
@@ -159,6 +163,8 @@ struct mox_ctx {
   size_t maxBatchPaths = 32u << 20;  // paths per wavefront (264 B each with 4 lights, bytesPerPath); measured 4 Mi -> 947, 32 Mi -> 980 Mrays/s at 4K
   bool overlapShadow = true;     // shadow rays of bounce b on a second stream, concurrent with the extend launch of bounce b+1 (MOX_OVERLAP_SHADOW=0: serial)
   bool brdfFast = true;          // approximate reciprocal / square root inside BRDF values (MOX_BRDF_IEEE=1: IEEE, the oracle's operations)
+  bool terminalQuery = true;     // the bounce past rayMaxDepth uses the light list and an any-hit query (MOX_TERMINAL_CLOSEST=1: closest hit)
+  uint32_t terminalDepth = 0;    // the batch's last bounce ran the terminal query: its ray counts come with the final counter copy
 };
 
 namespace {
@@ -372,6 +378,8 @@ int syncLights(mox_ctx* c) {
 
 inline uint32_t* bounceBlock(const PathBuffers& pb, uint32_t depth) { return pb.counters + C_WORDS + (depth % BOUNCE_RING) * C_BOUNCE_WORDS; }
 
+int finishBatch(mox_ctx* c);
+
 // Enqueue one bounce up to the point where the host needs numbers: extend (persistent traversal, ray count read on
 // the device), classify, and the read-back of the counters.
 int enqueueExtend(mox_ctx* c) {
@@ -383,6 +391,21 @@ int enqueueExtend(mox_ctx* c) {
   // bounce 1 traces exactly `bound` camera rays; later bounces read the number of spawned rays from the previous
   // bounce's counter block, `bound` (what was shaded) only sizes the grids
   const uint32_t* countPtr = depth == 1 ? nullptr : bounceBlock(c->pb, depth - 1) + C_NEXT;
+  // k_classify's test: every path of this bounce ends in it, whatever it hits (|payload colour| = sqrt(3))
+  const bool terminal = depth > c->rp.maxDepth || length(mk3(1.f)) < c->rp.minIntensity;
+  if (terminal && c->terminalQuery && c->nTerminalLights >= 0 && lc.scene.nodes8) {
+    TerminalLights tl;
+    tl.list = (const uint4*)c->dTerminalLights.p;
+    tl.n = c->nTerminalLights;
+    tl.missIsAbsorb = memcmp(&c->rp.bg, &c->rp.absorb, sizeof c->rp.bg) == 0;
+    tm.begin(ST_EXTEND, c->stream, depth);
+    launchTerminal(lc, depth == 1 ? nullptr : lc.pb.qCur, c->bound, countPtr, tl);
+    tm.end(c->stream);
+    c->extendLaunches++; c->kernelLaunches++;
+    // k_classify would queue nothing: no counts to wait for, the accumulation follows at once
+    c->terminalDepth = depth;
+    return finishBatch(c);
+  }
   tm.begin(ST_EXTEND, c->stream, depth);
   // camera rays are queued in path order (k_generate: qCur[p] = p): the traversal kernel skips the indirection
   launchExtend(lc, depth == 1 ? nullptr : lc.pb.qCur, c->bound, countPtr, depth);
@@ -409,6 +432,20 @@ int finishBatch(mox_ctx* c) {
   return MOX_OK;
 }
 
+// Exact number of rays bounce `depth` traced, and of shadow rays the bounce before it queued, from the counters in
+// hostCnt.
+void countBounceRays(mox_ctx* c, uint32_t depth) {
+  const uint32_t dIdx = std::min<uint32_t>(depth, MOX_STATS_DEPTHS - 1);
+  if (depth == 1) { c->raysPrimary += c->bound; c->raysDepth[1] += c->bound; }
+  else {
+    const uint32_t* prev = c->hostCnt + C_WORDS + ((depth - 1) % BOUNCE_RING) * C_BOUNCE_WORDS;
+    c->raysBounce += prev[C_NEXT];
+    c->raysShadowTraced += prev[C_SHQ];
+    c->raysDepth[dIdx] += prev[C_NEXT];
+    c->shadowDepth[std::min<uint32_t>(depth - 1, MOX_STATS_DEPTHS - 1)] += prev[C_SHQ];
+  }
+}
+
 // The counters of the bounce in flight have arrived: shade what was binned, trace the shadow rays, and enqueue
 // the next bounce — or the accumulation when nothing is left.
 int advanceBounce(mox_ctx* c) {
@@ -417,15 +454,7 @@ int advanceBounce(mox_ctx* c) {
   PathBuffers& pb = c->pb;
   const uint32_t depth = c->depth;
   const uint32_t* hostBounce = c->hostCnt + C_WORDS + (depth % BOUNCE_RING) * C_BOUNCE_WORDS;
-  const uint32_t dIdx = std::min<uint32_t>(depth, MOX_STATS_DEPTHS - 1);
-  if (depth == 1) { c->raysPrimary += c->bound; c->raysDepth[1] += c->bound; }
-  else {  // exact number of rays this bounce traced, and of shadow rays the previous one queued
-    const uint32_t* prev = c->hostCnt + C_WORDS + ((depth - 1) % BOUNCE_RING) * C_BOUNCE_WORDS;
-    c->raysBounce += prev[C_NEXT];
-    c->raysShadowTraced += prev[C_SHQ];
-    c->raysDepth[dIdx] += prev[C_NEXT];
-    c->shadowDepth[std::min<uint32_t>(depth - 1, MOX_STATS_DEPTHS - 1)] += prev[C_SHQ];
-  }
+  countBounceRays(c, depth);
   uint32_t any = 0;
   for (int k = 0; k < Q_COUNT; ++k) { c->matCount[k] = hostBounce[C_MAT0 + k]; any += c->matCount[k]; }
   if (!any) return finishBatch(c);
@@ -499,7 +528,7 @@ int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds) {
   lc.stream = c->stream;
   lc.pb.qCur = pb.qBuf[0]; lc.pb.qNext = pb.qBuf[1];
   lc.bc = bounceBlock(pb, 1);
-  c->batchSamples = S; c->bound = (uint32_t)P; c->depth = 1; c->batchDone = false; c->applyPending = false;
+  c->batchSamples = S; c->bound = (uint32_t)P; c->depth = 1; c->batchDone = false; c->applyPending = false; c->terminalDepth = 0;
   CUCK(c, cudaMemsetAsync(pb.counters, 0, kCounterWords * 4, c->stream));
   c->timer.begin(ST_GENERATE, c->stream);
   launchGenerate(lc, S);
@@ -513,6 +542,7 @@ int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds) {
   // the accumulation and the final counter read-back
   CUCK(c, cudaEventSynchronize(c->evReady));
   const uint32_t* host = c->hostCnt;
+  if (c->terminalDepth) countBounceRays(c, c->terminalDepth);
   c->timer.collect(c->msStage, c->msDepth);
   c->nonfinite += host[C_NONFINITE];
   c->shadowBlocked += host[C_SH_BLOCKED]; c->shadowTinted += host[C_SH_TINTED];
@@ -644,6 +674,32 @@ void buildShadeRecords(mox_ctx* c) {
                           (uint32_t)c->tris.size(), (float4*)c->dShadeRec.p, c->stream);
 }
 
+// The light primitives of the terminal query in id order, with their hit-record bits (k_pack gives a light material
+// shade class MOX_CLASS_LIGHT).  False when a mesh has a light material or there are more than
+// MOX_TERMINAL_LIGHTS_MAX of them.  Which ones the build kept is marked on the device (excludeUnbuiltLights).
+bool terminalLightList(const mox_ctx* c, std::vector<uint4>& out) {
+  out.clear();
+  auto isLight = [&](uint32_t id) { return c->mats[c->prims[id].typeMat >> 2].kind == MOX_MAT_LIGHT; };
+  for (const auto& m : c->meshes)
+    if (m.nFaces && isLight(m.firstPrim)) return false;
+  // the spheres and quads lie between the id ranges of the meshes (recorded in id order)
+  uint32_t id = 0;
+  auto scan = [&](uint32_t end) {
+    for (; id < end; ++id) {
+      if (!isLight(id)) continue;
+      const uint32_t type = c->prims[id].typeMat & 3u;
+      if (type == PT_TRI || out.size() == MOX_TERMINAL_LIGHTS_MAX) return false;
+      out.push_back(make_uint4(id | (MOX_CLASS_LIGHT << MOX_HIT_ID_BITS), type, c->prims[id].geom, 0u));
+    }
+    return true;
+  };
+  for (const auto& m : c->meshes) {
+    if (!scan(m.firstPrim)) return false;
+    id = m.firstPrim + m.nFaces;
+  }
+  return scan((uint32_t)c->prims.size());
+}
+
 constexpr int kRebuild = 1;   // refitAccel: nothing to refit, run the full build
 
 // MOX_ACCEL_REFIT (flags without it): refit the structure of the last full build in place.  Uploads only what
@@ -765,6 +821,7 @@ int mox_create(mox_ctx** out, int device_id) {
   if (const char* env = getenv("MOX_MAX_BATCH_PATHS")) { long long v = atoll(env); if (v > 0) c->maxBatchPaths = (size_t)v; }
   if (const char* env = getenv("MOX_OVERLAP_SHADOW")) c->overlapShadow = atoi(env) != 0;
   if (const char* env = getenv("MOX_BRDF_IEEE")) c->brdfFast = atoi(env) == 0;
+  if (const char* env = getenv("MOX_TERMINAL_CLOSEST")) c->terminalQuery = atoi(env) == 0;
   memset(&c->rp, 0, sizeof c->rp);
   c->rp.maxDepth = 256; c->rp.eps = 0.001f; c->rp.minIntensity = 0.001f;
   c->rp.bad = make_float3(1.f, 1.f, 1.f);
@@ -777,7 +834,7 @@ void mox_destroy(mox_ctx* c) {
   if (c->group) { groupDestroy(c->group); delete c; return; }
   cudaSetDevice(c->device);
   if (c->stream) cudaStreamSynchronize(c->stream);
-  for (DevBuf* b : {&c->dPrims, &c->dTris, &c->dVerts, &c->dNormals, &c->dUvs, &c->dAnalytic, &c->dMats, &c->dLights, &c->dLightN, &c->dShadeRec, &c->dQueryRays, &c->dQueryOut, &c->dQueryC, &c->dQueryO,
+  for (DevBuf* b : {&c->dPrims, &c->dTris, &c->dVerts, &c->dNormals, &c->dUvs, &c->dAnalytic, &c->dMats, &c->dLights, &c->dLightN, &c->dShadeRec, &c->dTerminalLights, &c->dQueryRays, &c->dQueryOut, &c->dQueryC, &c->dQueryO,
                    &c->dQueryD, &c->dQueryCounters}) b->release();
   for (auto& b : c->otherOwned) b.release();
   freeTextures(c);
@@ -978,6 +1035,7 @@ int mox_build_accel(mox_ctx* c, uint32_t flags, float* out_ms) {
   c->built = false;
   c->refitOk = false;
   c->wideBuilt = false;
+  c->nTerminalLights = -1;
   cudaStreamSynchronize(c->stream);
   if ((rc = upload(c, c->dPrims, c->prims))) return rc;
   if ((rc = upload(c, c->dTris, c->tris))) return rc;
@@ -1029,6 +1087,15 @@ int mox_build_accel(mox_ctx* c, uint32_t flags, float* out_ms) {
   c->built = true;
   c->refit = out.refit;
   c->refitOk = true;
+  {
+    std::vector<uint4> tl;
+    if (terminalLightList(c, tl)) {
+      if ((rc = upload(c, c->dTerminalLights, tl))) return rc;
+      excludeUnbuiltLights((uint4*)c->dTerminalLights.p, (int)tl.size(), c->refit, c->stream);
+      CUCK(c, cudaGetLastError());
+      c->nTerminalLights = (int)tl.size();
+    }
+  }
   if (out_ms) *out_ms = ms;
   return MOX_OK;
 }

@@ -30,3 +30,14 @@ struct TraceJob {
   int fetchThreshold;   // refill idle lanes when fewer than this many lanes are traversing
 };
 
+// Light primitives of the terminal query (the bounce past rayMaxDepth, traverse_wide.cuh), one uint4 each:
+//   x = primitive id | MOX_CLASS_LIGHT << 28 (the hit record's form), y = primitive type (PT_QUAD or PT_SPHERE; any
+//   other value marks a primitive the build left out, which is skipped), z = index into analytic[].
+#define MOX_TERMINAL_LIGHTS_MAX 32
+#define MOX_TERMINAL_EXCLUDED 3u
+struct TerminalLights {
+  const uint4* list = nullptr;
+  int n = 0;
+  int missIsAbsorb = 0;   // bgColor and absorbColor are bit-equal: a ray that hits no light needs no traversal
+};
+

@@ -74,8 +74,17 @@ MOX_D uint32_t bitSelect(uint32_t a, uint32_t b, uint32_t m) {
 // comes from the winning primitive's packed record — and beta / gamma are not carried (two registers less per
 // lane); the shade kernels recompute them from the same operands.  The raw query keeps the four-word record.
 // WT: the packed triangle records hold the raw vertices and the watertight test runs (MOX_ACCEL_WATERTIGHT).
-template <bool ANYHIT, bool COUNT, bool CLASSIFY = false, bool WT = false>
-__device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const TraceJob& job) {
+// TERMINAL (with CLASSIFY): the bounce past rayMaxDepth.  k_classify ends every such path and k_accumulate adds one
+// term chosen by the record's .y alone: miss -> bgColor, a light -> its emission, anything else -> absorbColor.  So
+// the refill finds the (t, id) minimum over the light list tl with the primitive step's tests and acceptance rule;
+// then an any-hit traversal bounded by that light (tBest = tL, tie id idL) ends at the first accepted hit, which
+// lies ahead of every light, so the closest hit is no light either.  Every primitive blocks.  The record is
+//   (t of the written primitive, id | class << 28) of that blocker, else of the light, else (tmax, MOX_HIT_MISS);
+// with no light hit and bgColor == absorbColor the ray ends at the refill with the miss record.  Nothing reads .x
+// of a terminal record.
+template <bool ANYHIT, bool COUNT, bool CLASSIFY = false, bool WT = false, bool TERMINAL = false>
+__device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const TraceJob& job, const TerminalLights& tl = TerminalLights()) {
+  static_assert(!TERMINAL || (CLASSIFY && !ANYHIT), "the terminal query writes the render path's hit record");
   const unsigned FULL = 0xffffffffu;
   const int lane = threadIdx.x & 31;
   const unsigned ltMask = (1u << lane) - 1u;
@@ -107,8 +116,10 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
   // touches yet — is issued when a pool runs dry, so what a refill waits for is one memory level (the ray itself)
   // instead of three (cursor, queue entry, ray); the whole warp sits in that wait, busy lanes included.  Measured:
   // shadow 90.6 -> 90.0 ms per step; the closest-hit kernel lost with it (69.3 -> 70.1 ms) and keeps one atomic
-  // per refill.
-  constexpr bool CHUNKED = ANYHIT;
+  // per refill.  The terminal query claims in chunks too: most of its rays end at the refill, and a warp that keeps a
+  // few lanes in an any-hit traversal refills its idle ones a few at a time, one atomic on the cursor each.  (Not its
+  // counting form: that one would spill at 56 registers, and the counts do not depend on how rays are claimed.)
+  constexpr bool CHUNKED = ANYHIT || (TERMINAL && !COUNT);
   uint32_t poolId = 0, poolPos = 0, poolCount = 0;   // poolPos / poolCount are warp-uniform
   bool moreChunks = true;
   while (true) {
@@ -156,6 +167,28 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
             gBase = 0; gBits = 0x80000000u;  // root: one pending child, imask 0 -> node index 0
             tBase = 0; tBits = 0;
             if (COUNT) { nv = 0; np = 0; shadowEnd = 0; }
+            if (TERMINAL) {
+              // closest light: same tests, same operands (the packed sphere record is analytic[].a) and same rule as
+              // the primitive step, so the minimum is the one the closest-hit traversal would find among the lights
+              for (int k = 0; k < tl.n; ++k) {
+                const uint4 e = __ldg(tl.list + k);
+                const bool tie = bPrim >= 0 && (e.x & MOX_HIT_ID_MASK) < ((uint32_t)bPrim & MOX_HIT_ID_MASK);
+                const Analytic* an = s.analytic + e.z;
+                float t = 0.f, a1, a2;
+                bool hit = false;
+                if (e.y == PT_SPHERE) hit = sphereTest(__ldg(&an->a), o, d, tmin, tBest, tie, t);
+                else if (e.y == PT_QUAD) {
+                  Analytic q;
+                  q.a = __ldg(&an->a); q.b = __ldg(&an->b); q.c = __ldg(&an->c); q.d = __ldg(&an->d);
+                  hit = quadTest(q, o, d, tmin, t, a1, a2) && (t < tBest || (t == tBest && tie));
+                }
+                if (hit) { tBest = t; bPrim = (int)e.x; }
+              }
+              if (bPrim < 0 && tl.missIsAbsorb) {   // miss and non-light end alike: nothing to traverse
+                MOX_ST_STREAM(job.hits2 + rayId, make_float2(tBest, __int_as_float(MOX_HIT_MISS)));
+                gBits = 0u;
+              }
+            }
           }
         }
         if (CHUNKED) {
@@ -319,6 +352,7 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
               tBest = t;
               if (CLASSIFY) bPrim = (int)((uint32_t)id | ((__float_as_uint(r1.w) >> MOX_CLASS_SHIFT) << MOX_HIT_ID_BITS));
               else { bPrim = id; bBeta = be; bGamma = ga; }
+              if (TERMINAL) { tBits = 0u; gBits = 0u; sp = 0; }   // the first hit ahead of the closest light decides
             }
           }
         };

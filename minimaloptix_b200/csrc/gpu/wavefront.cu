@@ -108,6 +108,15 @@ template <bool ANYHIT, bool COUNT, bool CLASSIFY>
 __global__ void __launch_bounds__(TRAV_TPB, MOX_WIDE_MINBLOCKS) k_traverse_wide(SceneView s, TraceJob job) {
   traverseWidePersistent<ANYHIT, COUNT, CLASSIFY>(s, job);
 }
+// The terminal bounce: closest light, then an any-hit query bounded by it (traverse_wide.cuh, TERMINAL).
+template <bool COUNT>
+__global__ void __launch_bounds__(TRAV_TPB, MOX_WIDE_MINBLOCKS) k_traverse_wide_terminal(SceneView s, TraceJob job, TerminalLights tl) {
+  traverseWidePersistent<false, COUNT, true, false, true>(s, job, tl);
+}
+template <bool COUNT>
+__global__ void __launch_bounds__(TRAV_TPB, 8) k_traverse_wide_wt_terminal(SceneView s, TraceJob job, TerminalLights tl) {
+  traverseWidePersistent<false, COUNT, true, true, true>(s, job, tl);
+}
 
 // Bins the paths of the current queue by the shade class in their hit record.  A miss, a light and a path
 // beyond rayMaxDepth end here without a write: their last term is added by k_accumulate from the same record.
@@ -662,6 +671,22 @@ void launchExtend(const LaunchCtx& c, const uint32_t* queue, uint32_t count, con
   job.rayO = c.pb.rayO; job.rayD = c.pb.rayD; job.queue = queue; job.count = count; job.countPtr = countPtr; job.originMod = 0;
   job.cursor = c.pb.counters + C_CURSOR; job.hits = nullptr; job.hits2 = c.pb.hit; job.shC = nullptr; job.counters = c.pb.counters;
   launchTraverse(c.scene, job, false, c.countTraversal, c.stream, true);
+}
+void launchTerminal(const LaunchCtx& c, const uint32_t* queue, uint32_t count, const uint32_t* countPtr, const TerminalLights& tl) {
+  if (!count) return;
+  TraceJob job;
+  job.rayO = c.pb.rayO; job.rayD = c.pb.rayD; job.queue = queue; job.count = count; job.countPtr = countPtr; job.originMod = 0;
+  job.cursor = c.pb.counters + C_CURSOR; job.hits = nullptr; job.hits2 = c.pb.hit; job.shC = nullptr; job.counters = c.pb.counters;
+  job.fetchThreshold = fetchThreshold(false, true);
+  job.originMagic = 0u;
+  cudaMemsetAsync(job.cursor, 0, 4, c.stream);
+  static std::atomic<int> bps{0}, bpsCount{0}, bpsWt{0}, bpsWtCount{0};
+  const SceneView& s = c.scene;
+  if (s.watertight) {
+    if (c.countTraversal) k_traverse_wide_wt_terminal<true><<<persistentGridFor(k_traverse_wide_wt_terminal<true>, count, bpsWtCount), TRAV_TPB, 0, c.stream>>>(s, job, tl);
+    else k_traverse_wide_wt_terminal<false><<<persistentGridFor(k_traverse_wide_wt_terminal<false>, count, bpsWt), TRAV_TPB, 0, c.stream>>>(s, job, tl);
+  } else if (c.countTraversal) k_traverse_wide_terminal<true><<<persistentGridFor(k_traverse_wide_terminal<true>, count, bpsCount), TRAV_TPB, 0, c.stream>>>(s, job, tl);
+  else k_traverse_wide_terminal<false><<<persistentGridFor(k_traverse_wide_terminal<false>, count, bps), TRAV_TPB, 0, c.stream>>>(s, job, tl);
 }
 void launchClassify(const LaunchCtx& c, const uint32_t* queue, uint32_t count, const uint32_t* countPtr, uint32_t depth) {
   if (count) k_classify<<<grid(count), TPB, 0, c.stream>>>(c, queue, count, countPtr, depth);

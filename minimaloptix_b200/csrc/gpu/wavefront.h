@@ -54,6 +54,9 @@ struct LaunchCtx {
 void launchGenerate(const LaunchCtx& c, uint32_t nSamples);
 // countPtr (may be null): exact ray count in device memory; `count` is then an upper bound used to size the grid.
 void launchExtend(const LaunchCtx& c, const uint32_t* queue, uint32_t count, const uint32_t* countPtr, uint32_t depth);
+// The bounce past rayMaxDepth on the wide BVH: the same hit records k_accumulate needs, from the light list tl and an
+// any-hit query instead of a closest-hit traversal.  k_classify is not needed after it (it would end every path).
+void launchTerminal(const LaunchCtx& c, const uint32_t* queue, uint32_t count, const uint32_t* countPtr, const TerminalLights& tl);
 void launchClassify(const LaunchCtx& c, const uint32_t* queue, uint32_t count, const uint32_t* countPtr, uint32_t depth);
 void launchShade(const LaunchCtx& c, int kind, uint32_t count, uint32_t depth);
 // The shadow traversal and k_apply may run on their own stream, overlapping the next bounce's extend launch.
