@@ -10,6 +10,8 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "build.h"
@@ -37,24 +39,100 @@ struct StageTimer {
   }
   void begin(int stage, cudaStream_t s, uint32_t depth = 0) { spans.push_back({stage, grab(s), 0, depth}); }
   void end(cudaStream_t s) { spans.back().e1 = grab(s); }
-  // msDepth[stage == ST_SHADOW][d]: the two traversal launches per path depth (mox_stats.ms_extend_depth / ms_shadow_depth)
-  void collect(double* ms, double (*msDepth)[MOX_STATS_DEPTHS]) {
+  // Adds the spans into the per-stage times, and the two traversal launches into the per-depth times.
+  void collect(mox_stats& st) {
+    double* ms[ST_COUNT] = {&st.ms_generate, &st.ms_extend, &st.ms_shade, &st.ms_shadow, &st.ms_accumulate};
     for (auto& sp : spans) {
       float t = 0;
       if (cudaEventElapsedTime(&t, pool[sp.e0], pool[sp.e1]) != cudaSuccess) continue;
-      ms[sp.stage] += t;
-      if (sp.depth) msDepth[sp.stage == ST_SHADOW ? 1 : 0][std::min<uint32_t>(sp.depth, MOX_STATS_DEPTHS - 1)] += t;
+      *ms[sp.stage] += t;
+      if (sp.depth) {
+        double* byDepth = sp.stage == ST_SHADOW ? st.ms_shadow_depth : st.ms_extend_depth;
+        byDepth[sp.depth < MOX_STATS_DEPTHS ? sp.depth : MOX_STATS_DEPTHS - 1] += t;
+      }
     }
     spans.clear(); used = 0;
   }
-  void release() { for (auto e : pool) cudaEventDestroy(e); pool.clear(); }
+  ~StageTimer() { for (auto e : pool) cudaEventDestroy(e); }
 };
 
-struct DevBuf {
-  void* p = nullptr;
+// Device (cudaMalloc) or pinned host (cudaMallocHost) memory: move-only, freed by its owner.  An empty one makes no
+// CUDA call, so the shell of a multi-GPU handle, which never binds a device, frees nothing.
+template <class T, bool HOST>
+struct OwnedMem {
+  T* p = nullptr;
   size_t bytes = 0;
-  void release() { if (p) cudaFree(p); p = nullptr; bytes = 0; }
+  OwnedMem() = default;
+  OwnedMem(OwnedMem&& o) noexcept : p(std::exchange(o.p, nullptr)), bytes(std::exchange(o.bytes, 0)) {}
+  OwnedMem& operator=(OwnedMem&& o) noexcept {
+    if (this != &o) { release(); p = std::exchange(o.p, nullptr); bytes = std::exchange(o.bytes, 0); }
+    return *this;
+  }
+  ~OwnedMem() { release(); }
+  void release() {
+    if (p) { if (HOST) cudaFreeHost((void*)p); else cudaFree((void*)p); }
+    p = nullptr; bytes = 0;
+  }
+  // Replaces the contents by n uninitialised bytes; empty on failure.
+  cudaError_t alloc(size_t n) {
+    release();
+    void* q = nullptr;
+    const cudaError_t e = HOST ? cudaMallocHost(&q, n) : cudaMalloc(&q, n);
+    if (e == cudaSuccess) { p = (T*)q; bytes = n; }
+    return e;
+  }
 };
+using DevBuf = OwnedMem<void, false>;
+template <class T> using DevArray = OwnedMem<T, false>;
+template <class T> using PinnedBuf = OwnedMem<T, true>;
+
+// A gather buffer: allocated here, opened from another process's export over CUDA IPC, or borrowed from another
+// context of this process, which frees it.
+struct GatherBuf {
+  enum Kind { own, ipc, borrowed };
+  float* p = nullptr;
+  Kind kind = own;
+  GatherBuf() = default;
+  GatherBuf(const GatherBuf&) = delete;
+  GatherBuf& operator=(const GatherBuf&) = delete;
+  ~GatherBuf() { release(); }
+  void release() {
+    if (p && kind == ipc) cudaIpcCloseMemHandle(p);
+    else if (p && kind == own) cudaFree(p);
+    p = nullptr; kind = own;
+  }
+};
+
+constexpr size_t kCounterWords = C_WORDS + BOUNCE_RING * C_BOUNCE_WORDS;
+
+// The layout of the wavefront state in one device block at `base` (null: sizes only): rays, hit, throughput,
+// radiance, RNG state, two queue buffers, four material queues and the second Disney queue; per light a direction,
+// a contribution and a queue entry, and one shadow origin per path when there are lights; the counters and the
+// launch seeds.  Every array starts 256-byte aligned, and one of 2 MiB or more on a 2 MiB boundary, where cudaMalloc
+// puts it: packed at 256 bytes, the path arrays measured 0.15 % slower.  Returns the block's size.
+size_t pathLayout(size_t paths, size_t nLights, size_t nSeeds, char* base, PathBuffers& pb) {
+  pb = PathBuffers();
+  size_t off = 0;
+  auto take = [&](auto*& a, size_t bytes) {
+    const size_t align = bytes >= (2u << 20) ? (2u << 20) : 256;
+    off = (off + align - 1) & ~(align - 1);
+    a = base ? (std::remove_reference_t<decltype(a)>)(base + off) : nullptr;
+    off += bytes;
+  };
+  const size_t slots = paths * nLights;
+  take(pb.rayO, paths * 16); take(pb.rayD, paths * 16); take(pb.hit, paths * 8); take(pb.thr, paths * 16);
+  take(pb.rad, paths * 16); take(pb.state, paths * 4);
+  for (auto& q : pb.qBuf) take(q, paths * 4);
+  for (auto& q : pb.qMat) take(q, paths * 4);
+  take(pb.qDisneyAlt, paths * 4);
+  if (slots) { take(pb.shO, paths * 16); take(pb.shD, slots * 16); take(pb.shC, slots * 16); take(pb.shQueue, slots * 4); }
+  take(pb.counters, kCounterWords * 4);
+  take(pb.seeds, nSeeds * 4);
+  pb.capacity = paths; pb.shadowSlots = slots; pb.seedCap = nSeeds;
+  return off;
+}
+
+inline uint64_t counter64(const uint32_t* words, int lo) { return ((uint64_t)words[lo + 1] << 32) | words[lo]; }
 }  // namespace
 
 struct mox_ctx {
@@ -93,30 +171,23 @@ struct mox_ctx {
   DevBuf dQueryO, dQueryD, dQueryCounters;  // raw ray queries
   DevBuf dQueryRays, dQueryOut, dQueryC;    // ... and their host-buffer forms: grow-only staging, no allocation per call
   DevBuf dTexObjs;
-  BvhNode2* dNodes = nullptr;
-  float4* dPacked = nullptr;
-  size_t nodesCap = 0, packedCap = 0;
-  BvhNode8* dNodes8 = nullptr;
-  float4* dPacked8 = nullptr;
-  size_t nodes8Cap = 0, packed8Cap = 0;
-  int nNodes8 = 0;
+  BuildOutput accel;   // its four node and record arrays belong to the context (freed in ~mox_ctx)
   bool wideBuilt = false, useWide = true;
   DeviceArena buildArena;
-  int nNodes = 0, nValid = 0;
   bool built = false, lightsDirty = true;
   uint32_t accelFlags = 0;
-  // The last full build succeeded and no primitive was added or removed since: MOX_ACCEL_REFIT may reuse its topology.
+  // The last full build succeeded and no primitive was added or removed since: MOX_ACCEL_REFIT may reuse its topology
+  // (accel.refit).
   bool refitOk = false;
-  RefitState refit;
   // Light primitives of the terminal query (traverse_job.h), from the last full build; nTerminalLights < 0: the scene
   // has a triangle-mesh light or more than MOX_TERMINAL_LIGHTS_MAX lights, and the terminal bounce runs closest hit.
   DevBuf dTerminalLights;
   int nTerminalLights = -1;
 
   // image
-  float* dAccu = nullptr;
+  DevArray<float> dAccu;
   uint32_t accuW = 0, accuH = 0;
-  uint32_t* dOwned = nullptr;
+  DevArray<uint32_t> dOwned;
   uint32_t nOwned = 0;
   bool ownedDirty = true;
   std::vector<DevBuf> otherOwned;  // cached owned lists of other ranks (unpack)
@@ -126,24 +197,23 @@ struct mox_ctx {
   // two persistent traversal launches are in flight while the host waits for a bounce's material counts.  Splitting
   // a batch into sub-batches on further streams measured no faster (1347 vs 1350 Mrays/s at full frame, slower on an
   // eighth of it) and was removed (DESIGN.md section 4; the code is in the git history).
-  PathBuffers pb;
+  PathBuffers pb;      // views into pathBlock (pathLayout)
+  DevBuf pathBlock;
   cudaStream_t shadowStream = nullptr;  // shadow traversal + k_apply of bounce b, overlapping extend + classify of bounce b+1
   cudaEvent_t evShaded = nullptr, evApplied = nullptr;
   bool applyPending = false;       // evApplied must be waited for before the next kernel that touches rad / the shadow buffers
   cudaEvent_t evReady = nullptr;   // the counters of the bounce in flight have landed in hostCnt
-  uint32_t* hostCnt = nullptr;     // pinned: C_WORDS + BOUNCE_RING * C_BOUNCE_WORDS
+  PinnedBuf<uint32_t> hostCnt;     // kCounterWords
   StageTimer timer;
   LaunchCtx lc;
   uint32_t batchSamples = 0, bound = 0, depth = 0, matCount[Q_COUNT] = {0, 0, 0, 0};
   bool batchDone = true;
-  float* pinned = nullptr;
-  size_t pinnedBytes = 0;
+  PinnedBuf<float> pinned;   // mox_map_accum's image
 
   // Gather / asynchronous read-back: two full-size device buffers (targets of the tile pushes, possibly of other
-  // GPUs), two pinned host images, a copy stream.  gatherPeer[w]: buffer w belongs to another rank (imported).
-  float* dGather[2] = {nullptr, nullptr};
-  int gatherPeer[2] = {0, 0};   // 0 own, 1 imported over CUDA IPC, 2 borrowed from another context of this process
-  float* hostGather[2] = {nullptr, nullptr};
+  // GPUs), two pinned host images, a copy stream.
+  GatherBuf dGather[2];
+  PinnedBuf<float> hostGather[2];
   size_t gatherBytes = 0;
   cudaStream_t copyStream = nullptr;
   cudaEvent_t evPushed = nullptr, evCopied[2] = {nullptr, nullptr};
@@ -152,19 +222,32 @@ struct mox_ctx {
 
   mox_group* group = nullptr; // set on the shell handle mox_create_multi returns
 
-  // stats
-  uint64_t raysPrimary = 0, raysBounce = 0, raysShadow = 0, nonfinite = 0, launches = 0, nodeVisits = 0, primTests = 0;
-  uint64_t nodeVisitsShadow = 0, primTestsShadow = 0, raysShadowTraced = 0, shadowBlocked = 0, shadowTinted = 0;
-  uint64_t raysDepth[MOX_STATS_DEPTHS] = {}, shadowDepth[MOX_STATS_DEPTHS] = {};
-  double msDepth[2][MOX_STATS_DEPTHS] = {};   // [0] extend, [1] shadow traversal launches per path depth
-  double msRender = 0, msBuild = 0;
-  double msStage[ST_COUNT] = {0, 0, 0, 0, 0};
-  uint64_t extendLaunches = 0, kernelLaunches = 0;
-  size_t maxBatchPaths = 32u << 20;  // paths per wavefront (264 B each with 4 lights, bytesPerPath); measured 4 Mi -> 947, 32 Mi -> 980 Mrays/s at 4K
+  // The counters and timings of mox_get_stats; the scene-derived fields are filled in there.  st.launches is also
+  // mox_render's seed counter.
+  mox_stats st{};
+  size_t maxBatchPaths = 32u << 20;  // paths per wavefront (264 B each with 4 lights, pathLayout); measured 4 Mi -> 947, 32 Mi -> 980 Mrays/s at 4K
   bool overlapShadow = true;     // shadow rays of bounce b on a second stream, concurrent with the extend launch of bounce b+1 (MOX_OVERLAP_SHADOW=0: serial)
   bool brdfFast = true;          // approximate reciprocal / square root inside BRDF values (MOX_BRDF_IEEE=1: IEEE, the oracle's operations)
   bool terminalQuery = true;     // the bounce past rayMaxDepth uses the light list and an any-hit query (MOX_TERMINAL_CLOSEST=1: closest hit)
   uint32_t terminalDepth = 0;    // the batch's last bounce ran the terminal query: its ray counts come with the final counter copy
+
+  // Frees what the context holds; the device buffers go with their owners.  mox_destroy binds the device and waits
+  // for the streams first.
+  ~mox_ctx() {
+    freeTextures();
+    for (void* a : {(void*)accel.nodes, (void*)accel.packed, (void*)accel.nodes8, (void*)accel.packed8})
+      if (a) cudaFree(a);
+    buildArena.release();
+    for (cudaEvent_t e : {ev0, ev1, evShaded, evApplied, evReady, evPushed, evCopied[0], evCopied[1]})
+      if (e) cudaEventDestroy(e);
+    for (cudaStream_t s : {stream, shadowStream, copyStream})
+      if (s) cudaStreamDestroy(s);
+  }
+  void freeTextures() {
+    for (auto t : texObjects) cudaDestroyTextureObject(t);
+    for (auto a : texArrays) cudaFreeArray(a);
+    texObjects.clear(); texArrays.clear();
+  }
 };
 
 namespace {
@@ -186,11 +269,11 @@ int bind(mox_ctx* c) {
   return MOX_OK;
 }
 
-int ensure(mox_ctx* c, DevBuf& b, size_t bytes) {
+// Grow-only: keeps b when it holds `bytes` already.
+template <class T, bool HOST>
+int ensure(mox_ctx* c, OwnedMem<T, HOST>& b, size_t bytes) {
   if (b.bytes >= bytes && b.p) return MOX_OK;
-  b.release();
-  CUCK(c, cudaMalloc(&b.p, std::max<size_t>(bytes, 16)));
-  b.bytes = std::max<size_t>(bytes, 16);
+  CUCK(c, b.alloc(std::max<size_t>(bytes, 16)));
   return MOX_OK;
 }
 
@@ -233,77 +316,41 @@ int refreshOwned(mox_ctx* c) {
   if (!c->ownedDirty) return MOX_OK;
   std::vector<uint32_t> l;
   ownedList(c->rp.W, c->rp.H, c->tile, c->world, c->rank, l);
-  if (c->dOwned) cudaFree(c->dOwned);
-  c->dOwned = nullptr;
-  CUCK(c, cudaMalloc(&c->dOwned, std::max<size_t>(l.size(), 1) * 4));
+  int rc = ensure(c, c->dOwned, l.size() * 4);
+  if (rc) return rc;
   // Stream-ordered upload: a plain cudaMemcpy from pageable memory may return before the DMA has landed, and
   // the context stream is non-blocking, so a kernel launched next could still read stale bytes.
-  if (!l.empty()) { CUCK(c, cudaMemcpyAsync(c->dOwned, l.data(), l.size() * 4, cudaMemcpyHostToDevice, c->stream)); CUCK(c, cudaStreamSynchronize(c->stream)); }
+  if (!l.empty()) { CUCK(c, cudaMemcpyAsync(c->dOwned.p, l.data(), l.size() * 4, cudaMemcpyHostToDevice, c->stream)); CUCK(c, cudaStreamSynchronize(c->stream)); }
   c->nOwned = (uint32_t)l.size();
-  for (auto& b : c->otherOwned) b.release();
   c->otherOwned.clear();
   c->ownedCount.clear();
   c->ownedDirty = false;
   return MOX_OK;
 }
 
-void freePaths(PathBuffers& pb) {
-  cudaFree(pb.rayO); cudaFree(pb.rayD); cudaFree(pb.hit); cudaFree(pb.thr); cudaFree(pb.rad); cudaFree(pb.state);
-  for (auto& q : pb.qBuf) cudaFree(q);
-  for (auto& q : pb.qMat) cudaFree(q);
-  cudaFree(pb.shO); cudaFree(pb.shD); cudaFree(pb.shC); cudaFree(pb.shQueue); cudaFree(pb.counters); cudaFree(pb.seeds); cudaFree(pb.qDisneyAlt);
+// The wavefront state of `paths` paths, nLights shadow slots per path and nSeeds launch seeds in c->pathBlock.
+int ensurePaths(mox_ctx* c, size_t paths, size_t nLights, size_t nSeeds) {
+  PathBuffers& pb = c->pb;
+  if (c->pathBlock.p && pb.capacity >= paths && pb.shadowSlots >= paths * nLights && pb.seedCap >= nSeeds) return MOX_OK;
+  cudaStreamSynchronize(c->stream);
+  // grow geometrically so that a slowly growing sample count does not reallocate on every call
+  if (pb.capacity && paths > pb.capacity) paths = std::max(paths, pb.capacity + pb.capacity / 2);
+  nSeeds = std::max(nSeeds, pb.seedCap);
+  c->pathBlock.release();
   pb = PathBuffers();
-}
-
-constexpr size_t kCounterWords = C_WORDS + BOUNCE_RING * C_BOUNCE_WORDS;
-
-// Bytes of wavefront state per path (see PathBuffers): rays, hit, throughput, radiance, RNG state, two queue
-// buffers, four material queues and the second Disney queue; per light a direction, a contribution and a queue
-// entry; one shadow origin when there are lights.
-size_t bytesPerPath(size_t nLights) { return 16 * 4 + 8 + 4 + 2 * 4 + 5 * 4 + (nLights ? 16 + nLights * 36 : 0); }
-
-int ensurePaths(mox_ctx* c, PathBuffers& pb, cudaStream_t stream, size_t paths, size_t nLights, size_t nSeeds) {
-  size_t slots = paths * nLights;
-  if (pb.capacity < paths || pb.shadowSlots < slots || !pb.counters) {
-    cudaStreamSynchronize(stream);
-    // grow geometrically so that a slowly growing sample count does not reallocate on every call
-    if (pb.capacity && paths > pb.capacity) paths = std::max(paths, pb.capacity + pb.capacity / 2);
-    slots = paths * nLights;
-    size_t seedCap = pb.seedCap;
-    int32_t* seeds = pb.seeds;
-    pb.seeds = nullptr;
-    freePaths(pb);
-    pb.seeds = seeds; pb.seedCap = seedCap;
-    CUCK(c, cudaMalloc(&pb.rayO, paths * 16)); CUCK(c, cudaMalloc(&pb.rayD, paths * 16));
-    CUCK(c, cudaMalloc(&pb.hit, paths * 8)); CUCK(c, cudaMalloc(&pb.thr, paths * 16));
-    CUCK(c, cudaMalloc(&pb.rad, paths * 16)); CUCK(c, cudaMalloc(&pb.state, paths * 4));
-    for (auto& q : pb.qBuf) CUCK(c, cudaMalloc(&q, paths * 4));
-    for (auto& q : pb.qMat) CUCK(c, cudaMalloc(&q, paths * 4));
-    CUCK(c, cudaMalloc(&pb.qDisneyAlt, paths * 4));
-    if (slots) {
-      CUCK(c, cudaMalloc(&pb.shO, paths * 16)); CUCK(c, cudaMalloc(&pb.shD, slots * 16)); CUCK(c, cudaMalloc(&pb.shC, slots * 16));
-      CUCK(c, cudaMalloc(&pb.shQueue, slots * 4));
-    }
-    CUCK(c, cudaMalloc(&pb.counters, kCounterWords * 4));
-    CUCK(c, cudaMemset(pb.counters, 0, kCounterWords * 4));
-    pb.capacity = paths; pb.shadowSlots = slots;
-  }
-  if (pb.seedCap < nSeeds) {
-    cudaStreamSynchronize(stream);
-    cudaFree(pb.seeds);
-    pb.seeds = nullptr;
-    CUCK(c, cudaMalloc(&pb.seeds, nSeeds * 4));
-    pb.seedCap = nSeeds;
-  }
+  const size_t bytes = pathLayout(paths, nLights, nSeeds, nullptr, pb);
+  CUCK(c, c->pathBlock.alloc(bytes));
+  pathLayout(paths, nLights, nSeeds, (char*)c->pathBlock.p, pb);
+  CUCK(c, cudaMemsetAsync(pb.counters, 0, kCounterWords * 4, c->stream));
   return MOX_OK;
 }
 
 SceneView sceneView(const mox_ctx* c) {
   SceneView s;
-  s.nodes = c->dNodes;
-  s.packed = c->dPacked;
-  s.nodes8 = (c->wideBuilt && c->useWide) ? c->dNodes8 : nullptr;
-  s.packed8 = c->dPacked8;
+  s.nodes = c->accel.nodes;
+  s.packed = c->accel.packed;
+  s.nodes8 = (c->wideBuilt && c->useWide) ? c->accel.nodes8 : nullptr;
+  s.packed8 = c->accel.packed8;
   s.analytic = (const Analytic*)c->dAnalytic.p;
   s.prims = (const PrimDesc*)c->dPrims.p;
   s.mats = (const GpuMaterial*)c->dMats.p;
@@ -317,15 +364,9 @@ SceneView sceneView(const mox_ctx* c) {
   s.textures = (const cudaTextureObject_t*)c->dTexObjs.p;
   s.nLights = (int)c->lights.size();
   s.nPrims = (int)c->prims.size();
-  s.nNodes8 = (uint32_t)c->nNodes8;
+  s.nNodes8 = (uint32_t)c->accel.nNodes8;
   s.watertight = (c->accelFlags & MOX_ACCEL_WATERTIGHT) ? 1 : 0;
   return s;
-}
-
-void freeTextures(mox_ctx* c) {
-  for (auto t : c->texObjects) cudaDestroyTextureObject(t);
-  for (auto a : c->texArrays) cudaFreeArray(a);
-  c->texObjects.clear(); c->texArrays.clear();
 }
 
 // createTextureSampler: REPEAT wrap, LINEAR filter, normalized coordinates, float4 texels
@@ -333,13 +374,13 @@ void freeTextures(mox_ctx* c) {
 int syncTextures(mox_ctx* c) {
   if (!c->texturesDirty) return MOX_OK;
   cudaStreamSynchronize(c->stream);
-  freeTextures(c);
+  c->freeTextures();
   for (auto& t : c->textures) {
     cudaChannelFormatDesc fmt = cudaCreateChannelDesc<float4>();
     cudaArray_t arr = nullptr;
     CUCK(c, cudaMallocArray(&arr, &fmt, t.w, t.h));
     c->texArrays.push_back(arr);
-    CUCK(c, cudaMemcpy2DToArray(arr, 0, 0, t.texels.data(), (size_t)t.w * 16, (size_t)t.w * 16, t.h, cudaMemcpyHostToDevice));
+    CUCK(c, cudaMemcpy2DToArrayAsync(arr, 0, 0, t.texels.data(), (size_t)t.w * 16, (size_t)t.w * 16, t.h, cudaMemcpyHostToDevice, c->stream));
     cudaResourceDesc res;
     memset(&res, 0, sizeof res);
     res.resType = cudaResourceTypeArray;
@@ -401,7 +442,7 @@ int enqueueExtend(mox_ctx* c) {
     tm.begin(ST_EXTEND, c->stream, depth);
     launchTerminal(lc, depth == 1 ? nullptr : lc.pb.qCur, c->bound, countPtr, tl);
     tm.end(c->stream);
-    c->extendLaunches++; c->kernelLaunches++;
+    c->st.extend_launches++; c->st.kernel_launches++;
     // k_classify would queue nothing: no counts to wait for, the accumulation follows at once
     c->terminalDepth = depth;
     return finishBatch(c);
@@ -413,8 +454,8 @@ int enqueueExtend(mox_ctx* c) {
   tm.begin(ST_SHADE, c->stream);
   launchClassify(lc, lc.pb.qCur, c->bound, countPtr, depth);
   tm.end(c->stream);
-  c->extendLaunches++; c->kernelLaunches += 2;
-  CUCK(c, cudaMemcpyAsync(c->hostCnt, c->pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, c->stream));
+  c->st.extend_launches++; c->st.kernel_launches += 2;
+  CUCK(c, cudaMemcpyAsync(c->hostCnt.p, c->pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, c->stream));
   CUCK(c, cudaEventRecord(c->evReady, c->stream));
   return MOX_OK;
 }
@@ -425,8 +466,8 @@ int finishBatch(mox_ctx* c) {
   tm.begin(ST_ACCUMULATE, c->stream);
   launchAccumulate(c->lc, c->batchSamples);
   tm.end(c->stream);
-  c->kernelLaunches++;
-  CUCK(c, cudaMemcpyAsync(c->hostCnt, c->pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, c->stream));
+  c->st.kernel_launches++;
+  CUCK(c, cudaMemcpyAsync(c->hostCnt.p, c->pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, c->stream));
   CUCK(c, cudaEventRecord(c->evReady, c->stream));
   c->batchDone = true;
   return MOX_OK;
@@ -435,14 +476,15 @@ int finishBatch(mox_ctx* c) {
 // Exact number of rays bounce `depth` traced, and of shadow rays the bounce before it queued, from the counters in
 // hostCnt.
 void countBounceRays(mox_ctx* c, uint32_t depth) {
+  mox_stats& st = c->st;
   const uint32_t dIdx = std::min<uint32_t>(depth, MOX_STATS_DEPTHS - 1);
-  if (depth == 1) { c->raysPrimary += c->bound; c->raysDepth[1] += c->bound; }
+  if (depth == 1) { st.rays_primary += c->bound; st.rays_depth[1] += c->bound; }
   else {
-    const uint32_t* prev = c->hostCnt + C_WORDS + ((depth - 1) % BOUNCE_RING) * C_BOUNCE_WORDS;
-    c->raysBounce += prev[C_NEXT];
-    c->raysShadowTraced += prev[C_SHQ];
-    c->raysDepth[dIdx] += prev[C_NEXT];
-    c->shadowDepth[std::min<uint32_t>(depth - 1, MOX_STATS_DEPTHS - 1)] += prev[C_SHQ];
+    const uint32_t* prev = c->hostCnt.p + C_WORDS + ((depth - 1) % BOUNCE_RING) * C_BOUNCE_WORDS;
+    st.rays_bounce += prev[C_NEXT];
+    st.rays_shadow_traced += prev[C_SHQ];
+    st.rays_depth[dIdx] += prev[C_NEXT];
+    st.shadow_traced_depth[std::min<uint32_t>(depth - 1, MOX_STATS_DEPTHS - 1)] += prev[C_SHQ];
   }
 }
 
@@ -453,7 +495,7 @@ int advanceBounce(mox_ctx* c) {
   StageTimer& tm = c->timer;
   PathBuffers& pb = c->pb;
   const uint32_t depth = c->depth;
-  const uint32_t* hostBounce = c->hostCnt + C_WORDS + (depth % BOUNCE_RING) * C_BOUNCE_WORDS;
+  const uint32_t* hostBounce = c->hostCnt.p + C_WORDS + (depth % BOUNCE_RING) * C_BOUNCE_WORDS;
   countBounceRays(c, depth);
   uint32_t any = 0;
   for (int k = 0; k < Q_COUNT; ++k) { c->matCount[k] = hostBounce[C_MAT0 + k]; any += c->matCount[k]; }
@@ -461,7 +503,7 @@ int advanceBounce(mox_ctx* c) {
   // the shade kernels touch the radiance and rewrite the shadow-ray buffers: the previous bounce's k_apply first
   if (c->applyPending) { CUCK(c, cudaStreamWaitEvent(c->stream, c->evApplied, 0)); c->applyPending = false; }
   tm.begin(ST_SHADE, c->stream);
-  for (int k = 0; k < Q_COUNT; ++k) { launchShade(lc, k, c->matCount[k], depth); if (c->matCount[k]) c->kernelLaunches++; }
+  for (int k = 0; k < Q_COUNT; ++k) { launchShade(lc, k, c->matCount[k], depth); if (c->matCount[k]) c->st.kernel_launches++; }
   tm.end(c->stream);
   if (c->matCount[Q_DISNEY] && lc.scene.nLights) {
     // Shadow rays and the NEE sum depend only on this bounce's shade kernels; the next extend launch does not
@@ -480,7 +522,7 @@ int advanceBounce(mox_ctx* c) {
     launchApply(lc, c->matCount[Q_DISNEY], ss);
     tm.end(ss);
     if (ss != c->stream) { CUCK(c, cudaEventRecord(c->evApplied, ss)); c->applyPending = true; }
-    c->kernelLaunches += 2;
+    c->st.kernel_launches += 2;
   }
   // the block bounce depth+1 will use was last written BOUNCE_RING bounces ago
   CUCK(c, cudaMemsetAsync(bounceBlock(pb, depth + 1), 0, C_BOUNCE_WORDS * 4, c->stream));
@@ -499,8 +541,8 @@ int prepareBatch(mox_ctx* c, uint32_t S) {
     CUCK(c, cudaEventCreateWithFlags(&c->evShaded, cudaEventDisableTiming));
     CUCK(c, cudaEventCreateWithFlags(&c->evApplied, cudaEventDisableTiming));
   }
-  if (!c->hostCnt) CUCK(c, cudaMallocHost(&c->hostCnt, kCounterWords * 4));
-  return ensurePaths(c, c->pb, c->stream, (size_t)S * c->nOwned, c->lights.size(), S);
+  int rc = ensure(c, c->hostCnt, kCounterWords * 4);
+  return rc ? rc : ensurePaths(c, (size_t)S * c->nOwned, c->lights.size(), S);
 }
 
 // One wavefront batch: `seeds.size()` samples of every owned pixel.  Generate, then advance bounce by bounce until
@@ -520,9 +562,9 @@ int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds) {
   lc.scene = sceneView(c);
   lc.rp = c->rp;
   lc.pb = pb;
-  lc.ownedPix = c->dOwned;
+  lc.ownedPix = c->dOwned.p;
   lc.nOwned = c->nOwned;
-  lc.accu = c->dAccu;
+  lc.accu = c->dAccu.p;
   lc.countTraversal = (c->accelFlags & MOX_ACCEL_COUNTERS) != 0;
   lc.brdfFast = c->brdfFast;
   lc.stream = c->stream;
@@ -533,7 +575,7 @@ int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds) {
   c->timer.begin(ST_GENERATE, c->stream);
   launchGenerate(lc, S);
   c->timer.end(c->stream);
-  c->kernelLaunches++;
+  c->st.kernel_launches++;
   if ((rc = enqueueExtend(c))) return rc;
   while (!c->batchDone) {
     CUCK(c, cudaEventSynchronize(c->evReady));
@@ -541,23 +583,24 @@ int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds) {
   }
   // the accumulation and the final counter read-back
   CUCK(c, cudaEventSynchronize(c->evReady));
-  const uint32_t* host = c->hostCnt;
+  const uint32_t* host = c->hostCnt.p;
+  mox_stats& st = c->st;
   if (c->terminalDepth) countBounceRays(c, c->terminalDepth);
-  c->timer.collect(c->msStage, c->msDepth);
-  c->nonfinite += host[C_NONFINITE];
-  c->shadowBlocked += host[C_SH_BLOCKED]; c->shadowTinted += host[C_SH_TINTED];
-  c->raysShadow += host[C_SHADOW];
-  c->nodeVisits += ((uint64_t)host[C_NODEVIS_HI] << 32) | host[C_NODEVIS_LO];
-  c->primTests += ((uint64_t)host[C_PRIMTEST_HI] << 32) | host[C_PRIMTEST_LO];
-  c->nodeVisitsShadow += ((uint64_t)host[C_NODEVIS_SH_LO + 1] << 32) | host[C_NODEVIS_SH_LO];
-  c->primTestsShadow += ((uint64_t)host[C_PRIMTEST_SH_LO + 1] << 32) | host[C_PRIMTEST_SH_LO];
+  c->timer.collect(st);
+  st.nonfinite_samples += host[C_NONFINITE];
+  st.rays_shadow_blocked += host[C_SH_BLOCKED]; st.rays_shadow_tinted += host[C_SH_TINTED];
+  st.rays_shadow += host[C_SHADOW];
+  st.node_visits += counter64(host, C_NODEVIS_LO);
+  st.prim_tests += counter64(host, C_PRIMTEST_LO);
+  st.node_visits_shadow += counter64(host, C_NODEVIS_SH_LO);
+  st.prim_tests_shadow += counter64(host, C_PRIMTEST_SH_LO);
   CUCK(c, cudaGetLastError());
-  c->launches += S;
+  st.launches += S;
   return MOX_OK;
 }
 
 // Paths per batch: the configured cap, lowered so that the wavefront state fits into 60 % of the free device
-// memory for this scene's light count (36 bytes per path and light).
+// memory (what the current block holds counts as free) for this scene's light count (36 bytes per path and light).
 size_t batchCap(mox_ctx* c, size_t wanted /* samples per pixel of this call */) {
   size_t cap = c->maxBatchPaths;
   const PathBuffers& pb = c->pb;
@@ -566,13 +609,15 @@ size_t batchCap(mox_ctx* c, size_t wanted /* samples per pixel of this call */) 
   if (c->nOwned) {
     const size_t S = std::min(std::max<size_t>(1, cap / c->nOwned), wanted), nL = c->lights.size();   // samples per batch at the full cap
     const size_t P = S * c->nOwned;
-    if (pb.counters && pb.capacity >= P && pb.shadowSlots >= P * nL && pb.seedCap >= S) return cap;
+    if (c->pathBlock.p && pb.capacity >= P && pb.shadowSlots >= P * nL && pb.seedCap >= S) return cap;
   }
   size_t freeB = 0, totalB = 0;
   if (cudaMemGetInfo(&freeB, &totalB) == cudaSuccess) {
-    const size_t have = pb.capacity * bytesPerPath(pb.capacity ? pb.shadowSlots / pb.capacity : 0);
-    size_t budget = (size_t)((freeB + have) * 0.6);
-    cap = std::min(cap, std::max<size_t>(budget / bytesPerPath(c->lights.size()), 65536));
+    // bytes per path: at 2^20 paths every array is a multiple of 2 MiB, and the counters add less than a byte
+    PathBuffers probe;
+    const size_t perPath = pathLayout(1u << 20, c->lights.size(), 0, nullptr, probe) >> 20;
+    size_t budget = (size_t)((freeB + c->pathBlock.bytes) * 0.6);
+    cap = std::min(cap, std::max<size_t>(budget / perPath, 65536));
   }
   return cap;
 }
@@ -586,7 +631,7 @@ int renderSeeds(mox_ctx* c, const std::vector<int32_t>& seeds) {
   if ((rc = refreshOwned(c))) return rc;
   if ((rc = syncLights(c))) return rc;
   if ((rc = syncTextures(c))) return rc;
-  if (c->nOwned == 0) { c->launches += seeds.size(); return MOX_OK; }
+  if (c->nOwned == 0) { c->st.launches += seeds.size(); return MOX_OK; }
   size_t perBatch = std::max<size_t>(1, batchCap(c, seeds.size()) / c->nOwned);
   rc = prepareBatch(c, (uint32_t)std::min(perBatch, seeds.size()));
   if (rc && rc != MOX_ERR_OOM) return rc;   // out of memory: the loop below retries with smaller batches
@@ -599,7 +644,8 @@ int renderSeeds(mox_ctx* c, const std::vector<int32_t>& seeds) {
       // the allocation failed after all (fragmentation, another context on the device): free the wavefront
       // state, halve the batch and render this chunk again (nothing of it was enqueued)
       cudaGetLastError();
-      { int32_t* sd = c->pb.seeds; c->pb.seeds = nullptr; freePaths(c->pb); cudaFree(sd); }
+      c->pathBlock.release();
+      c->pb = PathBuffers();
       perBatch = std::max<size_t>(1, perBatch / 2);
       continue;
     }
@@ -610,27 +656,23 @@ int renderSeeds(mox_ctx* c, const std::vector<int32_t>& seeds) {
   CUCK(c, cudaEventSynchronize(c->ev1));
   float ms = 0;
   CUCK(c, cudaEventElapsedTime(&ms, c->ev0, c->ev1));
-  c->msRender += ms;
+  c->st.ms_render += ms;
   return MOX_OK;
 }
 
 void freeGather(mox_ctx* c) {
-  for (int w = 0; w < 2; ++w) {
-    if (c->dGather[w]) { if (c->gatherPeer[w] == 1) cudaIpcCloseMemHandle(c->dGather[w]); else if (!c->gatherPeer[w]) cudaFree(c->dGather[w]); }
-    if (c->hostGather[w]) cudaFreeHost(c->hostGather[w]);
-    c->dGather[w] = nullptr; c->hostGather[w] = nullptr; c->gatherPeer[w] = 0;
-  }
+  for (int w = 0; w < 2; ++w) { c->dGather[w].release(); c->hostGather[w].release(); }
   c->gatherBytes = 0; c->readPending = -1;
 }
 
 // The two gather buffers of this context (allocated on first use, re-allocated when the image size changes).
 int ensureGather(mox_ctx* c, bool hostSide) {
-  if (!c->dAccu) return fail(c, MOX_ERR_STATE, "no accumulation buffer (mox_set_globals first)");
+  if (!c->dAccu.p) return fail(c, MOX_ERR_STATE, "no accumulation buffer (mox_set_globals first)");
   const size_t bytes = (size_t)c->accuW * c->accuH * 12;
   if (c->gatherBytes != bytes) {
     cudaStreamSynchronize(c->stream);
     if (c->copyStream) cudaStreamSynchronize(c->copyStream);
-    bool peer = c->gatherPeer[0] || c->gatherPeer[1];
+    bool peer = c->dGather[0].kind != GatherBuf::own || c->dGather[1].kind != GatherBuf::own;
     if (peer && c->gatherBytes) return fail(c, MOX_ERR_STATE, "image size changed after mox_gather_import");
     if (!peer) freeGather(c);
     c->gatherBytes = bytes;
@@ -639,18 +681,10 @@ int ensureGather(mox_ctx* c, bool hostSide) {
   if (!c->evPushed) CUCK(c, cudaEventCreateWithFlags(&c->evPushed, cudaEventDisableTiming));
   for (int w = 0; w < 2; ++w) {
     if (!c->evCopied[w]) CUCK(c, cudaEventCreateWithFlags(&c->evCopied[w], cudaEventDisableTiming));
-    if (!c->dGather[w]) { CUCK(c, cudaMalloc(&c->dGather[w], bytes)); CUCK(c, cudaMemsetAsync(c->dGather[w], 0, bytes, c->stream)); }
-    if (hostSide && !c->hostGather[w]) CUCK(c, cudaMallocHost(&c->hostGather[w], bytes));
+    GatherBuf& g = c->dGather[w];
+    if (!g.p) { CUCK(c, cudaMalloc(&g.p, bytes)); CUCK(c, cudaMemsetAsync(g.p, 0, bytes, c->stream)); }
+    if (hostSide && !c->hostGather[w].p) CUCK(c, c->hostGather[w].alloc(bytes));
   }
-  return MOX_OK;
-}
-
-int ensurePinned(mox_ctx* c, size_t bytes) {
-  if (c->pinnedBytes >= bytes) return MOX_OK;
-  if (c->pinned) cudaFreeHost(c->pinned);
-  c->pinned = nullptr; c->pinnedBytes = 0;
-  CUCK(c, cudaMallocHost(&c->pinned, bytes));
-  c->pinnedBytes = bytes;
   return MOX_OK;
 }
 
@@ -710,7 +744,7 @@ int refitAccel(mox_ctx* c, uint32_t flags, float* out_ms) {
     return fail(c, MOX_ERR_STATE, "MOX_ACCEL_REFIT needs a successful full build with no mox_add_* / mox_clear_scene after it");
   if (const char* env = getenv("MOX_WATERTIGHT")) { if (atoi(env)) flags |= MOX_ACCEL_WATERTIGHT; }
   if (flags != c->accelFlags) return fail(c, MOX_ERR_INVALID, "MOX_ACCEL_REFIT: the other flags differ from those of the last full build");
-  if (c->refit.path == RefitState::TRIVIAL) return kRebuild;
+  if (c->accel.refit.path == RefitState::TRIVIAL) return kRebuild;
   // A failed refit must not leave a context that still claims to be built, nor one that offers a refit again.
   c->built = false;
   c->refitOk = false;
@@ -726,18 +760,15 @@ int refitAccel(mox_ctx* c, uint32_t flags, float* out_ms) {
   if (rc) return rc;
   if (c->shadeRecBuilt) buildShadeRecords(c);   // ahead of the timed kernels, as in the full build
   BuildInput in = buildInput(c, flags);
-  BuildOutput out;
-  out.nodes = c->dNodes; out.packed = c->dPacked; out.nodes8 = c->dNodes8; out.packed8 = c->dPacked8;
-  out.refit = c->refit;
   std::string err;
   bool changed = false;
-  if (!refitBvh(in, out, c->stream, err, &changed)) return fail(c, MOX_ERR_CUDA, "build_accel (refit): " + err);
+  if (!refitBvh(in, c->accel, c->stream, err, &changed)) return fail(c, MOX_ERR_CUDA, "build_accel (refit): " + err);
   if (changed)
     return fail(c, MOX_ERR_STATE, "MOX_ACCEL_REFIT: a primitive became degenerate, or valid again, since the last full build; "
                                   "build without MOX_ACCEL_REFIT");
   float ms = 0;
   CUCK(c, cudaEventElapsedTime(&ms, c->ev0, c->ev1));
-  c->msBuild = ms;
+  c->st.ms_build = ms;
   c->built = true;
   c->refitOk = true;
   if (out_ms) *out_ms = ms;
@@ -833,29 +864,8 @@ void mox_destroy(mox_ctx* c) {
   if (!c) return;
   if (c->group) { groupDestroy(c->group); delete c; return; }
   cudaSetDevice(c->device);
-  if (c->stream) cudaStreamSynchronize(c->stream);
-  for (DevBuf* b : {&c->dPrims, &c->dTris, &c->dVerts, &c->dNormals, &c->dUvs, &c->dAnalytic, &c->dMats, &c->dLights, &c->dLightN, &c->dShadeRec, &c->dTerminalLights, &c->dQueryRays, &c->dQueryOut, &c->dQueryC, &c->dQueryO,
-                   &c->dQueryD, &c->dQueryCounters}) b->release();
-  for (auto& b : c->otherOwned) b.release();
-  freeTextures(c);
-  c->dTexObjs.release();
-  c->buildArena.release();
-  cudaFree(c->dNodes); cudaFree(c->dPacked); cudaFree(c->dNodes8); cudaFree(c->dPacked8); cudaFree(c->dAccu); cudaFree(c->dOwned);
-  if (c->shadowStream) { cudaStreamSynchronize(c->shadowStream); cudaStreamDestroy(c->shadowStream); }
-  if (c->evShaded) cudaEventDestroy(c->evShaded);
-  if (c->evApplied) cudaEventDestroy(c->evApplied);
-  freePaths(c->pb);
-  c->timer.release();
-  if (c->evReady) cudaEventDestroy(c->evReady);
-  if (c->hostCnt) cudaFreeHost(c->hostCnt);
-  if (c->pinned) cudaFreeHost(c->pinned);
-  freeGather(c);
-  if (c->copyStream) cudaStreamDestroy(c->copyStream);
-  if (c->evPushed) cudaEventDestroy(c->evPushed);
-  for (auto e : c->evCopied) if (e) cudaEventDestroy(e);
-  if (c->ev0) cudaEventDestroy(c->ev0);
-  if (c->ev1) cudaEventDestroy(c->ev1);
-  if (c->stream) cudaStreamDestroy(c->stream);
+  for (cudaStream_t s : {c->stream, c->shadowStream, c->copyStream})
+    if (s) cudaStreamSynchronize(s);
   delete c;
 }
 
@@ -867,14 +877,12 @@ int mox_set_globals(mox_ctx* c, uint32_t width, uint32_t height, uint32_t rayMax
   if ((uint64_t)width * height > 0x7fffffffull / 3) return fail(c, MOX_ERR_INVALID, "image too large");
   int rc = bind(c);
   if (rc) return rc;
-  if (width != c->accuW || height != c->accuH || !c->dAccu) {
+  if (width != c->accuW || height != c->accuH || !c->dAccu.p) {
     cudaStreamSynchronize(c->stream);
-    cudaFree(c->dAccu);
-    c->dAccu = nullptr;
-    CUCK(c, cudaMalloc(&c->dAccu, (size_t)width * height * 12));
-    CUCK(c, cudaMemset(c->dAccu, 0, (size_t)width * height * 12));
+    CUCK(c, c->dAccu.alloc((size_t)width * height * 12));
+    CUCK(c, cudaMemsetAsync(c->dAccu.p, 0, (size_t)width * height * 12, c->stream));
     c->accuW = width; c->accuH = height;
-    c->launches = 0;
+    c->st.launches = 0;
     c->ownedDirty = true;
   }
   c->rp.W = width; c->rp.H = height; c->rp.maxDepth = rayMaxDepth; c->rp.eps = rayEpsilonT; c->rp.minIntensity = rayMinIntensity;
@@ -1069,29 +1077,21 @@ int mox_build_accel(mox_ctx* c, uint32_t flags, float* out_ms) {
   c->useWide = (flags & MOX_ACCEL_BINARY) == 0;
   if (const char* env = getenv("MOX_FORCE_BINARY")) { if (atoi(env)) c->useWide = false; }
   in.useWide = c->useWide;
-  BuildOutput out;
-  out.nodes = c->dNodes; out.packed = c->dPacked; out.nodesCap = c->nodesCap; out.packedCap = c->packedCap;
-  out.nodes8 = c->dNodes8; out.packed8 = c->dPacked8; out.nodes8Cap = c->nodes8Cap; out.packed8Cap = c->packed8Cap;
   std::string err;
-  bool okBuild = buildBvh(in, out, c->stream, err);
-  c->dNodes = out.nodes; c->dPacked = out.packed; c->nodesCap = out.nodesCap; c->packedCap = out.packedCap;
-  c->dNodes8 = out.nodes8; c->dPacked8 = out.packed8; c->nodes8Cap = out.nodes8Cap; c->packed8Cap = out.packed8Cap;
-  c->nNodes8 = out.nNodes8; c->wideBuilt = okBuild && out.nNodes8 > 0;
-  if (!okBuild) return fail(c, MOX_ERR_CUDA, "build_accel: " + err);
+  if (!buildBvh(in, c->accel, c->stream, err)) return fail(c, MOX_ERR_CUDA, "build_accel: " + err);
+  c->wideBuilt = c->accel.nNodes8 > 0;
   CUCK(c, cudaEventSynchronize(c->ev1));
   float ms = 0;
   CUCK(c, cudaEventElapsedTime(&ms, c->ev0, c->ev1));
-  c->dNodes = out.nodes; c->dPacked = out.packed; c->nNodes = out.nNodes; c->nValid = out.nValid;
-  c->msBuild = ms;
+  c->st.ms_build = ms;
   c->accelFlags = flags;
   c->built = true;
-  c->refit = out.refit;
   c->refitOk = true;
   {
     std::vector<uint4> tl;
     if (terminalLightList(c, tl)) {
       if ((rc = upload(c, c->dTerminalLights, tl))) return rc;
-      excludeUnbuiltLights((uint4*)c->dTerminalLights.p, (int)tl.size(), c->refit, c->stream);
+      excludeUnbuiltLights((uint4*)c->dTerminalLights.p, (int)tl.size(), c->accel.refit, c->stream);
       CUCK(c, cudaGetLastError());
       c->nTerminalLights = (int)tl.size();
     }
@@ -1110,35 +1110,8 @@ int mox_render(mox_ctx* c, uint32_t spp, uint32_t seed) {
   if (!c) return MOX_ERR_INVALID;
   GROUP_PAR(c, mox_render(k, spp, seed));
   std::vector<int32_t> seeds(spp);
-  for (uint32_t i = 0; i < spp; ++i) seeds[i] = (int32_t)tea16((uint32_t)(c->launches + i), seed);
+  for (uint32_t i = 0; i < spp; ++i) seeds[i] = (int32_t)tea16((uint32_t)(c->st.launches + i), seed);
   return renderSeeds(c, seeds);
-}
-
-int mox_read_accum(mox_ctx* c, float* dst) {
-  if (!c) return MOX_ERR_INVALID;
-  if (c->group) {
-    const float* p = nullptr;
-    int rc_ = mox_read_accum_begin(c);
-    if (!rc_) rc_ = mox_read_accum_end(c, &p);
-    if (rc_) return rc_;
-    if (!dst) return fail(c, MOX_ERR_INVALID, "null destination");
-    mox_stats st;
-    uint64_t w = 0, h = 0;
-    (void)st;
-    mox_ctx* k0 = groupChild(c->group, 0);
-    w = k0->accuW; h = k0->accuH;
-    memcpy(dst, p, (size_t)w * h * 12);
-    return MOX_OK;
-  }
-  if (!dst || !c->dAccu) return fail(c, MOX_ERR_INVALID, "no accumulation buffer");
-  int rc = bind(c);
-  if (rc) return rc;
-  size_t bytes = (size_t)c->accuW * c->accuH * 12;
-  if ((rc = ensurePinned(c, bytes))) return rc;
-  CUCK(c, cudaMemcpyAsync(c->pinned, c->dAccu, bytes, cudaMemcpyDeviceToHost, c->stream));
-  CUCK(c, cudaStreamSynchronize(c->stream));
-  memcpy(dst, c->pinned, bytes);
-  return MOX_OK;
 }
 
 int mox_map_accum(mox_ctx* c, const float** out) {
@@ -1147,14 +1120,25 @@ int mox_map_accum(mox_ctx* c, const float** out) {
     int rc_ = mox_read_accum_begin(c);
     return rc_ ? rc_ : mox_read_accum_end(c, out);
   }
-  if (!out || !c->dAccu) return fail(c, MOX_ERR_INVALID, "no accumulation buffer");
+  if (!out || !c->dAccu.p) return fail(c, MOX_ERR_INVALID, "no accumulation buffer");
   int rc = bind(c);
   if (rc) return rc;
   size_t bytes = (size_t)c->accuW * c->accuH * 12;
-  if ((rc = ensurePinned(c, bytes))) return rc;
-  CUCK(c, cudaMemcpyAsync(c->pinned, c->dAccu, bytes, cudaMemcpyDeviceToHost, c->stream));
+  if ((rc = ensure(c, c->pinned, bytes))) return rc;
+  CUCK(c, cudaMemcpyAsync(c->pinned.p, c->dAccu.p, bytes, cudaMemcpyDeviceToHost, c->stream));
   CUCK(c, cudaStreamSynchronize(c->stream));
-  *out = c->pinned;
+  *out = c->pinned.p;
+  return MOX_OK;
+}
+
+int mox_read_accum(mox_ctx* c, float* dst) {
+  if (!c) return MOX_ERR_INVALID;
+  if (!dst) return fail(c, MOX_ERR_INVALID, "null destination");
+  const float* p = nullptr;
+  int rc = mox_map_accum(c, &p);
+  if (rc) return rc;
+  const mox_ctx* k = c->group ? groupChild(c->group, 0) : c;
+  memcpy(dst, p, (size_t)k->accuW * k->accuH * 12);
   return MOX_OK;
 }
 
@@ -1163,21 +1147,18 @@ int mox_unmap_accum(mox_ctx* c) { return c ? MOX_OK : MOX_ERR_INVALID; }
 // ---- asynchronous read-back and the peer-memory tile gather (see include/mox.h)
 float* ctxGatherBuffer(mox_ctx* c, int which) {
   if (bind(c) || ensureGather(c, true)) return nullptr;
-  if (c->gatherPeer[which]) { c->err = "gather buffer is imported"; return nullptr; }
+  if (c->dGather[which].kind != GatherBuf::own) { c->err = "gather buffer is imported"; return nullptr; }
   cudaStreamSynchronize(c->stream);   // the zero-fill of a fresh buffer
-  return c->dGather[which];
+  return c->dGather[which].p;
 }
 
 int ctxBorrowGatherTarget(mox_ctx* c, int which, float* ptr) {
-  if (c->dGather[which] == ptr) return MOX_OK;
+  if (c->dGather[which].p == ptr) return MOX_OK;
   if (bind(c)) return MOX_ERR_CUDA;
-  if (c->dGather[which]) {
-    cudaStreamSynchronize(c->stream);
-    if (c->gatherPeer[which] == 1) cudaIpcCloseMemHandle(c->dGather[which]);
-    else if (!c->gatherPeer[which]) cudaFree(c->dGather[which]);
-  }
-  c->dGather[which] = ptr;
-  c->gatherPeer[which] = 2;   // borrowed from another context of this process: never freed here
+  GatherBuf& g = c->dGather[which];
+  if (g.p) cudaStreamSynchronize(c->stream);
+  g.release();
+  g.p = ptr; g.kind = GatherBuf::borrowed;
   c->gatherBytes = (size_t)c->accuW * c->accuH * 12;
   return MOX_OK;
 }
@@ -1189,10 +1170,10 @@ int mox_gather_export(mox_ctx* c, int which, void* handle_out) {
   int rc = bind(c);
   if (rc) return rc;
   if ((rc = ensureGather(c, true))) return rc;
-  if (c->gatherPeer[which]) return fail(c, MOX_ERR_STATE, "this rank imported its gather buffer");
+  if (c->dGather[which].kind != GatherBuf::own) return fail(c, MOX_ERR_STATE, "this rank imported its gather buffer");
   CUCK(c, cudaStreamSynchronize(c->stream));
   static_assert(sizeof(cudaIpcMemHandle_t) == MOX_IPC_HANDLE_BYTES, "IPC handle size");
-  CUCK(c, cudaIpcGetMemHandle((cudaIpcMemHandle_t*)handle_out, c->dGather[which]));
+  CUCK(c, cudaIpcGetMemHandle((cudaIpcMemHandle_t*)handle_out, c->dGather[which].p));
   return MOX_OK;
 }
 
@@ -1200,21 +1181,17 @@ int mox_gather_import(mox_ctx* c, int which, const void* handle) {
   if (!c) return MOX_ERR_INVALID;
   GROUP_REFUSE(c, "the tile gather");
   if (!handle || which < 0 || which > 1) return fail(c, MOX_ERR_INVALID, "bad gather_import arguments");
-  if (!c->dAccu) return fail(c, MOX_ERR_STATE, "mox_gather_import before mox_set_globals");
+  if (!c->dAccu.p) return fail(c, MOX_ERR_STATE, "mox_gather_import before mox_set_globals");
   int rc = bind(c);
   if (rc) return rc;
-  if (c->dGather[which]) {
-    cudaStreamSynchronize(c->stream);
-    if (c->gatherPeer[which] == 1) cudaIpcCloseMemHandle(c->dGather[which]);
-    else if (!c->gatherPeer[which]) cudaFree(c->dGather[which]);
-    c->dGather[which] = nullptr;
-  }
+  GatherBuf& g = c->dGather[which];
+  if (g.p) cudaStreamSynchronize(c->stream);
+  g.release();
   cudaIpcMemHandle_t h;
   memcpy(&h, handle, sizeof h);
   void* p = nullptr;
   CUCK(c, cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess));
-  c->dGather[which] = (float*)p;
-  c->gatherPeer[which] = 1;
+  g.p = (float*)p; g.kind = GatherBuf::ipc;
   c->gatherBytes = (size_t)c->accuW * c->accuH * 12;
   return MOX_OK;
 }
@@ -1222,12 +1199,12 @@ int mox_gather_import(mox_ctx* c, int which, const void* handle) {
 int mox_gather_push(mox_ctx* c, int which) {
   if (!c) return MOX_ERR_INVALID;
   GROUP_REFUSE(c, "the tile gather");
-  if (which < 0 || which > 1 || !c->dAccu) return fail(c, MOX_ERR_INVALID, "bad gather_push");
+  if (which < 0 || which > 1 || !c->dAccu.p) return fail(c, MOX_ERR_INVALID, "bad gather_push");
   int rc = bind(c);
   if (rc) return rc;
   if ((rc = refreshOwned(c))) return rc;
-  if (!c->dGather[which] && (rc = ensureGather(c, false))) return rc;   // the root (or a single rank) pushes into its own buffer
-  launchPushOwned(c->dAccu, c->dOwned, c->nOwned, c->dGather[which], c->stream);
+  if (!c->dGather[which].p && (rc = ensureGather(c, false))) return rc;   // the root (or a single rank) pushes into its own buffer
+  launchPushOwned(c->dAccu.p, c->dOwned.p, c->nOwned, c->dGather[which].p, c->stream);
   CUCK(c, cudaStreamSynchronize(c->stream));   // the pixels have landed before a barrier tells the root to read them
   return MOX_OK;
 }
@@ -1239,11 +1216,11 @@ int mox_read_gathered_begin(mox_ctx* c, int which) {
   int rc = bind(c);
   if (rc) return rc;
   if ((rc = ensureGather(c, true))) return rc;
-  if (c->gatherPeer[which]) return fail(c, MOX_ERR_STATE, "only the rank that owns the gather buffer reads it");
+  if (c->dGather[which].kind != GatherBuf::own) return fail(c, MOX_ERR_STATE, "only the rank that owns the gather buffer reads it");
   // pushes of this rank are ordered by its stream, pushes of the others by the caller's barrier
   CUCK(c, cudaEventRecord(c->evPushed, c->stream));
   CUCK(c, cudaStreamWaitEvent(c->copyStream, c->evPushed, 0));
-  CUCK(c, cudaMemcpyAsync(c->hostGather[which], c->dGather[which], c->gatherBytes, cudaMemcpyDeviceToHost, c->copyStream));
+  CUCK(c, cudaMemcpyAsync(c->hostGather[which].p, c->dGather[which].p, c->gatherBytes, cudaMemcpyDeviceToHost, c->copyStream));
   CUCK(c, cudaEventRecord(c->evCopied[which], c->copyStream));
   return MOX_OK;
 }
@@ -1251,9 +1228,9 @@ int mox_read_gathered_begin(mox_ctx* c, int which) {
 int mox_read_gathered_end(mox_ctx* c, int which, const float** out) {
   if (!c) return MOX_ERR_INVALID;
   GROUP_REFUSE(c, "the tile gather");
-  if (which < 0 || which > 1 || !out || !c->hostGather[which]) return fail(c, MOX_ERR_INVALID, "bad read_gathered_end");
+  if (which < 0 || which > 1 || !out || !c->hostGather[which].p) return fail(c, MOX_ERR_INVALID, "bad read_gathered_end");
   CUCK(c, cudaEventSynchronize(c->evCopied[which]));
-  *out = c->hostGather[which];
+  *out = c->hostGather[which].p;
   return MOX_OK;
 }
 
@@ -1268,11 +1245,11 @@ int mox_read_accum_begin(mox_ctx* c) {
   if (rc) return rc;
   if ((rc = ensureGather(c, true))) return rc;
   const int which = c->readCur;
-  if (c->gatherPeer[which]) return fail(c, MOX_ERR_STATE, "this rank's gather buffers are imported: use mox_gather_push");
+  if (c->dGather[which].kind != GatherBuf::own) return fail(c, MOX_ERR_STATE, "this rank's gather buffers are imported: use mox_gather_push");
   // snapshot on the render stream (the next launch may start right away), copy on the copy stream; the snapshot
   // must not overwrite an image the copy stream is still sending
   CUCK(c, cudaStreamWaitEvent(c->stream, c->evCopied[which], 0));
-  CUCK(c, cudaMemcpyAsync(c->dGather[which], c->dAccu, c->gatherBytes, cudaMemcpyDeviceToDevice, c->stream));
+  CUCK(c, cudaMemcpyAsync(c->dGather[which].p, c->dAccu.p, c->gatherBytes, cudaMemcpyDeviceToDevice, c->stream));
   if ((rc = mox_read_gathered_begin(c, which))) return rc;
   c->readPending = which;
   c->readCur ^= 1;
@@ -1297,26 +1274,23 @@ int mox_clear_accum(mox_ctx* c) {
   GROUP_EACH(c, mox_clear_accum(k));
   int rc = bind(c);
   if (rc) return rc;
-  if (c->dAccu) CUCK(c, cudaMemsetAsync(c->dAccu, 0, (size_t)c->accuW * c->accuH * 12, c->stream));
+  if (c->dAccu.p) CUCK(c, cudaMemsetAsync(c->dAccu.p, 0, (size_t)c->accuW * c->accuH * 12, c->stream));
   CUCK(c, cudaStreamSynchronize(c->stream));
-  c->launches = 0; c->raysPrimary = c->raysBounce = c->raysShadow = c->nonfinite = c->nodeVisits = c->primTests = 0;
-  c->nodeVisitsShadow = c->primTestsShadow = c->raysShadowTraced = c->shadowBlocked = c->shadowTinted = 0;
-  c->msRender = 0;
-  for (double& m : c->msStage) m = 0;
-  for (int d = 0; d < MOX_STATS_DEPTHS; ++d) { c->raysDepth[d] = c->shadowDepth[d] = 0; c->msDepth[0][d] = c->msDepth[1][d] = 0; }
-  c->extendLaunches = c->kernelLaunches = 0;
+  const double msBuild = c->st.ms_build;   // describes the acceleration structure, not the image
+  c->st = mox_stats{};
+  c->st.ms_build = msBuild;
   return MOX_OK;
 }
 
 int mox_set_accum(mox_ctx* c, const float* src, uint64_t launches) {
   if (!c) return MOX_ERR_INVALID;
   GROUP_EACH(c, mox_set_accum(k, src, launches));   // every device keeps the pixels it owns
-  if (!src || !c->dAccu) return fail(c, MOX_ERR_INVALID, "no accumulation buffer");
+  if (!src || !c->dAccu.p) return fail(c, MOX_ERR_INVALID, "no accumulation buffer");
   int rc = bind(c);
   if (rc) return rc;
-  CUCK(c, cudaMemcpyAsync(c->dAccu, src, (size_t)c->accuW * c->accuH * 12, cudaMemcpyHostToDevice, c->stream));
+  CUCK(c, cudaMemcpyAsync(c->dAccu.p, src, (size_t)c->accuW * c->accuH * 12, cudaMemcpyHostToDevice, c->stream));
   CUCK(c, cudaStreamSynchronize(c->stream));
-  c->launches = launches;
+  c->st.launches = launches;
   return MOX_OK;
 }
 
@@ -1366,11 +1340,11 @@ int mox_owned_pixels(mox_ctx* c, uint32_t rank, uint64_t* out_n) {
 int mox_pack_owned(mox_ctx* c, void* dev_dst) {
   if (!c) return MOX_ERR_INVALID;
   GROUP_REFUSE(c, "the tile gather");
-  if (!dev_dst || !c->dAccu) return fail(c, MOX_ERR_INVALID, "bad pack_owned");
+  if (!dev_dst || !c->dAccu.p) return fail(c, MOX_ERR_INVALID, "bad pack_owned");
   int rc = bind(c);
   if (rc) return rc;
   if ((rc = refreshOwned(c))) return rc;
-  launchPackOwned(c->dAccu, c->dOwned, c->nOwned, (float*)dev_dst, c->stream);
+  launchPackOwned(c->dAccu.p, c->dOwned.p, c->nOwned, (float*)dev_dst, c->stream);
   CUCK(c, cudaStreamSynchronize(c->stream));
   return MOX_OK;
 }
@@ -1378,7 +1352,7 @@ int mox_pack_owned(mox_ctx* c, void* dev_dst) {
 int mox_unpack_owned(mox_ctx* c, uint32_t rank, const void* dev_src) {
   if (!c) return MOX_ERR_INVALID;
   GROUP_REFUSE(c, "the tile gather");
-  if (!dev_src || !c->dAccu || rank >= c->world) return fail(c, MOX_ERR_INVALID, "bad unpack_owned");
+  if (!dev_src || !c->dAccu.p || rank >= c->world) return fail(c, MOX_ERR_INVALID, "bad unpack_owned");
   int rc = bind(c);
   if (rc) return rc;
   if ((rc = refreshOwned(c))) return rc;
@@ -1391,7 +1365,7 @@ int mox_unpack_owned(mox_ctx* c, uint32_t rank, const void* dev_src) {
     if (!l.empty()) { CUCK(c, cudaMemcpyAsync(b.p, l.data(), l.size() * 4, cudaMemcpyHostToDevice, c->stream)); CUCK(c, cudaStreamSynchronize(c->stream)); }
     c->ownedCount[rank] = l.size();
   }
-  launchUnpackOwned(c->dAccu, (const uint32_t*)b.p, (uint32_t)c->ownedCount[rank], (const float*)dev_src, c->stream);
+  launchUnpackOwned(c->dAccu.p, (const uint32_t*)b.p, (uint32_t)c->ownedCount[rank], (const float*)dev_src, c->stream);
   CUCK(c, cudaStreamSynchronize(c->stream));
   return MOX_OK;
 }
@@ -1405,25 +1379,12 @@ int mox_get_stats(mox_ctx* c, mox_stats* s) {
     return rc_;
   }
   if (!s) return fail(c, MOX_ERR_INVALID, "null stats");
-  memset(s, 0, sizeof *s);
-  s->rays_primary = c->raysPrimary; s->rays_bounce = c->raysBounce; s->rays_shadow = c->raysShadow;
-  s->nonfinite_samples = c->nonfinite; s->launches = c->launches; s->node_visits = c->nodeVisits; s->prim_tests = c->primTests;
-  s->ms_render = c->msRender; s->ms_build = c->msBuild;
+  *s = c->st;
   s->n_prims = (uint32_t)c->prims.size(); s->n_triangles = (uint32_t)c->tris.size();
   s->n_spheres = c->nSpheres; s->n_quads = c->nQuads;
   const bool wide = c->wideBuilt && c->useWide;
-  s->n_nodes = (uint32_t)(wide ? c->nNodes8 : c->nNodes); s->node_bytes = wide ? sizeof(BvhNode8) : sizeof(BvhNode2); s->prim_bytes = 16 * MOX_PACKED_F4;
+  s->n_nodes = (uint32_t)(wide ? c->accel.nNodes8 : c->accel.nNodes); s->node_bytes = wide ? sizeof(BvhNode8) : sizeof(BvhNode2); s->prim_bytes = 16 * MOX_PACKED_F4;
   s->n_lights = (uint32_t)c->lights.size();
-  s->ms_generate = c->msStage[ST_GENERATE]; s->ms_extend = c->msStage[ST_EXTEND]; s->ms_shade = c->msStage[ST_SHADE];
-  s->ms_shadow = c->msStage[ST_SHADOW]; s->ms_accumulate = c->msStage[ST_ACCUMULATE];
-  s->extend_launches = c->extendLaunches; s->kernel_launches = c->kernelLaunches;
-  s->node_visits_shadow = c->nodeVisitsShadow; s->prim_tests_shadow = c->primTestsShadow;
-  s->rays_shadow_traced = c->raysShadowTraced;
-  s->rays_shadow_blocked = c->shadowBlocked; s->rays_shadow_tinted = c->shadowTinted;
-  for (int d = 0; d < MOX_STATS_DEPTHS; ++d) {
-    s->rays_depth[d] = c->raysDepth[d]; s->shadow_traced_depth[d] = c->shadowDepth[d];
-    s->ms_extend_depth[d] = c->msDepth[0][d]; s->ms_shadow_depth[d] = c->msDepth[1][d];
-  }
   return MOX_OK;
 }
 
@@ -1451,8 +1412,8 @@ int mox_trace_closest_device(mox_ctx* c, const void* dev_rays, size_t n, void* d
   CUCK(c, cudaMemsetAsync(counters, 0, C_WORDS * 4, c->stream));
   launchSplitRays((const float4*)dev_rays, (float4*)c->dQueryO.p, (float4*)c->dQueryD.p, n, c->stream);
   TraceJob job;
-  job.rayO = (const float4*)c->dQueryO.p; job.rayD = (const float4*)c->dQueryD.p; job.queue = nullptr; job.count = (uint32_t)n; job.countPtr = nullptr; job.originMod = 0;
-  job.cursor = counters + C_CURSOR; job.hits = (float4*)dev_hits; job.hits2 = nullptr; job.shC = nullptr; job.counters = counters;
+  job.rayO = (const float4*)c->dQueryO.p; job.rayD = (const float4*)c->dQueryD.p; job.count = (uint32_t)n;
+  job.cursor = counters + C_CURSOR; job.hits = (float4*)dev_hits; job.counters = counters;
   CUCK(c, cudaMemsetAsync(job.cursor, 0, 4, c->stream));
   CUCK(c, cudaEventRecord(c->ev0, c->stream));
   launchTraverse(sceneView(c), job, false, count, c->stream);
@@ -1464,9 +1425,10 @@ int mox_trace_closest_device(mox_ctx* c, const void* dev_rays, size_t n, void* d
   if (out_ms) *out_ms = ms;
   if (count) {
     uint32_t host[C_WORDS];
-    CUCK(c, cudaMemcpy(host, counters, sizeof host, cudaMemcpyDeviceToHost));
-    c->nodeVisits += ((uint64_t)host[C_NODEVIS_HI] << 32) | host[C_NODEVIS_LO];
-    c->primTests += ((uint64_t)host[C_PRIMTEST_HI] << 32) | host[C_PRIMTEST_LO];
+    CUCK(c, cudaMemcpyAsync(host, counters, sizeof host, cudaMemcpyDeviceToHost, c->stream));
+    CUCK(c, cudaStreamSynchronize(c->stream));
+    c->st.node_visits += counter64(host, C_NODEVIS_LO);
+    c->st.prim_tests += counter64(host, C_PRIMTEST_LO);
   }
   return MOX_OK;
 }
@@ -1484,7 +1446,8 @@ int mox_trace_closest(mox_ctx* c, const float* rays, size_t n, void* hits) {
   // stream-ordered: the traversal kernel runs on the (non-blocking) context stream
   CUCK(c, cudaMemcpyAsync(dRays, rays, n * 32, cudaMemcpyHostToDevice, c->stream));
   if ((rc = mox_trace_closest_device(c, dRays, n, dHits, nullptr))) return rc;
-  CUCK(c, cudaMemcpy(hits, dHits, n * 16, cudaMemcpyDeviceToHost));
+  CUCK(c, cudaMemcpyAsync(hits, dHits, n * 16, cudaMemcpyDeviceToHost, c->stream));
+  CUCK(c, cudaStreamSynchronize(c->stream));
   return MOX_OK;
 }
 
@@ -1502,18 +1465,19 @@ int mox_trace_shadow(mox_ctx* c, const float* rays, size_t n, float* out_rgb) {
     return rc;
   void *dRays = c->dQueryRays.p, *dOut = c->dQueryOut.p, *dC = c->dQueryC.p;
   uint32_t* counters = (uint32_t*)c->dQueryCounters.p;
-  cudaMemcpyAsync(dRays, rays, n * 32, cudaMemcpyHostToDevice, c->stream);   // stream-ordered, see mox_trace_closest
-  cudaMemsetAsync(counters, 0, C_WORDS * 4, c->stream);
+  CUCK(c, cudaMemcpyAsync(dRays, rays, n * 32, cudaMemcpyHostToDevice, c->stream));   // stream-ordered, see mox_trace_closest
+  CUCK(c, cudaMemsetAsync(counters, 0, C_WORDS * 4, c->stream));
   launchSplitRays((const float4*)dRays, (float4*)c->dQueryO.p, (float4*)c->dQueryD.p, n, c->stream);
   launchFillOnes((float4*)dC, n, c->stream);
   TraceJob job;
-  job.rayO = (const float4*)c->dQueryO.p; job.rayD = (const float4*)c->dQueryD.p; job.queue = nullptr; job.count = (uint32_t)n; job.countPtr = nullptr; job.originMod = 0;
-  job.cursor = counters + C_CURSOR; job.hits = nullptr; job.hits2 = nullptr; job.shC = (float4*)dC; job.counters = counters;
+  job.rayO = (const float4*)c->dQueryO.p; job.rayD = (const float4*)c->dQueryD.p; job.count = (uint32_t)n;
+  job.cursor = counters + C_CURSOR; job.shC = (float4*)dC; job.counters = counters;
   launchTraverse(sceneView(c), job, true, false, c->stream);
   launchCopyRgb((const float4*)dC, (float*)dOut, n, c->stream);
   cudaError_t e = cudaStreamSynchronize(c->stream);
   if (e == cudaSuccess) e = cudaGetLastError();
-  if (e == cudaSuccess) e = cudaMemcpy(out_rgb, dOut, n * 12, cudaMemcpyDeviceToHost);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(out_rgb, dOut, n * 12, cudaMemcpyDeviceToHost, c->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
   if (e != cudaSuccess) return fail(c, MOX_ERR_CUDA, cudaGetErrorString(e));
   return MOX_OK;
 }
@@ -1528,19 +1492,17 @@ extern "C" int mox_debug_radix_sort(mox_ctx* c, uint32_t* keys, uint32_t* vals, 
   if (!n) return MOX_OK;
   int rc = bind(c);
   if (rc) return rc;
-  uint32_t *dk = nullptr, *dv = nullptr;
-  CUCK(c, cudaMalloc(&dk, n * 4));
-  CUCK(c, cudaMalloc(&dv, n * 4));
-  CUCK(c, cudaMemcpyAsync(dk, keys, n * 4, cudaMemcpyHostToDevice, c->stream));
-  CUCK(c, cudaMemcpyAsync(dv, vals, n * 4, cudaMemcpyHostToDevice, c->stream));
+  DevArray<uint32_t> dk, dv;
+  CUCK(c, dk.alloc(n * 4));
+  CUCK(c, dv.alloc(n * 4));
+  CUCK(c, cudaMemcpyAsync(dk.p, keys, n * 4, cudaMemcpyHostToDevice, c->stream));
+  CUCK(c, cudaMemcpyAsync(dv.p, vals, n * 4, cudaMemcpyHostToDevice, c->stream));
   std::string err;
-  bool ok = radixSortPairs(dk, dv, (int)n, c->stream, err);
-  if (ok) {
-    cudaMemcpy(keys, dk, n * 4, cudaMemcpyDeviceToHost);
-    cudaMemcpy(vals, dv, n * 4, cudaMemcpyDeviceToHost);
-  }
-  cudaFree(dk); cudaFree(dv);
-  return ok ? MOX_OK : fail(c, MOX_ERR_CUDA, err);
+  if (!radixSortPairs(dk.p, dv.p, (int)n, c->stream, err)) return fail(c, MOX_ERR_CUDA, err);
+  CUCK(c, cudaMemcpyAsync(keys, dk.p, n * 4, cudaMemcpyDeviceToHost, c->stream));
+  CUCK(c, cudaMemcpyAsync(vals, dv.p, n * 4, cudaMemcpyDeviceToHost, c->stream));
+  CUCK(c, cudaStreamSynchronize(c->stream));
+  return MOX_OK;
 }
 
 extern "C" int mox_debug_read_accel(mox_ctx* c, int which, void* dst, size_t cap, size_t* out_bytes) {
@@ -1548,13 +1510,14 @@ extern "C" int mox_debug_read_accel(mox_ctx* c, int which, void* dst, size_t cap
   GROUP_FIRST(c, mox_debug_read_accel(k, which, dst, cap, out_bytes));
   if (!c->built) return fail(c, MOX_ERR_STATE, "debug_read_accel before mox_build_accel");
   const bool wide = c->wideBuilt && c->useWide;
+  const BuildOutput& a = c->accel;
   const void* src = nullptr;
   size_t bytes = 0;
   switch (which) {
-    case MOX_DEBUG_ACCEL_NODES: src = c->dNodes; bytes = (size_t)c->nNodes * sizeof(BvhNode2); break;
-    case MOX_DEBUG_ACCEL_NODES8: src = c->dNodes8; bytes = wide ? (size_t)c->nNodes8 * sizeof(BvhNode8) : 0; break;
-    case MOX_DEBUG_ACCEL_PACKED: src = c->dPacked; bytes = (size_t)c->nValid * 16 * MOX_PACKED_F4; break;
-    case MOX_DEBUG_ACCEL_PACKED8: src = c->dPacked8; bytes = wide ? (size_t)c->nValid * 16 * MOX_PACKED_F4 : 0; break;
+    case MOX_DEBUG_ACCEL_NODES: src = a.nodes; bytes = (size_t)a.nNodes * sizeof(BvhNode2); break;
+    case MOX_DEBUG_ACCEL_NODES8: src = a.nodes8; bytes = wide ? (size_t)a.nNodes8 * sizeof(BvhNode8) : 0; break;
+    case MOX_DEBUG_ACCEL_PACKED: src = a.packed; bytes = (size_t)a.nValid * 16 * MOX_PACKED_F4; break;
+    case MOX_DEBUG_ACCEL_PACKED8: src = a.packed8; bytes = wide ? (size_t)a.nValid * 16 * MOX_PACKED_F4 : 0; break;
     default: return fail(c, MOX_ERR_INVALID, "unknown acceleration array");
   }
   if (out_bytes) *out_bytes = bytes;

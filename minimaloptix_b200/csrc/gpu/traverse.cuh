@@ -310,12 +310,11 @@ __device__ __forceinline__ void traverseWarpPersistent(const SceneView& s, const
           MOX_ST_STREAM(job.hits + rayId, make_float4(tBest, __int_as_float(bPrim), bBeta, bGamma));
         }
         if (COUNT) {
-          // closest hit: words 10/12, shadow: 16/18 (CounterSlot in wavefront.h)
-          atomicAdd((unsigned long long*)(job.counters + (ANYHIT ? 16 : 10)), (unsigned long long)nv);
-          atomicAdd((unsigned long long*)(job.counters + (ANYHIT ? 18 : 12)), (unsigned long long)np);
-          if (ANYHIT) {   // words 20 / 21 (C_SH_BLOCKED / C_SH_TINTED): rays that touched their contribution record
-            if (atten.x == 0.f && atten.y == 0.f && atten.z == 0.f) atomicAdd(job.counters + 20, 1u);
-            else if (atten.x != 1.f || atten.y != 1.f || atten.z != 1.f) atomicAdd(job.counters + 21, 1u);
+          atomicAdd((unsigned long long*)(job.counters + (ANYHIT ? C_NODEVIS_SH_LO : C_NODEVIS_LO)), (unsigned long long)nv);
+          atomicAdd((unsigned long long*)(job.counters + (ANYHIT ? C_PRIMTEST_SH_LO : C_PRIMTEST_LO)), (unsigned long long)np);
+          if (ANYHIT) {   // rays that touched their contribution record
+            if (atten.x == 0.f && atten.y == 0.f && atten.z == 0.f) atomicAdd(job.counters + C_SH_BLOCKED, 1u);
+            else if (atten.x != 1.f || atten.y != 1.f || atten.z != 1.f) atomicAdd(job.counters + C_SH_TINTED, 1u);
           }
         }
         active = false;

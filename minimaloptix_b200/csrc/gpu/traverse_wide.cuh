@@ -392,9 +392,9 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
             MOX_ST_STREAM(job.hits + rayId, make_float4(tBest, __int_as_float(bPrim), bBeta, bGamma));
           }
           if (COUNT) {
-            atomicAdd((unsigned long long*)(job.counters + (ANYHIT ? 16 : 10)), (unsigned long long)nv);
-            atomicAdd((unsigned long long*)(job.counters + (ANYHIT ? 18 : 12)), (unsigned long long)np);
-            if (ANYHIT && shadowEnd) atomicAdd(job.counters + (shadowEnd == 1u ? 20 : 21), 1u);   // C_SH_BLOCKED / C_SH_TINTED
+            atomicAdd((unsigned long long*)(job.counters + (ANYHIT ? C_NODEVIS_SH_LO : C_NODEVIS_LO)), (unsigned long long)nv);
+            atomicAdd((unsigned long long*)(job.counters + (ANYHIT ? C_PRIMTEST_SH_LO : C_PRIMTEST_LO)), (unsigned long long)np);
+            if (ANYHIT && shadowEnd) atomicAdd(job.counters + (shadowEnd == 1u ? C_SH_BLOCKED : C_SH_TINTED), 1u);
           }
         }
       }

@@ -651,12 +651,18 @@ static void launchTraverseT(const SceneView& s, const TraceJob& job, cudaStream_
   else k_traverse<ANYHIT, COUNT, CLASSIFY><<<persistentGridFor(k_traverse<ANYHIT, COUNT, CLASSIFY>, job.count, bpsBinary), TRAV_TPB, 0, stream>>>(s, job);
 }
 
-void launchTraverse(const SceneView& s, const TraceJob& jobIn, bool anyHit, bool count, cudaStream_t stream, bool classify) {
-  if (!jobIn.count) return;
-  TraceJob job = jobIn;
-  job.fetchThreshold = fetchThreshold(anyHit, s.nodes8 != nullptr);
+// What every persistent traversal launch needs besides its rays: the refill threshold, the origin divisor and a zeroed
+// fetch cursor.
+static TraceJob preparedJob(TraceJob job, bool anyHit, bool wide, cudaStream_t stream) {
+  job.fetchThreshold = fetchThreshold(anyHit, wide);
   job.originMagic = job.originMod ? (uint32_t)(0x100000000ull / job.originMod) + 1u : 0u;
   cudaMemsetAsync(job.cursor, 0, 4, stream);
+  return job;
+}
+
+void launchTraverse(const SceneView& s, const TraceJob& jobIn, bool anyHit, bool count, cudaStream_t stream, bool classify) {
+  if (!jobIn.count) return;
+  const TraceJob job = preparedJob(jobIn, anyHit, s.nodes8 != nullptr, stream);
   if (anyHit && count) launchTraverseT<true, true, false>(s, job, stream);
   else if (anyHit) launchTraverseT<true, false, false>(s, job, stream);
   else if (classify && count) launchTraverseT<false, true, true>(s, job, stream);
@@ -665,21 +671,20 @@ void launchTraverse(const SceneView& s, const TraceJob& jobIn, bool anyHit, bool
   else launchTraverseT<false, false, false>(s, job, stream);
 }
 
-void launchExtend(const LaunchCtx& c, const uint32_t* queue, uint32_t count, const uint32_t* countPtr, uint32_t depth) {
-  if (!count) return;
+// The closest-hit rays of a bounce: path rays in, render-form hit records out.
+static TraceJob extendJob(const LaunchCtx& c, const uint32_t* queue, uint32_t count, const uint32_t* countPtr) {
   TraceJob job;
-  job.rayO = c.pb.rayO; job.rayD = c.pb.rayD; job.queue = queue; job.count = count; job.countPtr = countPtr; job.originMod = 0;
-  job.cursor = c.pb.counters + C_CURSOR; job.hits = nullptr; job.hits2 = c.pb.hit; job.shC = nullptr; job.counters = c.pb.counters;
-  launchTraverse(c.scene, job, false, c.countTraversal, c.stream, true);
+  job.rayO = c.pb.rayO; job.rayD = c.pb.rayD; job.queue = queue; job.count = count; job.countPtr = countPtr;
+  job.cursor = c.pb.counters + C_CURSOR; job.hits2 = c.pb.hit; job.counters = c.pb.counters;
+  return job;
+}
+
+void launchExtend(const LaunchCtx& c, const uint32_t* queue, uint32_t count, const uint32_t* countPtr, uint32_t depth) {
+  if (count) launchTraverse(c.scene, extendJob(c, queue, count, countPtr), false, c.countTraversal, c.stream, true);
 }
 void launchTerminal(const LaunchCtx& c, const uint32_t* queue, uint32_t count, const uint32_t* countPtr, const TerminalLights& tl) {
   if (!count) return;
-  TraceJob job;
-  job.rayO = c.pb.rayO; job.rayD = c.pb.rayD; job.queue = queue; job.count = count; job.countPtr = countPtr; job.originMod = 0;
-  job.cursor = c.pb.counters + C_CURSOR; job.hits = nullptr; job.hits2 = c.pb.hit; job.shC = nullptr; job.counters = c.pb.counters;
-  job.fetchThreshold = fetchThreshold(false, true);
-  job.originMagic = 0u;
-  cudaMemsetAsync(job.cursor, 0, 4, c.stream);
+  const TraceJob job = preparedJob(extendJob(c, queue, count, countPtr), false, true, c.stream);
   static std::atomic<int> bps{0}, bpsCount{0}, bpsWt{0}, bpsWtCount{0};
   const SceneView& s = c.scene;
   if (s.watertight) {
@@ -727,7 +732,7 @@ void launchShadow(const LaunchCtx& c, uint32_t disneyCount, cudaStream_t stream)
   // dense queue of the slots that need a ray; its length lives in device memory (no host sync)
   job.rayO = c.pb.shO; job.rayD = c.pb.shD; job.queue = c.pb.shQueue; job.count = (uint32_t)slots;
   job.countPtr = c.bc + C_SHQ; job.originMod = disneyCount;
-  job.cursor = c.pb.counters + C_CURSOR_SHADOW; job.hits = nullptr; job.hits2 = nullptr; job.shC = c.pb.shC; job.counters = c.pb.counters;
+  job.cursor = c.pb.counters + C_CURSOR_SHADOW; job.shC = c.pb.shC; job.counters = c.pb.counters;
   launchTraverse(c.scene, job, true, c.countTraversal, stream);
 }
 void launchApply(const LaunchCtx& c, uint32_t disneyCount, cudaStream_t stream) {

@@ -9,18 +9,6 @@
 // Material queues built by the extend kernel.
 enum ShadeQueue { Q_LAMBERT = 0, Q_METAL = 1, Q_DIELECTRIC = 2, Q_DISNEY = 3, Q_COUNT = 4 };
 
-// Device counters (uint32 words).  Words 0..7 exist once per bounce in a small ring (LaunchCtx::bc points at the
-// current bounce's block), so the host never has to zero them between two kernels of the same bounce loop:
-//   C_NEXT  rays spawned by this bounce's shade kernels (= the next extend launch's ray count, read on the device)
-//   C_MAT0+k paths binned into material queue k by this bounce's classify kernel
-//   C_SHQ   shadow rays queued by this bounce's Disney kernel
-// Words 8.. are per batch.
-enum CounterSlot { C_NEXT = 0, C_MAT0 = 1 /* ..4 */, C_SHQ = 5 /* shadow queue length */, C_BOUNCE_WORDS = 8,
-                   C_NONFINITE = 8, C_SHADOW = 9, C_NODEVIS_LO = 10, C_NODEVIS_HI = 11,
-                   C_PRIMTEST_LO = 12, C_PRIMTEST_HI = 13, C_CURSOR = 14, C_CURSOR_SHADOW = 15 /* the shadow launch may overlap the next extend launch */,
-                   C_NODEVIS_SH_LO = 16, C_PRIMTEST_SH_LO = 18, C_SH_BLOCKED = 20, C_SH_TINTED = 21, C_WORDS = 24 };
-constexpr int BOUNCE_RING = 4;   // per-bounce counter blocks kept alive at once
-
 struct PathBuffers {
   size_t capacity = 0;      // paths
   size_t shadowSlots = 0;   // capacity * nLights
