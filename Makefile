@@ -38,9 +38,9 @@ $(PKG)/libmox_host.so: $(HOST_SRCS) $(HOST_HDRS)
 $(PKG)/mox_cli: $(PKG)/libmox_host.so $(CSRC)/host/cli_main.cpp
 	$(CXX) $(CXXFLAGS) -o $@ $(CSRC)/host/cli_main.cpp -L$(PKG) -lmox_host -ldl -pthread -Wl,-rpath,'$$ORIGIN'
 
-# oracle/refit.cpp compiles oracle.cpp and adds the refit / mesh-update entry points around it.
-oracle/liboracle.so: oracle/refit.cpp oracle/oracle.cpp oracle/oracle.h oracle/device_spec.h oracle/vecmath.h include/mox.h include/mox_structs.h
-	$(CXX) $(ORCFLAGS) -shared -o $@ oracle/refit.cpp
+# oracle/adaptive.cpp compiles oracle/refit.cpp, which compiles oracle.cpp; each adds its entry points around the other.
+oracle/liboracle.so: oracle/adaptive.cpp oracle/refit.cpp oracle/oracle.cpp oracle/oracle.h oracle/device_spec.h oracle/vecmath.h include/mox.h include/mox_structs.h
+	$(CXX) $(ORCFLAGS) -shared -o $@ oracle/adaptive.cpp
 
 # Reference loader half (scene.cpp + tiny_obj_loader.h) compiled from /root/reference with a shim.
 oracle/_ref/libref_loader.so: oracle/ref_shim/ref_loader.cpp oracle/ref_shim/optix_world.h

@@ -202,6 +202,34 @@ int mox_launch(mox_ctx*, int32_t randSeed);
  * one wavefront; the result is bit-identical to spp calls of mox_launch. */
 int mox_render(mox_ctx*, uint32_t spp, uint32_t seed);
 
+/* Adaptive sampling: mox_render's launches for the pixels whose estimated error is still above a threshold.
+ *
+ * The call covers launches st.launches .. st.launches + spp - 1 of mox_render's seed schedule, and advances
+ * mox_stats.launches by spp even when every pixel has stopped.  A pixel's estimate uses only the samples it received
+ * from mox_render_adaptive since the last mox_clear_accum / mox_set_accum / size change; n is their number.  Each
+ * sample adds y = 0.2126 r + 0.7152 g + 0.0722 b (float32, in that order) of the colour the accumulation buffer
+ * receives (the clamped sample, or badColor for a non-finite one); S1 = sum y and S2 = sum y^2 are float64, in launch
+ * order.  With m = S1 / n, s^2 = max(0, (S2 - S1 m) / (n - 1)) and err = sqrt(s^2 / n), a pixel has converged when
+ * n >= max(min_spp, 2) and err < max(rel_error * m, abs_error) (strict: thresholds of 0 never stop a pixel).
+ *
+ * At the start of the call every owned pixel is checked; the active ones are rendered in rounds of round_spp
+ * launches (the last may be shorter) and checked after each round.  A pixel that has converged gets no further
+ * sample in this call; when none is left, the remaining launches run no kernel.  So a pixel that took k samples holds
+ * exactly what k launches of mox_render would have left in it.  *out_samples (may be NULL): pixel-samples traced.
+ * The first call allocates 24 bytes per pixel of statistics.  MOX_ERR_INVALID: null params, round_spp == 0, or a
+ * negative or non-finite threshold; MOX_ERR_STATE: as mox_render.  On a multi-GPU handle every device runs the
+ * rounds on its own tiles and finishes when they have converged. */
+typedef struct mox_adaptive {
+  uint32_t round_spp; /* launches between two convergence checks, >= 1 */
+  uint32_t min_spp;   /* adaptive samples a pixel needs before it may stop */
+  float rel_error;    /* stop when err < max(rel_error * mean, abs_error); both finite, >= 0 */
+  float abs_error;
+} mox_adaptive;
+int mox_render_adaptive(mox_ctx*, uint32_t spp, uint32_t seed, const mox_adaptive* params, uint64_t* out_samples);
+/* Samples per pixel (W*H, row 0 = bottom): mox_stats.launches minus the launches the pixel sat out in
+ * mox_render_adaptive; 0 for pixels of other ranks.  Divide the accumulation buffer by it to get the image. */
+int mox_read_sample_counts(mox_ctx*, uint32_t* dst);
+
 /* accuBuffer map()/unmap() (MinimalOptiX.cpp:44,60): W*H*3 floats, row 0 =
  * bottom of the image, un-normalised sums.  Pixels of other ranks are 0. */
 int mox_read_accum(mox_ctx*, float* dst_rgb);

@@ -73,6 +73,9 @@ int moxh_scene_apply_spheres(const moxh_scene*, const moxh_api*, void* ctx);
 /* updateContent (MinimalOptiX.cpp:43-66): out[H-1-i][j] = quantise(clamp(accu[i][j] / n, 0, 1)),
  * quantise(v) = round(v * 65535) >> 8 (QColor::setRedF -> RGB888).  out: W*H*3 bytes, row 0 = top. */
 void moxh_accum_to_rgb8(const float* accum, uint32_t width, uint32_t height, float n_accum, uint8_t* out);
+/* The same with a sample count per pixel (mox_read_sample_counts: W*H, row 0 = bottom) in place of n_accum, for
+ * images of mox_render_adaptive.  A count of 0 gives black. */
+void moxh_accum_to_rgb8_counts(const float* accum, uint32_t width, uint32_t height, const uint32_t* counts, uint8_t* out);
 /* saveCurrentFrame: PNG (RGB8, stored deflate) or binary PPM by extension. */
 int moxh_write_image(const char* path, const uint8_t* rgb, uint32_t width, uint32_t height);
 /* Raw float accumulator dump / load (resume + parity artefact): magic "MOXA", W, H, launches. */

@@ -37,6 +37,8 @@ SIGNATURES = {
     "build_accel": (C.c_int, [_vp, _u32, C.POINTER(_f32)]),
     "launch": (C.c_int, [_vp, _i32]),
     "render": (C.c_int, [_vp, _u32, _u32]),
+    "render_adaptive": (C.c_int, [_vp, _u32, _u32, C.POINTER(S.Adaptive), C.POINTER(_u64)]),
+    "read_sample_counts": (C.c_int, [_vp, _vp]),
     "read_accum": (C.c_int, [_vp, _vp]),
     "map_accum": (C.c_int, [_vp, C.POINTER(_fp)]),
     "unmap_accum": (C.c_int, [_vp]),
@@ -209,6 +211,20 @@ class Context:
 
     def render(self, spp, seed):
         self._ck(self.b.render(self.h, spp, seed & 0xFFFFFFFF), "render")
+
+    def render_adaptive(self, spp, seed, rel_error, abs_error=0.0, min_spp=16, round_spp=8):
+        """mox_render_adaptive: up to spp more samples per pixel, until its estimated error is below the threshold.
+        Returns the number of pixel-samples traced."""
+        p = S.Adaptive(round_spp, min_spp, rel_error, abs_error)
+        n = _u64()
+        self._ck(self.b.render_adaptive(self.h, spp, seed & 0xFFFFFFFF, C.byref(p), C.byref(n)), "render_adaptive")
+        return n.value
+
+    def read_sample_counts(self):
+        """Samples per pixel, (H, W) uint32, row 0 = bottom: divide the accumulation buffer by it."""
+        out = np.empty((self.height, self.width), dtype=np.uint32)
+        self._ck(self.b.read_sample_counts(self.h, _ptr(out)), "read_sample_counts")
+        return out
 
     def read_accum(self):
         out = np.empty((self.height, self.width, 3), dtype=np.float32)

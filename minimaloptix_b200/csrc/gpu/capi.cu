@@ -5,6 +5,7 @@
 //
 // There is no CPU path in this library: every compute entry point needs a usable sm_100 GPU.
 #include <algorithm>
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -230,6 +231,14 @@ struct mox_ctx {
   bool brdfFast = true;          // approximate reciprocal / square root inside BRDF values (MOX_BRDF_IEEE=1: IEEE, the oracle's operations)
   bool terminalQuery = true;     // the bounce past rayMaxDepth uses the light list and an any-hit query (MOX_TERMINAL_CLOSEST=1: closest hit)
   uint32_t terminalDepth = 0;    // the batch's last bounce ran the terminal query: its ray counts come with the final counter copy
+
+  // Adaptive sampling (mox_render_adaptive), allocated at its first call: per pixel the luminance sums, the sample
+  // count and the launches sat out (pixelStats, 24 bytes per pixel in one block), and the two active-pixel lists with
+  // the select kernels' tile sums and survivor word.
+  DevBuf adaptiveStats, adaptiveLists;
+  PixelStats pixelStats;
+  PinnedBuf<uint32_t> hostSurvivors;
+  const PixelStats* batchStats = nullptr;   // the batch in flight also accumulates these (null: mox_launch / mox_render)
 
   // Frees what the context holds; the device buffers go with their owners.  mox_destroy binds the device and waits
   // for the streams first.
@@ -464,7 +473,8 @@ int finishBatch(mox_ctx* c) {
   StageTimer& tm = c->timer;
   if (c->applyPending) { CUCK(c, cudaStreamWaitEvent(c->stream, c->evApplied, 0)); c->applyPending = false; }
   tm.begin(ST_ACCUMULATE, c->stream);
-  launchAccumulate(c->lc, c->batchSamples);
+  if (c->batchStats) launchAccumulateAdaptive(c->lc, c->batchSamples, *c->batchStats);
+  else launchAccumulate(c->lc, c->batchSamples);
   tm.end(c->stream);
   c->st.kernel_launches++;
   CUCK(c, cudaMemcpyAsync(c->hostCnt.p, c->pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, c->stream));
@@ -532,9 +542,9 @@ int advanceBounce(mox_ctx* c) {
   return enqueueExtend(c);
 }
 
-// Events, pinned counters and wavefront buffers for a batch of S samples per owned pixel.  renderSeeds calls it
+// Events, pinned counters and wavefront buffers for a batch of S samples of `count` pixels.  renderSeeds calls it
 // before its timed region, so the first launch of a context does not time its own allocations.
-int prepareBatch(mox_ctx* c, uint32_t S) {
+int prepareBatch(mox_ctx* c, uint32_t S, uint32_t count) {
   if (!c->evReady) CUCK(c, cudaEventCreateWithFlags(&c->evReady, cudaEventDisableTiming));
   if (c->overlapShadow && !c->shadowStream) {
     CUCK(c, cudaStreamCreateWithFlags(&c->shadowStream, cudaStreamNonBlocking));
@@ -542,28 +552,28 @@ int prepareBatch(mox_ctx* c, uint32_t S) {
     CUCK(c, cudaEventCreateWithFlags(&c->evApplied, cudaEventDisableTiming));
   }
   int rc = ensure(c, c->hostCnt, kCounterWords * 4);
-  return rc ? rc : ensurePaths(c, (size_t)S * c->nOwned, c->lights.size(), S);
+  return rc ? rc : ensurePaths(c, (size_t)S * count, c->lights.size(), S);
 }
 
-// One wavefront batch: `seeds.size()` samples of every owned pixel.  Generate, then advance bounce by bounce until
-// no path is left, then collect the counters.
-int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds) {
+// One wavefront batch: `seeds.size()` samples of each pixel of list[0, count).  Generate, then advance bounce by
+// bounce until no path is left, then collect the counters.
+int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds, const uint32_t* list, uint32_t count) {
   const uint32_t S = (uint32_t)seeds.size();
-  const size_t P = (size_t)S * c->nOwned;
+  const size_t P = (size_t)S * count;
   if (P == 0) return MOX_OK;
   if (P > 0xfffffff0ull) return fail(c, MOX_ERR_INVALID, "batch too large");
   int rc;
   // all allocations first: a failure (MOX_ERR_OOM -> the caller retries with a smaller batch) must not leave work
   // in flight
-  if ((rc = prepareBatch(c, S))) return rc;
+  if ((rc = prepareBatch(c, S, count))) return rc;
   PathBuffers& pb = c->pb;
   CUCK(c, cudaMemcpyAsync(pb.seeds, seeds.data(), S * 4, cudaMemcpyHostToDevice, c->stream));
   LaunchCtx& lc = c->lc;
   lc.scene = sceneView(c);
   lc.rp = c->rp;
   lc.pb = pb;
-  lc.ownedPix = c->dOwned.p;
-  lc.nOwned = c->nOwned;
+  lc.ownedPix = list;
+  lc.nOwned = count;
   lc.accu = c->dAccu.p;
   lc.countTraversal = (c->accelFlags & MOX_ACCEL_COUNTERS) != 0;
   lc.brdfFast = c->brdfFast;
@@ -601,14 +611,14 @@ int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds) {
 
 // Paths per batch: the configured cap, lowered so that the wavefront state fits into 60 % of the free device
 // memory (what the current block holds counts as free) for this scene's light count (36 bytes per path and light).
-size_t batchCap(mox_ctx* c, size_t wanted /* samples per pixel of this call */) {
+size_t batchCap(mox_ctx* c, size_t wanted /* samples per pixel of this call */, uint32_t count /* pixels */) {
   size_t cap = c->maxBatchPaths;
   const PathBuffers& pb = c->pb;
   // The buffers of an earlier call already hold such a batch: nothing will be allocated, so there is nothing to
   // budget.  (cudaMemGetInfo is a slow driver call — it was the 20-70 ms hiccup in front of some steps.)
-  if (c->nOwned) {
-    const size_t S = std::min(std::max<size_t>(1, cap / c->nOwned), wanted), nL = c->lights.size();   // samples per batch at the full cap
-    const size_t P = S * c->nOwned;
+  if (count) {
+    const size_t S = std::min(std::max<size_t>(1, cap / count), wanted), nL = c->lights.size();   // samples per batch at the full cap
+    const size_t P = S * count;
     if (c->pathBlock.p && pb.capacity >= P && pb.shadowSlots >= P * nL && pb.seedCap >= S) return cap;
   }
   size_t freeB = 0, totalB = 0;
@@ -622,7 +632,8 @@ size_t batchCap(mox_ctx* c, size_t wanted /* samples per pixel of this call */) 
   return cap;
 }
 
-int renderSeeds(mox_ctx* c, const std::vector<int32_t>& seeds) {
+// The preconditions of a render, then the device, the owned-pixel list, the lights and the textures.
+int beginRender(mox_ctx* c) {
   if (!c->built) return fail(c, MOX_ERR_STATE, "launch before mox_build_accel");
   if (!c->haveGlobals) return fail(c, MOX_ERR_STATE, "launch before mox_set_globals");
   if (!c->haveCamera) return fail(c, MOX_ERR_STATE, "launch before mox_set_camera");
@@ -630,16 +641,22 @@ int renderSeeds(mox_ctx* c, const std::vector<int32_t>& seeds) {
   if (rc) return rc;
   if ((rc = refreshOwned(c))) return rc;
   if ((rc = syncLights(c))) return rc;
-  if ((rc = syncTextures(c))) return rc;
-  if (c->nOwned == 0) { c->st.launches += seeds.size(); return MOX_OK; }
-  size_t perBatch = std::max<size_t>(1, batchCap(c, seeds.size()) / c->nOwned);
-  rc = prepareBatch(c, (uint32_t)std::min(perBatch, seeds.size()));
+  return syncTextures(c);
+}
+
+// One sample per seed for each pixel of list[0, count), in batches; with `stats`, the accumulation also adds every
+// sample's luminance to them.  beginRender first.
+int renderSeeds(mox_ctx* c, const std::vector<int32_t>& seeds, const uint32_t* list, uint32_t count, const PixelStats* stats = nullptr) {
+  if (count == 0) { c->st.launches += seeds.size(); return MOX_OK; }
+  c->batchStats = stats;
+  size_t perBatch = std::max<size_t>(1, batchCap(c, seeds.size(), count) / count);
+  int rc = prepareBatch(c, (uint32_t)std::min(perBatch, seeds.size()), count);
   if (rc && rc != MOX_ERR_OOM) return rc;   // out of memory: the loop below retries with smaller batches
   CUCK(c, cudaEventRecord(c->ev0, c->stream));
   for (size_t i = 0; i < seeds.size();) {
     const size_t n = std::min(perBatch, seeds.size() - i);
     std::vector<int32_t> chunk(seeds.begin() + i, seeds.begin() + i + n);
-    rc = renderBatch(c, chunk);
+    rc = renderBatch(c, chunk, list, count);
     if (rc == MOX_ERR_OOM && perBatch > 1) {
       // the allocation failed after all (fragmentation, another context on the device): free the wavefront
       // state, halve the batch and render this chunk again (nothing of it was enqueued)
@@ -732,6 +749,73 @@ bool terminalLightList(const mox_ctx* c, std::vector<uint4>& out) {
     id = m.firstPrim + m.nFaces;
   }
   return scan((uint32_t)c->prims.size());
+}
+
+// ---- adaptive sampling (mox_render_adaptive)
+
+// The per-pixel statistics (zeroed when allocated) and the active-pixel lists for the current image and partition.
+int ensureAdaptive(mox_ctx* c) {
+  const size_t nPix = (size_t)c->accuW * c->accuH;
+  if (!c->adaptiveStats.p) {
+    CUCK(c, c->adaptiveStats.alloc(nPix * 24));
+    char* b = (char*)c->adaptiveStats.p;
+    PixelStats& ps = c->pixelStats;
+    ps.s1 = (double*)b;
+    ps.s2 = (double*)(b + 8 * nPix);
+    ps.n = (uint32_t*)(b + 16 * nPix);
+    ps.skipped = ps.n + nPix;
+    CUCK(c, cudaMemsetAsync(b, 0, nPix * 24, c->stream));
+  }
+  const size_t words = 2 * (size_t)c->nOwned + adaptiveSelectTiles(c->nOwned) + 1;
+  int rc = ensure(c, c->adaptiveLists, words * 4);
+  return rc ? rc : ensure(c, c->hostSurvivors, 4);
+}
+
+// Forget every adaptive sample: the accumulation buffer was cleared or replaced.
+int resetAdaptive(mox_ctx* c) {
+  if (c->adaptiveStats.p) CUCK(c, cudaMemsetAsync(c->adaptiveStats.p, 0, c->adaptiveStats.bytes, c->stream));
+  return MOX_OK;
+}
+
+// Keeps the pixels of in[0, count) that have not converged under `rule`, in order, in `out`; the others sit out the
+// call's `remaining` launches.  Sets `active` to the number kept.
+int selectActive(mox_ctx* c, const AdaptiveRule& rule, const uint32_t* in, uint32_t count, uint32_t remaining, uint32_t* out,
+                 uint32_t& active) {
+  uint32_t* tileSums = (uint32_t*)c->adaptiveLists.p + 2 * (size_t)c->nOwned;
+  uint32_t* survivors = tileSums + adaptiveSelectTiles(c->nOwned);
+  if (count) {
+    launchAdaptiveSelect(c->pixelStats, rule, in, count, remaining, out, tileSums, survivors, c->stream);
+    c->st.kernel_launches += 2;
+  } else CUCK(c, cudaMemsetAsync(survivors, 0, 4, c->stream));
+  CUCK(c, cudaMemcpyAsync(c->hostSurvivors.p, survivors, 4, cudaMemcpyDeviceToHost, c->stream));
+  CUCK(c, cudaStreamSynchronize(c->stream));
+  CUCK(c, cudaGetLastError());
+  active = *c->hostSurvivors.p;
+  return MOX_OK;
+}
+
+// Launches st.launches .. st.launches + spp - 1 of mox_render's seed schedule for the pixels that have not converged,
+// in rounds of round_spp launches with a convergence check after each.  beginRender and ensureAdaptive first.
+int renderAdaptive(mox_ctx* c, uint32_t spp, uint32_t seed, const mox_adaptive& p, uint64_t& traced) {
+  const AdaptiveRule rule{std::max<uint32_t>(p.min_spp, 2u), (double)p.rel_error, (double)p.abs_error};
+  uint32_t* lists[2] = {(uint32_t*)c->adaptiveLists.p, (uint32_t*)c->adaptiveLists.p + c->nOwned};
+  const uint64_t first = c->st.launches;
+  uint32_t active = 0, cur = 0, done = 0;
+  int rc = selectActive(c, rule, c->dOwned.p, c->nOwned, spp, lists[0], active);
+  while (!rc && done < spp && active) {
+    const uint32_t r = std::min(p.round_spp, spp - done);
+    std::vector<int32_t> seeds(r);
+    for (uint32_t i = 0; i < r; ++i) seeds[i] = (int32_t)tea16((uint32_t)(first + done + i), seed);
+    if ((rc = renderSeeds(c, seeds, lists[cur], active, &c->pixelStats))) break;
+    traced += (uint64_t)r * active;
+    done += r;
+    if (done == spp) break;   // a pixel that converges now sits out no launch
+    rc = selectActive(c, rule, lists[cur], active, spp - done, lists[cur ^ 1], active);
+    cur ^= 1;
+  }
+  if (rc) return rc;
+  c->st.launches = first + spp;   // the launches no pixel needed still advance the seed schedule
+  return MOX_OK;
 }
 
 constexpr int kRebuild = 1;   // refitAccel: nothing to refit, run the full build
@@ -884,6 +968,9 @@ int mox_set_globals(mox_ctx* c, uint32_t width, uint32_t height, uint32_t rayMax
     c->accuW = width; c->accuH = height;
     c->st.launches = 0;
     c->ownedDirty = true;
+    c->adaptiveStats.release();   // allocated again, zeroed, at the next mox_render_adaptive
+    c->adaptiveLists.release();
+    c->pixelStats = PixelStats();
   }
   c->rp.W = width; c->rp.H = height; c->rp.maxDepth = rayMaxDepth; c->rp.eps = rayEpsilonT; c->rp.minIntensity = rayMinIntensity;
   c->rp.absorb = make_float3(absorbColor[0], absorbColor[1], absorbColor[2]);
@@ -1103,15 +1190,73 @@ int mox_build_accel(mox_ctx* c, uint32_t flags, float* out_ms) {
 int mox_launch(mox_ctx* c, int32_t randSeed) {
   if (!c) return MOX_ERR_INVALID;
   GROUP_PAR(c, mox_launch(k, randSeed));
-  return renderSeeds(c, std::vector<int32_t>{randSeed});
+  int rc = beginRender(c);
+  return rc ? rc : renderSeeds(c, std::vector<int32_t>{randSeed}, c->dOwned.p, c->nOwned);
 }
 
 int mox_render(mox_ctx* c, uint32_t spp, uint32_t seed) {
   if (!c) return MOX_ERR_INVALID;
   GROUP_PAR(c, mox_render(k, spp, seed));
+  int rc = beginRender(c);
+  if (rc) return rc;
   std::vector<int32_t> seeds(spp);
   for (uint32_t i = 0; i < spp; ++i) seeds[i] = (int32_t)tea16((uint32_t)(c->st.launches + i), seed);
-  return renderSeeds(c, seeds);
+  return renderSeeds(c, seeds, c->dOwned.p, c->nOwned);
+}
+
+int mox_render_adaptive(mox_ctx* c, uint32_t spp, uint32_t seed, const mox_adaptive* params, uint64_t* out_samples) {
+  if (!c) return MOX_ERR_INVALID;
+  if (out_samples) *out_samples = 0;
+  if (!params) return fail(c, MOX_ERR_INVALID, "null adaptive parameters");
+  if (!params->round_spp) return fail(c, MOX_ERR_INVALID, "mox_adaptive.round_spp must be at least 1");
+  if (!std::isfinite(params->rel_error) || !std::isfinite(params->abs_error) || params->rel_error < 0.f || params->abs_error < 0.f)
+    return fail(c, MOX_ERR_INVALID, "mox_adaptive thresholds must be finite and non-negative");
+  if (c->group) {
+    std::vector<uint64_t> n(groupCount(c->group), 0);
+    int rc_ = groupParallel(c->group, [&](mox_ctx* k, int i) { return mox_render_adaptive(k, spp, seed, params, &n[i]); });
+    if (rc_) { c->err = groupError(c->group); return rc_; }
+    if (out_samples) for (uint64_t v : n) *out_samples += v;
+    return MOX_OK;
+  }
+  int rc = beginRender(c);
+  if (rc) return rc;
+  if ((rc = ensureAdaptive(c))) return rc;
+  uint64_t traced = 0;
+  rc = renderAdaptive(c, spp, seed, *params, traced);
+  if (out_samples) *out_samples = traced;
+  return rc;
+}
+
+int mox_read_sample_counts(mox_ctx* c, uint32_t* dst) {
+  if (!c) return MOX_ERR_INVALID;
+  if (!dst) return fail(c, MOX_ERR_INVALID, "null destination");
+  if (c->group) {   // every pixel is owned by one device, the others hold 0 for it
+    const mox_ctx* k0 = groupChild(c->group, 0);
+    const size_t n = (size_t)k0->accuW * k0->accuH;
+    std::vector<uint32_t> part(n);
+    std::fill(dst, dst + n, 0u);
+    for (int i = 0; i < groupCount(c->group); ++i) {
+      mox_ctx* k = groupChild(c->group, i);
+      if (int rc_ = mox_read_sample_counts(k, part.data())) { c->err = mox_last_error(k); return rc_; }
+      for (size_t p = 0; p < n; ++p) dst[p] += part[p];
+    }
+    return MOX_OK;
+  }
+  if (!c->dAccu.p) return fail(c, MOX_ERR_STATE, "no accumulation buffer (mox_set_globals first)");
+  int rc = bind(c);
+  if (rc) return rc;
+  if ((rc = refreshOwned(c))) return rc;
+  const size_t n = (size_t)c->accuW * c->accuH;
+  std::vector<uint32_t> skipped(n, 0u);
+  if (c->adaptiveStats.p) {
+    CUCK(c, cudaMemcpyAsync(skipped.data(), c->pixelStats.skipped, n * 4, cudaMemcpyDeviceToHost, c->stream));
+    CUCK(c, cudaStreamSynchronize(c->stream));
+  }
+  std::fill(dst, dst + n, 0u);
+  std::vector<uint32_t> owned;
+  ownedList(c->accuW, c->accuH, c->tile, c->world, c->rank, owned);
+  for (uint32_t p : owned) dst[p] = (uint32_t)(c->st.launches - skipped[p]);
+  return MOX_OK;
 }
 
 int mox_map_accum(mox_ctx* c, const float** out) {
@@ -1275,6 +1420,7 @@ int mox_clear_accum(mox_ctx* c) {
   int rc = bind(c);
   if (rc) return rc;
   if (c->dAccu.p) CUCK(c, cudaMemsetAsync(c->dAccu.p, 0, (size_t)c->accuW * c->accuH * 12, c->stream));
+  if ((rc = resetAdaptive(c))) return rc;
   CUCK(c, cudaStreamSynchronize(c->stream));
   const double msBuild = c->st.ms_build;   // describes the acceleration structure, not the image
   c->st = mox_stats{};
@@ -1289,6 +1435,7 @@ int mox_set_accum(mox_ctx* c, const float* src, uint64_t launches) {
   int rc = bind(c);
   if (rc) return rc;
   CUCK(c, cudaMemcpyAsync(c->dAccu.p, src, (size_t)c->accuW * c->accuH * 12, cudaMemcpyHostToDevice, c->stream));
+  if ((rc = resetAdaptive(c))) return rc;   // the loaded buffer counts as a uniform render of `launches` samples
   CUCK(c, cudaStreamSynchronize(c->stream));
   c->st.launches = launches;
   return MOX_OK;

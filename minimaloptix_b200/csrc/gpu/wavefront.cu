@@ -475,14 +475,40 @@ __global__ void __launch_bounds__(TPB) k_apply(LaunchCtx c, uint32_t count) {
   c.pb.rad[path] = make_float4(r.x, r.y, r.z, 0.f);
 }
 
+// The luminance sums of adaptive sampling for one pixel: y = 0.2126 r + 0.7152 g + 0.0722 b rounded step by step in
+// float32 (no contraction, so a host model reproduces it), y and y^2 summed in float64 in launch order.
+template <bool ADAPTIVE>
+struct LumSums {
+  __device__ __forceinline__ LumSums(const PixelStats&, uint32_t) {}
+  __device__ __forceinline__ void add(float, float, float) {}
+  __device__ __forceinline__ void store(const PixelStats&, uint32_t, uint32_t) {}
+};
+template <>
+struct LumSums<true> {
+  double s1, s2;
+  __device__ __forceinline__ LumSums(const PixelStats& ps, uint32_t pix) : s1(ps.s1[pix]), s2(ps.s2[pix]) {}
+  __device__ __forceinline__ void add(float r, float g, float b) {
+    const float y = __fadd_rn(__fadd_rn(__fmul_rn(0.2126f, r), __fmul_rn(0.7152f, g)), __fmul_rn(0.0722f, b));
+    s1 = __dadd_rn(s1, (double)y);
+    s2 = __dadd_rn(s2, __dmul_rn((double)y, (double)y));
+  }
+  __device__ __forceinline__ void store(const PixelStats& ps, uint32_t pix, uint32_t nSamples) {
+    ps.s1[pix] = s1; ps.s2[pix] = s2; ps.n[pix] += nSamples;
+  }
+};
+
 // Camera.cu:39-41 — samples of one pixel are added in launch order, so a batch of S samples
-// gives bit-identical sums to S successive launches.
-__global__ void __launch_bounds__(TPB) k_accumulate(LaunchCtx c, uint32_t nSamples) {
+// gives bit-identical sums to S successive launches.  ADAPTIVE also adds every sample's luminance to ps; the image
+// is the same.  (The body stays in the kernel: moved into an inlined helper, the plain kernel compiled to different
+// instructions.)
+template <bool ADAPTIVE>
+__global__ void __launch_bounds__(TPB) k_accumulate(LaunchCtx c, uint32_t nSamples, PixelStats ps) {
   uint32_t j = blockIdx.x * TPB + threadIdx.x;
   if (j >= c.nOwned) return;
   uint32_t pix = c.ownedPix[j];
   float* a = c.accu + 3 * (size_t)pix;
   float3 acc = mk3(a[0], a[1], a[2]);
+  LumSums<ADAPTIVE> lum(ps, pix);
   uint32_t bad = 0;
   for (uint32_t s = 0; s < nSamples; ++s) {
     const size_t p = (size_t)s * c.nOwned + j;
@@ -509,14 +535,104 @@ __global__ void __launch_bounds__(TPB) k_accumulate(LaunchCtx c, uint32_t nSampl
       // sample, counted in mox_stats.nonfinite_samples (SURVEY App. A.8).
       bad++;
       acc.x += c.rp.bad.x; acc.y += c.rp.bad.y; acc.z += c.rp.bad.z;
+      lum.add(c.rp.bad.x, c.rp.bad.y, c.rp.bad.z);
       continue;
     }
-    acc.x += clampf(r.x, 0.f, 1.f);
-    acc.y += clampf(r.y, 0.f, 1.f);
-    acc.z += clampf(r.z, 0.f, 1.f);
+    const float cx = clampf(r.x, 0.f, 1.f), cy = clampf(r.y, 0.f, 1.f), cz = clampf(r.z, 0.f, 1.f);
+    acc.x += cx;
+    acc.y += cy;
+    acc.z += cz;
+    lum.add(cx, cy, cz);
   }
   a[0] = acc.x; a[1] = acc.y; a[2] = acc.z;
+  lum.store(ps, pix, nSamples);
   if (bad) atomicAdd(c.pb.counters + C_NONFINITE, bad);
+}
+
+// ------------------------------------------------------------------ adaptive sampling: the active-pixel list
+// One tile of the list per block: SEL_ITEMS consecutive entries per thread, so the survivors of a thread, a warp and
+// a block keep their order.
+constexpr int SEL_ITEMS = 8;
+constexpr int SEL_TILE = TPB * SEL_ITEMS;
+
+// The stopping rule of mox_render_adaptive (include/mox.h), rounded step by step in float64.
+__device__ __forceinline__ bool pixelConverged(const PixelStats& ps, const AdaptiveRule& rule, uint32_t pix) {
+  const uint32_t n = ps.n[pix];
+  if (n < rule.minSpp) return false;
+  const double dn = (double)n, s1 = ps.s1[pix], s2 = ps.s2[pix];
+  const double m = __ddiv_rn(s1, dn);
+  const double var = fmax(0.0, __ddiv_rn(__dsub_rn(s2, __dmul_rn(s1, m)), __dsub_rn(dn, 1.0)));
+  const double err = __dsqrt_rn(__ddiv_rn(var, dn));
+  return err < fmax(__dmul_rn(rule.rel, m), rule.abs);
+}
+
+__device__ __forceinline__ uint32_t blockSum(uint32_t v, uint32_t* sh) {
+  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  if (lane == 0) sh[warp] = v;
+  __syncthreads();
+  uint32_t t = 0;
+#pragma unroll
+  for (int w = 0; w < TPB / 32; ++w) t += sh[w];
+  return t;
+}
+
+// Evaluates the rule for the tile's pixels, adds `remaining` to the skipped launches of the converged ones and counts
+// the survivors of the tile.
+__global__ void __launch_bounds__(TPB) k_adaptive_select(PixelStats ps, AdaptiveRule rule, const uint32_t* __restrict__ list,
+                                                         uint32_t count, uint32_t remaining, uint32_t* __restrict__ tileSums) {
+  __shared__ uint32_t sh[TPB / 32];
+  const uint32_t base = blockIdx.x * SEL_TILE + threadIdx.x * SEL_ITEMS;
+  uint32_t keep = 0;
+#pragma unroll
+  for (int k = 0; k < SEL_ITEMS; ++k) {
+    const uint32_t i = base + k;
+    if (i >= count) break;
+    const uint32_t pix = list[i];
+    if (pixelConverged(ps, rule, pix)) ps.skipped[pix] += remaining;
+    else keep++;
+  }
+  const uint32_t t = blockSum(keep, sh);
+  if (threadIdx.x == 0) tileSums[blockIdx.x] = t;
+}
+
+// Writes the survivors in list order: the tile's offset is the sum of the tile counts in front of it (a few thousand
+// words at most, L2-resident), the offset inside the tile a block scan.  The last tile writes the total.
+__global__ void __launch_bounds__(TPB) k_adaptive_compact(PixelStats ps, AdaptiveRule rule, const uint32_t* __restrict__ list,
+                                                          uint32_t count, const uint32_t* __restrict__ tileSums,
+                                                          uint32_t* __restrict__ out, uint32_t* __restrict__ survivors) {
+  __shared__ uint32_t sh[TPB / 32];
+  __shared__ uint32_t warpOff[TPB / 32];
+  uint32_t part = 0;
+  for (uint32_t t = threadIdx.x; t < blockIdx.x; t += TPB) part += tileSums[t];
+  const uint32_t tileOffset = blockSum(part, sh);
+  __syncthreads();   // sh is reused below
+  const uint32_t base = blockIdx.x * SEL_TILE + threadIdx.x * SEL_ITEMS;
+  uint32_t keepMask = 0, v = 0;
+#pragma unroll
+  for (int k = 0; k < SEL_ITEMS; ++k) {
+    const uint32_t i = base + k;
+    if (i < count && !pixelConverged(ps, rule, list[i])) { keepMask |= 1u << k; v++; }
+  }
+  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+  uint32_t incl = v;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= (uint32_t)o) incl += t; }
+  if (lane == 31) sh[warp] = incl;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    uint32_t run = 0;
+    for (int w = 0; w < TPB / 32; ++w) { warpOff[w] = run; run += sh[w]; }
+    if (blockIdx.x == gridDim.x - 1) *survivors = tileOffset + run;
+  }
+  __syncthreads();
+  uint32_t pos = tileOffset + warpOff[warp] + incl - v;
+  while (keepMask) {
+    const int k = __ffs(keepMask) - 1;
+    keepMask &= keepMask - 1u;
+    out[pos++] = list[base + k];
+  }
 }
 
 // ------------------------------------------------------------------ raw ray queries
@@ -739,7 +855,18 @@ void launchApply(const LaunchCtx& c, uint32_t disneyCount, cudaStream_t stream) 
   if (disneyCount && c.scene.nLights) k_apply<<<grid(disneyCount), TPB, 0, stream>>>(c, disneyCount);
 }
 void launchAccumulate(const LaunchCtx& c, uint32_t nSamples) {
-  if (c.nOwned) k_accumulate<<<grid(c.nOwned), TPB, 0, c.stream>>>(c, nSamples);
+  if (c.nOwned) k_accumulate<false><<<grid(c.nOwned), TPB, 0, c.stream>>>(c, nSamples, PixelStats());
+}
+void launchAccumulateAdaptive(const LaunchCtx& c, uint32_t nSamples, const PixelStats& ps) {
+  if (c.nOwned) k_accumulate<true><<<grid(c.nOwned), TPB, 0, c.stream>>>(c, nSamples, ps);
+}
+size_t adaptiveSelectTiles(uint32_t count) { return ((size_t)count + SEL_TILE - 1) / SEL_TILE; }
+void launchAdaptiveSelect(const PixelStats& ps, const AdaptiveRule& rule, const uint32_t* listIn, uint32_t count, uint32_t remaining,
+                          uint32_t* listOut, uint32_t* tileSums, uint32_t* survivors, cudaStream_t stream) {
+  if (!count) return;
+  const unsigned tiles = (unsigned)adaptiveSelectTiles(count);
+  k_adaptive_select<<<tiles, TPB, 0, stream>>>(ps, rule, listIn, count, remaining, tileSums);
+  k_adaptive_compact<<<tiles, TPB, 0, stream>>>(ps, rule, listIn, count, tileSums, listOut, survivors);
 }
 void launchSplitRays(const float4* rays, float4* o, float4* d, size_t n, cudaStream_t stream) {
   if (n) k_split_rays<<<grid(n), TPB, 0, stream>>>(rays, o, d, n);

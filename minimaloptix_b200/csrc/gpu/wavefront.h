@@ -51,6 +51,27 @@ void launchShade(const LaunchCtx& c, int kind, uint32_t count, uint32_t depth);
 void launchShadow(const LaunchCtx& c, uint32_t disneyCount, cudaStream_t stream);
 void launchApply(const LaunchCtx& c, uint32_t disneyCount, cudaStream_t stream);
 void launchAccumulate(const LaunchCtx& c, uint32_t nSamples);
+
+// Adaptive sampling (mox_render_adaptive).  Per pixel, over the samples it received from adaptive renders since the
+// last reset: the sum of the luminances y and of y^2 in float64, their number, and the launches the pixel sat out.
+struct PixelStats {
+  double *s1 = nullptr, *s2 = nullptr;
+  uint32_t *n = nullptr, *skipped = nullptr;
+};
+// The stopping rule: converged when n >= minSpp (at least 2) and sqrt(s^2 / n) < max(rel * mean, abs).
+struct AdaptiveRule {
+  uint32_t minSpp;
+  double rel, abs;
+};
+// k_accumulate, which also adds each sample's luminance to ps (same image, bit for bit).
+void launchAccumulateAdaptive(const LaunchCtx& c, uint32_t nSamples, const PixelStats& ps);
+// Words of tile sums launchAdaptiveSelect needs for `count` pixels.
+size_t adaptiveSelectTiles(uint32_t count);
+// Drops the converged pixels of listIn[0, count), adding `remaining` to their skipped launches, and writes the others
+// to listOut in their order; their number goes to *survivors.  tileSums: adaptiveSelectTiles(count) words.  Launches
+// nothing for count == 0 (*survivors is then not written).
+void launchAdaptiveSelect(const PixelStats& ps, const AdaptiveRule& rule, const uint32_t* listIn, uint32_t count, uint32_t remaining,
+                          uint32_t* listOut, uint32_t* tileSums, uint32_t* survivors, cudaStream_t stream);
 // Persistent traversal over one batch of rays (closest hit or shadow transmittance).
 void launchTraverse(const SceneView& s, const TraceJob& job, bool anyHit, bool count, cudaStream_t stream, bool classify = false);
 void launchSplitRays(const float4* rays, float4* o, float4* d, size_t n, cudaStream_t stream);

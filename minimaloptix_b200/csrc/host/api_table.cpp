@@ -22,5 +22,7 @@ bool loadMoxApi(const char* libPath, const char* prefix, MoxApi& api, std::strin
   api.read_accum_end = (int (*)(mox_ctx*, const float**))dlsym(lib, (std::string(prefix) + "read_accum_end").c_str());
   api.device_count = (int (*)(const mox_ctx*))dlsym(lib, (std::string(prefix) + "device_count").c_str());
   api.get_device_stats = (int (*)(mox_ctx*, int, mox_stats*))dlsym(lib, (std::string(prefix) + "get_device_stats").c_str());
+  api.render_adaptive = (int (*)(mox_ctx*, uint32_t, uint32_t, const mox_adaptive*, uint64_t*))dlsym(lib, (std::string(prefix) + "render_adaptive").c_str());
+  api.read_sample_counts = (int (*)(mox_ctx*, uint32_t*))dlsym(lib, (std::string(prefix) + "read_sample_counts").c_str());
   return ok;
 }

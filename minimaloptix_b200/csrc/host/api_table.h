@@ -35,6 +35,8 @@ struct MoxApi {
   int (*read_accum_end)(mox_ctx*, const float**) = nullptr;
   int (*device_count)(const mox_ctx*) = nullptr;
   int (*get_device_stats)(mox_ctx*, int, mox_stats*) = nullptr;
+  int (*render_adaptive)(mox_ctx*, uint32_t, uint32_t, const mox_adaptive*, uint64_t*) = nullptr;
+  int (*read_sample_counts)(mox_ctx*, uint32_t*) = nullptr;
 };
 
 // prefix is "mox_" for the product library.  Returns false and fills err on failure.

@@ -18,12 +18,16 @@ static void usage() {
   fprintf(stderr,
           "usage: mox_cli --scene NAME [--scene-dir DIR] [--width W --height H] [--spp N] [--max-depth D]\n"
           "               [--seed S] [--rng ref|philox] [--out PREFIX] [--snapshots] [--dump-accum] [--resume FILE.moxa] [--device K | --gpus N]\n"
-          "               [--param P] [--lib PATH] [--watertight]\n"
+          "               [--param P] [--lib PATH] [--watertight] [--adaptive REL[,ABS] [--adaptive-min N] [--adaptive-round N]]\n"
           "  NAME: spheres_lens spheres_pinhole random_spheres interior soup, or a folder under DIR\n"
           "        holding NAME.scene (coffee, cornell, ...).  Defaults are the reference's constants\n"
           "        (1920x1080, 32 spp, depth 256; MinimalOptiX.h:82-89); a .scene file's properties{width,height}\n"
           "        replace 1920x1080.  --gpus N renders on devices 0..N-1 of this process (tile-split, scene\n"
-          "        replicated, tiles gathered over NVLink into device 0).  --watertight: MOX_ACCEL_WATERTIGHT (include/mox.h).\n");
+          "        replicated, tiles gathered over NVLink into device 0).  --watertight: MOX_ACCEL_WATERTIGHT (include/mox.h).\n"
+          "  --adaptive REL[,ABS]: render with mox_render_adaptive up to --spp: a pixel stops once the standard error of its\n"
+          "        luminance is below max(REL * mean, ABS) (ABS default 0); the image is divided by each pixel's sample count.\n"
+          "        --adaptive-min N: samples before a pixel may stop (default 16); --adaptive-round N: launches between two\n"
+          "        checks (default 8).  Not combined with --snapshots, --resume or --dump-accum.\n");
 }
 
 int main(int argc, char** argv) {
@@ -31,7 +35,8 @@ int main(int argc, char** argv) {
   uint32_t W = 0, H = 0, spp = 32, depth = 256, seed = 0xC0FFEE;
   uint64_t param = 0;
   int device = 0, gpus = 0;
-  bool snapshots = false, dumpAccum = false, watertight = false;
+  bool snapshots = false, dumpAccum = false, watertight = false, adaptive = false;
+  mox_adaptive ad{8u, 16u, 0.f, 0.f};   // round_spp, min_spp, rel_error, abs_error
   for (int i = 1; i < argc; ++i) {
     std::string a = argv[i];
     auto val = [&]() -> const char* { if (i + 1 >= argc) { usage(); exit(2); } return argv[++i]; };
@@ -52,7 +57,22 @@ int main(int argc, char** argv) {
     else if (a == "--gpus") gpus = atoi(val());
     else if (a == "--param") param = strtoull(val(), nullptr, 0);
     else if (a == "--lib") lib = val();
+    else if (a == "--adaptive") {
+      const char* v = val();
+      char* end = nullptr;
+      adaptive = true;
+      ad.rel_error = strtof(v, &end);
+      if (*end == ',') ad.abs_error = strtof(end + 1, &end);
+      if (*end) { fprintf(stderr, "--adaptive wants REL or REL,ABS, got %s\n", v); return 2; }
+    }
+    else if (a == "--adaptive-min") ad.min_spp = (uint32_t)atoi(val());
+    else if (a == "--adaptive-round") ad.round_spp = (uint32_t)atoi(val());
     else { usage(); return 2; }
+  }
+  if (adaptive && (snapshots || !resume.empty() || dumpAccum)) {
+    fprintf(stderr, "--adaptive renders a different number of samples per pixel; it cannot be combined with --snapshots, --resume "
+                    "or --dump-accum, which assume the same count everywhere\n");
+    return 2;
   }
   if (lib.empty()) {
     std::string self = argv[0];
@@ -81,6 +101,7 @@ int main(int argc, char** argv) {
     for (int i = 0; i < gpus; ++i) ids[i] = i;
     if (api.create_multi(&ctx, ids.data(), gpus)) { fprintf(stderr, "mox_create_multi: %s\n", api.last_error(nullptr)); return 1; }
   } else if (api.create(&ctx, device)) { fprintf(stderr, "mox_create: %s\n", api.last_error(nullptr)); return 1; }
+  if (adaptive && !(api.render_adaptive && api.read_sample_counts)) { fprintf(stderr, "%s has no mox_render_adaptive\n", lib.c_str()); return 1; }
   api.set_rng_mode(ctx, rng == "philox" ? MOX_RNG_PHILOX : MOX_RNG_REF);
   if (!moxh::uploadScene(sc, api, ctx, W, H, depth, err)) { fprintf(stderr, "upload: %s\n", err.c_str()); return 1; }
   float buildMs = 0;
@@ -88,6 +109,7 @@ int main(int argc, char** argv) {
 
   std::vector<float> accum((size_t)W * H * 3);
   std::vector<uint8_t> rgb((size_t)W * H * 3);
+  std::vector<uint32_t> counts(adaptive ? (size_t)W * H : 0);
   // a snapshot = updateContent (MinimalOptiX.cpp:556-560): map the accumulation buffer (on several GPUs: gather the
   // tiles into device 0 over NVLink), quantise, write the image
   double readSec = 0, writeSec = 0;
@@ -96,7 +118,10 @@ int main(int argc, char** argv) {
     auto a0 = std::chrono::steady_clock::now();
     api.read_accum(ctx, accum.data());
     auto a1 = std::chrono::steady_clock::now();
-    moxh_accum_to_rgb8(accum.data(), W, H, (float)n, rgb.data());
+    if (adaptive) {
+      api.read_sample_counts(ctx, counts.data());
+      moxh_accum_to_rgb8_counts(accum.data(), W, H, counts.data(), rgb.data());
+    } else moxh_accum_to_rgb8(accum.data(), W, H, (float)n, rgb.data());
     if (moxh_write_image((name + ".png").c_str(), rgb.data(), W, H)) fprintf(stderr, "write: %s\n", moxh_last_error());
     readSec += std::chrono::duration<double>(a1 - a0).count();
     writeSec += std::chrono::duration<double>(std::chrono::steady_clock::now() - a1).count();
@@ -110,7 +135,12 @@ int main(int argc, char** argv) {
     done = (uint32_t)std::min<uint64_t>(launches, spp);
     while (checkpoint <= done) checkpoint *= 2;
   }
+  uint64_t samples = (uint64_t)W * H * (spp - done);
   auto t0 = std::chrono::steady_clock::now();
+  if (adaptive) {
+    if (api.render_adaptive(ctx, spp, seed, &ad, &samples)) { fprintf(stderr, "render_adaptive: %s\n", api.last_error(ctx)); return 1; }
+    done = spp;
+  }
   while (done < spp) {  // renderScene: snapshots at 1, 2, 4, ... (MinimalOptiX.cpp:543-553)
     uint32_t n = snapshots ? std::min(spp, checkpoint) - done : spp - done;
     if (api.render(ctx, n, seed)) { fprintf(stderr, "render: %s\n", api.last_error(ctx)); return 1; }
@@ -122,18 +152,25 @@ int main(int argc, char** argv) {
   if (dumpAccum) moxh_write_accum((out + ".moxa").c_str(), accum.data(), W, H, spp);
   mox_stats st;
   api.get_stats(ctx, &st);
+  // share of the pixels that received every launch (1 for a uniform render)
+  double activeEnd = 1.0;
+  if (adaptive) {
+    uint64_t full = 0;
+    for (uint32_t n : counts) full += n == spp;
+    activeEnd = (double)full / ((double)W * H);
+  }
   double rays = (double)(st.rays_primary + st.rays_bounce);
   printf("{\"scene\": \"%s\", \"width\": %u, \"height\": %u, \"spp\": %u, \"max_depth\": %u, \"seed\": %u, \"rng\": \"%s\", "
          "\"triangles\": %u, \"prims\": %u, \"bvh_build_ms\": %.3f, \"render_ms\": %.3f, \"wall_s\": %.3f, "
          "\"rays_primary\": %llu, \"rays_bounce\": %llu, \"rays_shadow\": %llu, \"mrays_per_s\": %.2f, \"mshadow_per_s\": %.2f, "
          "\"spp_per_s\": %.3f, \"nonfinite\": %llu, \"gpus\": %d, \"ms_extend\": %.2f, \"ms_shade\": %.2f, \"ms_shadow\": %.2f, "
          "\"kernel_launches\": %llu, \"snapshots\": %u, \"gather_and_readback_s\": %.4f, \"quantise_and_png_s\": %.3f, "
-         "\"render_ms_per_gpu\": [",
+         "\"samples\": %llu, \"active_fraction_end\": %.4f, \"render_ms_per_gpu\": [",
          scene.c_str(), W, H, spp, depth, seed, rng.c_str(), st.n_triangles, st.n_prims, buildMs, st.ms_render, sec,
          (unsigned long long)st.rays_primary, (unsigned long long)st.rays_bounce, (unsigned long long)st.rays_shadow,
          rays / (st.ms_render * 1e3), (double)st.rays_shadow / (st.ms_render * 1e3), spp / (st.ms_render * 1e-3),
          (unsigned long long)st.nonfinite_samples, gpus > 0 ? gpus : 1, st.ms_extend, st.ms_shade, st.ms_shadow,
-         (unsigned long long)st.kernel_launches, nSnapshots, readSec, writeSec);
+         (unsigned long long)st.kernel_launches, nSnapshots, readSec, writeSec, (unsigned long long)samples, activeEnd);
   const int nDev = api.device_count ? api.device_count(ctx) : 1;
   for (int i = 0; i < nDev; ++i) {
     mox_stats ds = st;

@@ -155,6 +155,9 @@ int moxh_scene_apply_spheres(const moxh_scene* s, const moxh_api* api, void* ctx
 }
 
 void moxh_accum_to_rgb8(const float* accum, uint32_t w, uint32_t h, float n, uint8_t* out) { accumToRgb8(accum, w, h, n, out); }
+void moxh_accum_to_rgb8_counts(const float* accum, uint32_t w, uint32_t h, const uint32_t* counts, uint8_t* out) {
+  accumToRgb8Counts(accum, w, h, counts, out);
+}
 int moxh_write_image(const char* path, const uint8_t* rgb, uint32_t w, uint32_t h) {
   std::string err;
   return writeImage(path, rgb, w, h, err) ? 0 : fail(err);

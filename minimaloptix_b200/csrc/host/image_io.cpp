@@ -32,6 +32,20 @@ void accumToRgb8(const float* accum, uint32_t W, uint32_t H, float nAccum, uint8
     }
 }
 
+void accumToRgb8Counts(const float* accum, uint32_t W, uint32_t H, const uint32_t* counts, uint8_t* out) {
+  for (uint32_t i = 0; i < H; ++i)
+    for (uint32_t j = 0; j < W; ++j) {
+      const size_t p = (size_t)i * W + j;
+      const float* src = accum + 3 * p;
+      uint8_t* dst = out + 3 * ((size_t)(H - 1 - i) * W + j);
+      if (!counts[p]) { dst[0] = dst[1] = dst[2] = 0; continue; }   // a pixel nobody rendered
+      const float n = (float)counts[p];
+      dst[0] = quantise(src[0] / n);
+      dst[1] = quantise(src[1] / n);
+      dst[2] = quantise(src[2] / n);
+    }
+}
+
 namespace {
 uint32_t crcTable[256];
 bool crcInit = false;

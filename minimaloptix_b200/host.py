@@ -54,6 +54,7 @@ def lib():
         L.moxh_scene_animate.argtypes = [_vp, C.c_float]
         L.moxh_scene_apply_spheres.argtypes = [_vp, _vp, _vp]
         L.moxh_accum_to_rgb8.argtypes = [_vp, _u32, _u32, C.c_float, _vp]
+        L.moxh_accum_to_rgb8_counts.argtypes = [_vp, _u32, _u32, _vp, _vp]
         L.moxh_write_image.argtypes = [C.c_char_p, _vp, _u32, _u32]
         L.moxh_write_accum.argtypes = [C.c_char_p, _vp, _u32, _u32, _u64]
         L.moxh_read_accum.argtypes = [C.c_char_p, _vp, _u32, _u32, C.POINTER(_u64)]
@@ -213,6 +214,18 @@ def accum_to_rgb8(accum, n_accum):
     h, w = a.shape[:2]
     out = np.empty((h, w, 3), dtype=np.uint8)
     lib().moxh_accum_to_rgb8(a.ctypes.data_as(_vp), w, h, float(n_accum), out.ctypes.data_as(_vp))
+    return out
+
+
+def accum_to_rgb8_counts(accum, counts):
+    """accum_to_rgb8 with a sample count per pixel ((H, W), as read_sample_counts returns it); 0 gives black."""
+    a = np.ascontiguousarray(accum, dtype=np.float32)
+    n = np.ascontiguousarray(counts, dtype=np.uint32)
+    h, w = a.shape[:2]
+    if n.shape != (h, w):
+        raise ValueError(f"counts of shape {n.shape} for a {h}x{w} image")
+    out = np.empty((h, w, 3), dtype=np.uint8)
+    lib().moxh_accum_to_rgb8_counts(a.ctypes.data_as(_vp), w, h, n.ctypes.data_as(_vp), out.ctypes.data_as(_vp))
     return out
 
 

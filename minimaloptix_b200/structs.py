@@ -82,12 +82,17 @@ class Stats(C.Structure):
         return {k: (list(getattr(self, k)) if hasattr(getattr(self, k), "__len__") else getattr(self, k)) for k, _ in self._fields_}
 
 
+class Adaptive(C.Structure):
+    """mox_adaptive: the rounds and thresholds of mox_render_adaptive."""
+    _fields_ = [("round_spp", C.c_uint32), ("min_spp", C.c_uint32), ("rel_error", C.c_float), ("abs_error", C.c_float)]
+
+
 MAT_LAMBERTIAN, MAT_METAL, MAT_GLASS, MAT_DISNEY, MAT_LIGHT = range(5)
 RNG_REF, RNG_PHILOX = 0, 1
 ACCEL_DEFAULT, ACCEL_LBVH, ACCEL_COUNTERS, ACCEL_BINARY, ACCEL_WATERTIGHT = 0, 1, 2, 4, 8
 ACCEL_REFIT = 16   # refit the last full build in place (mox.h MOX_ACCEL_REFIT)
 
 SIZES = {Payload: 32, CamParams: 76, SphereParams: 28, QuadParams: 64, LambertianParams: 12, MetalParams: 16,
-         GlassParams: 16, DisneyParams: 72, LightParams: 72}
+         GlassParams: 16, DisneyParams: 72, LightParams: 72, Adaptive: 16}
 for _t, _s in SIZES.items():
     assert C.sizeof(_t) == _s, (_t.__name__, C.sizeof(_t), _s)
