@@ -63,8 +63,12 @@ struct PlocScratch {
 };
 size_t plocScratchBytes(int n);
 bool plocAlloc(PlocScratch& s, int n, DeviceArena& arena, std::string& err);
-bool plocBuild(PlocScratch& s, int n, const uint32_t* sortedIds, const float4* primLo, const float4* primHi, int radius,
-               BvhNode2* outNodes, float rootLo[3], float rootHi[3], int* maxDepthOut, cudaStream_t stream, std::string& err);
+// NOT_CONVERGED: the clustering ran out of iterations before one cluster was left (many primitives with the same box
+// merge one pair per iteration); the caller builds another hierarchy.  ERROR: a CUDA error or an inconsistent state,
+// described in err.
+enum class PlocResult { OK, NOT_CONVERGED, ERROR };
+PlocResult plocBuild(PlocScratch& s, int n, const uint32_t* sortedIds, const float4* primLo, const float4* primHi, int radius,
+                     BvhNode2* outNodes, float rootLo[3], float rootHi[3], int* maxDepthOut, cudaStream_t stream, std::string& err);
 
 // What an in-place refit (refitBvh) needs from the last full build.  Every pointer is a slice of the build's
 // DeviceArena.  Nothing takes from the arena between two full builds, so the slices stay valid until the next

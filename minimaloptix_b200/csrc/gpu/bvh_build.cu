@@ -585,8 +585,10 @@ bool buildBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::
   out.nNodes = nInner;
   if (in.usePloc) {
     std::string perr;
-    if (!plocBuild(ploc, nValid, vin, boxLo, boxHi, in.plocRadius > 0 ? in.plocRadius : (nValid > 2000000 ? 16 : 32), out.nodes, out.sceneLo, out.sceneHi, &out.maxDepth, stream, perr)) return bail(perr);
-    if (out.maxDepth <= MOX_TRAVERSAL_STACK - 2) {
+    const PlocResult pr = plocBuild(ploc, nValid, vin, boxLo, boxHi, in.plocRadius > 0 ? in.plocRadius : (nValid > 2000000 ? 16 : 32),
+                                    out.nodes, out.sceneLo, out.sceneHi, &out.maxDepth, stream, perr);
+    if (pr == PlocResult::ERROR) return bail(perr);
+    if (pr == PlocResult::OK && out.maxDepth <= MOX_TRAVERSAL_STACK - 2) {
     k_pack<<<divUp(nValid, B), B, 0, stream>>>(nValid, ploc.orderedIds, in.prims, in.tris, in.verts, in.analytic, in.mats, out.packed, in.watertight);
     if (wantWide) {
       uint32_t* ordered8 = nullptr;
@@ -604,7 +606,8 @@ bool buildBvh(const BuildInput& in, BuildOutput& out, cudaStream_t stream, std::
     rs.path = RefitState::PLOC;
     return true;
     }
-    // too deep for the traversal stack: fall through to the radix tree (depth <= 62)
+    // PLOC did not converge (many coincident primitives), or its tree is too deep for the traversal stack: fall through
+    // to the radix tree (depth <= 62)
     k_pack<<<divUp(nValid, B), B, 0, stream>>>(nValid, vin, in.prims, in.tris, in.verts, in.analytic, in.mats, out.packed, in.watertight);
   }
   k_karras<<<divUp(nInner, B), B, 0, stream>>>(nValid, kin, children, range, parentInternal, parentLeaf);

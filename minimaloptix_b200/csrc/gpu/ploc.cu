@@ -363,7 +363,8 @@ inline int divUp(size_t a, size_t b) { return (int)((a + b - 1) / b); }
 
 }  // namespace
 
-#define PCK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { err = std::string(#x) + ": " + cudaGetErrorString(e_); return false; } } while (0)
+// On a CUDA error: describe it in err and return `failed`.
+#define PCK(x, failed) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { err = std::string(#x) + ": " + cudaGetErrorString(e_); return failed; } } while (0)
 
 size_t plocScratchBytes(int n) {
   const size_t nn = (size_t)std::max(n, 2);
@@ -391,8 +392,8 @@ bool plocAlloc(PlocScratch& s, int n, DeviceArena& a, std::string& err) {
 
 // n >= 2 valid primitives in Morton order (sortedIds); primLo/primHi indexed by primitive id.
 // Writes n-1 nodes to outNodes (root = node 0) and the leaf-ordered ids to s.orderedIds.
-bool plocBuild(PlocScratch& s, int n, const uint32_t* sortedIds, const float4* primLo, const float4* primHi, int radius,
-               BvhNode2* outNodes, float rootLo[3], float rootHi[3], int* maxDepthOut, cudaStream_t stream, std::string& err) {
+PlocResult plocBuild(PlocScratch& s, int n, const uint32_t* sortedIds, const float4* primLo, const float4* primHi, int radius,
+                     BvhNode2* outNodes, float rootLo[3], float rootHi[3], int* maxDepthOut, cudaStream_t stream, std::string& err) {
   radius = std::max(1, std::min(radius, PL_MAX_RADIUS));
   const int B = 256;
   k_ploc_init<<<divUp(n, B), B, 0, stream>>>(n, sortedIds, primLo, primHi, s.cid[0], s.cLo[0], s.cHi[0], s.nodeLo, s.nodeHi, s.size);
@@ -404,11 +405,13 @@ bool plocBuild(PlocScratch& s, int n, const uint32_t* sortedIds, const float4* p
   {
     PlocState s0{n, 0u, 0u, 0u};
     *hostState = s0;
-    PCK(cudaMemcpyAsync(st, hostState, sizeof s0, cudaMemcpyHostToDevice, stream));
+    PCK(cudaMemcpyAsync(st, hostState, sizeof s0, cudaMemcpyHostToDevice, stream), PlocResult::ERROR);
   }
   int it = 0;
   while (count > PL_TAIL) {
-    if (it + PL_BATCH >= PL_MAX_ITERS) { err = "PLOC made no progress"; return false; }
+    // Out of state slots.  Many primitives with the same box get here: equal merged areas tie towards the smaller
+    // index, so each iteration merges a single pair of them.
+    if (it + PL_BATCH >= PL_MAX_ITERS) return PlocResult::NOT_CONVERGED;
     // PL_BATCH iterations on the device's own counts; grids cover `count`, the last value the host has seen
     const int nTiles = divUp(count, PL_TILE);
     for (int b = 0; b < PL_BATCH; ++b, ++it) {
@@ -419,10 +422,10 @@ bool plocBuild(PlocScratch& s, int n, const uint32_t* sortedIds, const float4* p
                                                        s.cid[c ^ 1], s.cLo[c ^ 1], s.cHi[c ^ 1], s.nodeLo, s.nodeHi, s.children,
                                                        s.parent, s.size);
     }
-    PCK(cudaMemcpyAsync(hostState, st + it, sizeof(PlocState), cudaMemcpyDeviceToHost, stream));
-    PCK(cudaStreamSynchronize(stream));
+    PCK(cudaMemcpyAsync(hostState, st + it, sizeof(PlocState), cudaMemcpyDeviceToHost, stream), PlocResult::ERROR);
+    PCK(cudaStreamSynchronize(stream), PlocResult::ERROR);
     const PlocState got = *hostState;
-    if (got.count >= count || got.count < 1 || (int)got.nodeBase != n - got.count) { err = "PLOC made no progress"; return false; }
+    if (got.count >= count || got.count < 1 || (int)got.nodeBase != n - got.count) { err = "PLOC made no progress"; return PlocResult::ERROR; }
     count = got.count;
     nodeBase = got.nodeBase;
     cur = (int)(got.iters & 1u);   // iterations that ran (the no-op ones at the end of a batch do not swap buffers)
@@ -432,35 +435,35 @@ bool plocBuild(PlocScratch& s, int n, const uint32_t* sortedIds, const float4* p
     k_ploc_tail<<<1, PL_TAIL, 0, stream>>>(count, n, radius, nodeBase, s.cid[cur], s.cLo[cur], s.cHi[cur], s.nodeLo, s.nodeHi, s.children,
                                            s.parent, s.size, dCreated);
     uint32_t created = 0;
-    PCK(cudaMemcpyAsync(&created, dCreated, 4, cudaMemcpyDeviceToHost, stream));
-    PCK(cudaStreamSynchronize(stream));
+    PCK(cudaMemcpyAsync(&created, dCreated, 4, cudaMemcpyDeviceToHost, stream), PlocResult::ERROR);
+    PCK(cudaStreamSynchronize(stream), PlocResult::ERROR);
     nodeBase = created;
   }
   const int nInner = n - 1;
-  if ((int)nodeBase != nInner) { err = "PLOC node count mismatch"; return false; }
+  if ((int)nodeBase != nInner) { err = "PLOC node count mismatch"; return PlocResult::ERROR; }
   const uint32_t root = (uint32_t)(n + nInner - 1);
   uint32_t* dDepth = (uint32_t*)(dTotal + 1);
-  PCK(cudaMemsetAsync(dDepth, 0, 4, stream));
+  PCK(cudaMemsetAsync(dDepth, 0, 4, stream), PlocResult::ERROR);
   k_ploc_leaf_order<<<divUp(n, B), B, 0, stream>>>(n, root, s.parent, s.children, s.size, sortedIds, s.leafPos, s.orderedIds, s.firstPos, dDepth);
   k_ploc_emit<<<divUp(nInner, B), B, 0, stream>>>(n, nInner, root, s.parent, s.children, s.size, s.leafPos, s.firstPos, s.nodeLo, s.nodeHi, outNodes);
   float4 lo, hi;
-  PCK(cudaMemcpyAsync(&lo, s.nodeLo + root, 16, cudaMemcpyDeviceToHost, stream));
-  PCK(cudaMemcpyAsync(&hi, s.nodeHi + root, 16, cudaMemcpyDeviceToHost, stream));
+  PCK(cudaMemcpyAsync(&lo, s.nodeLo + root, 16, cudaMemcpyDeviceToHost, stream), PlocResult::ERROR);
+  PCK(cudaMemcpyAsync(&hi, s.nodeHi + root, 16, cudaMemcpyDeviceToHost, stream), PlocResult::ERROR);
   uint32_t depth = 0;
-  PCK(cudaMemcpyAsync(&depth, dDepth, 4, cudaMemcpyDeviceToHost, stream));
-  PCK(cudaStreamSynchronize(stream));
-  PCK(cudaGetLastError());
+  PCK(cudaMemcpyAsync(&depth, dDepth, 4, cudaMemcpyDeviceToHost, stream), PlocResult::ERROR);
+  PCK(cudaStreamSynchronize(stream), PlocResult::ERROR);
+  PCK(cudaGetLastError(), PlocResult::ERROR);
   *maxDepthOut = (int)depth;
   rootLo[0] = lo.x; rootLo[1] = lo.y; rootLo[2] = lo.z;
   rootHi[0] = hi.x; rootHi[1] = hi.y; rootHi[2] = hi.z;
-  return true;
+  return PlocResult::OK;
 }
 
 bool plocRefit(const PlocScratch& s, int n, const uint32_t* sortedIds, const float4* primLo, const float4* primHi, uint32_t* arrivals,
                BvhNode2* outNodes, cudaStream_t stream, std::string& err) {
   const int B = 256, nInner = n - 1;
   const uint32_t root = (uint32_t)(n + nInner - 1);
-  PCK(cudaMemsetAsync(arrivals, 0, (size_t)nInner * 4, stream));
+  PCK(cudaMemsetAsync(arrivals, 0, (size_t)nInner * 4, stream), false);
   k_ploc_refit<<<divUp(n, B), B, 0, stream>>>(n, root, sortedIds, primLo, primHi, s.children, s.parent, s.nodeLo, s.nodeHi, arrivals);
   k_ploc_emit<<<divUp(nInner, B), B, 0, stream>>>(n, nInner, root, s.parent, s.children, s.size, s.leafPos, s.firstPos, s.nodeLo, s.nodeHi, outNodes);
   return true;

@@ -46,12 +46,35 @@ def check_ids(o, g, rays, name):
     return len(bad), int((io >= 0).sum())
 
 
-@pytest.mark.parametrize("n", [1, 31, 4096, 4097, 100000, (1 << 20) + 17])
-def test_radix_sort_matches_stable_sort(gpu_backend, n):
+def _sort_keys(rng, n, kind):
+    if kind == "morton":   # 30-bit Morton-like keys with heavy duplication in the low bits
+        return (rng.integers(0, 1 << 30, size=n, dtype=np.uint32) & np.uint32(0x3FFF00FF)).astype(np.uint32)
+    if kind == "full32":   # every digit of every pass, 0 and 0xFFFFFFFF included
+        keys = rng.integers(0, 1 << 32, size=n, dtype=np.uint64).astype(np.uint32)
+        keys[rng.integers(0, n, size=min(n, 8))] = 0xFFFFFFFF
+        keys[rng.integers(0, n, size=min(n, 8))] = 0
+        return keys
+    if kind == "invalid":  # Morton codes with k_morton's key of an invalid primitive mixed in
+        keys = rng.integers(0, 1 << 30, size=n, dtype=np.uint32)
+        keys[rng.random(n) < 0.2] = 0x40000000
+        return keys
+    if kind == "equal":
+        return np.full(n, 0x2AAAAAAA, np.uint32)
+    if kind == "descending":
+        return (np.uint32(0xFFFFFFFF) - np.arange(n, dtype=np.uint32) * np.uint32(977)).astype(np.uint32)
+    raise ValueError(kind)
+
+
+# n at the edges of the 4096-key sort tile (256 threads x 16 keys)
+@pytest.mark.parametrize("n, kind", [pytest.param(n, "morton", id=str(n)) for n in [1, 31, 4096, 4097, 100000, (1 << 20) + 17]]
+                         + [pytest.param(n, k, id=f"{k}-{n}") for k, n in [("full32", 4095), ("full32", 8193), ("full32", (1 << 20) + 17),
+                                                                          ("invalid", 4096), ("invalid", 100000), ("equal", 1), ("equal", 8192),
+                                                                          ("equal", 12289), ("descending", 4097), ("descending", 65536),
+                                                                          ("morton", 4095), ("morton", 8191), ("morton", 8192)]])
+def test_radix_sort_matches_stable_sort(gpu_backend, n, kind):
     g = gpu_backend.context(0)
     rng = np.random.default_rng(n)
-    # 30-bit Morton-like keys with heavy duplication in the low bits
-    keys = (rng.integers(0, 1 << 30, size=n, dtype=np.uint32) & np.uint32(0x3FFF00FF)).astype(np.uint32)
+    keys = _sort_keys(rng, n, kind)
     vals = np.arange(n, dtype=np.uint32)
     k, v = g.debug_radix_sort(keys, vals)
     order = np.argsort(keys, kind="stable")
