@@ -111,13 +111,34 @@ MOX_D float slabRcp(float x) {
   asm("rcp.approx.f32 %0, %1;" : "=f"(r) : "f"(x));
   return r;
 }
+// A component of magnitude at most 1e-30 counts as zero: the ray then stays in that axis' slab for every t when
+// lo <= o <= hi and never otherwise (oracle.cpp::slab).  What 1/d becomes for it depends on the slab test that reads it.
+//  * boxEntry (binary BVH, WIDE = false): +-inf.  A plane term is then +-inf, or NaN (0 * inf) for an origin on the
+//    plane, which boxEntry drops from its near or its far side: the axis culls exactly by the rule above.
+//  * the wide node step (WIDE = true): +1e30 whatever the sign of the zero, so that the axis keeps culling with finite
+//    terms and its far planes are the high ones.  A far term is 0 only for a plane through the origin, and the node
+//    step's 2^-21 slack of the origin term (planeTerms) lifts every far plane above the node's own origin plane to a
+//    huge t; what is left is a child flat at the node's origin plane with the ray running in that plane.  Every
+//    primitive of such a child lies in the ray's plane, and no primitive test accepts a ray lying in its plane (the
+//    product of the ray with the plane normal is exactly 0).  With the sign kept (-1e30 for -0) the far planes of
+//    such a ray would be the low ones, and every child starting at the node's origin plane would be culled.
+// (A clamp of +-1e30 with the sign kept culled both kinds of hit: (hi - o) * 1e30 = 0 put the far plane at t = 0.)
+template <bool WIDE>
 MOX_D RayPre prepRay(const float3& o, const float3& d, float tmin) {
   RayPre r;
   r.o = o; r.d = d; r.tmin = tmin;
   const float tiny = 1e-30f;
-  r.idir.x = slabRcp(fabsf(d.x) > tiny ? d.x : copysignf(tiny, d.x));
-  r.idir.y = slabRcp(fabsf(d.y) > tiny ? d.y : copysignf(tiny, d.y));
-  r.idir.z = slabRcp(fabsf(d.z) > tiny ? d.z : copysignf(tiny, d.z));
+  const float rx = slabRcp(d.x), ry = slabRcp(d.y), rz = slabRcp(d.z);   // (unconditionally: selects, no branches)
+  if (WIDE) {
+    r.idir.x = fabsf(d.x) > tiny ? rx : 1e30f;
+    r.idir.y = fabsf(d.y) > tiny ? ry : 1e30f;
+    r.idir.z = fabsf(d.z) > tiny ? rz : 1e30f;
+  } else {
+    const float inf = __int_as_float(0x7f800000);
+    r.idir.x = fabsf(d.x) > tiny ? rx : copysignf(inf, d.x);
+    r.idir.y = fabsf(d.y) > tiny ? ry : copysignf(inf, d.y);
+    r.idir.z = fabsf(d.z) > tiny ? rz : copysignf(inf, d.z);
+  }
   return r;
 }
 
@@ -130,13 +151,17 @@ MOX_D uint32_t originIndex(const TraceJob& job, uint32_t id) {
   return (int32_t)r < 0 ? r + job.originMod : r;
 }
 
-// Entry distance of the slab test, or +inf when the box is missed within [tmin, tcur].
+// Entry distance of the slab test, or +inf when the box is missed within [tmin, tcur].  Near and far planes are
+// picked by the sign of 1/d, so that a NaN term (zero component, origin on the plane) is dropped from the near side
+// or from the far side as it belongs; fminf / fmaxf of the two terms of an axis would turn (-inf, NaN) into an
+// empty slab.
 MOX_D float boxEntry(const RayPre& r, float lox, float hix, float loy, float hiy, float loz, float hiz, float tcur) {
-  float x0 = (lox - r.o.x) * r.idir.x, x1 = (hix - r.o.x) * r.idir.x;
-  float y0 = (loy - r.o.y) * r.idir.y, y1 = (hiy - r.o.y) * r.idir.y;
-  float z0 = (loz - r.o.z) * r.idir.z, z1 = (hiz - r.o.z) * r.idir.z;
-  float tn = fmaxf(fmaxf(fminf(x0, x1), fminf(y0, y1)), fmaxf(fminf(z0, z1), r.tmin));
-  float tf = fminf(fminf(fmaxf(x0, x1), fmaxf(y0, y1)), fminf(fmaxf(z0, z1), tcur)) * 1.00001f;
+  const bool nx = r.idir.x < 0.f, ny = r.idir.y < 0.f, nz = r.idir.z < 0.f;
+  float x0 = ((nx ? hix : lox) - r.o.x) * r.idir.x, x1 = ((nx ? lox : hix) - r.o.x) * r.idir.x;
+  float y0 = ((ny ? hiy : loy) - r.o.y) * r.idir.y, y1 = ((ny ? loy : hiy) - r.o.y) * r.idir.y;
+  float z0 = ((nz ? hiz : loz) - r.o.z) * r.idir.z, z1 = ((nz ? loz : hiz) - r.o.z) * r.idir.z;
+  float tn = fmaxf(fmaxf(x0, y0), fmaxf(z0, r.tmin));
+  float tf = fminf(fminf(x1, y1), fminf(z1, tcur)) * 1.00001f;
   return tn <= tf ? tn : __int_as_float(0x7f800000);
 }
 
@@ -205,7 +230,7 @@ __device__ __forceinline__ void traverseWarpPersistent(const SceneView& s, const
             const uint32_t oId = originIndex(job, rayId);
             float4 ro = MOX_LD_STREAM(job.rayO + oId), rd = MOX_LD_STREAM(job.rayD + rayId);
             if (!(ANYHIT && rd.w < 0.f)) {
-              r = prepRay(mk3(ro), mk3(rd), ro.w);
+              r = prepRay<false>(mk3(ro), mk3(rd), ro.w);
               if (WT) wr = wtPrep(r.d);
               tBest = rd.w; bPrim = -1; bBeta = 0.f; bGamma = 0.f;
               atten = mk3(1.f);

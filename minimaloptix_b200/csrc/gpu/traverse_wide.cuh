@@ -156,10 +156,10 @@ __device__ __forceinline__ void traverseWidePersistent(const SceneView& s, const
           const uint32_t oId = originIndex(job, rayId);
           float4 ro = MOX_LD_STREAM(job.rayO + oId), rd = MOX_LD_STREAM(job.rayD + rayId);
           if (!(ANYHIT && rd.w < 0.f)) {
-            RayPre r = prepRay(mk3(ro), mk3(rd), ro.w);
+            RayPre r = prepRay<true>(mk3(ro), mk3(rd), ro.w);
             o = r.o; d = r.d; idir = r.idir; tmin = r.tmin;
             if (WT) wr = wtPrep(d);
-            octinv = 7u ^ ((idir.x < 0.f ? 4u : 0u) | (idir.y < 0.f ? 2u : 0u) | (idir.z < 0.f ? 1u : 0u));   // (-0.0 counts as negative here)
+            octinv = 7u ^ ((idir.x < 0.f ? 4u : 0u) | (idir.y < 0.f ? 2u : 0u) | (idir.z < 0.f ? 1u : 0u));   // (a zero component counts as positive, prepRay)
             tBest = rd.w; bPrim = -1;
             if (!CLASSIFY) { bBeta = 0.f; bGamma = 0.f; }
             tinted = false;

@@ -291,14 +291,26 @@ inline void testPrimClosest(const orc_ctx& c, int id, const Ray& ray, HitAttr& b
   }
 }
 
+// One axis of the slab test.  A direction component of magnitude at most 1e-30 (where the GPU's prepRay stops
+// taking 1/d) counts as zero: the ray then stays in the slab for every t when lo <= o <= hi, and never otherwise.
+// (With 1/d itself, an origin on a plane gives (lo - o) * inf = 0 * inf = NaN; with 1/d clamped, a ray on the far
+// plane whose component is "+0 outwards" leaves the slab at t = 0.  Both culled hits on the plane that the
+// primitive test accepts.)
+inline bool slab(float lo, float hi, float o, float d, float inv, float& tn, float& tf) {
+  if (fabsf(d) <= 1e-30f) return lo <= o && o <= hi;
+  float t0 = (lo - o) * inv, t1 = (hi - o) * inv;
+  tn = fmaxf(tn, fminf(t0, t1));
+  tf = fminf(tf, fmaxf(t0, t1));
+  return true;
+}
+
 // Slab test, padded so it never rejects a box whose primitive test could accept.
-inline bool hitBox(const float3& lo, const float3& hi, const float3& o, const float3& inv, float tmin, float tmax) {
-  float tx0 = (lo.x - o.x) * inv.x, tx1 = (hi.x - o.x) * inv.x;
-  float ty0 = (lo.y - o.y) * inv.y, ty1 = (hi.y - o.y) * inv.y;
-  float tz0 = (lo.z - o.z) * inv.z, tz1 = (hi.z - o.z) * inv.z;
-  // fmin/fmax drop NaNs (0 * inf) the conservative way.
-  float tn = fmaxf(fmaxf(fminf(tx0, tx1), fminf(ty0, ty1)), fmaxf(fminf(tz0, tz1), tmin));
-  float tf = fminf(fminf(fmaxf(tx0, tx1), fmaxf(ty0, ty1)), fminf(fmaxf(tz0, tz1), tmax));
+inline bool hitBox(const float3& lo, const float3& hi, const float3& o, const float3& d, const float3& inv, float tmin,
+                   float tmax) {
+  float tn = tmin, tf = tmax;
+  if (!slab(lo.x, hi.x, o.x, d.x, inv.x, tn, tf) || !slab(lo.y, hi.y, o.y, d.y, inv.y, tn, tf) ||
+      !slab(lo.z, hi.z, o.z, d.z, inv.z, tn, tf))
+    return false;
   // tn >= tmin >= 0 here; widen the interval by a relative 1e-5 on both ends (the stated
   // epsilon-tie tolerance) so rounding in the slab arithmetic can never cull a primitive
   // the exact test would accept.
@@ -319,7 +331,7 @@ bool closestHit(const orc_ctx& c, const Ray& ray, HitAttr& out) {
     stack[sp++] = 0;
     while (sp) {
       const BvhNode& nd = c.nodes[stack[--sp]];
-      if (!hitBox(nd.lo, nd.hi, ray.origin, inv, ray.tmin, best.t)) continue;
+      if (!hitBox(nd.lo, nd.hi, ray.origin, ray.direction, inv, ray.tmin, best.t)) continue;
       if (nd.count > 0) {
         for (int k = 0; k < nd.count; ++k) testPrimClosest(c, c.order[nd.first + k], ray, best, bestN);
       } else {
@@ -371,7 +383,7 @@ float3 shadowTransmittance(const orc_ctx& c, const Ray& ray) {
     stack[sp++] = 0;
     while (sp && !blocked) {
       const BvhNode& nd = c.nodes[stack[--sp]];
-      if (!hitBox(nd.lo, nd.hi, ray.origin, inv, ray.tmin, ray.tmax)) continue;
+      if (!hitBox(nd.lo, nd.hi, ray.origin, ray.direction, inv, ray.tmin, ray.tmax)) continue;
       if (nd.count > 0) {
         for (int k = 0; k < nd.count && !blocked; ++k) testPrimShadow(c, c.order[nd.first + k], ray, atten, blocked);
       } else {

@@ -184,9 +184,14 @@ def test_quantised_box_test_is_conservative(mix):
     d += rng.normal(size=(n, 3)) * 1e-3 * np.linalg.norm(d, axis=1, keepdims=True)   # graze: not all through the centre
     d /= np.maximum(np.linalg.norm(d, axis=1, keepdims=True), 1e-30)
     d = d.astype(f)
-    axis_aligned = rng.random((n, 3)) < 0.02
-    d[axis_aligned] = 0.0
+    # axis-parallel components, +0 and -0, many of them with the origin on a plane of the child or of the node
+    axis_aligned = rng.random((n, 3)) < 0.05
+    d[axis_aligned] = np.where(rng.random(int(axis_aligned.sum())) < 0.5, f(-0.0), f(0.0))
     d[np.all(d == 0, axis=1)] = f(1.0)
+    axis_aligned = d == 0
+    plane = rng.integers(0, 4, size=(n, 3))
+    o = np.where(axis_aligned & (plane == 0), lo, np.where(axis_aligned & (plane == 1), hi,
+                 np.where(axis_aligned & (plane == 2), blo, o))).astype(f)
     tmin = f(1e-3)
     tbest = np.where(rng.random(n) < 0.5, f(1e27), (10.0 ** rng.uniform(-2, 4, size=n)).astype(f)).astype(f)
 
@@ -202,11 +207,13 @@ def test_quantised_box_test_is_conservative(mix):
     tf_true = np.minimum(far.min(axis=1), tbest)
     hit_true = tn_true <= tf_true
 
-    # ---- the kernel's arithmetic (float32)
-    dd = np.where(np.abs(d) > f(1e-30), d, np.copysign(f(1e-30), d)).astype(f)
-    idir = (f(1.0) / dd).astype(f)
+    # ---- the kernel's arithmetic (float32); traverse.cuh::prepRay<true>: a zero component, +0 or -0, gets 1/d = +1e30
+    zero_d = np.abs(d) <= f(1e-30)
+    with np.errstate(divide="ignore"):
+        idir = (f(1.0) / d).astype(f)
     ulp = rng.integers(-1, 2, size=idir.shape)                               # rcp.approx: 1 ulp
     idir = np.where(ulp > 0, np.nextafter(idir, f(np.inf)), np.where(ulp < 0, np.nextafter(idir, f(-np.inf)), idir)).astype(f)
+    idir = np.where(zero_d, f(1e30), idir).astype(f)
     ia = (s * idir).astype(f)
     oa = ((blo - o).astype(f) * idir).astype(f)
     neg = idir < 0
@@ -232,7 +239,11 @@ def test_quantised_box_test_is_conservative(mix):
     diff = _fma(tf, np.full(n, f(1.00001)), -tn)                             # the sign bit decides
     hit_kernel = ~np.signbit(diff)
     assert hit_true.sum() > n // 10                                          # the sample does exercise hits
-    missed = hit_true & ~hit_kernel
+    # What the node step may cull: a child flat at the node's origin plane of a zero axis, with the ray running in that
+    # plane.  Its primitives all lie in the ray's plane, and no primitive test accepts a ray lying in its plane.
+    coplanar = np.any(zero_d & (o == blo) & (qh == 0), axis=1)
+    missed = hit_true & ~hit_kernel & ~coplanar
+    assert (hit_true & zero_d.any(axis=1) & ((o == lo) | (o == hi)).any(axis=1)).sum() > n // 200   # on-plane rays hit
     assert not missed.any(), f"{missed.sum()} exact hits culled, e.g. index {np.flatnonzero(missed)[:5]}"
     # and it is a box test, not a constant: most exact misses stay misses
     assert (hit_kernel & ~hit_true).sum() < 0.5 * (~hit_true).sum()
