@@ -28,6 +28,7 @@ gpu: $(PKG)/libmox.so
 host: $(PKG)/libmox_host.so $(PKG)/mox_cli
 oracle: oracle/liboracle.so
 ref: oracle/_ref/libref_loader.so oracle/_ref/libref_render.so
+probe: tests/probe/libshading_probe.so
 
 $(PKG)/libmox.so: $(GPU_SRCS) $(GPU_HDRS)
 	$(NVCC) $(NVFLAGS) -shared -o $@ $(GPU_SRCS) -lcudart
@@ -41,6 +42,11 @@ $(PKG)/mox_cli: $(PKG)/libmox_host.so $(CSRC)/host/cli_main.cpp
 # oracle/adaptive.cpp compiles oracle/refit.cpp, which compiles oracle.cpp; each adds its entry points around the other.
 oracle/liboracle.so: oracle/adaptive.cpp oracle/refit.cpp oracle/oracle.cpp oracle/oracle.h oracle/device_spec.h oracle/vecmath.h include/mox.h include/mox_structs.h
 	$(CXX) $(ORCFLAGS) -shared -o $@ oracle/adaptive.cpp
+
+# Test infrastructure: the device shading math behind a C ABI for tests/test_shading_math.py, compiled with the
+# flags of libmox.so from the same headers.
+tests/probe/libshading_probe.so: tests/probe/shading_probe.cu $(GPU_HDRS)
+	$(NVCC) $(NVFLAGS) -Xptxas -v -shared -o $@ tests/probe/shading_probe.cu -lcudart
 
 # Reference loader half (scene.cpp + tiny_obj_loader.h) compiled from /root/reference with a shim.
 oracle/_ref/libref_loader.so: oracle/ref_shim/ref_loader.cpp oracle/ref_shim/optix_world.h
@@ -59,7 +65,7 @@ oracle/_ref/libref_render.so: oracle/ref_shim/ref_render.cpp oracle/ref_shim/ren
 	else echo "reference not present: skipping oracle/_ref"; fi
 
 clean:
-	rm -f $(PKG)/libmox.so $(PKG)/libmox_host.so $(PKG)/mox_cli oracle/liboracle.so
+	rm -f $(PKG)/libmox.so $(PKG)/libmox_host.so $(PKG)/mox_cli oracle/liboracle.so tests/probe/libshading_probe.so
 	rm -rf oracle/_ref
 
-.PHONY: all gpu host oracle ref clean
+.PHONY: all gpu host oracle ref probe clean
