@@ -194,21 +194,17 @@ struct mox_ctx {
   std::vector<DevBuf> otherOwned;  // cached owned lists of other ranks (unpack)
   std::vector<uint64_t> ownedCount; // cached |owned pixels| per rank of the current partition
 
-  // Wavefront state of the batch in flight.  The shadow rays of a bounce run on their own stream (overlapShadow), so
-  // two persistent traversal launches are in flight while the host waits for a bounce's material counts.  Splitting
-  // a batch into sub-batches on further streams measured no faster (1347 vs 1350 Mrays/s at full frame, slower on an
-  // eighth of it) and was removed (DESIGN.md section 4; the code is in the git history).
+  // Wavefront buffers, streams and events of renderBatch.  The shadow rays of a bounce run on their own stream
+  // (overlapShadow), so two persistent traversal launches are in flight while the host waits for a bounce's material
+  // counts.  Splitting a batch into sub-batches on further streams measured no faster (1347 vs 1350 Mrays/s at full
+  // frame, slower on an eighth of it) and was removed (DESIGN.md section 4; the code is in the git history).
   PathBuffers pb;      // views into pathBlock (pathLayout)
   DevBuf pathBlock;
   cudaStream_t shadowStream = nullptr;  // shadow traversal + k_apply of bounce b, overlapping extend + classify of bounce b+1
   cudaEvent_t evShaded = nullptr, evApplied = nullptr;
-  bool applyPending = false;       // evApplied must be waited for before the next kernel that touches rad / the shadow buffers
   cudaEvent_t evReady = nullptr;   // the counters of the bounce in flight have landed in hostCnt
   PinnedBuf<uint32_t> hostCnt;     // kCounterWords
   StageTimer timer;
-  LaunchCtx lc;
-  uint32_t batchSamples = 0, bound = 0, depth = 0, matCount[Q_COUNT] = {0, 0, 0, 0};
-  bool batchDone = true;
   PinnedBuf<float> pinned;   // mox_map_accum's image
 
   // Gather / asynchronous read-back: two full-size device buffers (targets of the tile pushes, possibly of other
@@ -230,7 +226,6 @@ struct mox_ctx {
   bool overlapShadow = true;     // shadow rays of bounce b on a second stream, concurrent with the extend launch of bounce b+1 (MOX_OVERLAP_SHADOW=0: serial)
   bool brdfFast = true;          // approximate reciprocal / square root inside BRDF values (MOX_BRDF_IEEE=1: IEEE, the oracle's operations)
   bool terminalQuery = true;     // the bounce past rayMaxDepth uses the light list and an any-hit query (MOX_TERMINAL_CLOSEST=1: closest hit)
-  uint32_t terminalDepth = 0;    // the batch's last bounce ran the terminal query: its ray counts come with the final counter copy
 
   // Adaptive sampling (mox_render_adaptive), allocated at its first call: per pixel the luminance sums, the sample
   // count and the launches sat out (pixelStats, 24 bytes per pixel in one block), and the two active-pixel lists with
@@ -238,7 +233,6 @@ struct mox_ctx {
   DevBuf adaptiveStats, adaptiveLists;
   PixelStats pixelStats;
   PinnedBuf<uint32_t> hostSurvivors;
-  const PixelStats* batchStats = nullptr;   // the batch in flight also accumulates these (null: mox_launch / mox_render)
 
   // Frees what the context holds; the device buffers go with their owners.  mox_destroy binds the device and waits
   // for the streams first.
@@ -337,10 +331,16 @@ int refreshOwned(mox_ctx* c) {
   return MOX_OK;
 }
 
+// c->pathBlock already holds `paths` paths, nLights shadow slots per path and nSeeds launch seeds.
+bool pathsFit(const mox_ctx* c, size_t paths, size_t nLights, size_t nSeeds) {
+  const PathBuffers& pb = c->pb;
+  return c->pathBlock.p && pb.capacity >= paths && pb.shadowSlots >= paths * nLights && pb.seedCap >= nSeeds;
+}
+
 // The wavefront state of `paths` paths, nLights shadow slots per path and nSeeds launch seeds in c->pathBlock.
 int ensurePaths(mox_ctx* c, size_t paths, size_t nLights, size_t nSeeds) {
+  if (pathsFit(c, paths, nLights, nSeeds)) return MOX_OK;
   PathBuffers& pb = c->pb;
-  if (c->pathBlock.p && pb.capacity >= paths && pb.shadowSlots >= paths * nLights && pb.seedCap >= nSeeds) return MOX_OK;
   cudaStreamSynchronize(c->stream);
   // grow geometrically so that a slowly growing sample count does not reallocate on every call
   if (pb.capacity && paths > pb.capacity) paths = std::max(paths, pb.capacity + pb.capacity / 2);
@@ -426,120 +426,23 @@ int syncLights(mox_ctx* c) {
   return MOX_OK;
 }
 
-inline uint32_t* bounceBlock(const PathBuffers& pb, uint32_t depth) { return pb.counters + C_WORDS + (depth % BOUNCE_RING) * C_BOUNCE_WORDS; }
+// The counter block of bounce `depth` in the device counters (pb.counters) or in their host copy (hostCnt): after the
+// C_WORDS batch words, a ring of BOUNCE_RING blocks.
+inline uint32_t* bounceBlock(uint32_t* counters, uint32_t depth) { return counters + C_WORDS + (depth % BOUNCE_RING) * C_BOUNCE_WORDS; }
 
-int finishBatch(mox_ctx* c);
-
-// Enqueue one bounce up to the point where the host needs numbers: extend (persistent traversal, ray count read on
-// the device), classify, and the read-back of the counters.
-int enqueueExtend(mox_ctx* c) {
-  LaunchCtx& lc = c->lc;
-  StageTimer& tm = c->timer;
-  const uint32_t depth = c->depth;
-  lc.bc = bounceBlock(c->pb, depth);
-  lc.pb.qMat[Q_DISNEY] = (depth & 1u) ? c->pb.qMat[Q_DISNEY] : c->pb.qDisneyAlt;   // k_apply of bounce depth-1 may still read the other one
-  // bounce 1 traces exactly `bound` camera rays; later bounces read the number of spawned rays from the previous
-  // bounce's counter block, `bound` (what was shaded) only sizes the grids
-  const uint32_t* countPtr = depth == 1 ? nullptr : bounceBlock(c->pb, depth - 1) + C_NEXT;
-  // k_classify's test: every path of this bounce ends in it, whatever it hits (|payload colour| = sqrt(3))
-  const bool terminal = depth > c->rp.maxDepth || length(mk3(1.f)) < c->rp.minIntensity;
-  if (terminal && c->terminalQuery && c->nTerminalLights >= 0 && lc.scene.nodes8) {
-    TerminalLights tl;
-    tl.list = (const uint4*)c->dTerminalLights.p;
-    tl.n = c->nTerminalLights;
-    tl.missIsAbsorb = memcmp(&c->rp.bg, &c->rp.absorb, sizeof c->rp.bg) == 0;
-    tm.begin(ST_EXTEND, c->stream, depth);
-    launchTerminal(lc, depth == 1 ? nullptr : lc.pb.qCur, c->bound, countPtr, tl);
-    tm.end(c->stream);
-    c->st.extend_launches++; c->st.kernel_launches++;
-    // k_classify would queue nothing: no counts to wait for, the accumulation follows at once
-    c->terminalDepth = depth;
-    return finishBatch(c);
-  }
-  tm.begin(ST_EXTEND, c->stream, depth);
-  // camera rays are queued in path order (k_generate: qCur[p] = p): the traversal kernel skips the indirection
-  launchExtend(lc, depth == 1 ? nullptr : lc.pb.qCur, c->bound, countPtr, depth);
-  tm.end(c->stream);
-  tm.begin(ST_SHADE, c->stream);
-  launchClassify(lc, lc.pb.qCur, c->bound, countPtr, depth);
-  tm.end(c->stream);
-  c->st.extend_launches++; c->st.kernel_launches += 2;
-  CUCK(c, cudaMemcpyAsync(c->hostCnt.p, c->pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, c->stream));
-  CUCK(c, cudaEventRecord(c->evReady, c->stream));
-  return MOX_OK;
-}
-
-int finishBatch(mox_ctx* c) {
-  StageTimer& tm = c->timer;
-  if (c->applyPending) { CUCK(c, cudaStreamWaitEvent(c->stream, c->evApplied, 0)); c->applyPending = false; }
-  tm.begin(ST_ACCUMULATE, c->stream);
-  if (c->batchStats) launchAccumulateAdaptive(c->lc, c->batchSamples, *c->batchStats);
-  else launchAccumulate(c->lc, c->batchSamples);
-  tm.end(c->stream);
-  c->st.kernel_launches++;
-  CUCK(c, cudaMemcpyAsync(c->hostCnt.p, c->pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, c->stream));
-  CUCK(c, cudaEventRecord(c->evReady, c->stream));
-  c->batchDone = true;
-  return MOX_OK;
-}
-
-// Exact number of rays bounce `depth` traced, and of shadow rays the bounce before it queued, from the counters in
-// hostCnt.
-void countBounceRays(mox_ctx* c, uint32_t depth) {
+// Exact number of rays bounce `depth` traced (`bound` camera rays at depth 1), and of shadow rays the bounce before it
+// queued, from the counters in hostCnt.
+void countBounceRays(mox_ctx* c, uint32_t depth, uint32_t bound) {
   mox_stats& st = c->st;
   const uint32_t dIdx = std::min<uint32_t>(depth, MOX_STATS_DEPTHS - 1);
-  if (depth == 1) { st.rays_primary += c->bound; st.rays_depth[1] += c->bound; }
+  if (depth == 1) { st.rays_primary += bound; st.rays_depth[1] += bound; }
   else {
-    const uint32_t* prev = c->hostCnt.p + C_WORDS + ((depth - 1) % BOUNCE_RING) * C_BOUNCE_WORDS;
+    const uint32_t* prev = bounceBlock(c->hostCnt.p, depth - 1);
     st.rays_bounce += prev[C_NEXT];
     st.rays_shadow_traced += prev[C_SHQ];
     st.rays_depth[dIdx] += prev[C_NEXT];
     st.shadow_traced_depth[std::min<uint32_t>(depth - 1, MOX_STATS_DEPTHS - 1)] += prev[C_SHQ];
   }
-}
-
-// The counters of the bounce in flight have arrived: shade what was binned, trace the shadow rays, and enqueue
-// the next bounce — or the accumulation when nothing is left.
-int advanceBounce(mox_ctx* c) {
-  LaunchCtx& lc = c->lc;
-  StageTimer& tm = c->timer;
-  PathBuffers& pb = c->pb;
-  const uint32_t depth = c->depth;
-  const uint32_t* hostBounce = c->hostCnt.p + C_WORDS + (depth % BOUNCE_RING) * C_BOUNCE_WORDS;
-  countBounceRays(c, depth);
-  uint32_t any = 0;
-  for (int k = 0; k < Q_COUNT; ++k) { c->matCount[k] = hostBounce[C_MAT0 + k]; any += c->matCount[k]; }
-  if (!any) return finishBatch(c);
-  // the shade kernels touch the radiance and rewrite the shadow-ray buffers: the previous bounce's k_apply first
-  if (c->applyPending) { CUCK(c, cudaStreamWaitEvent(c->stream, c->evApplied, 0)); c->applyPending = false; }
-  tm.begin(ST_SHADE, c->stream);
-  for (int k = 0; k < Q_COUNT; ++k) { launchShade(lc, k, c->matCount[k], depth); if (c->matCount[k]) c->st.kernel_launches++; }
-  tm.end(c->stream);
-  if (c->matCount[Q_DISNEY] && lc.scene.nLights) {
-    // Shadow rays and the NEE sum depend only on this bounce's shade kernels; the next extend launch does not
-    // depend on them.  On a second stream the two persistent traversal launches overlap: each one's last CTAs
-    // drain while the other's first CTAs already run.
-    cudaStream_t ss = c->stream;
-    if (c->overlapShadow && c->shadowStream) {
-      ss = c->shadowStream;
-      CUCK(c, cudaEventRecord(c->evShaded, c->stream));
-      CUCK(c, cudaStreamWaitEvent(ss, c->evShaded, 0));
-    }
-    tm.begin(ST_SHADOW, ss, depth);
-    launchShadow(lc, c->matCount[Q_DISNEY], ss);
-    tm.end(ss);
-    tm.begin(ST_SHADE, ss);
-    launchApply(lc, c->matCount[Q_DISNEY], ss);
-    tm.end(ss);
-    if (ss != c->stream) { CUCK(c, cudaEventRecord(c->evApplied, ss)); c->applyPending = true; }
-    c->st.kernel_launches += 2;
-  }
-  // the block bounce depth+1 will use was last written BOUNCE_RING bounces ago
-  CUCK(c, cudaMemsetAsync(bounceBlock(pb, depth + 1), 0, C_BOUNCE_WORDS * 4, c->stream));
-  std::swap(lc.pb.qCur, lc.pb.qNext);
-  c->bound = any;   // every shaded path spawns at most one ray
-  c->depth = depth + 1;
-  return enqueueExtend(c);
 }
 
 // Events, pinned counters and wavefront buffers for a batch of S samples of `count` pixels.  renderSeeds calls it
@@ -555,10 +458,10 @@ int prepareBatch(mox_ctx* c, uint32_t S, uint32_t count) {
   return rc ? rc : ensurePaths(c, (size_t)S * count, c->lights.size(), S);
 }
 
-// One wavefront batch: `seeds.size()` samples of each pixel of list[0, count).  Generate, then advance bounce by
-// bounce until no path is left, then collect the counters.
-int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds, const uint32_t* list, uint32_t count) {
-  const uint32_t S = (uint32_t)seeds.size();
+// One wavefront batch: the S samples seeds[0, S) of each pixel of list[0, count); with `stats`, the accumulation also
+// adds every sample's luminance to them.  Generate, then bounce by bounce until no path is left: extend, classify,
+// wait for the material counts, shade, shadow.  Then accumulate and collect the counters.
+int renderBatch(mox_ctx* c, const int32_t* seeds, uint32_t S, const uint32_t* list, uint32_t count, const PixelStats* stats) {
   const size_t P = (size_t)S * count;
   if (P == 0) return MOX_OK;
   if (P > 0xfffffff0ull) return fail(c, MOX_ERR_INVALID, "batch too large");
@@ -567,8 +470,10 @@ int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds, const uint32_t* l
   // in flight
   if ((rc = prepareBatch(c, S, count))) return rc;
   PathBuffers& pb = c->pb;
-  CUCK(c, cudaMemcpyAsync(pb.seeds, seeds.data(), S * 4, cudaMemcpyHostToDevice, c->stream));
-  LaunchCtx& lc = c->lc;
+  StageTimer& tm = c->timer;
+  mox_stats& st = c->st;
+  CUCK(c, cudaMemcpyAsync(pb.seeds, seeds, S * 4, cudaMemcpyHostToDevice, c->stream));
+  LaunchCtx lc;
   lc.scene = sceneView(c);
   lc.rp = c->rp;
   lc.pb = pb;
@@ -579,24 +484,102 @@ int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds, const uint32_t* l
   lc.brdfFast = c->brdfFast;
   lc.stream = c->stream;
   lc.pb.qCur = pb.qBuf[0]; lc.pb.qNext = pb.qBuf[1];
-  lc.bc = bounceBlock(pb, 1);
-  c->batchSamples = S; c->bound = (uint32_t)P; c->depth = 1; c->batchDone = false; c->applyPending = false; c->terminalDepth = 0;
+  lc.bc = bounceBlock(pb.counters, 1);
   CUCK(c, cudaMemsetAsync(pb.counters, 0, kCounterWords * 4, c->stream));
-  c->timer.begin(ST_GENERATE, c->stream);
+  tm.begin(ST_GENERATE, c->stream);
   launchGenerate(lc, S);
-  c->timer.end(c->stream);
-  c->st.kernel_launches++;
-  if ((rc = enqueueExtend(c))) return rc;
-  while (!c->batchDone) {
+  tm.end(c->stream);
+  st.kernel_launches++;
+  // k_apply of a bounce may still run on the shadow stream (evApplied): the next kernel of the context stream that
+  // touches the radiance or the shadow-ray buffers waits for it
+  bool applyPending = false;
+  auto waitApplied = [&]() -> int {
+    if (applyPending) { CUCK(c, cudaStreamWaitEvent(c->stream, c->evApplied, 0)); applyPending = false; }
+    return MOX_OK;
+  };
+  uint32_t bound = (uint32_t)P;   // rays this bounce traces at most: every shaded path spawns at most one
+  bool ranTerminal = false;       // the last bounce ran the terminal query: its ray counts come with the final counter copy
+  uint32_t depth;
+  for (depth = 1;; ++depth) {
+    lc.bc = bounceBlock(pb.counters, depth);
+    lc.pb.qMat[Q_DISNEY] = (depth & 1u) ? pb.qMat[Q_DISNEY] : pb.qDisneyAlt;   // k_apply of bounce depth-1 may still read the other one
+    // bounce 1 traces exactly `bound` camera rays; later bounces read the number of spawned rays from the previous
+    // bounce's counter block, `bound` (what was shaded) only sizes the grids
+    const uint32_t* countPtr = depth == 1 ? nullptr : bounceBlock(pb.counters, depth - 1) + C_NEXT;
+    // k_classify's test: every path of this bounce ends in it, whatever it hits (|payload colour| = sqrt(3))
+    const bool terminal = depth > c->rp.maxDepth || length(mk3(1.f)) < c->rp.minIntensity;
+    if (terminal && c->terminalQuery && c->nTerminalLights >= 0 && lc.scene.nodes8) {
+      TerminalLights tl;
+      tl.list = (const uint4*)c->dTerminalLights.p;
+      tl.n = c->nTerminalLights;
+      tl.missIsAbsorb = memcmp(&c->rp.bg, &c->rp.absorb, sizeof c->rp.bg) == 0;
+      tm.begin(ST_EXTEND, c->stream, depth);
+      launchTerminal(lc, depth == 1 ? nullptr : lc.pb.qCur, bound, countPtr, tl);
+      tm.end(c->stream);
+      st.extend_launches++; st.kernel_launches++;
+      // k_classify would queue nothing: no counts to wait for, the accumulation follows at once
+      ranTerminal = true;
+      break;
+    }
+    tm.begin(ST_EXTEND, c->stream, depth);
+    // camera rays are queued in path order (k_generate: qCur[p] = p): the traversal kernel skips the indirection
+    launchExtend(lc, depth == 1 ? nullptr : lc.pb.qCur, bound, countPtr, depth);
+    tm.end(c->stream);
+    tm.begin(ST_SHADE, c->stream);
+    launchClassify(lc, lc.pb.qCur, bound, countPtr, depth);
+    tm.end(c->stream);
+    st.extend_launches++; st.kernel_launches += 2;
+    CUCK(c, cudaMemcpyAsync(c->hostCnt.p, pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, c->stream));
+    CUCK(c, cudaEventRecord(c->evReady, c->stream));
+    // the material counts size the shade launches: the host waits for them
     CUCK(c, cudaEventSynchronize(c->evReady));
-    if ((rc = advanceBounce(c))) return rc;
+    countBounceRays(c, depth, bound);
+    const uint32_t* hostBounce = bounceBlock(c->hostCnt.p, depth);
+    uint32_t binned[Q_COUNT], any = 0;
+    for (int k = 0; k < Q_COUNT; ++k) { binned[k] = hostBounce[C_MAT0 + k]; any += binned[k]; }
+    if (!any) break;
+    // the shade kernels touch the radiance and rewrite the shadow-ray buffers: the previous bounce's k_apply first
+    if ((rc = waitApplied())) return rc;
+    tm.begin(ST_SHADE, c->stream);
+    for (int k = 0; k < Q_COUNT; ++k) { launchShade(lc, k, binned[k], depth); if (binned[k]) st.kernel_launches++; }
+    tm.end(c->stream);
+    if (binned[Q_DISNEY] && lc.scene.nLights) {
+      // Shadow rays and the NEE sum depend only on this bounce's shade kernels; the next extend launch does not
+      // depend on them.  On a second stream the two persistent traversal launches overlap: each one's last CTAs
+      // drain while the other's first CTAs already run.
+      cudaStream_t ss = c->stream;
+      if (c->overlapShadow && c->shadowStream) {
+        ss = c->shadowStream;
+        CUCK(c, cudaEventRecord(c->evShaded, c->stream));
+        CUCK(c, cudaStreamWaitEvent(ss, c->evShaded, 0));
+      }
+      tm.begin(ST_SHADOW, ss, depth);
+      launchShadow(lc, binned[Q_DISNEY], ss);
+      tm.end(ss);
+      tm.begin(ST_SHADE, ss);
+      launchApply(lc, binned[Q_DISNEY], ss);
+      tm.end(ss);
+      if (ss != c->stream) { CUCK(c, cudaEventRecord(c->evApplied, ss)); applyPending = true; }
+      st.kernel_launches += 2;
+    }
+    // the block bounce depth+1 will use was last written BOUNCE_RING bounces ago
+    CUCK(c, cudaMemsetAsync(bounceBlock(pb.counters, depth + 1), 0, C_BOUNCE_WORDS * 4, c->stream));
+    std::swap(lc.pb.qCur, lc.pb.qNext);
+    bound = any;
   }
-  // the accumulation and the final counter read-back
+  if ((rc = waitApplied())) return rc;
+  tm.begin(ST_ACCUMULATE, c->stream);
+  if (stats) launchAccumulateAdaptive(lc, S, *stats);
+  else launchAccumulate(lc, S);
+  tm.end(c->stream);
+  st.kernel_launches++;
+  // the final counter read-back
+  CUCK(c, cudaMemcpyAsync(c->hostCnt.p, pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, c->stream));
+  CUCK(c, cudaEventRecord(c->evReady, c->stream));
   CUCK(c, cudaEventSynchronize(c->evReady));
   const uint32_t* host = c->hostCnt.p;
-  mox_stats& st = c->st;
-  if (c->terminalDepth) countBounceRays(c, c->terminalDepth);
-  c->timer.collect(st);
+  if (ranTerminal) countBounceRays(c, depth, bound);
+  tm.collect(st);
   st.nonfinite_samples += host[C_NONFINITE];
   st.rays_shadow_blocked += host[C_SH_BLOCKED]; st.rays_shadow_tinted += host[C_SH_TINTED];
   st.rays_shadow += host[C_SHADOW];
@@ -613,13 +596,11 @@ int renderBatch(mox_ctx* c, const std::vector<int32_t>& seeds, const uint32_t* l
 // memory (what the current block holds counts as free) for this scene's light count (36 bytes per path and light).
 size_t batchCap(mox_ctx* c, size_t wanted /* samples per pixel of this call */, uint32_t count /* pixels */) {
   size_t cap = c->maxBatchPaths;
-  const PathBuffers& pb = c->pb;
   // The buffers of an earlier call already hold such a batch: nothing will be allocated, so there is nothing to
   // budget.  (cudaMemGetInfo is a slow driver call — it was the 20-70 ms hiccup in front of some steps.)
   if (count) {
-    const size_t S = std::min(std::max<size_t>(1, cap / count), wanted), nL = c->lights.size();   // samples per batch at the full cap
-    const size_t P = S * count;
-    if (c->pathBlock.p && pb.capacity >= P && pb.shadowSlots >= P * nL && pb.seedCap >= S) return cap;
+    const size_t S = std::min(std::max<size_t>(1, cap / count), wanted);   // samples per batch at the full cap
+    if (pathsFit(c, S * count, c->lights.size(), S)) return cap;
   }
   size_t freeB = 0, totalB = 0;
   if (cudaMemGetInfo(&freeB, &totalB) == cudaSuccess) {
@@ -648,15 +629,13 @@ int beginRender(mox_ctx* c) {
 // sample's luminance to them.  beginRender first.
 int renderSeeds(mox_ctx* c, const std::vector<int32_t>& seeds, const uint32_t* list, uint32_t count, const PixelStats* stats = nullptr) {
   if (count == 0) { c->st.launches += seeds.size(); return MOX_OK; }
-  c->batchStats = stats;
   size_t perBatch = std::max<size_t>(1, batchCap(c, seeds.size(), count) / count);
   int rc = prepareBatch(c, (uint32_t)std::min(perBatch, seeds.size()), count);
   if (rc && rc != MOX_ERR_OOM) return rc;   // out of memory: the loop below retries with smaller batches
   CUCK(c, cudaEventRecord(c->ev0, c->stream));
   for (size_t i = 0; i < seeds.size();) {
     const size_t n = std::min(perBatch, seeds.size() - i);
-    std::vector<int32_t> chunk(seeds.begin() + i, seeds.begin() + i + n);
-    rc = renderBatch(c, chunk, list, count);
+    rc = renderBatch(c, seeds.data() + i, (uint32_t)n, list, count, stats);
     if (rc == MOX_ERR_OOM && perBatch > 1) {
       // the allocation failed after all (fragmentation, another context on the device): free the wavefront
       // state, halve the batch and render this chunk again (nothing of it was enqueued)
