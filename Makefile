@@ -39,9 +39,10 @@ $(PKG)/libmox_host.so: $(HOST_SRCS) $(HOST_HDRS)
 $(PKG)/mox_cli: $(PKG)/libmox_host.so $(CSRC)/host/cli_main.cpp
 	$(CXX) $(CXXFLAGS) -o $@ $(CSRC)/host/cli_main.cpp -L$(PKG) -lmox_host -ldl -pthread -Wl,-rpath,'$$ORIGIN'
 
-# oracle/adaptive.cpp compiles oracle/refit.cpp, which compiles oracle.cpp; each adds its entry points around the other.
-oracle/liboracle.so: oracle/adaptive.cpp oracle/refit.cpp oracle/oracle.cpp oracle/oracle.h oracle/device_spec.h oracle/vecmath.h include/mox.h include/mox_structs.h
-	$(CXX) $(ORCFLAGS) -shared -o $@ oracle/adaptive.cpp
+# oracle/denoise.cpp compiles oracle/adaptive.cpp, which compiles oracle/refit.cpp, which compiles oracle.cpp; each adds
+# its entry points around the other.
+oracle/liboracle.so: oracle/denoise.cpp oracle/adaptive.cpp oracle/refit.cpp oracle/oracle.cpp oracle/oracle.h oracle/device_spec.h oracle/vecmath.h include/mox.h include/mox_structs.h
+	$(CXX) $(ORCFLAGS) -shared -o $@ oracle/denoise.cpp
 
 # Test infrastructure: the device shading math behind a C ABI for tests/test_shading_math.py, compiled with the
 # flags of libmox.so from the same headers.

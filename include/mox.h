@@ -244,6 +244,61 @@ int mox_clear_accum(mox_ctx*);
  * MinimalOptiX.cpp:543-558; this is the "dump/resume" row of SURVEY.md §8 f-2). */
 int mox_set_accum(mox_ctx*, const float* src_rgb, uint64_t launches);
 
+/* ---- first-hit AOVs and the denoiser --------------------------------------- */
+
+/* AOVs ("arbitrary output variables"): per-pixel buffers besides the colour.  mox_set_aovs(ctx, 1) allocates and
+ * zeroes 36 bytes per pixel of sums on the device; from then on every camera sample that mox_launch, mox_render or
+ * mox_render_adaptive traces adds one record, taken at the closest hit of its depth-1 ray:
+ *   albedo  Lambertian, metal, glass: albedo; Disney: the base colour (texture or color, not linearised); light:
+ *           emission clamped to [0, 1]; miss: bgColor clamped to [0, 1]
+ *   normal  the shading normal turned towards the viewer, faceforward(Ns, -d, Ng); 0 for a miss
+ *   depth   the ray's t, counted for hits only
+ * The AOVs keep their own sample and hit counts per pixel, so they may be switched on after some samples.  The sums
+ * are reset by mox_clear_accum, mox_set_accum and a size change in mox_set_globals; mox_set_aovs(ctx, 0) frees them.
+ * The image itself does not change: with AOVs on or off the accumulation buffer, the sample counts and the ray counts
+ * are bit-identical.  On a multi-GPU handle the switch is replicated to every device. */
+int mox_set_aovs(mox_ctx*, int enable);
+/* The per-pixel means, W*H*k floats with row 0 = bottom (k = 3, 3, 1); any pointer may be NULL.  Each mean is one
+ * float32 division of the sum by its count: albedo and normal by the AOV sample count, depth by the hit count.  A pixel
+ * without a sample, and the depth of a pixel without a hit, read 0.  These are exactly the guides mox_denoise uses.
+ * On a multi-GPU handle: the sum over the devices (each pixel is non-zero on its owner only).  MOX_ERR_STATE: AOVs off. */
+int mox_read_aovs(mox_ctx*, float* albedo_rgb, float* normal_xyz, float* depth);
+
+/* Edge-avoiding a-trous wavelet filter (Dammertz, Hanika, Keller 2010) of the mean colour, guided by the AOVs.
+ *
+ * c_p = accum_p / n_p is the mean colour (n_p from mox_read_sample_counts, so adaptive renders work; 0 where n_p = 0),
+ * a, N, z are the AOV means of mox_read_aovs.  All arithmetic is float32, evaluated in the order written, without
+ * fused multiply-adds:
+ *   e0_p      = c_p / (a_p + 0.001)                                          per channel (demodulation)
+ *   for i = 0 .. K-1, with step s = 2^i and sigma_i = sigma_color * 2^-i:
+ *   e(i+1)_p  = sum_q h(dx) h(dy) w_pq e(i)_q / sum_q h(dx) h(dy) w_pq,  q = p + s (dx, dy)
+ *               dy = -2..2 in the outer loop, dx = -2..2 in the inner one; taps outside the image are skipped
+ *               (not clamped); h = (1/16, 1/4, 3/8, 1/4, 1/16); each sum adds h(dx) h(dy) w_pq (and its product
+ *               with e(i)_q) in tap order
+ *   w_pq      = exp(-(|e(i)_p - e(i)_q|^2 / sigma_i^2 + max(0, 1 - N_p . N_q) / sigma_normal
+ *                     + |z_p - z_q| / (sigma_depth * max(z_p, z_q) + 1e-30)))
+ *               with |v|^2 = (x*x + y*y) + z*z, N_p . N_q = (x*x' + y*y') + z*z', sigma_i^2 = sigma_i * sigma_i; the
+ *               centre tap has w = 1; two misses (z = 0) compare as equal depth
+ *   out_p     = e(K)_p * (a_p + 0.001)                                       (remodulation)
+ *
+ * dst_rgb: W*H*3 floats, row 0 = bottom.  params == NULL selects the defaults MOX_DENOISE_DEFAULT_*.  *out_ms (may be
+ * NULL): device time of the denoise kernels (CUDA events).  Two calls on the same state give bit-identical results.
+ * MOX_ERR_INVALID: iterations outside 1..10, or a sigma that is not finite and > 0.  MOX_ERR_STATE: AOVs off, no
+ * camera sample rendered with AOVs on since the last reset (a buffer loaded by mox_set_accum alone has no guides), or a
+ * context with mox_set_partition world > 1 (the filter needs the whole frame; a mox_create_multi handle gathers it into
+ * device 0 and filters there). */
+typedef struct mox_denoise_params {
+  uint32_t iterations;   /* 1 .. 10 */
+  float sigma_color;     /* colour (irradiance) edge stop of iteration 0; halved every iteration */
+  float sigma_normal;    /* normal edge stop */
+  float sigma_depth;     /* depth edge stop, relative to the larger depth */
+} mox_denoise_params;
+#define MOX_DENOISE_DEFAULT_ITERATIONS 5
+#define MOX_DENOISE_DEFAULT_SIGMA_COLOR 1.0f
+#define MOX_DENOISE_DEFAULT_SIGMA_NORMAL 0.5f
+#define MOX_DENOISE_DEFAULT_SIGMA_DEPTH 0.05f
+int mox_denoise(mox_ctx*, const mox_denoise_params* params, float* dst_rgb, float* out_ms);
+
 /* Multi-GPU gather plumbing (device pointers on this context's GPU).
  * mox_owned_pixels: number of pixels rank `rank` of the current partition owns.
  * mox_pack_owned: copy this rank's owned pixels (tile order) to dev_dst

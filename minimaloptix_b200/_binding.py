@@ -56,6 +56,9 @@ SIGNATURES = {
     "read_accum_end": (C.c_int, [_vp, C.POINTER(_fp)]),
     "trace_closest": (C.c_int, [_vp, _vp, C.c_size_t, _vp]),
     "trace_shadow": (C.c_int, [_vp, _vp, C.c_size_t, _vp]),
+    "set_aovs": (C.c_int, [_vp, C.c_int]),
+    "read_aovs": (C.c_int, [_vp, _vp, _vp, _vp]),
+    "denoise": (C.c_int, [_vp, C.POINTER(S.DenoiseParams), _vp, C.POINTER(_f32)]),
 }
 # Only the GPU library has the device-pointer query.
 GPU_ONLY = {"create_multi": (C.c_int, [C.POINTER(_vp), C.POINTER(C.c_int), C.c_int]),
@@ -225,6 +228,28 @@ class Context:
         out = np.empty((self.height, self.width), dtype=np.uint32)
         self._ck(self.b.read_sample_counts(self.h, _ptr(out)), "read_sample_counts")
         return out
+
+    def set_aovs(self, on):
+        """mox_set_aovs: accumulate every camera sample's first-hit albedo, normal and depth (on) or free them (off)."""
+        self._ck(self.b.set_aovs(self.h, 1 if on else 0), "set_aovs")
+
+    def read_aovs(self):
+        """The AOV means, row 0 = bottom: (albedo (H, W, 3), normal (H, W, 3), depth (H, W))."""
+        a = np.empty((self.height, self.width, 3), dtype=np.float32)
+        n = np.empty((self.height, self.width, 3), dtype=np.float32)
+        z = np.empty((self.height, self.width), dtype=np.float32)
+        self._ck(self.b.read_aovs(self.h, _ptr(a), _ptr(n), _ptr(z)), "read_aovs")
+        return a, n, z
+
+    def denoise(self, iterations=S.DENOISE_DEFAULTS["iterations"], sigma_color=S.DENOISE_DEFAULTS["sigma_color"],
+                sigma_normal=S.DENOISE_DEFAULTS["sigma_normal"], sigma_depth=S.DENOISE_DEFAULTS["sigma_depth"]):
+        """mox_denoise: the edge-avoiding a-trous filter of the mean colour, guided by the AOVs.
+        Returns (image (H, W, 3), ms of the filter kernels)."""
+        p = S.DenoiseParams(iterations, sigma_color, sigma_normal, sigma_depth)
+        out = np.empty((self.height, self.width, 3), dtype=np.float32)
+        ms = _f32()
+        self._ck(self.b.denoise(self.h, C.byref(p), _ptr(out), C.byref(ms)), "denoise")
+        return out, ms.value
 
     def read_accum(self):
         out = np.empty((self.height, self.width, 3), dtype=np.float32)

@@ -16,6 +16,7 @@
 #include <vector>
 
 #include "build.h"
+#include "denoise.h"
 #include "group.h"
 #include "mox.h"
 #include "mox_debug.h"
@@ -233,6 +234,15 @@ struct mox_ctx {
   DevBuf adaptiveStats, adaptiveLists;
   PixelStats pixelStats;
   PinnedBuf<uint32_t> hostSurvivors;
+
+  // First-hit AOVs (mox_set_aovs): the sums in one block (aovLayout), allocated while aovOn and the image size is
+  // known.  Grow-only scratch of mox_denoise: the filter's buffers and its output; on device 0 of a multi-GPU handle
+  // also the frame the devices gather their inputs into (denoiseFrame: colour, skipped launches, AOV sums).
+  bool aovOn = false;
+  bool aovRecorded = false;   // a camera sample added its record since the sums were last zeroed
+  DevBuf aovBlock;
+  AovBuffers aov;
+  DevBuf denoiseScratch, denoiseOut, denoiseFrame;
 
   // Frees what the context holds; the device buffers go with their owners.  mox_destroy binds the device and waits
   // for the streams first.
@@ -508,7 +518,9 @@ int renderBatch(mox_ctx* c, const int32_t* seeds, uint32_t S, const uint32_t* li
     const uint32_t* countPtr = depth == 1 ? nullptr : bounceBlock(pb.counters, depth - 1) + C_NEXT;
     // k_classify's test: every path of this bounce ends in it, whatever it hits (|payload colour| = sqrt(3))
     const bool terminal = depth > c->rp.maxDepth || length(mk3(1.f)) < c->rp.minIntensity;
-    if (terminal && c->terminalQuery && c->nTerminalLights >= 0 && lc.scene.nodes8) {
+    // the AOVs need the camera rays' closest hits, which the terminal query does not record
+    const bool aovHere = depth == 1 && c->aovBlock.p;
+    if (terminal && c->terminalQuery && c->nTerminalLights >= 0 && lc.scene.nodes8 && !aovHere) {
       TerminalLights tl;
       tl.list = (const uint4*)c->dTerminalLights.p;
       tl.n = c->nTerminalLights;
@@ -529,6 +541,7 @@ int renderBatch(mox_ctx* c, const int32_t* seeds, uint32_t S, const uint32_t* li
     launchClassify(lc, lc.pb.qCur, bound, countPtr, depth);
     tm.end(c->stream);
     st.extend_launches++; st.kernel_launches += 2;
+    if (aovHere) { launchAov(lc, S, c->aov); st.kernel_launches++; c->aovRecorded = true; }
     CUCK(c, cudaMemcpyAsync(c->hostCnt.p, pb.counters, kCounterWords * 4, cudaMemcpyDeviceToHost, c->stream));
     CUCK(c, cudaEventRecord(c->evReady, c->stream));
     // the material counts size the shade launches: the host waits for them
@@ -613,7 +626,9 @@ size_t batchCap(mox_ctx* c, size_t wanted /* samples per pixel of this call */, 
   return cap;
 }
 
-// The preconditions of a render, then the device, the owned-pixel list, the lights and the textures.
+int ensureAovs(mox_ctx* c);
+
+// The preconditions of a render, then the device, the owned-pixel list, the lights, the AOV sums and the textures.
 int beginRender(mox_ctx* c) {
   if (!c->built) return fail(c, MOX_ERR_STATE, "launch before mox_build_accel");
   if (!c->haveGlobals) return fail(c, MOX_ERR_STATE, "launch before mox_set_globals");
@@ -622,6 +637,7 @@ int beginRender(mox_ctx* c) {
   if (rc) return rc;
   if ((rc = refreshOwned(c))) return rc;
   if ((rc = syncLights(c))) return rc;
+  if ((rc = ensureAovs(c))) return rc;
   return syncTextures(c);
 }
 
@@ -797,6 +813,125 @@ int renderAdaptive(mox_ctx* c, uint32_t spp, uint32_t seed, const mox_adaptive& 
   return MOX_OK;
 }
 
+// ---- first-hit AOVs and the denoiser (mox_set_aovs, mox_read_aovs, mox_denoise)
+
+constexpr size_t kAovBytesPerPixel = 36;
+
+// The AOV arrays of nPix pixels in one block at `base`: albedo xyz, normal xyz, depth, sample count, hit count.
+AovBuffers aovLayout(void* base, size_t nPix) {
+  AovBuffers a;
+  float* f = (float*)base;
+  a.albedo = f; a.normal = f + 3 * nPix; a.depth = f + 6 * nPix;
+  a.n = (uint32_t*)(f + 7 * nPix); a.hits = a.n + nPix;
+  return a;
+}
+
+// Allocates and zeroes the sums while AOVs are on and the image size is known.
+int ensureAovs(mox_ctx* c) {
+  if (!c->aovOn || c->aovBlock.p || !c->dAccu.p) return MOX_OK;
+  const size_t nPix = (size_t)c->accuW * c->accuH;
+  CUCK(c, c->aovBlock.alloc(nPix * kAovBytesPerPixel));
+  c->aov = aovLayout(c->aovBlock.p, nPix);
+  CUCK(c, cudaMemsetAsync(c->aovBlock.p, 0, nPix * kAovBytesPerPixel, c->stream));
+  c->aovRecorded = false;
+  return MOX_OK;
+}
+
+// Forget every AOV record: the accumulation buffer was cleared or replaced.
+int resetAovs(mox_ctx* c) {
+  if (c->aovBlock.p) CUCK(c, cudaMemsetAsync(c->aovBlock.p, 0, c->aovBlock.bytes, c->stream));
+  c->aovRecorded = false;
+  return MOX_OK;
+}
+
+// The AOV means of this context (full frame; pixels of other ranks read 0) into the destinations that are not null.
+int readAovMeans(mox_ctx* c, float* albedo, float* normal, float* depth) {
+  if (!c->aovOn) return fail(c, MOX_ERR_STATE, "AOVs are off (mox_set_aovs)");
+  if (!c->aovBlock.p) return fail(c, MOX_ERR_STATE, "no accumulation buffer (mox_set_globals first)");
+  int rc = bind(c);
+  if (rc) return rc;
+  const size_t nPix = (size_t)c->accuW * c->accuH;
+  std::vector<float> h(nPix * (kAovBytesPerPixel / 4));
+  CUCK(c, cudaMemcpyAsync(h.data(), c->aovBlock.p, nPix * kAovBytesPerPixel, cudaMemcpyDeviceToHost, c->stream));
+  CUCK(c, cudaStreamSynchronize(c->stream));
+  const AovBuffers s = aovLayout(h.data(), nPix);
+  for (size_t p = 0; p < nPix; ++p) {
+    const float n = (float)s.n[p];
+    for (int k = 0; k < 3; ++k) {
+      if (albedo) albedo[3 * p + k] = s.n[p] ? s.albedo[3 * p + k] / n : 0.f;
+      if (normal) normal[3 * p + k] = s.n[p] ? s.normal[3 * p + k] / n : 0.f;
+    }
+    if (depth) depth[p] = s.hits[p] ? s.depth[p] / (float)s.hits[p] : 0.f;
+  }
+  return MOX_OK;
+}
+
+// params (null: the defaults) checked and converted.
+int denoiseParams(mox_ctx* c, const mox_denoise_params* in, DenoiseParams& p) {
+  mox_denoise_params d{MOX_DENOISE_DEFAULT_ITERATIONS, MOX_DENOISE_DEFAULT_SIGMA_COLOR, MOX_DENOISE_DEFAULT_SIGMA_NORMAL,
+                       MOX_DENOISE_DEFAULT_SIGMA_DEPTH};
+  if (in) d = *in;
+  if (d.iterations < 1 || d.iterations > 10) return fail(c, MOX_ERR_INVALID, "mox_denoise_params.iterations must be 1..10");
+  for (float s : {d.sigma_color, d.sigma_normal, d.sigma_depth})
+    if (!std::isfinite(s) || !(s > 0.f)) return fail(c, MOX_ERR_INVALID, "mox_denoise_params sigmas must be finite and > 0");
+  p = DenoiseParams{d.iterations, d.sigma_color, d.sigma_normal, d.sigma_depth};
+  return MOX_OK;
+}
+
+// The launches pixel p sat out in adaptive renders (null: none).
+const uint32_t* skippedLaunches(const mox_ctx* c) { return c->adaptiveStats.p ? c->pixelStats.skipped : nullptr; }
+
+// Filters the frame `in` on c's device (bound) into dst (host, W*H*3 floats).
+int runDenoise(mox_ctx* c, const DenoiseInput& in, const DenoiseParams& p, float* dst, float* out_ms) {
+  const size_t nPix = (size_t)in.W * in.H;
+  int rc = ensure(c, c->denoiseScratch, denoiseScratchBytes(in.W, in.H));
+  if (rc || (rc = ensure(c, c->denoiseOut, nPix * 12))) return rc;
+  CUCK(c, cudaEventRecord(c->ev0, c->stream));
+  launchDenoise(in, p, c->denoiseScratch.p, (float*)c->denoiseOut.p, c->stream);
+  CUCK(c, cudaEventRecord(c->ev1, c->stream));
+  CUCK(c, cudaMemcpyAsync(dst, c->denoiseOut.p, nPix * 12, cudaMemcpyDeviceToHost, c->stream));
+  CUCK(c, cudaStreamSynchronize(c->stream));
+  CUCK(c, cudaGetLastError());
+  float ms = 0;
+  CUCK(c, cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+  if (out_ms) *out_ms = ms;
+  return MOX_OK;
+}
+
+// mox_denoise on a multi-GPU handle: every device stores the inputs of the pixels it owns into device 0's frame (peer
+// stores), then device 0 filters the whole frame.  Errors are reported on the shell c.
+int denoiseGroup(mox_ctx* c, const DenoiseParams& p, float* dst, float* out_ms) {
+  mox_group* g = c->group;
+  mox_ctx* k0 = groupChild(g, 0);
+  for (int i = 0; i < groupCount(g); ++i)
+    if (!groupChild(g, i)->aovOn || !groupChild(g, i)->aovBlock.p) return fail(c, MOX_ERR_STATE, "AOVs are off (mox_set_aovs)");
+  bool recorded = false;
+  for (int i = 0; i < groupCount(g); ++i) recorded = recorded || groupChild(g, i)->aovRecorded;
+  if (!recorded) return fail(c, MOX_ERR_STATE, "mox_denoise before any sample was rendered with AOVs on");
+  auto err0 = [&](int rc) { c->err = mox_last_error(k0); return rc; };
+  int rc = bind(k0);
+  if (rc) return err0(rc);
+  const size_t nPix = (size_t)k0->accuW * k0->accuH;
+  if ((rc = ensure(k0, k0->denoiseFrame, nPix * (12 + 4 + kAovBytesPerPixel)))) return err0(rc);
+  float* frameAccu = (float*)k0->denoiseFrame.p;
+  uint32_t* frameSkipped = (uint32_t*)(frameAccu + 3 * nPix);
+  const AovBuffers frameAov = aovLayout(frameSkipped + nPix, nPix);
+  if (cudaStreamSynchronize(k0->stream) != cudaSuccess) return fail(c, MOX_ERR_CUDA, "device 0 stream");
+  rc = groupParallel(g, [&](mox_ctx* k, int) -> int {
+    int r = bind(k);
+    if (r || (r = refreshOwned(k))) return r;
+    launchPushDenoiseInput(k->dOwned.p, k->nOwned, k->dAccu.p, skippedLaunches(k), k->aov, frameAccu, frameSkipped, frameAov, k->stream);
+    CUCK(k, cudaStreamSynchronize(k->stream));   // the pixels have landed before device 0 reads them
+    CUCK(k, cudaGetLastError());
+    return MOX_OK;
+  });
+  if (rc) { c->err = groupError(g); return rc; }
+  if ((rc = bind(k0))) return err0(rc);
+  const DenoiseInput in{frameAccu, frameSkipped, (uint32_t)k0->st.launches, frameAov, k0->accuW, k0->accuH};
+  if ((rc = runDenoise(k0, in, p, dst, out_ms))) return err0(rc);
+  return MOX_OK;
+}
+
 constexpr int kRebuild = 1;   // refitAccel: nothing to refit, run the full build
 
 // MOX_ACCEL_REFIT (flags without it): refit the structure of the last full build in place.  Uploads only what
@@ -950,13 +1085,15 @@ int mox_set_globals(mox_ctx* c, uint32_t width, uint32_t height, uint32_t rayMax
     c->adaptiveStats.release();   // allocated again, zeroed, at the next mox_render_adaptive
     c->adaptiveLists.release();
     c->pixelStats = PixelStats();
+    c->aovBlock.release();       // allocated again, zeroed, for the new size (ensureAovs below)
+    c->aov = AovBuffers();
   }
   c->rp.W = width; c->rp.H = height; c->rp.maxDepth = rayMaxDepth; c->rp.eps = rayEpsilonT; c->rp.minIntensity = rayMinIntensity;
   c->rp.absorb = make_float3(absorbColor[0], absorbColor[1], absorbColor[2]);
   c->rp.bad = make_float3(badColor[0], badColor[1], badColor[2]);
   c->rp.bg = make_float3(bgColor[0], bgColor[1], bgColor[2]);
   c->haveGlobals = true;
-  return MOX_OK;
+  return ensureAovs(c);
 }
 
 int mox_set_camera(mox_ctx* c, const CamParams* cam) {
@@ -1399,7 +1536,7 @@ int mox_clear_accum(mox_ctx* c) {
   int rc = bind(c);
   if (rc) return rc;
   if (c->dAccu.p) CUCK(c, cudaMemsetAsync(c->dAccu.p, 0, (size_t)c->accuW * c->accuH * 12, c->stream));
-  if ((rc = resetAdaptive(c))) return rc;
+  if ((rc = resetAdaptive(c)) || (rc = resetAovs(c))) return rc;
   CUCK(c, cudaStreamSynchronize(c->stream));
   const double msBuild = c->st.ms_build;   // describes the acceleration structure, not the image
   c->st = mox_stats{};
@@ -1414,10 +1551,68 @@ int mox_set_accum(mox_ctx* c, const float* src, uint64_t launches) {
   int rc = bind(c);
   if (rc) return rc;
   CUCK(c, cudaMemcpyAsync(c->dAccu.p, src, (size_t)c->accuW * c->accuH * 12, cudaMemcpyHostToDevice, c->stream));
-  if ((rc = resetAdaptive(c))) return rc;   // the loaded buffer counts as a uniform render of `launches` samples
+  if ((rc = resetAdaptive(c)) || (rc = resetAovs(c))) return rc;   // the loaded buffer counts as a uniform render of `launches` samples
   CUCK(c, cudaStreamSynchronize(c->stream));
   c->st.launches = launches;
   return MOX_OK;
+}
+
+int mox_set_aovs(mox_ctx* c, int enable) {
+  if (!c) return MOX_ERR_INVALID;
+  GROUP_EACH(c, mox_set_aovs(k, enable));
+  int rc = bind(c);
+  if (rc) return rc;
+  if (enable) {   // already on: the sums are kept
+    c->aovOn = true;
+    if ((rc = ensureAovs(c))) return rc;
+    CUCK(c, cudaStreamSynchronize(c->stream));
+    return MOX_OK;
+  }
+  c->aovOn = false;
+  CUCK(c, cudaStreamSynchronize(c->stream));
+  c->aovBlock.release();
+  c->aov = AovBuffers();
+  return MOX_OK;
+}
+
+int mox_read_aovs(mox_ctx* c, float* albedo, float* normal, float* depth) {
+  if (!c) return MOX_ERR_INVALID;
+  if (c->group) {   // every pixel is owned by one device, the others hold 0 for it
+    const mox_ctx* k0 = groupChild(c->group, 0);
+    const size_t n = (size_t)k0->accuW * k0->accuH;
+    std::vector<float> a(albedo ? 3 * n : 0), nr(normal ? 3 * n : 0), z(depth ? n : 0);
+    if (albedo) std::fill(albedo, albedo + 3 * n, 0.f);
+    if (normal) std::fill(normal, normal + 3 * n, 0.f);
+    if (depth) std::fill(depth, depth + n, 0.f);
+    for (int i = 0; i < groupCount(c->group); ++i) {
+      mox_ctx* k = groupChild(c->group, i);
+      if (int rc_ = readAovMeans(k, albedo ? a.data() : nullptr, normal ? nr.data() : nullptr, depth ? z.data() : nullptr)) {
+        c->err = mox_last_error(k);
+        return rc_;
+      }
+      for (size_t p = 0; p < a.size(); ++p) albedo[p] += a[p];
+      for (size_t p = 0; p < nr.size(); ++p) normal[p] += nr[p];
+      for (size_t p = 0; p < z.size(); ++p) depth[p] += z[p];
+    }
+    return MOX_OK;
+  }
+  return readAovMeans(c, albedo, normal, depth);
+}
+
+int mox_denoise(mox_ctx* c, const mox_denoise_params* params, float* dst, float* out_ms) {
+  if (!c) return MOX_ERR_INVALID;
+  if (out_ms) *out_ms = 0.f;
+  DenoiseParams p;
+  int rc = denoiseParams(c, params, p);
+  if (rc) return rc;
+  if (!dst) return fail(c, MOX_ERR_INVALID, "null destination");
+  if (c->group) return denoiseGroup(c, p, dst, out_ms);
+  if (c->world > 1) return fail(c, MOX_ERR_STATE, "mox_denoise needs the whole frame: this context renders one rank of a partition");
+  if (!c->aovOn || !c->aovBlock.p) return fail(c, MOX_ERR_STATE, "AOVs are off (mox_set_aovs)");
+  if (!c->aovRecorded) return fail(c, MOX_ERR_STATE, "mox_denoise before any sample was rendered with AOVs on");
+  if ((rc = bind(c))) return rc;
+  const DenoiseInput in{c->dAccu.p, skippedLaunches(c), (uint32_t)c->st.launches, c->aov, c->accuW, c->accuH};
+  return runDenoise(c, in, p, dst, out_ms);
 }
 
 int mox_update_sphere(mox_ctx* c, uint32_t prim_id, const SphereParams* s) {

@@ -549,6 +549,51 @@ __global__ void __launch_bounds__(TPB) k_accumulate(LaunchCtx c, uint32_t nSampl
   if (bad) atomicAdd(c.pb.counters + C_NONFINITE, bad);
 }
 
+// ------------------------------------------------------------------ first-hit AOVs (mox_set_aovs)
+// One thread per pixel of the batch's list: its samples s * nOwned + j are added in launch order, so the sums do not
+// depend on the batching.  Runs at depth 1 after k_classify, when rayO / rayD still hold the camera rays and hit their
+// closest hits; the shade kernels overwrite both.
+__global__ void __launch_bounds__(TPB) k_aov(LaunchCtx c, uint32_t nSamples, AovBuffers aov) {
+  const uint32_t j = blockIdx.x * TPB + threadIdx.x;
+  if (j >= c.nOwned) return;
+  const uint32_t pix = c.ownedPix[j];
+  float3 alb = mk3(aov.albedo[3 * (size_t)pix], aov.albedo[3 * (size_t)pix + 1], aov.albedo[3 * (size_t)pix + 2]);
+  float3 nrm = mk3(aov.normal[3 * (size_t)pix], aov.normal[3 * (size_t)pix + 1], aov.normal[3 * (size_t)pix + 2]);
+  float depth = aov.depth[pix];
+  uint32_t hits = aov.hits[pix];
+  const float3 bg = mk3(fmaxf(0.f, fminf(c.rp.bg.x, 1.f)), fmaxf(0.f, fminf(c.rp.bg.y, 1.f)), fmaxf(0.f, fminf(c.rp.bg.z, 1.f)));
+  for (uint32_t s = 0; s < nSamples; ++s) {
+    const size_t p = (size_t)s * c.nOwned + j;
+    const float2 h = c.pb.hit[p];
+    const int bits = __float_as_int(h.y);
+    if (bits < 0) { alb = alb + bg; continue; }   // miss: normal 0, no depth
+    const PrimDesc pd = c.scene.prims[(uint32_t)bits & MOX_HIT_ID_MASK];
+    const GpuMaterial* m = c.scene.mats + (pd.typeMat >> 2);
+    const float3 o = mk3(c.pb.rayO[p]), d = mk3(c.pb.rayD[p]);
+    const Attr a = hitAttributes(c.scene, pd, o, d, h.x, true);
+    float3 A;
+    switch (m->kind) {
+      case MOX_MAT_LAMBERTIAN: A = f3(m->lam.albedo); break;
+      case MOX_MAT_METAL: A = f3(m->met.albedo); break;
+      case MOX_MAT_GLASS: A = f3(m->gls.albedo); break;
+      case MOX_MAT_DISNEY: A = disneyBaseColor(c.scene, m->dis, a.u, a.v); break;
+      default: {
+        const float3 e = f3(m->lgt.emission);
+        A = mk3(fmaxf(0.f, fminf(e.x, 1.f)), fmaxf(0.f, fminf(e.y, 1.f)), fmaxf(0.f, fminf(e.z, 1.f)));
+      }
+    }
+    alb = alb + A;
+    nrm = nrm + faceforward3(a.Ns, -d, a.Ng);
+    depth += h.x;
+    hits++;
+  }
+  aov.albedo[3 * (size_t)pix] = alb.x; aov.albedo[3 * (size_t)pix + 1] = alb.y; aov.albedo[3 * (size_t)pix + 2] = alb.z;
+  aov.normal[3 * (size_t)pix] = nrm.x; aov.normal[3 * (size_t)pix + 1] = nrm.y; aov.normal[3 * (size_t)pix + 2] = nrm.z;
+  aov.depth[pix] = depth;
+  aov.hits[pix] = hits;
+  aov.n[pix] += nSamples;
+}
+
 // ------------------------------------------------------------------ adaptive sampling: the active-pixel list
 // One tile of the list per block: SEL_ITEMS consecutive entries per thread, so the survivors of a thread, a warp and
 // a block keep their order.
@@ -859,6 +904,9 @@ void launchAccumulate(const LaunchCtx& c, uint32_t nSamples) {
 }
 void launchAccumulateAdaptive(const LaunchCtx& c, uint32_t nSamples, const PixelStats& ps) {
   if (c.nOwned) k_accumulate<true><<<grid(c.nOwned), TPB, 0, c.stream>>>(c, nSamples, ps);
+}
+void launchAov(const LaunchCtx& c, uint32_t nSamples, const AovBuffers& aov) {
+  if (c.nOwned) k_aov<<<grid(c.nOwned), TPB, 0, c.stream>>>(c, nSamples, aov);
 }
 size_t adaptiveSelectTiles(uint32_t count) { return ((size_t)count + SEL_TILE - 1) / SEL_TILE; }
 void launchAdaptiveSelect(const PixelStats& ps, const AdaptiveRule& rule, const uint32_t* listIn, uint32_t count, uint32_t remaining,

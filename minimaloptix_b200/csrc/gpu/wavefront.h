@@ -72,6 +72,15 @@ size_t adaptiveSelectTiles(uint32_t count);
 // nothing for count == 0 (*survivors is then not written).
 void launchAdaptiveSelect(const PixelStats& ps, const AdaptiveRule& rule, const uint32_t* listIn, uint32_t count, uint32_t remaining,
                           uint32_t* listOut, uint32_t* tileSums, uint32_t* survivors, cudaStream_t stream);
+// First-hit AOV sums (mox_set_aovs), full-frame arrays indexed by pixel: albedo and normal xyz (3 floats per pixel),
+// depth, the AOV sample count and the hit count.  36 bytes per pixel.
+struct AovBuffers {
+  float *albedo = nullptr, *normal = nullptr, *depth = nullptr;
+  uint32_t *n = nullptr, *hits = nullptr;
+};
+// k_aov: adds the record of every camera sample of the batch (depth 1, after k_classify, before any shade kernel) to
+// aov, per pixel in launch order.
+void launchAov(const LaunchCtx& c, uint32_t nSamples, const AovBuffers& aov);
 // Persistent traversal over one batch of rays (closest hit or shadow transmittance).
 void launchTraverse(const SceneView& s, const TraceJob& job, bool anyHit, bool count, cudaStream_t stream, bool classify = false);
 void launchSplitRays(const float4* rays, float4* o, float4* d, size_t n, cudaStream_t stream);

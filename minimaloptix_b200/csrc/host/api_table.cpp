@@ -24,5 +24,8 @@ bool loadMoxApi(const char* libPath, const char* prefix, MoxApi& api, std::strin
   api.get_device_stats = (int (*)(mox_ctx*, int, mox_stats*))dlsym(lib, (std::string(prefix) + "get_device_stats").c_str());
   api.render_adaptive = (int (*)(mox_ctx*, uint32_t, uint32_t, const mox_adaptive*, uint64_t*))dlsym(lib, (std::string(prefix) + "render_adaptive").c_str());
   api.read_sample_counts = (int (*)(mox_ctx*, uint32_t*))dlsym(lib, (std::string(prefix) + "read_sample_counts").c_str());
+  api.set_aovs = (int (*)(mox_ctx*, int))dlsym(lib, (std::string(prefix) + "set_aovs").c_str());
+  api.read_aovs = (int (*)(mox_ctx*, float*, float*, float*))dlsym(lib, (std::string(prefix) + "read_aovs").c_str());
+  api.denoise = (int (*)(mox_ctx*, const mox_denoise_params*, float*, float*))dlsym(lib, (std::string(prefix) + "denoise").c_str());
   return ok;
 }

@@ -37,6 +37,9 @@ struct MoxApi {
   int (*get_device_stats)(mox_ctx*, int, mox_stats*) = nullptr;
   int (*render_adaptive)(mox_ctx*, uint32_t, uint32_t, const mox_adaptive*, uint64_t*) = nullptr;
   int (*read_sample_counts)(mox_ctx*, uint32_t*) = nullptr;
+  int (*set_aovs)(mox_ctx*, int) = nullptr;
+  int (*read_aovs)(mox_ctx*, float*, float*, float*) = nullptr;
+  int (*denoise)(mox_ctx*, const mox_denoise_params*, float*, float*) = nullptr;
 };
 
 // prefix is "mox_" for the product library.  Returns false and fills err on failure.

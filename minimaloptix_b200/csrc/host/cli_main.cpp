@@ -19,6 +19,7 @@ static void usage() {
           "usage: mox_cli --scene NAME [--scene-dir DIR] [--width W --height H] [--spp N] [--max-depth D]\n"
           "               [--seed S] [--rng ref|philox] [--out PREFIX] [--snapshots] [--dump-accum] [--resume FILE.moxa] [--device K | --gpus N]\n"
           "               [--param P] [--lib PATH] [--watertight] [--adaptive REL[,ABS] [--adaptive-min N] [--adaptive-round N]]\n"
+          "               [--denoise [ITER]]\n"
           "  NAME: spheres_lens spheres_pinhole random_spheres interior soup, or a folder under DIR\n"
           "        holding NAME.scene (coffee, cornell, ...).  Defaults are the reference's constants\n"
           "        (1920x1080, 32 spp, depth 256; MinimalOptiX.h:82-89); a .scene file's properties{width,height}\n"
@@ -27,7 +28,10 @@ static void usage() {
           "  --adaptive REL[,ABS]: render with mox_render_adaptive up to --spp: a pixel stops once the standard error of its\n"
           "        luminance is below max(REL * mean, ABS) (ABS default 0); the image is divided by each pixel's sample count.\n"
           "        --adaptive-min N: samples before a pixel may stop (default 16); --adaptive-round N: launches between two\n"
-          "        checks (default 8).  Not combined with --snapshots, --resume or --dump-accum.\n");
+          "        checks (default 8).  Not combined with --snapshots, --resume or --dump-accum.\n"
+          "  --denoise [ITER]: accumulate first-hit albedo, normal and depth (mox_set_aovs) and filter the final image with\n"
+          "        mox_denoise (ITER a-trous iterations, default 5): writes PREFIX_denoised.png, PREFIX_albedo.png and\n"
+          "        PREFIX_normal.png (0.5 + 0.5 N) and adds ms_denoise to the JSON line.\n");
 }
 
 int main(int argc, char** argv) {
@@ -35,7 +39,9 @@ int main(int argc, char** argv) {
   uint32_t W = 0, H = 0, spp = 32, depth = 256, seed = 0xC0FFEE;
   uint64_t param = 0;
   int device = 0, gpus = 0;
-  bool snapshots = false, dumpAccum = false, watertight = false, adaptive = false;
+  bool snapshots = false, dumpAccum = false, watertight = false, adaptive = false, denoise = false;
+  mox_denoise_params dn{MOX_DENOISE_DEFAULT_ITERATIONS, MOX_DENOISE_DEFAULT_SIGMA_COLOR, MOX_DENOISE_DEFAULT_SIGMA_NORMAL,
+                        MOX_DENOISE_DEFAULT_SIGMA_DEPTH};
   mox_adaptive ad{8u, 16u, 0.f, 0.f};   // round_spp, min_spp, rel_error, abs_error
   for (int i = 1; i < argc; ++i) {
     std::string a = argv[i];
@@ -64,6 +70,10 @@ int main(int argc, char** argv) {
       ad.rel_error = strtof(v, &end);
       if (*end == ',') ad.abs_error = strtof(end + 1, &end);
       if (*end) { fprintf(stderr, "--adaptive wants REL or REL,ABS, got %s\n", v); return 2; }
+    }
+    else if (a == "--denoise") {
+      denoise = true;
+      if (i + 1 < argc && argv[i + 1][0] >= '0' && argv[i + 1][0] <= '9') dn.iterations = (uint32_t)atoi(argv[++i]);
     }
     else if (a == "--adaptive-min") ad.min_spp = (uint32_t)atoi(val());
     else if (a == "--adaptive-round") ad.round_spp = (uint32_t)atoi(val());
@@ -102,6 +112,10 @@ int main(int argc, char** argv) {
     if (api.create_multi(&ctx, ids.data(), gpus)) { fprintf(stderr, "mox_create_multi: %s\n", api.last_error(nullptr)); return 1; }
   } else if (api.create(&ctx, device)) { fprintf(stderr, "mox_create: %s\n", api.last_error(nullptr)); return 1; }
   if (adaptive && !(api.render_adaptive && api.read_sample_counts)) { fprintf(stderr, "%s has no mox_render_adaptive\n", lib.c_str()); return 1; }
+  if (denoise && !(api.set_aovs && api.read_aovs && api.denoise && api.read_sample_counts)) {
+    fprintf(stderr, "%s has no mox_denoise\n", lib.c_str());
+    return 1;
+  }
   api.set_rng_mode(ctx, rng == "philox" ? MOX_RNG_PHILOX : MOX_RNG_REF);
   if (!moxh::uploadScene(sc, api, ctx, W, H, depth, err)) { fprintf(stderr, "upload: %s\n", err.c_str()); return 1; }
   float buildMs = 0;
@@ -127,6 +141,7 @@ int main(int argc, char** argv) {
     writeSec += std::chrono::duration<double>(std::chrono::steady_clock::now() - a1).count();
     nSnapshots++;
   };
+  if (denoise && api.set_aovs(ctx, 1)) { fprintf(stderr, "set_aovs: %s\n", api.last_error(ctx)); return 1; }
   uint32_t done = 0, checkpoint = 1;
   if (!resume.empty()) {  // continue a previous run: same seed schedule, samples [launches, spp)
     uint64_t launches = 0;
@@ -150,6 +165,21 @@ int main(int argc, char** argv) {
   double sec = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
   save(out, spp);
   if (dumpAccum) moxh_write_accum((out + ".moxa").c_str(), accum.data(), W, H, spp);
+  // the denoised image and its guides, each written through the same quantisation as the image (n = 1)
+  float denoiseMs = 0;
+  if (denoise) {
+    std::vector<float> img((size_t)W * H * 3), nrm((size_t)W * H * 3);
+    if (api.denoise(ctx, &dn, img.data(), &denoiseMs)) { fprintf(stderr, "denoise: %s\n", api.last_error(ctx)); return 1; }
+    auto write = [&](const char* suffix, const float* v) {
+      moxh_accum_to_rgb8(v, W, H, 1.f, rgb.data());
+      if (moxh_write_image((out + suffix).c_str(), rgb.data(), W, H)) fprintf(stderr, "write: %s\n", moxh_last_error());
+    };
+    write("_denoised.png", img.data());
+    if (api.read_aovs(ctx, img.data(), nrm.data(), nullptr)) { fprintf(stderr, "read_aovs: %s\n", api.last_error(ctx)); return 1; }
+    write("_albedo.png", img.data());
+    for (float& v : nrm) v = 0.5f + 0.5f * v;
+    write("_normal.png", nrm.data());
+  }
   mox_stats st;
   api.get_stats(ctx, &st);
   // share of the pixels that received every launch (1 for a uniform render)
@@ -177,7 +207,9 @@ int main(int argc, char** argv) {
     if (api.get_device_stats) api.get_device_stats(ctx, i, &ds);
     printf("%s%.2f", i ? ", " : "", ds.ms_render);
   }
-  printf("]}\n");
+  printf("]");
+  if (denoise) printf(", \"ms_denoise\": %.3f, \"denoise_iterations\": %u", denoiseMs, dn.iterations);
+  printf("}\n");
   api.destroy(ctx);
   return 0;
 }

@@ -87,6 +87,14 @@ class Adaptive(C.Structure):
     _fields_ = [("round_spp", C.c_uint32), ("min_spp", C.c_uint32), ("rel_error", C.c_float), ("abs_error", C.c_float)]
 
 
+class DenoiseParams(C.Structure):
+    """mox_denoise_params: the iterations and edge stops of mox_denoise."""
+    _fields_ = [("iterations", C.c_uint32), ("sigma_color", C.c_float), ("sigma_normal", C.c_float), ("sigma_depth", C.c_float)]
+
+
+# mox.h MOX_DENOISE_DEFAULT_*
+DENOISE_DEFAULTS = {"iterations": 5, "sigma_color": 1.0, "sigma_normal": 0.5, "sigma_depth": 0.05}
+
 MAT_LAMBERTIAN, MAT_METAL, MAT_GLASS, MAT_DISNEY, MAT_LIGHT = range(5)
 RNG_REF, RNG_PHILOX = 0, 1
 ACCEL_DEFAULT, ACCEL_LBVH, ACCEL_COUNTERS, ACCEL_BINARY, ACCEL_WATERTIGHT = 0, 1, 2, 4, 8
